@@ -2,6 +2,7 @@
 """Benchmark of the N-HANS inference hot path on B200 (contract: see the task statement / DESIGN.md §6).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg1..cfg5] [--utts U]
+                  [--dump-outputs DIR]
 
 Metric (BASELINE.json): audio-seconds denoised / separated per wall-second.  A step = one pass of the hot path
 (STFT -> embedding towers -> conditioned residual network -> iSTFT/overlap-add) over one batch of synthetic 16 kHz
@@ -17,6 +18,11 @@ utterances.  Workloads are BASELINE.json's `configs`:
 `value` is measured with the inputs resident in HBM (CUDA events on the engine's stream); `e2e` goes through
 nhans_enhance_batch with pinned host buffers, H2D and D2H inside the timed region.  `--impl reference` times the
 reference's own structure (oracle faithful mode: both towers per window, mb = 100) on the host cores.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller (rank 0's batch), so that two builds
+can be compared output for output on identical inputs: out_i16.npy (the int16 PCM, as float32), out_f32.npy (the
+float32 samples of the same batch) and out_offsets.npy (utterance boundaries, float64).  Above DUMP_BYTES a fixed,
+seeded sample of sample positions is written instead, listed in sample_index.npy (float64).
 """
 import argparse
 import json
@@ -47,6 +53,7 @@ CONFIGS = {
     "cfg5": (0, 256, 10.0, "neg", "nhans_denoiser, utterance-sharded 8192 x 10 s sweep: 1024 clips per GPU, one step = a 256-clip slice of "
                                   "the GPU's shard + --neg clips (BASELINE config 5)"),
 }
+DUMP_BYTES = 64 * 10 ** 6
 
 
 class ClockSampler:
@@ -117,6 +124,26 @@ def contexts(variant, kind, u):
     return synth.speaker_clip(u, "interference"), synth.speaker_clip(u, "target")
 
 
+def dump_outputs(out_dir, eng, out_i16, out_offs):
+    """Write the outputs of the batch the engine processed last (see the module docstring) under out_dir."""
+    out_f32 = np.zeros(out_i16.shape, np.float32)
+    eng.download(out_f32=out_f32)
+    eng.sync()
+    arrays = {"out_i16": out_i16.astype(np.float32), "out_f32": out_f32}
+    n = len(out_f32)
+    header = 128                                        # bytes of an .npy header
+    fixed = 3 * header + 8 * len(out_offs)
+    if fixed + 8 * n > DUMP_BYTES:
+        k = (DUMP_BYTES - fixed - header) // 16         # two float32 values and one float64 index per sampled position
+        idx = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+        arrays = {name: a[idx] for name, a in arrays.items()}
+        arrays["sample_index"] = idx.astype(np.float64)
+    arrays["out_offsets"] = np.asarray(out_offs, np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_baseline(weights, variant, kind, seconds, steps=1, warmup=0, dedup=True):
     """The reference's own structure on the host cores: oracle faithful mode (mb = 100, both towers per
     window, materialised windows), torch-CPU fp32, all threads; plus the algorithmically de-duplicated mode
@@ -159,7 +186,13 @@ def main():
     ap.add_argument("--seconds", type=float, default=0.0)
     ap.add_argument("--win-capacity", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as .npy files under DIR (--impl ours, rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -293,6 +326,8 @@ def main():
     wall_e2e = time.perf_counter() - t_host
     ms_e2e, ms_e2e_all = over_ranks(eng.event_elapsed_ms(2, 3))
     e2e = world * a.steps * audio_s / (ms_e2e / 1e3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, eng, p_out.array, oo)
 
     if rank == 0:
         tf_peak, hbm_peak, which = peaks()

@@ -1,7 +1,6 @@
-"""Regenerates tests/golden/ckpt_index_{sn,ss}.json from the reference checkpoints' .index files
-(run in the authoring container, where /root/reference is mounted):
+"""Regenerates tests/golden/ckpt_index_{sn,ss}.json from the reference checkpoints' .index files:
 
-    python tests/golden/make_ckpt_index.py
+    python tests/golden/make_ckpt_index.py <reference checkout>
 
 The JSON holds name -> [dtype, shape, offset, size] for every entry of
 N_HANS___Selective_Noise/trained_model/81448_0-1000000.index and
@@ -15,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from nhans_b200 import weights as W  # noqa: E402
 
-REF = "/root/reference"
+REF = sys.argv[1]
 for tag, prefix in (("sn", "N_HANS___Selective_Noise/trained_model/81448_0-1000000"),
                     ("ss", "N_HANS___Source_Separation/trained_model/81457_2-545000")):
     e = W.read_bundle_index(os.path.join(REF, prefix + ".index"))

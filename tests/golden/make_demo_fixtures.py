@@ -2,14 +2,15 @@
 266-353, shipped under DEMO_N-HANS/) into tests/golden/demo_relations.npz.  They are the only reference-produced
 numerical artefacts in the tree; tests/test_reference_artifacts.py uses them to pin the restatement of domixing
 (SN/reader.py:131-180): the scaling quirk of target / noise signals and the SNR convention.
-Run in the build container (needs /root/reference): python tests/golden/make_demo_fixtures.py"""
+Needs a checkout of the reference project:  python tests/golden/make_demo_fixtures.py <reference checkout>"""
 import glob
 import os
+import sys
 
 import numpy as np
 from scipy.io import wavfile
 
-REF = "/root/reference/DEMO_N-HANS"
+REF = os.path.join(sys.argv[1], "DEMO_N-HANS")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "demo_relations.npz")
 N = 4000                                                   # samples per excerpt (interior of the file)
 

@@ -1,7 +1,7 @@
 """Round-2 parity additions (VERDICT r1 item 4): elementwise mask error against the fp32 oracle, the spectra the
 FUSED path keeps in HBM (reciprocal-multiply normalisation, log of |X| via rsqrt, unit phasors) against the oracle's
-arrays, stereo clips through the float entry points, `removed` relative to the output level, and a dormant
-end-to-end test that switches on when a real trained checkpoint is mounted."""
+arrays, stereo clips through the float entry points, `removed` relative to the output level, and an end-to-end
+test from a checkpoint in the reference's tensor-bundle format."""
 import os
 
 import numpy as np
@@ -125,40 +125,22 @@ def test_removed_relative_to_output_level(engine_sn, oracle_sn):
     assert _snr(comp, post["compensated"][0]) >= 40.0
 
 
-def _real_checkpoint(sub):
-    for root in (os.environ.get("NHANS_CHECKPOINT_ROOT"), "/root/reference"):
-        if not root:
-            continue
-        d = os.path.join(root, sub, "trained_model")
-        prefix = W.find_checkpoint(d) if os.path.isdir(d) else None
-        if prefix:
-            try:
-                W.load_bundle(prefix)
-                return root, d
-            except Exception:
-                continue
-    return None, None
-
-
-def test_trained_checkpoint_end_to_end_when_mounted():
-    """Dormant unless a REAL trained checkpoint is mounted (NHANS_CHECKPOINT_ROOT or /root/reference with the LFS blobs
-    pulled): restores the reference's separator checkpoint through the tensor-bundle reader and runs the shipped
-    audio_examples triple (SS/apply.py:28-34) through the engine and the oracle."""
-    root, d = _real_checkpoint("N_HANS___Source_Separation")
-    if root is None:
-        pytest.skip("no real trained checkpoint mounted (the reference's .data files are git-LFS pointers)")
-    from nhans_b200.wavio import read_wav
-    w, src = W.load_or_init(W.SEPARATOR, d, allow_random=False)
+def test_checkpoint_bundle_end_to_end(tmp_path):
+    """A separator checkpoint in the reference's tensor-bundle format (seeded weights of the identical architecture:
+    the reference distributes its trained data shards as git-LFS pointers only) restored through the bundle reader,
+    then a mixture with interference and target speaker clips (the triple SS/apply.py:28-34 takes) through the engine
+    and the oracle."""
+    from test_weights import _write_bundle
+    d = tmp_path / "trained_model"
+    os.makedirs(str(d))
+    _write_bundle(str(d / "81457_2-545000"), W.seeded_init(W.SEPARATOR, 3))
+    w, src = W.load_or_init(W.SEPARATOR, str(d), allow_random=False)
     assert src == "checkpoint"
-    ex = os.path.join(root, "N_HANS___Source_Separation", "audio_examples")
-    mix, tgt, itf = (read_wav(os.path.join(ex, n)) for n in ("mixed.wav", "target_speaker.wav", "noise_speaker.wav"))
+    mix, tgt, itf = synth.mixture(2.5, 51), synth.speaker_clip(51, "target"), synth.speaker_clip(51, "interference")
     eng = Engine(0, W.SEPARATOR)
     try:
         eng.load_weights(w, src)
-        if all(a.dtype == np.int16 for a in (mix, tgt, itf)):
-            got = eng.enhance([mix], [itf], [tgt])["f32"][0]
-        else:
-            got = eng.enhance_float(mix, itf, tgt)["f32"]
+        got = eng.enhance([mix], [itf], [tgt])["f32"][0]
     finally:
         eng.close()
     ref = O.apply_arrays(O.Net(w, W.SEPARATOR), mix, itf, tgt)

@@ -29,18 +29,27 @@ def test_inventory_matches_reference_checkpoint_index(tag, variant):
     assert all(offs[i][0] + offs[i][1] == offs[i + 1][0] for i in range(len(offs) - 1))   # contiguous
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference mount absent")
-def test_index_reader_on_reference_files():
-    e = W.read_bundle_index("/root/reference/N_HANS___Selective_Noise/trained_model/81448_0-1000000.index")
+def test_index_reader_on_reference_files(tmp_path):
+    """The reference's selective-noise checkpoint as its repository ships it: the .index (every entry of
+    tests/golden/ckpt_index_sn.json, laid out like TF's table builder writes it: prefix-compressed keys, a restart
+    point every 16 entries, ~4 KiB data blocks) next to a git-LFS pointer in place of the data shard."""
     idx = json.load(open(os.path.join(GOLD, "ckpt_index_sn.json")))
+    d = str(tmp_path / "trained_model")
+    os.makedirs(d)
+    prefix = os.path.join(d, "81448_0-1000000")
+    entries = [(k.encode(), _entry_proto(*v)) for k, v in sorted(idx.items())]
+    _write_table(prefix + ".index", [(b"", _BUNDLE_HEADER)] + entries, block_size=4096, restart_interval=16)
+    with open(prefix + ".data-00000-of-00001", "wb") as f:
+        f.write(b"version https://git-lfs.github.com/spec/v1\noid sha256:0\nsize 115999524\n")
+    e = W.read_bundle_index(prefix + ".index")
     assert {k: [v["dtype"], list(v["shape"]), v["offset"], v["size"]] for k, v in e.items()} == idx
     with pytest.raises(FileNotFoundError):                           # the data shard is an LFS pointer
-        W.load_bundle("/root/reference/N_HANS___Selective_Noise/trained_model/81448_0-1000000")
+        W.load_bundle(prefix)
     # like the reference (SN/apply.py:428-432), a checkpoint that cannot be restored is an error ...
     with pytest.raises(W.CheckpointMissing):
-        W.load_or_init(0, "/root/reference/N_HANS___Selective_Noise/trained_model", allow_random=False)
+        W.load_or_init(0, d, allow_random=False)
     # ... unless random-init weights of the identical architecture are explicitly allowed
-    w, src = W.load_or_init(0, "/root/reference/N_HANS___Selective_Noise/trained_model", allow_random=True)
+    w, src = W.load_or_init(0, d, allow_random=True)
     assert src == "random-init" and len(w) == 571
 
 
@@ -54,36 +63,66 @@ def _varint(n):
             return out
 
 
-def _block(entries):
-    body = b""
-    for k, v in entries:                      # no prefix compression, single restart
-        body += _varint(0) + _varint(len(k)) + _varint(len(v)) + k + v
-    body += struct.pack("<I", 0) + struct.pack("<I", 1)
-    return body
+_BUNDLE_HEADER = b"\x08\x01"                  # BundleHeaderProto: num_shards = 1
+
+
+def _block(entries, restart_interval=1):
+    """LevelDB block: keys share their prefix with the previous key except at restart points."""
+    body, restarts, prev = b"", [], b""
+    for i, (k, v) in enumerate(entries):
+        shared = 0
+        if i % restart_interval == 0:
+            restarts.append(len(body))
+        else:
+            while shared < min(len(k), len(prev)) and k[shared] == prev[shared]:
+                shared += 1
+        body += _varint(shared) + _varint(len(k) - shared) + _varint(len(v)) + k[shared:] + v
+        prev = k
+    restarts = restarts or [0]
+    return body + b"".join(struct.pack("<I", r) for r in restarts) + struct.pack("<I", len(restarts))
+
+
+def _write_table(path, entries, block_size=1 << 62, restart_interval=1):
+    """LevelDB table of sorted (key, value) pairs: uncompressed data blocks of about `block_size` bytes, an empty
+    meta-index block, the index block and the footer."""
+    f, index, pending = b"", [], []
+
+    def put(blk):
+        nonlocal f
+        handle = _varint(len(f)) + _varint(len(blk))
+        f += blk + b"\x00" + b"\x00" * 4                 # trailer: type (uncompressed) + crc32c (not checked)
+        return handle
+    for i, (k, v) in enumerate(entries):
+        pending.append((k, v))
+        if i == len(entries) - 1 or sum(len(a) + len(b) for a, b in pending) >= block_size:
+            index.append((k, put(_block(pending, restart_interval))))
+            pending = []
+    meta = put(_block([]))
+    idx = put(_block(index))
+    footer = meta + idx
+    footer += b"\x00" * (40 - len(footer)) + struct.pack("<Q", 0xDB4775248B80FB57)
+    with open(path, "wb") as out:
+        out.write(f + footer)
+
+
+def _entry_proto(dtype, shape, offset, size):
+    """BundleEntryProto: dtype, shape, offset, size and a crc32c field (a stand-in value: the reader ignores it)."""
+    dims = b"".join(b"\x12" + _varint(len(d)) + d for d in (b"\x08" + _varint(s) for s in shape))
+    return (b"\x08" + _varint(dtype) + b"\x12" + _varint(len(dims)) + dims + b"\x20" + _varint(offset) + b"\x28" + _varint(size)
+            + b"\x35" + struct.pack("<I", 0x5EED))
 
 
 def _write_bundle(prefix, tensors):
     """Minimal TF tensor-bundle writer (one data block) to round-trip the reader."""
-    data = b""
-    entries = [(b"", b"\x08\x01")]
+    chunks, off, entries = [], 0, [(b"", _BUNDLE_HEADER)]
     for name in sorted(tensors):
         a = np.ascontiguousarray(tensors[name], "<f4")
-        shape = b"".join(b"\x12" + _varint(len(d)) + d for d in (b"\x08" + _varint(s) for s in a.shape))
-        proto = b"\x08\x01" + b"\x12" + _varint(len(shape)) + shape + b"\x20" + _varint(len(data)) + b"\x28" + _varint(a.nbytes)
-        entries.append((name.encode(), proto))
-        data += a.tobytes()
-    blk = _block(entries)
-    f = blk + b"\x00" + b"\x00" * 4
-    meta_off = len(f)
-    meta = _block([])
-    f += meta + b"\x00" + b"\x00" * 4
-    idx_off = len(f)
-    idx = _block([(b"\xff", _varint(0) + _varint(len(blk)))])
-    f += idx + b"\x00" + b"\x00" * 4
-    footer = _varint(meta_off) + _varint(len(meta)) + _varint(idx_off) + _varint(len(idx))
-    footer += b"\x00" * (40 - len(footer)) + struct.pack("<Q", 0xDB4775248B80FB57)
-    open(prefix + ".index", "wb").write(f + footer)
-    open(prefix + ".data-00000-of-00001", "wb").write(data)
+        entries.append((name.encode(), _entry_proto(1, a.shape, off, a.nbytes)))
+        chunks.append(a.tobytes())
+        off += a.nbytes
+    _write_table(prefix + ".index", entries)
+    with open(prefix + ".data-00000-of-00001", "wb") as f:
+        f.write(b"".join(chunks))
 
 
 def test_bundle_roundtrip(tmp_path):
