@@ -129,9 +129,7 @@ struct nhans_ctx {
   std::vector<ProfRec> prof;
   std::vector<cudaEvent_t> ev_pool;
   double prof_acc[5][4] = {};
-  int debug_skip_epilogue = 0;
   unsigned long long* debug_stats = nullptr;   // [128][8] per-layer wait-cycle counters (NHANS_DEBUG_STATS=1)
-  int desc_mode = 0;
   // NHANS_DEBUG_TIMELINE=1: timing events on the three streams for every batch (nhans_debug_timeline)
   bool timeline = false;
   cudaEvent_t tl_origin = nullptr;
@@ -206,7 +204,7 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
     net.bufs[i] = reinterpret_cast<__half*>(p);
   }
   int rc;
-  if (P.cond.n_cols > 0 && !getenv("NHANS_NO_FRAMECONV")) {
+  if (P.cond.n_cols > 0) {
     // main net: room for the frames of one pass plus 34 virtual frames per utterance (utterances of >= 17 frames on
     // average; a pass of shorter ones falls back to the per-window kernel)
     net.crow_cap = 3LL * P.capacity + 64;
@@ -372,7 +370,6 @@ EpiDev make_epi(const NetDev& net, const Epilogue& E, const Grid& out, const flo
   e.r1_vec = r1_vec; e.r1_sh = E.r1_sh; e.r1_sw = E.r1_sw; e.raw_oh = E.raw_oh;
   e.raw = raw;
   e.relu = E.relu; e.head = E.head;
-  e.pair = E.pair; e.n_real = E.n_real; e.pair_W = E.pair_W; e.res_off0 = E.res_off[0]; e.res_off1 = E.res_off[1];
   fill_out(e, net, out);
   e.out_f32 = out_f32;
   return e;
@@ -452,7 +449,7 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
     g.epi.ttab16 = reinterpret_cast<const __half*>(D.ttab16);
     g.epi.ftab16 = reinterpret_cast<const __half*>(D.ftab16);
     g.epi.tab_H = L.Ho;
-    g.epi.tab_W = L.epi.pair ? L.epi.pair_W : L.Wo;
+    g.epi.tab_W = L.Wo;
     g.err_flag = ctx->err_flag_dev;
     g.ksplit = 1;
     // last_dense: 16 row tiles per 2048-window pass but K = 13312 - split K over the idle SMs (deterministic two-stage sum)
@@ -460,7 +457,6 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
     // share the pass)
     const bool split_head = L.epi.head && net.head_scratch && (int)L.groups.size() % kHeadSplit == 0;
     if (split_head) { g.ksplit = kHeadSplit; g.split_scratch = net.head_scratch; }
-    g.debug_skip_epilogue = ctx->debug_skip_epilogue;
     g.debug_stats = ctx->debug_stats ? ctx->debug_stats + 8 * ((&net == &ctx->tower ? 64 : 0) + (int)i) : nullptr;
     ProfScope ps(ctx, 0, 2.0 * L.macs_per_unit * units, 0, (&net == &ctx->tower ? 64 : 0) + (int)i);
     if (L.walk && D.w_walk && ctx->use_walk) {
@@ -479,7 +475,7 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
       continue;
     }
     {
-      cudaError_t le = launch_gemm(ctx->stream, ctx->n_sm, D.mapA0, D.mapA1, D.mapB, D.mapBhalf, g, ctx->desc_mode);
+      cudaError_t le = launch_gemm(ctx->stream, ctx->n_sm, D.mapA0, D.mapA1, D.mapB, D.mapBhalf, g);
       if (le != cudaSuccess)
         return fail(ctx, NHANS_ERR_CUDA, "launch of layer " + L.name + " (M " + std::to_string(g.M) + ", BN " + std::to_string(g.BN) + "): " + cudaGetErrorString(le));
       if (split_head) {
@@ -615,8 +611,6 @@ int nhans_create(int device, int variant, int win_capacity, int row_capacity, nh
   ctx->variant = variant;
   if (win_capacity > 0) ctx->win_cap = win_capacity;
   if (row_capacity > 0) ctx->row_cap = row_capacity;
-  if (const char* dbg = getenv("NHANS_DEBUG_SKIP_EPILOGUE")) ctx->debug_skip_epilogue = atoi(dbg);
-  if (const char* dbg = getenv("NHANS_DESC_MODE")) ctx->desc_mode = atoi(dbg);
   if (const char* dbg = getenv("NHANS_DEBUG_TIMELINE")) ctx->timeline = atoi(dbg) != 0;
   if (const char* dbg = getenv("NHANS_NO_WALK")) ctx->use_walk = atoi(dbg) == 0;
   if (const char* dbg = getenv("NHANS_NO_GEN")) ctx->use_gen = atoi(dbg) == 0;
@@ -639,7 +633,6 @@ int nhans_create(int device, int variant, int win_capacity, int row_capacity, nh
   if ((e = cudaHostAlloc((void**)&ctx->err_flag_host, sizeof(int), cudaHostAllocMapped)) != cudaSuccess) return bail(cudaGetErrorString(e));
   *ctx->err_flag_host = 0;
   if ((e = cudaHostGetDevicePointer((void**)&ctx->err_flag_dev, ctx->err_flag_host, 0)) != cudaSuccess) return bail(cudaGetErrorString(e));
-  if ((e = gemm_configure()) != cudaSuccess) return bail(std::string("gemm_configure: ") + cudaGetErrorString(e));
   if ((e = dsp_init_tables()) != cudaSuccess) return bail(std::string("dsp_init_tables: ") + cudaGetErrorString(e));
   for (auto& ev : ctx->events) cudaEventCreate(&ev);
   *out = c.release();

@@ -463,7 +463,7 @@ cudaError_t launch_flavour(cudaStream_t s, int grid, const CUtensorMap& a, const
 cudaError_t launch_walk(cudaStream_t s, int n_sm, const CUtensorMap& mapA, const CUtensorMap& mapB, const WalkDev& p) {
   if (p.plane_rows <= 0) return cudaSuccess;
   const EpiDev& e = p.epi;
-  if (p.H < 1 || p.H > kMaxH || p.pt < 0 || p.pt > kWalkKH - 1 || e.head || e.pair || e.o_mode != 0 || e.out_C != 64 ||
+  if (p.H < 1 || p.H > kMaxH || p.pt < 0 || p.pt > kWalkKH - 1 || e.head || e.o_mode != 0 || e.out_C != 64 ||
       (e.res && e.res_C != 64) || (e.res && e.r1_vec))
     return cudaErrorInvalidValue;
   const int tiles = (p.plane_rows + 127) / 128;

@@ -110,10 +110,7 @@ __device__ __forceinline__ void warp_pass_b(float2* __restrict__ z, int nfw, int
 // ((1, 0) where X = 0) instead of the angle - what the fused path keeps between the two transforms (SURVEY.md A.3:
 // no atan2 here, no sincos in the inverse).
 template <bool PHASOR>
-#ifndef NHANS_STFT_MINB
-#define NHANS_STFT_MINB 6
-#endif
-__global__ void __launch_bounds__(kSW * 32, NHANS_STFT_MINB)
+__global__ void __launch_bounds__(kSW * 32, 6)
 stft_kernel(const int16_t* __restrict__ pcm, const float* __restrict__ xf, const long long* __restrict__ offs,
             const long long* __restrict__ frame_offs, const int* __restrict__ peak, float* __restrict__ logmag,
             float* __restrict__ phase) {
@@ -121,13 +118,8 @@ stft_kernel(const int16_t* __restrict__ pcm, const float* __restrict__ xf, const
   __shared__ __align__(16) float2 s_z[kSW][kFW * 200];
   // TMA landing zone of the int16 span (16-byte aligned start and size): the FFT buffers, which nobody touches
   // before the samples are converted
-#ifdef NHANS_STFT_NOALIAS
-  __shared__ __align__(16) int16_t s_raw_buf[kSpanF + 16];
-  int16_t* s_raw = s_raw_buf;
-#else
   int16_t* s_raw = reinterpret_cast<int16_t*>(&s_z[0][0]);
   static_assert(sizeof(float2) * kSW * kFW * 200 >= (kSpanF + 16) * sizeof(int16_t), "raw span must fit the FFT buffers");
-#endif
   __shared__ __align__(8) uint64_t s_bar;
   const int u = blockIdx.y;
   const int T = (int)(frame_offs[u + 1] - frame_offs[u]);

@@ -23,20 +23,19 @@
 //                           releases ring slots / publishes accumulators in both CTAs; split-K for the head
 //   warps 0-7 epilogue      two flavours (kEpiRow): row-per-thread for BN <= 128 (thread = TMEM lane = GEMM
 //                           row, 16 channels per step, 256-bit residual loads and stores, fp16 tables and
-//                           per-channel vectors in shared memory, no staging) and transposing for BN = 256
-//                           (tcgen05.ld -> XOR-swizzled fp32 transpose -> 4 lanes per row, coalesced).
+//                           per-channel vectors in shared memory, no staging) and transposing for BN = 256 and
+//                           the head (tcgen05.ld -> XOR-swizzled fp32 transpose -> 4 lanes per row, coalesced).
 //                           + per-utterance conditioning bias + time / frequency embedding tables + scaled
 //                           identity residual / rank-1 transform -> ReLU -> fp16 into the consumer's grid
 //                           (or, for the head, raw fp32 partial sums of one K split: head_reduce_kernel
 //                           adds the splits, the column scale, the bias and the centre frame)
 //
 // The 64-channel stride-1 layers of the mask network run on conv_walk.cu instead (this kernel remains their
-// NHANS_NO_WALK fallback as a plain N = 64 GEMM, and round 1's pixel-pair form behind NHANS_STAGE1=pair).
+// NHANS_NO_WALK fallback as a plain N = 64 GEMM).
 //
 // The epilogue is the fusion of blocks.py:104-108 (batch-norm), main.py:166,172 (conditioning adds),
 // main.py:184-186 (residual add, ReLU) folded as in SURVEY.md App. A.6.
 #include <cstdio>
-#include <cstdlib>
 
 #include "kernels.h"
 #include "ptx.cuh"
@@ -54,11 +53,7 @@ constexpr int kEpiBytes = kEpiWarps * kEpiWarpBytes;
 constexpr int kMaxGroups = 212;
 constexpr int kMaxA = 8, kMaxB = 16;
 constexpr int kSmemLimit = 227 * 1024;
-#ifdef NHANS_ISSUERS_FIRST
-constexpr int kWarpA = 0, kWarpB = 1, kWarpMma = 2, kEpiWarp0 = 3;
-#else
-constexpr int kWarpA = 8, kWarpB = 9, kWarpMma = 10, kEpiWarp0 = 0;
-#endif
+constexpr int kWarpA = 8, kWarpB = 9, kWarpMma = 10;
 
 struct __align__(8) Ctrl {
   uint64_t a_full[kMaxA], a_empty[kMaxA];
@@ -87,7 +82,7 @@ __device__ __forceinline__ void mma_issuer(Ctrl* ctrl, const GemmDev& p, const G
   const int MT = cfg.mt;
   const int num_groups = p.num_groups;
   // CTA pairs: M = 256 (bit 24.. holds M >> 4), issued by the leader for both CTAs
-  const uint32_t idesc = ptx::umma_idesc_f16((uint32_t)(cfg.dbg & 4 ? p.BN >> 1 : p.BN)) + (CTA2 ? (8u << 24) : 0u);
+  const uint32_t idesc = ptx::umma_idesc_f16((uint32_t)p.BN) + (CTA2 ? (8u << 24) : 0u);
   const uint64_t desc_hi = ptx::umma_desc_sw128(0, 0);             // everything but the address field
   const uint32_t a_base = ptx::smem_u32(smem_a) >> 4, b_base = ptx::smem_u32(smem_b) >> 4;
   const uint32_t b_step = (uint32_t)b_bytes >> 4;
@@ -174,36 +169,28 @@ __device__ __forceinline__ void mma_issuer(Ctrl* ctrl, const GemmDev& p, const G
 }
 
 // Epilogue flavours (compile-time: the epilogue is instruction bound, every runtime flag costs issue slots)
-constexpr int kEpiPair = 1;       // pixel-pair rows (plan.h Epilogue::pair)
 constexpr int kEpiRes = 2;        // + res_scale[c] * x (identity residual)
 constexpr int kEpiR1 = 4;         // + r1_vec[c] * raw spectrogram value (1x1 transform with Cin = 1)
-constexpr int kEpiTabS = 8;       // time / frequency embedding tables (fp16) resident in shared memory
-constexpr int kEpiTabG = 16;      // combined fp32 embedding table read from global memory
+constexpr int kEpiTabS = 8;       // time / frequency embedding tables (fp16) resident in shared memory (row flavour)
+constexpr int kEpiTabG = 16;      // combined fp32 embedding table read from global memory (transposing flavour)
 constexpr int kEpiHead = 32;      // last_dense: fp32 out + centre frame
 constexpr int kEpiRow = 64;       // row-per-thread epilogue (below) instead of the transposing one
 
-// One epilogue warp.  ew = 0..7: TMEM lane quarter q = ew & 3, and the two warps of a quarter (half = ew >> 2)
-// take alternate 16-column chunks.  Per chunk: tcgen05.ld (thread = row) -> XOR-swizzled 32 x 16 fp32 transpose
-// in shared memory -> 4 lanes per row x 4 channels, so that global loads / stores are coalesced.  The loads
-// of chunk k + 1 are in flight while chunk k is processed; slot metadata is computed one slot ahead.
+// One epilogue warp of the BN > 128 layers (a CTA tile is one sub-tile of 128 rows: mt = 1).  ew = 0..7: TMEM lane
+// quarter q = ew & 3, and the two warps of a quarter (half = ew >> 2) take alternate 16-column chunks.  Per chunk:
+// tcgen05.ld (thread = row) -> XOR-swizzled 32 x 16 fp32 transpose in shared memory -> 4 lanes per row x 4 channels,
+// so that global loads / stores are coalesced.  The loads of chunk k + 1 are in flight while chunk k is processed.
 template <int EPI, bool CTA2>
-__device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, const GemmCfg& cfg, int ew, int lane,
-                                              uint32_t tmem_base, int num_tiles, int n_tiles, const __half* s_ttab,
-                                              const __half* s_ftab, uint32_t rank) {
-  constexpr bool kPair = EPI & kEpiPair, kRes = EPI & kEpiRes, kR1 = EPI & kEpiR1, kTabS = EPI & kEpiTabS,
-                 kTabG = EPI & kEpiTabG, kHead = EPI & kEpiHead;
+__device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, int ew, int lane, uint32_t tmem_base,
+                                              int num_tiles, int n_tiles, uint32_t rank) {
+  constexpr bool kRes = EPI & kEpiRes, kR1 = EPI & kEpiR1, kTabG = EPI & kEpiTabG, kHead = EPI & kEpiHead;
   const EpiDev& e = p.epi;
-  const int MT = cfg.mt;
   const int q = ew & 3, half = ew >> 2;
   uint8_t* epi_base = reinterpret_cast<uint8_t*>(ctrl) + kCtrlBytes + ew * kEpiWarpBytes;
   uint4* stage = reinterpret_cast<uint4*>(epi_base);                 // [32 rows][4 x 16 B], XOR swizzled
   int4* meta = reinterpret_cast<int4*>(epi_base + 32 * 64);          // [32] {pixel, (ho << 16) | wo, utt, raw bits}
   const int sub = lane >> 2;                // row within a group of 8
   const int jc = lane & 3;                  // 16-byte column slot: channels 4 jc .. 4 jc + 3 of the chunk
-  const int NV = kPair ? 2 * MT : MT;       // slots per tile: sub-tile i, or (sub-tile i, pixel j) for pair rows
-  const int vcols = kPair ? e.n_real : p.BN;
-  const int tab_C = kPair ? e.n_real : p.N; // row pitch of the embedding tables
-  const int tab_W = kPair ? e.pair_W : p.Wo;
   struct LoadSet {
     float4 b[4], t[4];
     uint2 x[4];
@@ -224,29 +211,23 @@ __device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, cons
     const uint32_t acc = it & 1, acc_phase = (it >> 1) & 1;
     const int tile_sp = tile / p.ksplit, split = tile - tile_sp * p.ksplit;
     const int n0 = (tile_sp % n_tiles) * p.BN;
-    if (p.debug_skip_epilogue == 1) {
+    // tile -> (row chunk, image row) with the image row fastest (kernels.h GemmDev)
+    const int mtile = tile_sp / n_tiles;
+    const int tchunk = mtile / p.Ho, ho = mtile - tchunk * p.Ho;
+    const int local0 = tchunk * sub_rows + (int)rank * 128;      // first row of this CTA within the plane
+    const int tile_m0 = ho * p.plane_pitch + local0;
+    if (local0 >= p.plane_rows) {           // the second CTA of a pair past the plane's last row
       ptx::mbar_wait(&ctrl->tmem_full[acc], acc_phase, p.err_flag, 4);
       release_acc(acc);
       continue;
     }
-    // tile -> (row chunk, image row) with the image row fastest (kernels.h GemmDev)
-    const int mtile = tile_sp / n_tiles;
-    const int tchunk = mtile / p.Ho, ho = mtile - tchunk * p.Ho;
-    const int local0 = tchunk * (MT * sub_rows) + (int)rank * 128;      // first row of this CTA within the plane
-    const int tile_m0 = ho * p.plane_pitch + local0;
-    // metadata of the row this thread owns in slot v (its TMEM lane)
-    auto slot_meta = [&](int v) -> int4 {
-      if (v >= NV) return make_int4(-1, 0, 0, 0);
-      const int i = kPair ? (v >> 1) : v, j = kPair ? (v & 1) : 0;
-      const int r = local0 + i * sub_rows + q * 32 + lane;
+    // metadata of the row this thread owns (its TMEM lane)
+    auto slot_meta = [&]() -> int4 {
+      const int r = local0 + q * 32 + lane;
       if (r >= p.plane_rows) return make_int4(-1, 0, 0, 0);
       const int unit = r / p.Wq;
-      int wo = r - unit * p.Wq;
+      const int wo = r - unit * p.Wq;
       if (wo >= p.Wo) return make_int4(-1, 0, 0, 0);
-      if (kPair) {
-        wo = 2 * wo + j;
-        if (wo >= e.pair_W) return make_int4(-1, 0, 0, 0);
-      }
       int pix, utt = p.units.utt[unit];
       float rawv = 0.f;
       if (kR1) {
@@ -265,137 +246,110 @@ __device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, cons
       }
       return make_int4(pix, (ho << 16) | wo, utt, __float_as_int(rawv));
     };
-    bool waited = false;
-    int4 md_next = slot_meta(0);
-#pragma unroll 1
-    for (int v = 0; v < NV; ++v) {
-      const int i = kPair ? (v >> 1) : v;
-      const int m0 = tile_m0 + i * sub_rows;
-      if (local0 + i * sub_rows >= p.plane_rows) break;
-      const int4 md_cur = md_next;
-      md_next = slot_meta(v + 1);             // its loads are in flight while slot v is processed
-      __syncwarp();
-      meta[lane] = md_cur;
-      __syncwarp();
-      // per row group g (row 8 g + sub of the warp's 32 rows): element offsets hoisted out of the chunk loop
-      bool ok[4];
-      float raws[4];
-      size_t o_out[4], o_res[4], o_bias[4], o_tf[4];
-      int o_t[4], o_f[4];
-      const int col0 = n0 + 4 * jc;
+    __syncwarp();
+    meta[lane] = slot_meta();
+    __syncwarp();
+    // per row group g (row 8 g + sub of the warp's 32 rows): element offsets hoisted out of the chunk loop
+    bool ok[4];
+    float raws[4];
+    size_t o_out[4], o_res[4], o_bias[4], o_tf[4];
+    const int col0 = n0 + 4 * jc;
+#pragma unroll
+    for (int g = 0; g < 4; ++g) {
+      const int4 mm = meta[g * 8 + sub];
+      ok[g] = mm.x >= 0;
+      raws[g] = __int_as_float(mm.w);
+      const int ho = mm.y >> 16, wo = mm.y & 0xffff;
+      o_out[g] = (size_t)mm.x * (kHead ? 201 : e.out_C) + col0;
+      o_bias[g] = (size_t)mm.z * (kHead ? 201 : e.bias_stride) + col0;   // head: mm.z = centre frame row of raw
+      if (kRes) o_res[g] = (size_t)((long long)tile_m0 + q * 32 + g * 8 + sub) * e.res_C + col0;
+      if (kTabG) o_tf[g] = (size_t)(ho * p.Wo + wo) * p.N + col0;
+    }
+    auto issue_loads = [&](LoadSet& L, int c0) {
+      if (kHead || c0 >= p.BN) return;
 #pragma unroll
       for (int g = 0; g < 4; ++g) {
-        const int4 mm = meta[g * 8 + sub];
-        ok[g] = mm.x >= 0;
-        raws[g] = __int_as_float(mm.w);
-        const int ho = mm.y >> 16, wo = mm.y & 0xffff;
-        o_out[g] = (size_t)mm.x * (kHead ? 201 : e.out_C) + col0;
-        o_bias[g] = (size_t)mm.z * (kHead ? 201 : e.bias_stride) + col0;   // head: mm.z = centre frame row of raw
+        if (!ok[g]) continue;
+        L.b[g] = __ldg(reinterpret_cast<const float4*>(e.bias + o_bias[g] + c0));
+        if (kTabG) L.t[g] = __ldg(reinterpret_cast<const float4*>(e.tftab + o_tf[g] + c0));
+        if (kRes) L.x[g] = __ldg(reinterpret_cast<const uint2*>(e.res + o_res[g] + c0));
+      }
+    };
+    const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * 256;
+    auto process = [&](const LoadSet& L, int c0) {
+      {
+        uint32_t tv[16];
+        ptx::tmem_ld16(t_addr + c0, tv);
+        ptx::tmem_ld_wait();
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          stage[lane * 4 + ((j ^ (lane >> 1)) & 3)] = make_uint4(tv[4 * j], tv[4 * j + 1], tv[4 * j + 2], tv[4 * j + 3]);
+      }
+      __syncwarp();
+      float4 rs, r1;
+      if (kRes) rs = __ldg(reinterpret_cast<const float4*>(e.res_scale + col0 + c0));
+      if (kR1) r1 = __ldg(reinterpret_cast<const float4*>(e.r1_vec + col0 + c0));
+#pragma unroll
+      for (int g = 0; g < 4; ++g) {
+        if (!ok[g]) continue;
+        const int r = g * 8 + sub;
+        const uint4 u = stage[r * 4 + ((jc ^ (r >> 1)) & 3)];
+        float4 f = make_float4(__uint_as_float(u.x), __uint_as_float(u.y), __uint_as_float(u.z), __uint_as_float(u.w));
+        if (kHead && p.ksplit > 1) {
+          // split-K: raw partial sums of this split, [split][unit][N]; o_out = unit * 201 + col0
+          const size_t unit = (o_out[g] - col0) / 201;
+          *reinterpret_cast<float4*>(p.split_scratch + ((size_t)split * (p.plane_rows / p.Wq) + unit) * p.N + col0 + c0) = f;
+          continue;
+        }
+        if (kHead) {
+          const int col = col0 + c0;
+          const float4 b = __ldg(reinterpret_cast<const float4*>(e.bias + col));
+          const float4 sc = __ldg(reinterpret_cast<const float4*>(e.res_scale + col));   // inverse weight scale of the column
+          const float* raw_row = e.raw + o_bias[g] - col0;
+          float* o = e.out_f32 + o_out[g] - col0;
+          if (col < 201) o[col] = f.x * sc.x + b.x + raw_row[col];
+          if (col + 1 < 201) o[col + 1] = f.y * sc.y + b.y + raw_row[col + 1];
+          if (col + 2 < 201) o[col + 2] = f.z * sc.z + b.z + raw_row[col + 2];
+          if (col + 3 < 201) o[col + 3] = f.w * sc.w + b.w + raw_row[col + 3];
+          continue;
+        }
+        f.x += L.b[g].x; f.y += L.b[g].y; f.z += L.b[g].z; f.w += L.b[g].w;
+        if (kTabG) { f.x += L.t[g].x; f.y += L.t[g].y; f.z += L.t[g].z; f.w += L.t[g].w; }
         if (kRes) {
-          const long long rr = (long long)m0 + q * 32 + g * 8 + sub + (kPair ? ((v & 1) ? e.res_off1 : e.res_off0) : 0);
-          o_res[g] = (size_t)rr * e.res_C + col0;
+          const float2 x0 = __half22float2(*reinterpret_cast<const __half2*>(&L.x[g].x));
+          const float2 x1 = __half22float2(*reinterpret_cast<const __half2*>(&L.x[g].y));
+          f.x = fmaf(rs.x, x0.x, f.x); f.y = fmaf(rs.y, x0.y, f.y);
+          f.z = fmaf(rs.z, x1.x, f.z); f.w = fmaf(rs.w, x1.y, f.w);
         }
-        if (kTabS) { o_t[g] = ho * tab_C + col0; o_f[g] = wo * tab_C + col0; }
-        if (kTabG) o_tf[g] = (size_t)(ho * tab_W + wo) * tab_C + col0;
+        if (kR1) {
+          f.x = fmaf(r1.x, raws[g], f.x); f.y = fmaf(r1.y, raws[g], f.y);
+          f.z = fmaf(r1.z, raws[g], f.z); f.w = fmaf(r1.w, raws[g], f.w);
+        }
+        if (e.relu) {
+          f.x = fmaxf(f.x, 0.f); f.y = fmaxf(f.y, 0.f); f.z = fmaxf(f.z, 0.f); f.w = fmaxf(f.w, 0.f);
+        }
+        uint2 o;
+        o.x = pack_half2(f.x, f.y);
+        o.y = pack_half2(f.z, f.w);
+        *reinterpret_cast<uint2*>(e.out + o_out[g] + c0) = o;
       }
-      auto issue_loads = [&](LoadSet& L, int c0) {
-        if (kHead || c0 >= vcols || p.debug_skip_epilogue == 2) return;
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-          if (!ok[g]) continue;
-          L.b[g] = __ldg(reinterpret_cast<const float4*>(e.bias + o_bias[g] + c0));
-          if (kTabG) L.t[g] = __ldg(reinterpret_cast<const float4*>(e.tftab + o_tf[g] + c0));
-          if (kRes) L.x[g] = __ldg(reinterpret_cast<const uint2*>(e.res + o_res[g] + c0));
-        }
-      };
-      const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * 256 + i * p.BN + (kPair ? (v & 1) * e.n_real : 0);
-      auto process = [&](const LoadSet& L, int c0) {
-        {
-          uint32_t tv[16];
-          ptx::tmem_ld16(t_addr + c0, tv);
-          ptx::tmem_ld_wait();
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            stage[lane * 4 + ((j ^ (lane >> 1)) & 3)] = make_uint4(tv[4 * j], tv[4 * j + 1], tv[4 * j + 2], tv[4 * j + 3]);
-        }
-        __syncwarp();
-        float4 rs, r1;
-        if (kRes) rs = __ldg(reinterpret_cast<const float4*>(e.res_scale + col0 + c0));
-        if (kR1) r1 = __ldg(reinterpret_cast<const float4*>(e.r1_vec + col0 + c0));
-#pragma unroll
-        for (int g = 0; g < 4; ++g) {
-          if (!ok[g]) continue;
-          const int r = g * 8 + sub;
-          const uint4 u = stage[r * 4 + ((jc ^ (r >> 1)) & 3)];
-          float4 f = make_float4(__uint_as_float(u.x), __uint_as_float(u.y), __uint_as_float(u.z), __uint_as_float(u.w));
-          if (kHead && p.ksplit > 1) {
-            // split-K: raw partial sums of this split, [split][unit][N]; o_out = unit * 201 + col0
-            const size_t unit = (o_out[g] - col0) / 201;
-            *reinterpret_cast<float4*>(p.split_scratch + ((size_t)split * (p.plane_rows / p.Wq) + unit) * p.N + col0 + c0) = f;
-            continue;
-          }
-          if (kHead) {
-            const int col = col0 + c0;
-            const float4 b = __ldg(reinterpret_cast<const float4*>(e.bias + col));
-            const float4 sc = __ldg(reinterpret_cast<const float4*>(e.res_scale + col));   // inverse weight scale of the column
-            const float* raw_row = e.raw + o_bias[g] - col0;
-            float* o = e.out_f32 + o_out[g] - col0;
-            if (col < 201) o[col] = f.x * sc.x + b.x + raw_row[col];
-            if (col + 1 < 201) o[col + 1] = f.y * sc.y + b.y + raw_row[col + 1];
-            if (col + 2 < 201) o[col + 2] = f.z * sc.z + b.z + raw_row[col + 2];
-            if (col + 3 < 201) o[col + 3] = f.w * sc.w + b.w + raw_row[col + 3];
-            continue;
-          }
-          if (p.debug_skip_epilogue != 2) { f.x += L.b[g].x; f.y += L.b[g].y; f.z += L.b[g].z; f.w += L.b[g].w; }
-          if (kTabG && p.debug_skip_epilogue != 2) { f.x += L.t[g].x; f.y += L.t[g].y; f.z += L.t[g].z; f.w += L.t[g].w; }
-          if (kTabS) {
-            // fp16 tables: add time + frequency rows as half2, then widen once
-            const uint2 tv = *reinterpret_cast<const uint2*>(s_ttab + o_t[g] + c0);
-            const uint2 fv = *reinterpret_cast<const uint2*>(s_ftab + o_f[g] + c0);
-            const float2 s0 = __half22float2(__hadd2(*reinterpret_cast<const __half2*>(&tv.x), *reinterpret_cast<const __half2*>(&fv.x)));
-            const float2 s1 = __half22float2(__hadd2(*reinterpret_cast<const __half2*>(&tv.y), *reinterpret_cast<const __half2*>(&fv.y)));
-            f.x += s0.x; f.y += s0.y; f.z += s1.x; f.w += s1.y;
-          }
-          if (kRes && p.debug_skip_epilogue != 2) {
-            const float2 x0 = __half22float2(*reinterpret_cast<const __half2*>(&L.x[g].x));
-            const float2 x1 = __half22float2(*reinterpret_cast<const __half2*>(&L.x[g].y));
-            f.x = fmaf(rs.x, x0.x, f.x); f.y = fmaf(rs.y, x0.y, f.y);
-            f.z = fmaf(rs.z, x1.x, f.z); f.w = fmaf(rs.w, x1.y, f.w);
-          }
-          if (kR1) {
-            f.x = fmaf(r1.x, raws[g], f.x); f.y = fmaf(r1.y, raws[g], f.y);
-            f.z = fmaf(r1.z, raws[g], f.z); f.w = fmaf(r1.w, raws[g], f.w);
-          }
-          if (e.relu) {
-            f.x = fmaxf(f.x, 0.f); f.y = fmaxf(f.y, 0.f); f.z = fmaxf(f.z, 0.f); f.w = fmaxf(f.w, 0.f);
-          }
-          uint2 o;
-          o.x = pack_half2(f.x, f.y);
-          o.y = pack_half2(f.z, f.w);
-          if (p.debug_skip_epilogue != 3) *reinterpret_cast<uint2*>(e.out + o_out[g] + c0) = o;
-        }
-        __syncwarp();                         // staging is overwritten by the next chunk
-      };
-      // chunks of this warp: the two warps of a quarter alternate 16-column chunks
-      LoadSet A, B;
-      int c0 = ((half + v) & 1) * 16;
-      issue_loads(A, c0);
-      if (!waited) {
-        ptx::mbar_wait_timed(&ctrl->tmem_full[acc], acc_phase, p.err_flag, 4, &w_full);
-        ptx::tc_fence_after();
-        waited = true;
-      }
+      __syncwarp();                         // staging is overwritten by the next chunk
+    };
+    // chunks of this warp: the two warps of a quarter alternate 16-column chunks
+    LoadSet A, B;
+    int c0 = half * 16;
+    issue_loads(A, c0);
+    ptx::mbar_wait_timed(&ctrl->tmem_full[acc], acc_phase, p.err_flag, 4, &w_full);
+    ptx::tc_fence_after();
 #pragma unroll 1
-      for (; c0 < vcols; c0 += 64) {
-        issue_loads(B, c0 + 32);              // in flight while chunk c0 is processed (no-op past the end)
-        process(A, c0);
-        if (c0 + 32 < vcols) {
-          issue_loads(A, c0 + 64);
-          process(B, c0 + 32);
-        }
+    for (; c0 < p.BN; c0 += 64) {
+      issue_loads(B, c0 + 32);              // in flight while chunk c0 is processed (no-op past the end)
+      process(A, c0);
+      if (c0 + 32 < p.BN) {
+        issue_loads(A, c0 + 64);
+        process(B, c0 + 32);
       }
     }
-    if (!waited) ptx::mbar_wait(&ctrl->tmem_full[acc], acc_phase, p.err_flag, 4);
     release_acc(acc);
   }
   if (p.debug_stats && ew == 0 && lane == 0) atomicAdd(p.debug_stats + 3, (unsigned long long)w_full);
@@ -423,19 +377,13 @@ template <int EPI, bool CTA2>
 __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, const GemmCfg& cfg, int ew, int lane,
                                                   uint32_t tmem_base, int num_tiles, int n_tiles, const __half* s_ttab,
                                                   const __half* s_ftab, const float* s_rs, const float* s_r1, uint32_t rank) {
-  constexpr bool kPair = EPI & kEpiPair, kRes = EPI & kEpiRes, kR1 = EPI & kEpiR1, kTabS = EPI & kEpiTabS,
-                 kTabG = EPI & kEpiTabG;
+  constexpr bool kRes = EPI & kEpiRes, kR1 = EPI & kEpiR1, kTabS = EPI & kEpiTabS;
   const EpiDev& e = p.epi;
   const int MT = cfg.mt;
   const int q = ew & 3, half = ew >> 2;
-  const int NV = kPair ? 2 * MT : MT;
-  const int vcols = kPair ? e.n_real : p.BN;
-  const int tab_C = kPair ? e.n_real : p.N;
-  const int tab_W = kPair ? e.pair_W : p.Wo;
-  const int f_pitch = tab_C + 8;
-  const int half_W = (tab_W + 1) >> 1;
+  const int f_pitch = p.N + 8;
   struct LoadSet {
-    float4 b[4], t[4];
+    float4 b[4];
     uint4 x[2];
   };
   const int cta_shift = CTA2 ? 1 : 0;
@@ -453,35 +401,24 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
   for (int tile = blockIdx.x >> cta_shift; tile < num_tiles; tile += gridDim.x >> cta_shift, ++it) {
     const uint32_t acc = it & 1, acc_phase = (it >> 1) & 1;
     const int n0 = (tile % n_tiles) * p.BN;
-    if (p.debug_skip_epilogue == 1) {
-      ptx::mbar_wait(&ctrl->tmem_full[acc], acc_phase, p.err_flag, 4);
-      release_acc(acc);
-      continue;
-    }
     const int mtile = tile / n_tiles;
     const int tchunk = mtile / p.Ho, ho = mtile - tchunk * p.Ho;      // image row fastest (kernels.h GemmDev)
     const int local0 = tchunk * (MT * sub_rows) + (int)rank * 128;
     const int tile_m0 = ho * p.plane_pitch + local0;
     bool waited = false;
-    bool row_ok = false;
-    int unit = 0, wb = 0, utt = 0;
 #pragma unroll 1
-    for (int v = 0; v < NV; ++v) {
-      const int i = kPair ? (v >> 1) : v, j = kPair ? (v & 1) : 0;
+    for (int i = 0; i < MT; ++i) {
       const int m0 = tile_m0 + i * sub_rows;
       if (local0 + i * sub_rows >= p.plane_rows) break;
       const int m = m0 + q * 32 + lane;
-      if (!kPair || j == 0) {                 // the row this thread owns in sub-tile i
-        const int r = local0 + i * sub_rows + q * 32 + lane;
-        unit = r / p.Wq;
-        wb = r - unit * p.Wq;
-        row_ok = r < p.plane_rows && wb < p.Wo;
-        utt = row_ok ? p.units.utt[unit] : 0;
-      }
-      const int wo = kPair ? 2 * wb + j : wb;
-      const bool ok = row_ok && (!kPair || wo < e.pair_W);
+      // the row this thread owns in sub-tile i
+      const int r = local0 + i * sub_rows + q * 32 + lane;
+      const int unit = r / p.Wq;
+      const int wo = r - unit * p.Wq;
+      const bool ok = r < p.plane_rows && wo < p.Wo;
+      const int utt = ok ? p.units.utt[unit] : 0;
       float rawv = 0.f;
-      size_t o_out = 0, o_bias = 0, o_res = 0, o_tf = 0;
+      size_t o_out = 0, o_bias = 0, o_res = 0;
       int o_t = 0, o_f = 0;
       if (ok) {
         if (kR1) {
@@ -498,24 +435,19 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
         }
         o_out = (size_t)pix * e.out_C + n0;
         o_bias = (size_t)utt * e.bias_stride + n0;
-        if (kRes) o_res = (size_t)((long long)m + (kPair ? (j ? e.res_off1 : e.res_off0) : 0)) * e.res_C + n0;
+        if (kRes) o_res = (size_t)m * e.res_C + n0;
         if (kTabS) {
-          o_t = ho * tab_C + n0;
-          o_f = (kPair ? ((wo & 1) * half_W + (wo >> 1)) : wo) * f_pitch + n0;    // pair tables are stored by column parity
+          o_t = ho * p.N + n0;
+          o_f = wo * f_pitch + n0;
         }
-        if (kTabG) o_tf = (size_t)(ho * tab_W + wo) * tab_C + n0;
       }
       auto issue_loads = [&](LoadSet& L, int c0) {
-        if (c0 >= vcols || !ok || p.debug_skip_epilogue == 2) return;
+        if (c0 >= p.BN || !ok) return;
         const float4* bp = reinterpret_cast<const float4*>(e.bias + o_bias + c0);
         L.b[0] = __ldg(bp); L.b[1] = __ldg(bp + 1); L.b[2] = __ldg(bp + 2); L.b[3] = __ldg(bp + 3);
-        if (kTabG) {
-          const float4* tp = reinterpret_cast<const float4*>(e.tftab + o_tf + c0);
-          L.t[0] = __ldg(tp); L.t[1] = __ldg(tp + 1); L.t[2] = __ldg(tp + 2); L.t[3] = __ldg(tp + 3);
-        }
         if (kRes) ldg256(e.res + o_res + c0, L.x[0], L.x[1]);
       };
-      const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * 256 + i * p.BN + (kPair ? j * e.n_real : 0);
+      const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * 256 + i * p.BN;
       auto process = [&](const LoadSet& L, int c0) {
         uint32_t tv[16];
         ptx::tmem_ld16(t_addr + c0, tv);
@@ -524,14 +456,8 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
         float f[16];
 #pragma unroll
         for (int k = 0; k < 16; ++k) f[k] = __uint_as_float(tv[k]);
-        if (p.debug_skip_epilogue != 2) {
 #pragma unroll
-          for (int k = 0; k < 4; ++k) { f[4 * k] += L.b[k].x; f[4 * k + 1] += L.b[k].y; f[4 * k + 2] += L.b[k].z; f[4 * k + 3] += L.b[k].w; }
-          if (kTabG) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k) { f[4 * k] += L.t[k].x; f[4 * k + 1] += L.t[k].y; f[4 * k + 2] += L.t[k].z; f[4 * k + 3] += L.t[k].w; }
-          }
-        }
+        for (int k = 0; k < 4; ++k) { f[4 * k] += L.b[k].x; f[4 * k + 1] += L.b[k].y; f[4 * k + 2] += L.b[k].z; f[4 * k + 3] += L.b[k].w; }
         if (kTabS) {
           uint4 tt[2], ff[2];
           tt[0] = *reinterpret_cast<const uint4*>(s_ttab + o_t + c0);
@@ -547,7 +473,7 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
             f[2 * k + 1] += s2.y;
           }
         }
-        if (kRes && p.debug_skip_epilogue != 2) {
+        if (kRes) {
           const __half2* xh = reinterpret_cast<const __half2*>(L.x);
           const float4* rs = reinterpret_cast<const float4*>(s_rs + n0 + c0);
 #pragma unroll
@@ -574,10 +500,10 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
         uint4 o0, o1;
         o0.x = pack_half2(f[0], f[1]); o0.y = pack_half2(f[2], f[3]); o0.z = pack_half2(f[4], f[5]); o0.w = pack_half2(f[6], f[7]);
         o1.x = pack_half2(f[8], f[9]); o1.y = pack_half2(f[10], f[11]); o1.z = pack_half2(f[12], f[13]); o1.w = pack_half2(f[14], f[15]);
-        if (p.debug_skip_epilogue != 3) stg256(e.out + o_out + c0, o0, o1);
+        stg256(e.out + o_out + c0, o0, o1);
       };
       LoadSet A, B;
-      int c0 = ((half + v) & 1) * 16;
+      int c0 = ((half + i) & 1) * 16;
       issue_loads(A, c0);
       if (!waited) {
         ptx::mbar_wait_timed(&ctrl->tmem_full[acc], acc_phase, p.err_flag, 4, &w_full);
@@ -585,10 +511,10 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
         waited = true;
       }
 #pragma unroll 1
-      for (; c0 < vcols; c0 += 64) {
+      for (; c0 < p.BN; c0 += 64) {
         issue_loads(B, c0 + 32);
         process(A, c0);
-        if (c0 + 32 < vcols) {
+        if (c0 + 32 < p.BN) {
           issue_loads(A, c0 + 64);
           process(B, c0 + 32);
         }
@@ -624,40 +550,32 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
   const int num_groups = p.num_groups;
 
   for (int i = threadIdx.x; i < num_groups; i += blockDim.x) ctrl->groups[i] = p.groups[i];
-  // optional shared-memory copies of the fp16 time / frequency embedding tables (after the epilogue staging)
+  // row flavour: shared-memory copies of the fp16 time / frequency embedding tables (frequency rows padded by 8
+  // halfs), then the per-channel residual scale / rank-1 vectors as fp32, after the control block
   constexpr bool kRow = (EPI & kEpiRow) != 0;
-  uint8_t* tab_base = reinterpret_cast<uint8_t*>(ctrl) + kCtrlBytes + (kRow ? 0 : kEpiBytes);
-  __half* s_ttab = reinterpret_cast<__half*>(tab_base);
-  const int tab_C = p.epi.pair ? p.epi.n_real : p.N;
-  __half* s_ftab = s_ttab + p.epi.tab_H * tab_C;
+  __half* s_ttab = nullptr;
+  __half* s_ftab = nullptr;
   float* s_rs = nullptr;
   float* s_r1 = nullptr;
   if (kRow) {
-    // row flavour: frequency rows padded by 8 halfs (pair layers: rows ordered by column parity, so that the rows of
-    // consecutive GEMM rows are consecutive), then the per-channel residual scale / rank-1 vectors as fp32
-    const bool tabs = (EPI & kEpiTabS) != 0;
-    const int f_pitch = tab_C + 8;
-    const int half_W = (p.epi.tab_W + 1) >> 1;
-    if (!tabs) s_ftab = s_ttab;
-    float* vec = reinterpret_cast<float*>(tabs ? reinterpret_cast<uint8_t*>(s_ftab) + (((size_t)p.epi.tab_W * f_pitch * 2 + 15) & ~(size_t)15)
-                                               : tab_base);
-    s_rs = vec;
-    s_r1 = vec + p.N;
-    if (tabs) {
-      const int nt = p.epi.tab_H * tab_C / 8, c8 = tab_C / 8;
+    uint8_t* tab_base = reinterpret_cast<uint8_t*>(ctrl) + kCtrlBytes;
+    float* vec = reinterpret_cast<float*>(tab_base);
+    if (EPI & kEpiTabS) {
+      const int f_pitch = p.N + 8;
+      s_ttab = reinterpret_cast<__half*>(tab_base);
+      s_ftab = s_ttab + p.epi.tab_H * p.N;
+      vec = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(s_ftab) + (((size_t)p.epi.tab_W * f_pitch * 2 + 15) & ~(size_t)15));
+      const int nt = p.epi.tab_H * p.N / 8, c8 = p.N / 8;
       for (int i = threadIdx.x; i < nt; i += blockDim.x) reinterpret_cast<uint4*>(s_ttab)[i] = reinterpret_cast<const uint4*>(p.epi.ttab16)[i];
       for (int i = threadIdx.x; i < p.epi.tab_W * c8; i += blockDim.x) {
         const int w = i / c8, c = i - w * c8;
-        const int r = p.epi.pair ? ((w & 1) * half_W + (w >> 1)) : w;
-        *reinterpret_cast<uint4*>(s_ftab + (size_t)r * f_pitch + c * 8) = reinterpret_cast<const uint4*>(p.epi.ftab16)[i];
+        *reinterpret_cast<uint4*>(s_ftab + (size_t)w * f_pitch + c * 8) = reinterpret_cast<const uint4*>(p.epi.ftab16)[i];
       }
     }
+    s_rs = vec;
+    s_r1 = vec + p.N;
     if (EPI & kEpiRes) for (int i = threadIdx.x; i < p.N; i += blockDim.x) s_rs[i] = p.epi.res_scale[i];
     if (EPI & kEpiR1) for (int i = threadIdx.x; i < p.N; i += blockDim.x) s_r1[i] = p.epi.r1_vec[i];
-  } else if (cfg.tab_bytes) {
-    const int nt = p.epi.tab_H * tab_C / 8, nf = p.epi.tab_W * tab_C / 8;       // 16-byte units
-    for (int i = threadIdx.x; i < nt; i += blockDim.x) reinterpret_cast<uint4*>(s_ttab)[i] = reinterpret_cast<const uint4*>(p.epi.ttab16)[i];
-    for (int i = threadIdx.x; i < nf; i += blockDim.x) reinterpret_cast<uint4*>(s_ftab)[i] = reinterpret_cast<const uint4*>(p.epi.ftab16)[i];
   }
   if (threadIdx.x == 0) {
     for (int s = 0; s < cfg.na; ++s) { ptx::mbar_init(&ctrl->a_full[s], 1); ptx::mbar_init(&ctrl->a_empty[s], 1); }
@@ -698,9 +616,7 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
         uint64_t* gbar = &ctrl->a_full[slot];               // the group's slabs complete on its first slab's barrier
         for (int i = 0; i < MT; ++i) {
           ptx::mbar_wait(&ctrl->a_empty[slot], phase ^ 1, p.err_flag, 1);
-          if (cfg.dbg & 1) {
-            if (rank == 0 && i == 0 && ptx::elect_one()) ptx::mbar_arrive(gbar);
-          } else if (ptx::elect_one()) {
+          if (ptx::elect_one()) {
             if (CTA2) {
               // both CTAs' slabs are credited to the leader's barrier
               if (rank == 0 && i == 0) ptx::mbar_expect_tx(gbar, 2 * MT * kSlabBytes);
@@ -741,9 +657,7 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
           for (int t = 0; t < ntaps; ++t) {
             const int bk = ctrl->groups[g].bk[t];
             ptx::mbar_wait(&ctrl->b_empty[slot], phase ^ 1, p.err_flag, 5);
-            if (cfg.dbg & 2) {
-              if (rank == 0 && t == 0 && ptx::elect_one()) ptx::mbar_arrive(gbar);
-            } else if (ptx::elect_one()) {
+            if (ptx::elect_one()) {
               if (CTA2) {
                 if (rank == 0 && t == 0) ptx::mbar_expect_tx(gbar, 2u * (uint32_t)(ntaps * b_bytes));
                 ptx::tma_load_2d_2sm(smem_b + (size_t)slot * b_bytes, &mapB, gbar, bk * 64, n0);
@@ -763,18 +677,16 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     if (rank != 0) {
       // the peer CTA of a pair only lends its shared memory / TMEM; the leader issues for both
     } else if (cfg.resident) {
-      if (cfg.il == 4) mma_issuer<4, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
-      else if (cfg.il == 2) mma_issuer<2, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
+      if (cfg.il == 2) mma_issuer<2, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
       else mma_issuer<1, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
     } else {
-      if (cfg.il == 4) mma_issuer<4, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
-      else if (cfg.il == 2) mma_issuer<2, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
+      if (cfg.il == 2) mma_issuer<2, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
       else mma_issuer<1, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
     }
   } else {
     // ===================== epilogue (warps 0..7) =====================
-    if (kRow) epilogue_warp_row<EPI, CTA2>(ctrl, p, cfg, warp - kEpiWarp0, lane, tmem_base, num_tiles, n_tiles, s_ttab, s_ftab, s_rs, s_r1, rank);
-    else epilogue_warp<EPI, CTA2>(ctrl, p, cfg, warp - kEpiWarp0, lane, tmem_base, num_tiles, n_tiles, s_ttab, s_ftab, rank);
+    if (kRow) epilogue_warp_row<EPI, CTA2>(ctrl, p, cfg, warp, lane, tmem_base, num_tiles, n_tiles, s_ttab, s_ftab, s_rs, s_r1, rank);
+    else epilogue_warp<EPI, CTA2>(ctrl, p, warp, lane, tmem_base, num_tiles, n_tiles, rank);
   }
 
   ptx::tc_fence_before();
@@ -794,24 +706,18 @@ int gemm_smem_bytes(int BN, int num_kb, int tab_bytes, int cta2, int row, GemmCf
   GemmCfg c;
   c.cta2 = cta2;
   c.row = row;
-  // shared-memory tables only where the epilogue is the critical path (short main loops: BN <= 128); the row
-  // flavour's tab_bytes (padded tables + per-channel vectors) is computed by the caller and always taken
-  c.tab_bytes = ((BN <= 128 || row) && tab_bytes > 0) ? ((tab_bytes + 127) & ~127) : 0;
+  c.tab_bytes = (tab_bytes + 127) & ~127;       // the row flavour's padded tables + per-channel vectors, else 0
   c.mt = 256 / BN < 1 ? 1 : 256 / BN;
   // A ring: 4 slabs = 4 groups ahead for BN = 256 (one slab per group).  BN <= 128 tiles take two slabs per group and
   // the stride-2 layers consume a group in ~1000 cycles, less than a TMA round trip: 6 slabs (3 groups ahead) cut the
   // issuer's a_full stalls there (B tiles are 8 KB in these layers, the B ring stays >= 9 deep)
-  static const int na_env = getenv("NHANS_NA") ? atoi(getenv("NHANS_NA")) : 0;
   c.na = BN <= 128 ? 6 : 4;
-  if (na_env > 0 && na_env <= kMaxA && na_env % c.mt == 0) c.na = na_env;
   if (c.na % c.mt != 0) c.na = 4;
   const int epi_bytes = row ? 0 : kEpiBytes;
   const int budget = kSmemLimit - 1024 - kCtrlBytes - epi_bytes - c.tab_bytes - c.na * kSlabBytes;
   c.nb = budget / b_bytes;
   if (c.nb > kMaxB) c.nb = kMaxB;
   c.resident = (num_kb <= c.nb && !cta2) ? 1 : 0;
-  c.desc_mode = 0;
-  c.dbg = 0;
   c.il = c.mt >= 2 ? 2 : 1;
   if (cfg) *cfg = c;
   return 1024 + c.na * kSlabBytes + c.nb * b_bytes + kCtrlBytes + epi_bytes + c.tab_bytes;
@@ -843,81 +749,58 @@ cudaError_t launch_flavour(cudaStream_t s, int grid, int smem, const CUtensorMap
     }
     return le;
   }
-  static bool configured = false;           // per process; every device of one box runs the same binary
   cudaError_t e = cudaFuncSetAttribute(gemm_shift_kernel<EPI, CTA2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
   if (e != cudaSuccess) return e;
-  configured = true;
-  (void)configured;
   gemm_shift_kernel<EPI, CTA2><<<grid, kGemmThreads, smem, s>>>(a0, a1, b, p, cfg);
   return cudaGetLastError();
 }
 }  // namespace
 
-cudaError_t gemm_configure() { return cudaSuccess; }
-
 cudaError_t launch_gemm(cudaStream_t s, int n_sm, const CUtensorMap& mapA0, const CUtensorMap& mapA1,
-                        const CUtensorMap& mapB_full, const CUtensorMap& mapB_half, const GemmDev& p, int desc_mode) {
+                        const CUtensorMap& mapB_full, const CUtensorMap& mapB_half, const GemmDev& p) {
   if (p.M <= 0) return cudaSuccess;
   if (p.num_groups > kMaxGroups || p.BN % 16 != 0 || p.BN > 256 || p.N % p.BN != 0) return cudaErrorInvalidValue;
+  const EpiDev& e = p.epi;
   GemmCfg cfg;
-  static const int row_env = getenv("NHANS_EPI_ROW") ? atoi(getenv("NHANS_EPI_ROW")) : 1;
-  // bit 0: row-per-thread epilogue for the 64/128-channel layers (BN <= 128), bit 1: for the BN = 256 layers too
-  const int row = (!p.epi.head && ((p.BN <= 128 && (row_env & 1)) || (p.BN > 128 && (row_env & 2)))) ? 1 : 0;
-  const int tab_C = p.epi.pair ? p.epi.n_real : p.N;
-  const bool tabs_fit = p.epi.ttab16 && p.epi.ftab16 && p.BN <= 128;
-  int tab_bytes = (p.epi.ttab16 && p.epi.ftab16) ? (p.epi.tab_H + p.epi.tab_W) * tab_C * 2 : 0;
-  if (row) tab_bytes = (tabs_fit ? p.epi.tab_H * tab_C * 2 + ((p.epi.tab_W * (tab_C + 8) * 2 + 15) & ~15) : 0) + 2 * p.N * 4;
-  // CTA pairs whenever there is enough work for every pair and B splits into two legal boxes (debug: bit 4 of desc_mode disables)
-  const int cta2 = (!(desc_mode & 16) && (p.BN % 32) == 0 && !p.epi.head && p.M >= 256 * (n_sm / 2)) ? 1 : 0;
+  // row-per-thread epilogue for the 64/128-channel layers, transposing epilogue for BN = 256 and the head
+  const int row = (!e.head && p.BN <= 128) ? 1 : 0;
+  // the row flavour keeps the fp16 tables (frequency rows padded by 8 halfs) and two per-channel vectors in shared memory
+  const bool tabs = e.ttab16 && e.ftab16;
+  const int tab_bytes = row ? (tabs ? e.tab_H * p.N * 2 + ((e.tab_W * (p.N + 8) * 2 + 15) & ~15) : 0) + 2 * p.N * 4 : 0;
+  // CTA pairs whenever there is enough work for every pair and B splits into two legal boxes
+  const int cta2 = ((p.BN % 32) == 0 && !e.head && p.M >= 256 * (n_sm / 2)) ? 1 : 0;
   const int smem = gemm_smem_bytes(p.BN, p.num_kb, tab_bytes, cta2, row, &cfg);
   const CUtensorMap& mapB = cta2 ? mapB_half : mapB_full;
   if (p.N != p.BN) cfg.resident = 0;
-  cfg.desc_mode = desc_mode & 1;
-  cfg.dbg = (desc_mode >> 6) & 7;
-  if ((desc_mode >> 1) & 7) { cfg.il = (desc_mode >> 1) & 7; if (cfg.il > cfg.mt) cfg.il = cfg.mt; }   // debug override
   if (cfg.nb < 4 || cfg.na % cfg.mt != 0) return cudaErrorInvalidValue;   // a group has up to 4 taps in flight; its slabs never wrap the A ring
+  if (!row && cfg.mt != 1) return cudaErrorInvalidValue;                   // the transposing epilogue handles one sub-tile per tile
   const int tile_rows = (cfg.mt * 128) << cta2;
-  if (p.ksplit < 1 || (p.ksplit > 1 && (!p.epi.head || !p.split_scratch || cfg.resident))) return cudaErrorInvalidValue;
+  if (p.ksplit < 1 || (p.ksplit > 1 && (!e.head || !p.split_scratch || cfg.resident))) return cudaErrorInvalidValue;
   const int tiles = p.Ho * ((p.plane_rows + tile_rows - 1) / tile_rows) * (p.N / p.BN) * p.ksplit;
   int grid = tiles < (n_sm >> cta2) ? tiles : (n_sm >> cta2);
   grid <<= cta2;                              // CTA pairs: two CTAs per tile
-  const EpiDev& e = p.epi;
   int fl = 0;
   if (e.head) fl = kEpiHead;
   else {
-    if (e.pair) fl |= kEpiPair;
     if (e.res) fl |= kEpiRes;
     if (e.r1_vec) fl |= kEpiR1;
-    if (e.tftab) fl |= (row ? tabs_fit : cfg.tab_bytes != 0) ? kEpiTabS : kEpiTabG;
+    if (e.tftab) fl |= (row && tabs) ? kEpiTabS : kEpiTabG;
     if (row) fl |= kEpiRow;
   }
 #define NHANS_FLAVOUR(F) \
   case F:                \
     return cta2 ? launch_flavour<F, true>(s, grid, smem, mapA0, mapA1, mapB, p, cfg) : launch_flavour<F, false>(s, grid, smem, mapA0, mapA1, mapB, p, cfg);
   switch (fl) {
-    NHANS_FLAVOUR(0)                                   // tower conv1 / conv2 with GEMM transform, last_conv
-    NHANS_FLAVOUR(kEpiR1)                              // tower block-1 conv2
-    NHANS_FLAVOUR(kEpiHead)                            // last_dense
-    NHANS_FLAVOUR(kEpiTabS)                            // conditioned conv1 / conv2+GEMM transform, BN <= 128
-    NHANS_FLAVOUR(kEpiTabS | kEpiRes)
-    NHANS_FLAVOUR(kEpiTabS | kEpiR1)
-    NHANS_FLAVOUR(kEpiTabG)                            // the same with BN = 256 (tables stay in global memory)
+    NHANS_FLAVOUR(0)                                   // tower layers with 256 / 512 channels, last_conv
+    NHANS_FLAVOUR(kEpiTabG)                            // conditioned layers with BN = 256 (tables stay in global memory)
     NHANS_FLAVOUR(kEpiTabG | kEpiRes)
-    NHANS_FLAVOUR(kEpiTabG | kEpiR1)
-    NHANS_FLAVOUR(kEpiPair | kEpiTabS)                 // pixel-pair rows (64-channel stage)
-    NHANS_FLAVOUR(kEpiPair | kEpiTabS | kEpiRes)
-    NHANS_FLAVOUR(kEpiPair | kEpiTabS | kEpiR1)
-    NHANS_FLAVOUR(kEpiRow)
-    NHANS_FLAVOUR(kEpiRow | kEpiR1)
-    NHANS_FLAVOUR(kEpiRow | kEpiTabS)
+    case kEpiHead:                                     // last_dense (never on CTA pairs)
+      return launch_flavour<kEpiHead, false>(s, grid, smem, mapA0, mapA1, mapB, p, cfg);
+    NHANS_FLAVOUR(kEpiRow)                             // tower layers with 64 / 128 channels
+    NHANS_FLAVOUR(kEpiRow | kEpiR1)                    // tower block-1 conv2
+    NHANS_FLAVOUR(kEpiRow | kEpiTabS)                  // conditioned conv1 / conv2 + GEMM transform, BN <= 128
     NHANS_FLAVOUR(kEpiRow | kEpiTabS | kEpiRes)
-    NHANS_FLAVOUR(kEpiRow | kEpiTabS | kEpiR1)
-    NHANS_FLAVOUR(kEpiRow | kEpiTabG)
-    NHANS_FLAVOUR(kEpiRow | kEpiTabG | kEpiRes)
-    NHANS_FLAVOUR(kEpiRow | kEpiTabG | kEpiR1)
-    NHANS_FLAVOUR(kEpiRow | kEpiPair | kEpiTabS)
-    NHANS_FLAVOUR(kEpiRow | kEpiPair | kEpiTabS | kEpiRes)
-    NHANS_FLAVOUR(kEpiRow | kEpiPair | kEpiTabS | kEpiR1)
+    NHANS_FLAVOUR(kEpiRow | kEpiTabS | kEpiR1)         // resblock1_1_conv2 without the row-walk kernel
     default: return cudaErrorInvalidValue;
   }
 #undef NHANS_FLAVOUR

@@ -33,8 +33,6 @@ struct EpiDev {
   const float* raw;         // fp32 spectrogram rows [frame][201]
   int relu;
   int head;                 // 1: out_f32[n][201] = acc + bias + raw[frame(n)]
-  int pair, n_real, pair_W; // pixel-pair rows: column = j * n_real + c (plan.h Epilogue)
-  long long res_off0, res_off1;
   // output grid (plan.h Grid)
   __half* out;
   int out_C;
@@ -54,9 +52,7 @@ struct GemmCfg {              // chosen by the host per layer shape
   int mt;                     // 128-row sub-tiles per CTA tile (256 / BN)
   int na, nb;                 // A slab ring / B tile ring depth
   int resident;               // all k-blocks of B fit in the ring: load once
-  int desc_mode;              // 1: set the descriptor base-offset field for row-shifted slabs
-  int dbg;                    // timing experiments, results are garbage (NHANS_DESC_MODE bits 6-8): 1 no A loads, 2 no B loads, 4 MMAs of half the N
-  int il;                     // sub-tiles whose MMAs are interleaved (1, 2 or 4; divides mt, <= na)
+  int il;                     // sub-tiles whose MMAs are interleaved (1 or 2; divides mt, <= na)
   int tab_bytes;              // > 0: the fp16 time / frequency tables are staged in shared memory
   int cta2;                   // 1: CTA pairs (cta_group::2): M = 256 MMAs, each CTA loads half of B
   int row;                    // 1: row-per-thread epilogue (no shared-memory transpose), see gemm_tc.cu
@@ -82,7 +78,6 @@ struct GemmDev {
   int ksplit;
   float* split_scratch;
   int* err_flag;
-  int debug_skip_epilogue;  // measurement aid: epilogue warps only release the accumulator
   unsigned long long* debug_stats;   // optional [8] cycle counters (wait times per role), or null
 };
 
@@ -116,9 +111,8 @@ struct DirectDev {
 
 constexpr int kGemmThreads = 352;     // A producer, B producer, MMA issuer, 8 epilogue warps
 int gemm_smem_bytes(int BN, int num_kb, int tab_bytes, int cta2, int row, GemmCfg* cfg);
-cudaError_t gemm_configure();   // sets the dynamic shared-memory attribute once
 cudaError_t launch_gemm(cudaStream_t s, int n_sm, const CUtensorMap& mapA0, const CUtensorMap& mapA1,
-                        const CUtensorMap& mapB, const CUtensorMap& mapBhalf, const GemmDev& p, int desc_mode);
+                        const CUtensorMap& mapB, const CUtensorMap& mapBhalf, const GemmDev& p);
 cudaError_t launch_direct_conv(cudaStream_t s, const DirectDev& p);
 // mapA: the input grid as [pixels][64] (box 136 x 64), mapB: repacked weights [4 kernel-row blocks x 64][4 x 64] (box 256 x 64)
 cudaError_t launch_walk(cudaStream_t s, int n_sm, const CUtensorMap& mapA, const CUtensorMap& mapB, const WalkDev& p);

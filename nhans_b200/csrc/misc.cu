@@ -3,8 +3,6 @@
 // per-unit lookup tables.
 #include "kernels.h"
 
-#include <cstdlib>
-
 namespace nhans {
 
 namespace {
@@ -477,7 +475,7 @@ __global__ void units_rows_kernel(int r0, int n_units, int rows, int* frame, int
 cudaError_t launch_direct_conv(cudaStream_t s, const DirectDev& p) {
   if (p.units <= 0) return cudaSuccess;
   if (p.N != 64) return cudaErrorInvalidValue;
-  if (p.kw == 4 && p.kh == 4 && !getenv("NHANS_DIRECT_FMA")) {
+  if (p.kw == 4 && p.kh == 4) {
     const int segs = (p.Wo + 15) / 16;
     const long long rows = (long long)p.units * p.Ho;
     if (rows > 0x7fffffffLL) return cudaErrorInvalidValue;

@@ -9,7 +9,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <stdexcept>
 
@@ -131,7 +130,6 @@ std::vector<double> cont_embed(const WeightMap& w, const std::string& scope, int
 struct BlockSpec {
   std::string scope;
   int kh, kw, sh, sw, C;
-  bool pair = false;                   // pixel-pair GEMM rows (stride-1 blocks with 64 channels)
 };
 
 struct BlockGeom {
@@ -274,37 +272,9 @@ struct Builder {
     L->K = Knew;
   }
 
-  // Pixel-pair variant of add_conv_taps for a stride-1 (kh x kw) convolution: GEMM row = pixels (h, 2 w'),
-  // (h, 2 w' + 1); the virtual kernel has kw + 1 column taps t' (padded column 2 w' + t') and 2 C output
-  // columns (j, n) with W'[i][t'][c][(j, n)] = w[i][t' - j][c][n] (zero outside 0 <= t' - j < kw).
-  void add_conv_taps_pair(GemmLayer* L, const Grid& src, const std::vector<float>& wt, int kh, int kw, int Cin, int C,
-                          int pt, int pl, const std::vector<double>& scale) {
-    if (!L->kb.empty() || src.sw != 2 || src.sh != 1) throw std::runtime_error("pair taps need a fresh layer on a column-split grid");
-    L->a_rowlen[0] = Cin;
-    const int kwv = kw + 1;
-    const int K = kh * kwv * Cin;
-    L->N = 2 * C;
-    L->w.assign((size_t)L->N * K, 0);
-    for (int i = 0; i < kh; ++i)
-      for (int t = 0; t < kwv; ++t) {
-        const int32_t off = tap_offset(src, i - pt, t - pl);
-        for (int c0 = 0; c0 < Cin; c0 += kTileK) L->kb.push_back({off, (int16_t)0, (int16_t)c0});
-        for (int j = 0; j < 2; ++j) {
-          const int tj = t - j;
-          if (tj < 0 || tj >= kw) continue;
-          for (int c = 0; c < Cin; ++c)
-            for (int n = 0; n < C; ++n) {
-              const double v = (double)wt[(((size_t)i * kw + tj) * Cin + c) * C + n] * scale[n];
-              L->w[(size_t)(j * C + n) * K + (i * kwv + t) * Cin + c] = f32_to_f16_bits((float)v);
-            }
-        }
-      }
-    L->K = K;
-  }
-
   // Stride-1 4 x 4 convolutions with 64 channels in and out can be executed by the row-walk kernel.
   static void mark_walk(GemmLayer* L, const BlockSpec& b, int Cin, int C, int pt, int pl) {
-    if (b.pair || b.kh != 4 || b.kw != 4 || b.sh != 1 || b.sw != 1 || Cin != 64 || C != 64) return;
+    if (b.kh != 4 || b.kw != 4 || b.sh != 1 || b.sw != 1 || Cin != 64 || C != 64) return;
     L->walk = 1;
     L->c_kh = b.kh; L->c_kw = b.kw; L->c_pt = pt; L->c_pl = pl;
   }
@@ -319,10 +289,8 @@ struct Builder {
     const auto& w2 = get(w, b.scope + "_conv2/w", (size_t)b.kh * b.kw * C * C);
     const auto& b2 = get(w, b.scope + "_conv2/b", C);
 
-    Grid h = b.pair ? make_grid(-1, g.Ho, g.Wo, C, 1, 2, 0, g.pl2, g.Hq, g.Wq, cap)
-                    : make_grid(-1, g.Ho, g.Wo, C, 1, 1, 0, 0, g.Hq, g.Wq, cap);
+    Grid h = make_grid(-1, g.Ho, g.Wo, C, 1, 1, 0, 0, g.Hq, g.Wq, cap);
     h.buf = new_buf(h);
-    const int Wo_rows = b.pair ? (g.Wo + 1) / 2 : g.Wo;        // GEMM rows per image row
 
     // ---- conv1 (no bias) + conditioning -> BN -> ReLU ----
     Epilogue e1;
@@ -344,15 +312,10 @@ struct Builder {
     } else {
       GemmLayer L;
       L.name = b.scope + "_conv1";
-      L.Hq = g.Hq; L.Wq = g.Wq; L.Ho = g.Ho; L.Wo = Wo_rows;
+      L.Hq = g.Hq; L.Wq = g.Wq; L.Ho = g.Ho; L.Wo = g.Wo;
       L.a_buf[0] = x.buf;
-      if (b.pair) {
-        add_conv_taps_pair(&L, x, w1, b.kh, b.kw, Cin, C, g.pt, g.pl, bn1.s);
-        e1.pair = 1; e1.n_real = C; e1.pair_W = g.Wo;
-      } else {
-        L.N = C;
-        add_conv_taps(&L, x, 0, w1, b.kh, b.kw, Cin, C, g.pt, g.pl, bn1.s);
-      }
+      L.N = C;
+      add_conv_taps(&L, x, 0, w1, b.kh, b.kw, Cin, C, g.pt, g.pl, bn1.s);
       L.BN = pick_bn(L.N);
       L.epi = e1;
       L.out = h;
@@ -365,30 +328,18 @@ struct Builder {
     // ---- conv2 (+b) + conditioning + identity/transform -> BN -> ReLU ----
     GemmLayer L;
     L.name = b.scope + "_conv2";
-    L.Hq = g.Hq; L.Wq = g.Wq; L.Ho = g.Ho; L.Wo = Wo_rows;
+    L.Hq = g.Hq; L.Wq = g.Wq; L.Ho = g.Ho; L.Wo = g.Wo;
     L.a_buf[0] = h.buf;
-    if (b.pair) {
-      add_conv_taps_pair(&L, h, w2, b.kh, b.kw, C, C, g.pt2, g.pl2, bnA.s);
-    } else {
-      L.N = C;
-      add_conv_taps(&L, h, 0, w2, b.kh, b.kw, C, C, g.pt2, g.pl2, bnA.s);
-    }
+    L.N = C;
+    add_conv_taps(&L, h, 0, w2, b.kh, b.kw, C, C, g.pt2, g.pl2, bnA.s);
     L.BN = pick_bn(L.N);
     L.macs_per_unit = (double)g.Ho * g.Wo * b.kh * b.kw * C * C;
     std::vector<double> constant(C);
     for (int c = 0; c < C; ++c) constant[c] = bnA.s[c] * (double)b2[c] + bnA.o[c];
     Epilogue e2;
     e2.relu = 1;
-    if (b.pair) {
-      e2.pair = 1; e2.n_real = C; e2.pair_W = g.Wo;
-      if (Cin != C && Cin != 1) throw std::runtime_error("pair mode has no GEMM transform path");
-    }
     if (Cin == C) {
       if (b.sh != 1 || b.sw != 1) throw std::runtime_error("identity path with stride");
-      if (b.pair) {                                        // pixel (h, 2 w' + j) of x relative to the GEMM row
-        e2.res_off[0] = tap_offset(x, 0, 0);
-        e2.res_off[1] = tap_offset(x, 0, 1);
-      }
       e2.res_buf = x.buf;
       e2.res_scale.resize(C);
       for (int c = 0; c < C; ++c) e2.res_scale[c] = (float)bnA.s[c];
@@ -428,11 +379,7 @@ std::vector<BlockGeom> block_geometry(const std::vector<BlockSpec>& blocks, int 
     same_pads(g.Wo, b.kw, 1, &o, &g.pl2, &g.pr2);
     g.Hq = g.Ho + std::max(g.pt2, g.pb2);
     g.Wq = g.Wo + std::max(g.pl2, g.pr2);
-    if (b.pair) {
-      if (b.sh != 1 || b.sw != 1) throw std::runtime_error("pair mode needs a stride-1 block");
-      // columns are phase-split by parity; a pair row reads padded columns 2 w' .. 2 w' + kw
-      g.Wq = (g.Wo + g.pl2 + g.pr2 + 1 + 1) / 2;
-    } else if (Cin > 1) {
+    if (Cin > 1) {
       int hx, wx;
       if (b.sh == 1 && b.sw == 1) {
         hx = H + std::max(g.pt, g.pb);
@@ -452,7 +399,6 @@ std::vector<BlockGeom> block_geometry(const std::vector<BlockSpec>& blocks, int 
 
 // Grid of the tensor entering block `i` (written by block i-1), laid out for block i's convolutions.
 Grid input_grid(const BlockSpec& b, const BlockGeom& g, int cap) {
-  if (b.pair) return make_grid(-1, g.H, g.W, g.Cin, 1, 2, 0, g.pl, g.Hq, g.Wq, cap);
   if (b.sh == 1 && b.sw == 1) return make_grid(-1, g.H, g.W, g.Cin, 1, 1, 0, 0, g.Hq, g.Wq, cap);
   return make_grid(-1, g.H, g.W, g.Cin, b.sh, b.sw, g.pt, g.pl, g.Hq, g.Wq, cap);
 }
@@ -541,12 +487,8 @@ NetPlan build_main_plan(const WeightMap& w, int variant, int capacity) {
   Builder B(w, capacity, true);
   if (variant == 0) { B.sa = "_noise_pos_emb"; B.sb = "_noise_neg_emb"; }
   else              { B.sa = "_noise_emb";     B.sb = "_clean_emb"; }
-  // 64-channel stage: plain pixel rows executed by the row-walk kernel (default), or the pixel-pair GEMM rows of
-  // round 1 (NHANS_STAGE1=pair; kept for A/B measurements)
-  const char* s1 = getenv("NHANS_STAGE1");
-  const bool pair1 = s1 && std::string(s1) == "pair";
   std::vector<BlockSpec> blocks = {                      // main.py:221-229
-      {"resblock1_1", 4, 4, 1, 1, 64, pair1},  {"resblock1_2", 4, 4, 1, 1, 64, pair1},
+      {"resblock1_1", 4, 4, 1, 1, 64},  {"resblock1_2", 4, 4, 1, 1, 64},
       {"resblock2_1", 4, 4, 2, 2, 128}, {"resblock2_2", 4, 4, 1, 1, 128},
       {"resblock3_1", 3, 3, 2, 2, 256}, {"resblock3_2", 3, 3, 1, 1, 256},
       {"resblock4_1", 3, 3, 2, 2, 512}, {"resblock4_2", 3, 3, 1, 1, 512}};

@@ -95,13 +95,6 @@ struct Epilogue {
   std::vector<float> r1_vec;      // rank-1 term on the raw spectrogram (1x1 transform with Cin = 1)
   int r1_sh = 1, r1_sw = 1;       // raw frame = win_frame[n] + ho * r1_sh + raw_oh, bin = wo * r1_sw
   int raw_oh = 0;
-  // Pixel-pair mode (64-channel stride-1 blocks): a GEMM row is the pixel pair (h, 2 w'), (h, 2 w' + 1) and
-  // column n = j * n_real + c is channel c of pixel j, so that the MMA runs with N = 128 (an M = 128 MMA with
-  // N = 64 costs as much as N = 128).  Tables / res_scale / r1_vec are indexed by c.
-  int pair = 0;
-  int n_real = 0;                 // channels per pixel (pair mode), else N
-  int pair_W = 0;                 // logical width: pixel j of a pair is valid when 2 w' + j < pair_W
-  int64_t res_off[2] = {0, 0};    // residual row of pixel j relative to the GEMM row
   int relu = 1;
   int head = 0;                   // 1: fp32 output [n][201] = acc * res_scale + bias + raw[center frame] (main.py:238-242;
                                   //    res_scale = inverse of the per-column power-of-two weight scale)

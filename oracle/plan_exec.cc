@@ -138,15 +138,7 @@ void run_net(Net& net, int units_n, const Units& units, const float* raw, const 
           }
         }
       }
-      if (L.epi.pair) {
-        // pixel-pair rows: columns [j * C, (j + 1) * C) are pixel (ho, 2 wo + j)
-        const int C = L.epi.n_real;
-        for (int j = 0; j < 2; ++j)
-          if (2 * wo + j < L.epi.pair_W)
-            epilogue(c, L.epi, L.out, C, L.epi.pair_W, unit, ho, 2 * wo + j, m + L.epi.res_off[j], acc.data() + j * C, net.bufs);
-      } else {
-        epilogue(c, L.epi, L.out, L.N, L.Wo, unit, ho, wo, m, acc.data(), net.bufs);
-      }
+      epilogue(c, L.epi, L.out, L.N, L.Wo, unit, ho, wo, m, acc.data(), net.bufs);
     }
   }
 }

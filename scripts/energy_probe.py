@@ -1,5 +1,5 @@
 """Energy per pass of the mask network on a GPU box: NVML's total-energy counter around N engine runs.
-   python scripts/energy_probe.py [utts] [seconds] [runs]   (NHANS_DESC_MODE debug switches apply)"""
+   python scripts/energy_probe.py [utts] [seconds] [runs]"""
 import os
 import sys
 import time
@@ -40,5 +40,5 @@ t1 = time.perf_counter()
 e1 = pynvml.nvmlDeviceGetTotalEnergyConsumption(dev)
 ms = eng.event_elapsed_ms(0, 1) / runs
 joule = (e1 - e0) / 1000.0 / runs
-print("mode %s: %.1f ms/run  %.1f J/run  %.0f W avg  sm clock samples %s  -> %.1f audio-s/s" % (
-    os.environ.get("NHANS_DESC_MODE", "0"), ms, joule, joule / (ms / 1000.0), clk, utts * secs / (ms / 1000.0)))
+print("%.1f ms/run  %.1f J/run  %.0f W avg  sm clock samples %s  -> %.1f audio-s/s" % (
+    ms, joule, joule / (ms / 1000.0), clk, utts * secs / (ms / 1000.0)))

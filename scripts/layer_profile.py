@@ -1,5 +1,5 @@
 """Per-layer timing of the tensor-core layers on a GPU box (CUDA events around every launch).
-   python scripts/layer_profile.py [utts] [seconds]   -> table + gpurun_out/layers.json"""
+   python scripts/layer_profile.py [utts] [seconds] [layers.json]   -> table (+ the per-layer records as JSON)"""
 import json
 import os
 import sys
@@ -13,6 +13,7 @@ from nhans_b200.engine import Engine, pack  # noqa: E402
 
 utts = int(sys.argv[1]) if len(sys.argv) > 1 else 64
 secs = float(sys.argv[2]) if len(sys.argv) > 2 else 4.0
+json_out = sys.argv[3] if len(sys.argv) > 3 else None
 eng = Engine(0, 0, win_capacity=int(os.environ.get("NHANS_WIN_CAPACITY", "0")))
 eng.load_weights(W.seeded_init(0, 0))
 base = [synth.mixture(secs, u) for u in range(8)]
@@ -38,13 +39,14 @@ _c = [c for c in _c if c[1] > 400]
 print('clocks under load: median sm %.0f MHz, median power %.0f W (%d samples)' % (np.median([c[0] for c in _c]) if _c else 0, np.median([c[1] for c in _c]) if _c else 0, len(_c)))
 layers = eng.profile_layers(0)
 tot = sum(l["ms"] for l in layers)
-print("skip_epilogue=%s  %d x %.0f s: %.1f ms/run -> %.1f audio-s/s" % (os.environ.get("NHANS_DEBUG_SKIP_EPILOGUE", "0"), utts, secs, ms / 2, utts * secs / (ms / 2e3)))
+print("%d x %.0f s: %.1f ms/run -> %.1f audio-s/s" % (utts, secs, ms / 2, utts * secs / (ms / 2e3)))
 for l in layers:
     print("%-22s K=%5d N=%3d  %8.2f ms  %5.1f%%  %7.1f TFLOP/s" % (l["name"], l["K"], l["N"], l["ms"] / 6, 100 * l["ms"] / tot, l["tflops"]))
 st = eng.profile_get(0)
 print("all GEMM layers: %.1f ms, %.1f TFLOP/s;  direct conv %.1f ms" % (st["ms"] / 6, st["flops"] / st["ms"] / 1e9, eng.profile_get(3)["ms"] / 6))
-os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-json.dump(layers, open(os.path.join(ROOT, "gpurun_out", "layers_skip%s.json" % os.environ.get("NHANS_DEBUG_SKIP_EPILOGUE", "0")), "w"))
+if json_out:
+    with open(json_out, "w") as f:
+        json.dump(layers, f)
 if os.environ.get("NHANS_DEBUG_STATS"):
     import ctypes
     print("wait cycles per layer (sum over 148 CTAs, %): tmem_empty | a_full | b_full | epi waits tmem_full | of MMA-warp total")
