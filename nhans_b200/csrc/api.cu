@@ -11,6 +11,7 @@
 #include <cstring>
 #include <memory>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "kernels.h"
@@ -92,13 +93,22 @@ struct IoSlot {
   bool d2h_pending = false;
 };
 
-struct Batch {
+// Layout of a batch of U utterances (batch_geometry).  Sample offsets are relative to the first sample of each array;
+// a_offs / b_offs are empty when the batch has no such context.
+struct Geometry {
   int U = 0;
+  std::vector<long long> mix_offs;  // [u < U]: first sample of utterance u's kept frames; [U]: samples in the array
+  std::vector<long long> a_offs, b_offs;
+  std::vector<long long> frame_offs, out_offs;   // kept mixture frames and output samples of each utterance
+  std::vector<long long> ctx_frame_offs;         // u * 200: the context frames the towers read
+  int max_frames = 0;
+  long long total_frames = 0, total_out = 0;
+};
+
+struct Batch {
+  Geometry geo;
   bool has_a = false;
   bool staged = false, done = false;
-  std::vector<long long> mix_offs, a_offs, b_offs, frame_offs, out_offs, ctx_frame_offs;
-  long long total_frames = 0, total_out = 0;
-  int max_frames = 0;
   IoSlot io[2];
   int cur = 0;                      // set the staged / running batch uses
   DBuf peak_mix, peak_a, peak_b;
@@ -123,7 +133,6 @@ struct nhans_ctx {
   bool silent_ready = false;
   Batch batch;
   DBuf tmp[8];
-  DBuf fbuf[12];                    // nhans_enhance_f32 staging (float clips, offsets, compacted spectra)
   cudaEvent_t events[16] = {};
   bool profile = false;
   std::vector<ProfRec> prof;
@@ -567,6 +576,50 @@ int check_kernel_flag(nhans_ctx* ctx) {
 
 int frames_of(long long n) { return n >= 400 ? (int)(1 + (n - 400) / 160) : 0; }
 
+// samples the inverse STFT returns for T frames
+long long out_len(long long T) { return T > 0 ? (T - 1) * 160 + 400 : 0; }
+
+constexpr int kWholeClips = -1;     // batch_geometry: keep every frame, and allow mixtures shorter than one frame
+
+// Lays out a batch from the caller's sample offsets (a_offs / b_offs may be null: no such context).  Mixture frames
+// [start_frame, T_u) are kept, and every mixture must have more than start_frame frames; frame t of x[160 s:] is
+// frame t + s of x, so the kept frames are transformed from mix_offs[u] + 160 * start_frame on.  Every context must
+// yield the 200 frames the towers read.
+int batch_geometry(nhans_ctx* ctx, const int64_t* mix_offs, const int64_t* a_offs, const int64_t* b_offs, int U,
+                   int start_frame, Geometry& g) {
+  auto rel = [&](const int64_t* o, std::vector<long long>& v) {
+    v.clear();
+    if (o) for (int u = 0; u <= U; ++u) v.push_back(o[u] - o[0]);
+  };
+  auto short_ctx = [](const std::vector<long long>& o, int u) { return !o.empty() && frames_of(o[u + 1] - o[u]) < kCtxFrames; };
+  g.U = U;
+  rel(mix_offs, g.mix_offs);
+  rel(a_offs, g.a_offs);
+  rel(b_offs, g.b_offs);
+  g.frame_offs.assign(U + 1, 0);
+  g.out_offs.assign(U + 1, 0);
+  g.ctx_frame_offs.resize(U + 1);
+  g.max_frames = 0;
+  const int skip = std::max(start_frame, 0);
+  for (int u = 0; u < U; ++u) {
+    const int T = frames_of(g.mix_offs[u + 1] - g.mix_offs[u]);
+    if (start_frame != kWholeClips && T <= start_frame)
+      return fail(ctx, NHANS_ERR_ARG, "utterance " + std::to_string(u) + " has " + std::to_string(T) + " <= start_frame frames");
+    if (short_ctx(g.b_offs, u) || short_ctx(g.a_offs, u))
+      return fail(ctx, NHANS_ERR_CONTEXT_TOO_SHORT,
+                  "context clip of utterance " + std::to_string(u) + " yields fewer than 200 STFT frames (needs >= 32240 samples)");
+    const int kept = T - skip;
+    g.max_frames = std::max(g.max_frames, kept);
+    g.frame_offs[u + 1] = g.frame_offs[u] + kept;
+    g.out_offs[u + 1] = g.out_offs[u] + out_len(kept);
+  }
+  for (int u = 0; u < U; ++u) g.mix_offs[u] += 160LL * skip;
+  for (int u = 0; u <= U; ++u) g.ctx_frame_offs[u] = (long long)u * kCtxFrames;
+  g.total_frames = g.frame_offs[U];
+  g.total_out = g.out_offs[U];
+  return 0;
+}
+
 int to_device_offs(nhans_ctx* ctx, DBuf& d, const std::vector<long long>& h, cudaStream_t stream = nullptr) {
   CK(d.ensure(h.size() * sizeof(long long)));
   CK(cudaMemcpyAsync(d.p, h.data(), h.size() * sizeof(long long), cudaMemcpyHostToDevice, stream ? stream : ctx->stream));
@@ -576,6 +629,148 @@ int to_device_offs(nhans_ctx* ctx, DBuf& d, const std::vector<long long>& h, cud
 int need_weights(nhans_ctx* ctx) {
   if (!ctx->main_net.ready || !ctx->tower.ready) return fail(ctx, NHANS_ERR_STATE, "nhans_load_weights has not been called");
   return 0;
+}
+
+// STFT of int16 PCM (scaled by 1 / (peak + 1e-6) on the fly) or of float samples (as they are)
+cudaError_t launch_stft_of(cudaStream_t s, const int16_t* pcm, const long long* offs, const long long* frame_offs, int U,
+                           const int* peak, int max_frames, float* logmag, float* phase, bool phasor) {
+  return launch_stft(s, pcm, offs, frame_offs, U, peak, max_frames, logmag, phase, phasor);
+}
+cudaError_t launch_stft_of(cudaStream_t s, const float* x, const long long* offs, const long long* frame_offs, int U,
+                           const int*, int max_frames, float* logmag, float* phase, bool phasor) {
+  return launch_stft_f32(s, x, offs, frame_offs, U, max_frames, logmag, phase, phasor);
+}
+
+// Copies a batch's clips (int16 or float samples) and its offset arrays into `io` on `stream`.  ctx_a may be null.
+template <class T>
+int stage_batch(nhans_ctx* ctx, IoSlot& io, const Geometry& g, const T* mix, const int64_t* mix_offs, const T* ctx_a,
+                const int64_t* a_offs, const T* ctx_b, const int64_t* b_offs, cudaStream_t stream) {
+  auto clips = [&](DBuf& d, const T* x, const int64_t* offs, long long n) {
+    CK(d.ensure(n * sizeof(T) + 32));
+    CK(cudaMemcpyAsync(d.p, x + offs[0], n * sizeof(T), cudaMemcpyHostToDevice, stream));
+    return 0;
+  };
+  const int U = g.U;
+  int rc;
+  if ((rc = clips(io.mix, mix, mix_offs, g.mix_offs[U]))) return rc;
+  if ((rc = clips(io.b, ctx_b, b_offs, g.b_offs[U]))) return rc;
+  if (ctx_a) {
+    if ((rc = clips(io.a, ctx_a, a_offs, g.a_offs[U]))) return rc;
+    if ((rc = to_device_offs(ctx, io.d_a_offs, g.a_offs, stream))) return rc;
+  }
+  if ((rc = to_device_offs(ctx, io.d_mix_offs, g.mix_offs, stream))) return rc;
+  if ((rc = to_device_offs(ctx, io.d_b_offs, g.b_offs, stream))) return rc;
+  if ((rc = to_device_offs(ctx, io.d_frame_offs, g.frame_offs, stream))) return rc;
+  if ((rc = to_device_offs(ctx, io.d_out_offs, g.out_offs, stream))) return rc;
+  if ((rc = to_device_offs(ctx, io.d_ctx_frame_offs, g.ctx_frame_offs, stream))) return rc;
+  return 0;
+}
+
+// The fused path up to the inverse STFT, on the compute stream, for the batch staged in `io` (int16 or float samples):
+// a2-a4 for the mixture and the first 200 frames of each context (SN/apply.py:359-387), the embedding towers, the
+// conditioning table and the mask network.  Leaves batch.logmag / phase / den filled.
+template <class T>
+int run_fused(nhans_ctx* ctx, IoSlot& io) {
+  constexpr bool pcm = std::is_same<T, int16_t>::value;
+  Batch& b = ctx->batch;
+  const Geometry& g = b.geo;
+  const int U = g.U;
+  const size_t sbytes = (size_t)g.total_frames * kBins * 4;
+  const size_t cbytes = (size_t)U * kCtxFrames * kBins * 4;
+  const int n_cols = ctx->main_net.plan.cond.n_cols;
+  cudaStream_t st = ctx->stream;
+  CK(b.peak_mix.ensure(sizeof(int) * U));
+  CK(b.logmag.ensure(sbytes + 4));
+  CK(b.phase.ensure(2 * sbytes + 8));          // unit phasors (float2 per bin) between the two transforms
+  CK(b.den.ensure(sbytes + 4));
+  CK(b.ctxlm_b.ensure(cbytes));
+  CK(b.emb_b.ensure((size_t)U * 512 * 4));
+  CK(b.cond.ensure((size_t)U * n_cols * 4));
+  if (b.has_a) {
+    CK(b.ctxlm_a.ensure(cbytes));
+    CK(b.emb_a.ensure((size_t)U * 512 * 4));
+  }
+  if (pcm) {
+    CK(b.peak_a.ensure(sizeof(int) * U));
+    CK(b.peak_b.ensure(sizeof(int) * U));
+    CK(launch_peaks(st, io.mix.as<int16_t>(), io.d_mix_offs.as<long long>(), U, b.peak_mix.as<int>()));
+    CK(launch_peaks(st, io.b.as<int16_t>(), io.d_b_offs.as<long long>(), U, b.peak_b.as<int>()));
+    ctx->launches += 2;
+  } else {
+    CK(cudaMemsetAsync(b.peak_mix.p, 0, sizeof(int) * U, st));     // the inverse STFT reads it; no int16 output here
+  }
+  {
+    ProfScope ps(ctx, 1, 0, (double)sizeof(T) * g.mix_offs[U] + 3.0 * sbytes);
+    CK(launch_stft_of(st, io.mix.as<T>(), io.d_mix_offs.as<long long>(), io.d_frame_offs.as<long long>(), U,
+                      b.peak_mix.as<int>(), g.max_frames, b.logmag.as<float>(), b.phase.as<float>(), true));
+  }
+  {
+    ProfScope ps(ctx, 4, 0, 0);
+    CK(launch_stft_of(st, io.b.as<T>(), io.d_b_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U,
+                      b.peak_b.as<int>(), kCtxFrames, b.ctxlm_b.as<float>(), nullptr, false));
+  }
+  const float* emb_a = ctx->silent_emb.as<float>();
+  int stride_a = 0;
+  int rc;
+  if (b.has_a) {
+    if (pcm) {
+      CK(launch_peaks(st, io.a.as<int16_t>(), io.d_a_offs.as<long long>(), U, b.peak_a.as<int>()));
+      ctx->launches += 1;
+    }
+    {
+      ProfScope ps(ctx, 4, 0, 0);
+      CK(launch_stft_of(st, io.a.as<T>(), io.d_a_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U,
+                        b.peak_a.as<int>(), kCtxFrames, b.ctxlm_a.as<float>(), nullptr, false));
+    }
+    // embedding towers: once per distinct context clip (SURVEY.md F6), not once per window
+    if ((rc = run_tower(ctx, b.ctxlm_a.as<float>(), U, b.emb_a.as<float>()))) return rc;
+    emb_a = b.emb_a.as<float>();
+    stride_a = 512;
+  }
+  if ((rc = run_tower(ctx, b.ctxlm_b.as<float>(), U, b.emb_b.as<float>()))) return rc;
+  {
+    ProfScope ps(ctx, 4, 0, 0);
+    CK(launch_cond_table(st, emb_a, stride_a, b.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb,
+                         ctx->main_net.c, n_cols, b.cond.as<float>()));
+  }
+  return run_masknet(ctx, b.logmag.as<float>(), io.d_frame_offs.as<long long>(), g.frame_offs.data(), U, g.total_frames,
+                     b.cond.as<float>(), b.den.as<float>());
+}
+
+// nhans_stft / nhans_stft_f32
+template <class T>
+int stft_entry(nhans_ctx* ctx, const T* x, const int64_t* offs, int U, float* logmag, float* phase, int64_t* frame_offs,
+               int32_t* peak) {
+  constexpr bool pcm = std::is_same<T, int16_t>::value;
+  if (!ctx || !x || !offs || !frame_offs || U <= 0) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  CK(cudaSetDevice(ctx->device));
+  Geometry g;
+  int rc;
+  if ((rc = batch_geometry(ctx, offs, nullptr, nullptr, U, kWholeClips, g))) return rc;
+  std::copy(g.frame_offs.begin(), g.frame_offs.end(), frame_offs);
+  if (!logmag && !phase && !peak) return NHANS_OK;
+  const long long total = g.mix_offs[U];
+  CK(ctx->tmp[0].ensure(total * sizeof(T) + 32));
+  CK(cudaMemcpyAsync(ctx->tmp[0].p, x + offs[0], total * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = to_device_offs(ctx, ctx->tmp[1], g.mix_offs))) return rc;
+  if ((rc = to_device_offs(ctx, ctx->tmp[2], g.frame_offs))) return rc;
+  const size_t sbytes = (size_t)g.total_frames * kBins * 4;
+  CK(ctx->tmp[4].ensure(sbytes + 4));
+  CK(ctx->tmp[5].ensure(sbytes + 4));
+  if (pcm) {
+    CK(ctx->tmp[3].ensure(sizeof(int) * U));
+    CK(launch_peaks(ctx->stream, ctx->tmp[0].as<int16_t>(), ctx->tmp[1].as<long long>(), U, ctx->tmp[3].as<int>()));
+  }
+  {
+    ProfScope ps(ctx, 1, 0, (double)sizeof(T) * total + 2.0 * sbytes);
+    CK(launch_stft_of(ctx->stream, ctx->tmp[0].as<T>(), ctx->tmp[1].as<long long>(), ctx->tmp[2].as<long long>(), U,
+                      ctx->tmp[3].as<int>(), g.max_frames, ctx->tmp[4].as<float>(), ctx->tmp[5].as<float>(), false));
+  }
+  if (logmag) CK(cudaMemcpyAsync(logmag, ctx->tmp[4].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (phase) CK(cudaMemcpyAsync(phase, ctx->tmp[5].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (peak) CK(cudaMemcpyAsync(peak, ctx->tmp[3].p, sizeof(int) * U, cudaMemcpyDeviceToHost, ctx->stream));
+  CK(cudaStreamSynchronize(ctx->stream));
+  return NHANS_OK;
 }
 
 }  // namespace
@@ -659,7 +854,6 @@ void nhans_destroy(nhans_ctx* ctx) {
                   &b.snr, &ctx->silent_emb})
     d->release();
   for (auto& t : ctx->tmp) t.release();
-  for (auto& t : ctx->fbuf) t.release();
   for (auto& ev : ctx->events) if (ev) cudaEventDestroy(ev);
   for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
   for (auto& ev : ctx->ev_pool) cudaEventDestroy(ev);
@@ -703,11 +897,9 @@ int nhans_load_weights(nhans_ctx* ctx, const char* const* names, const int64_t* 
 
 int nhans_output_offsets(const int64_t* mix_offs, int U, int64_t* out_offs) {
   if (!mix_offs || !out_offs || U < 0) return NHANS_ERR_ARG;
-  out_offs[0] = 0;
-  for (int u = 0; u < U; ++u) {
-    int T = frames_of(mix_offs[u + 1] - mix_offs[u]);
-    out_offs[u + 1] = out_offs[u] + (T > 0 ? (long long)(T - 1) * 160 + 400 : 0);
-  }
+  Geometry g;
+  batch_geometry(nullptr, mix_offs, nullptr, nullptr, U, kWholeClips, g);     // checks nothing without contexts
+  std::copy(g.out_offs.begin(), g.out_offs.end(), out_offs);
   return NHANS_OK;
 }
 
@@ -741,73 +933,12 @@ int nhans_normalise(nhans_ctx* ctx, const int16_t* pcm, const int64_t* offs, int
 
 int nhans_stft(nhans_ctx* ctx, const int16_t* pcm, const int64_t* offs, int U, float* logmag, float* phase,
                int64_t* frame_offs, int32_t* peak) {
-  if (!ctx || !pcm || !offs || !frame_offs || U <= 0) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  CK(cudaSetDevice(ctx->device));
-  std::vector<long long> rel(U + 1), fo(U + 1, 0);
-  int max_frames = 0;
-  for (int u = 0; u <= U; ++u) rel[u] = offs[u] - offs[0];
-  for (int u = 0; u < U; ++u) {
-    int T = frames_of(offs[u + 1] - offs[u]);
-    max_frames = std::max(max_frames, T);
-    fo[u + 1] = fo[u] + T;
-  }
-  for (int u = 0; u <= U; ++u) frame_offs[u] = fo[u];
-  if (!logmag && !phase && !peak) return NHANS_OK;
-  const long long total = rel[U];
-  CK(ctx->tmp[0].ensure(total * 2 + 32));
-  CK(cudaMemcpyAsync(ctx->tmp[0].p, pcm + offs[0], total * 2, cudaMemcpyHostToDevice, ctx->stream));
-  int rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[1], rel))) return rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[2], fo))) return rc;
-  CK(ctx->tmp[3].ensure(sizeof(int) * U));
-  const size_t sbytes = (size_t)fo[U] * kBins * 4;
-  CK(ctx->tmp[4].ensure(sbytes + 4));
-  CK(ctx->tmp[5].ensure(sbytes + 4));
-  CK(launch_peaks(ctx->stream, ctx->tmp[0].as<int16_t>(), ctx->tmp[1].as<long long>(), U, ctx->tmp[3].as<int>()));
-  {
-    ProfScope ps(ctx, 1, 0, 2.0 * total + 2.0 * sbytes);
-    CK(launch_stft(ctx->stream, ctx->tmp[0].as<int16_t>(), ctx->tmp[1].as<long long>(), ctx->tmp[2].as<long long>(), U,
-                   ctx->tmp[3].as<int>(), max_frames, fo[U], ctx->tmp[4].as<float>(), ctx->tmp[5].as<float>()));
-  }
-  if (logmag) CK(cudaMemcpyAsync(logmag, ctx->tmp[4].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
-  if (phase) CK(cudaMemcpyAsync(phase, ctx->tmp[5].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
-  if (peak) CK(cudaMemcpyAsync(peak, ctx->tmp[3].p, sizeof(int) * U, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return NHANS_OK;
+  return stft_entry(ctx, pcm, offs, U, logmag, phase, frame_offs, peak);
 }
 
 int nhans_stft_f32(nhans_ctx* ctx, const float* x, const int64_t* offs, int U, float* logmag, float* phase,
                    int64_t* frame_offs) {
-  if (!ctx || !x || !offs || !frame_offs || U <= 0) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  CK(cudaSetDevice(ctx->device));
-  std::vector<long long> rel(U + 1), fo(U + 1, 0);
-  int max_frames = 0;
-  for (int u = 0; u <= U; ++u) rel[u] = offs[u] - offs[0];
-  for (int u = 0; u < U; ++u) {
-    int T = frames_of(offs[u + 1] - offs[u]);
-    max_frames = std::max(max_frames, T);
-    fo[u + 1] = fo[u] + T;
-  }
-  for (int u = 0; u <= U; ++u) frame_offs[u] = fo[u];
-  if (!logmag && !phase) return NHANS_OK;
-  const long long total = rel[U];
-  CK(ctx->tmp[0].ensure(total * 4 + 8));
-  CK(cudaMemcpyAsync(ctx->tmp[0].p, x + offs[0], total * 4, cudaMemcpyHostToDevice, ctx->stream));
-  int rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[1], rel))) return rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[2], fo))) return rc;
-  const size_t sbytes = (size_t)fo[U] * kBins * 4;
-  CK(ctx->tmp[4].ensure(sbytes + 4));
-  CK(ctx->tmp[5].ensure(sbytes + 4));
-  {
-    ProfScope ps(ctx, 1, 0, 4.0 * total + 2.0 * sbytes);
-    CK(launch_stft_f32(ctx->stream, ctx->tmp[0].as<float>(), ctx->tmp[1].as<long long>(), ctx->tmp[2].as<long long>(), U,
-                       max_frames, ctx->tmp[4].as<float>(), ctx->tmp[5].as<float>()));
-  }
-  if (logmag) CK(cudaMemcpyAsync(logmag, ctx->tmp[4].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
-  if (phase) CK(cudaMemcpyAsync(phase, ctx->tmp[5].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
-  CK(cudaStreamSynchronize(ctx->stream));
-  return NHANS_OK;
+  return stft_entry(ctx, x, offs, U, logmag, phase, frame_offs, nullptr);
 }
 
 int nhans_eval_loss(nhans_ctx* ctx, const float* denoised, const float* target, int64_t n_frames, float* example_loss) {
@@ -887,7 +1018,7 @@ int nhans_istft(nhans_ctx* ctx, const float* logmag, const float* phase, const i
   for (int u = 0; u < U; ++u) {
     int T = (int)(fo[u + 1] - fo[u]);
     max_frames = std::max(max_frames, T);
-    oo[u + 1] = oo[u] + (T > 0 ? (long long)(T - 1) * 160 + 400 : 0);
+    oo[u + 1] = oo[u] + out_len(T);
   }
   for (int u = 0; u <= U; ++u) out_offs[u] = oo[u];
   if (!wav_f32 && !wav_i16) return NHANS_OK;
@@ -908,7 +1039,7 @@ int nhans_istft(nhans_ctx* ctx, const float* logmag, const float* phase, const i
   {
     ProfScope ps(ctx, 2, 0, 2.0 * sbytes + (wav_f32 ? 4.0 : 0.0) * oo[U] + (wav_i16 ? 2.0 : 0.0) * oo[U]);
     CK(launch_istft(ctx->stream, ctx->tmp[0].as<float>(), ctx->tmp[1].as<float>(), ctx->tmp[2].as<long long>(),
-                    ctx->tmp[3].as<long long>(), U, ctx->tmp[4].as<int>(), 0, max_frames, wav_f32 ? ctx->tmp[5].as<float>() : nullptr,
+                    ctx->tmp[3].as<long long>(), U, ctx->tmp[4].as<int>(), max_frames, wav_f32 ? ctx->tmp[5].as<float>() : nullptr,
                     wav_i16 ? ctx->tmp[6].as<int16_t>() : nullptr));
   }
   if (wav_f32) CK(cudaMemcpyAsync(wav_f32, ctx->tmp[5].p, oo[U] * 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -928,51 +1059,15 @@ int nhans_upload(nhans_ctx* ctx, const int16_t* mix, const int64_t* mix_offs, in
   if ((rc = need_weights(ctx))) return rc;
   Batch& b = ctx->batch;
   b.staged = false; b.done = false;
-  b.U = U;
   b.has_a = ctx_a != nullptr;
-  auto rel = [&](const int64_t* o, std::vector<long long>& v) {
-    v.resize(U + 1);
-    for (int u = 0; u <= U; ++u) v[u] = o[u] - o[0];
-  };
-  rel(mix_offs, b.mix_offs);
-  rel(b_offs, b.b_offs);
-  if (b.has_a) rel(a_offs, b.a_offs);
-  b.frame_offs.assign(U + 1, 0);
-  b.out_offs.assign(U + 1, 0);
-  b.ctx_frame_offs.resize(U + 1);
-  b.max_frames = 0;
-  for (int u = 0; u < U; ++u) {
-    const int T = frames_of(b.mix_offs[u + 1] - b.mix_offs[u]);
-    b.max_frames = std::max(b.max_frames, T);
-    b.frame_offs[u + 1] = b.frame_offs[u] + T;
-    b.out_offs[u + 1] = b.out_offs[u] + (T > 0 ? (long long)(T - 1) * 160 + 400 : 0);
-    if (frames_of(b.b_offs[u + 1] - b.b_offs[u]) < kCtxFrames || (b.has_a && frames_of(b.a_offs[u + 1] - b.a_offs[u]) < kCtxFrames))
-      return fail(ctx, NHANS_ERR_CONTEXT_TOO_SHORT,
-                  "context clip of utterance " + std::to_string(u) + " yields fewer than 200 STFT frames (needs >= 32240 samples)");
-  }
-  for (int u = 0; u <= U; ++u) b.ctx_frame_offs[u] = (long long)u * kCtxFrames;
-  b.total_frames = b.frame_offs[U];
-  b.total_out = b.out_offs[U];
+  if ((rc = batch_geometry(ctx, mix_offs, ctx_a ? a_offs : nullptr, b_offs, U, kWholeClips, b.geo))) return rc;
   // stage into the set the previous batch does NOT use; its last user (two batches ago) must have finished
   b.cur ^= 1;
   IoSlot& io = b.io[b.cur];
   cudaStream_t hs = ctx->h2d_stream;
   CK(cudaStreamWaitEvent(hs, io.consumed, 0));
   tl_mark(ctx, 0, hs);
-  CK(io.mix.ensure(b.mix_offs[U] * 2 + 32));
-  CK(cudaMemcpyAsync(io.mix.p, mix + mix_offs[0], b.mix_offs[U] * 2, cudaMemcpyHostToDevice, hs));
-  CK(io.b.ensure(b.b_offs[U] * 2 + 32));
-  CK(cudaMemcpyAsync(io.b.p, ctx_b + b_offs[0], b.b_offs[U] * 2, cudaMemcpyHostToDevice, hs));
-  if (b.has_a) {
-    CK(io.a.ensure(b.a_offs[U] * 2 + 32));
-    CK(cudaMemcpyAsync(io.a.p, ctx_a + a_offs[0], b.a_offs[U] * 2, cudaMemcpyHostToDevice, hs));
-    if ((rc = to_device_offs(ctx, io.d_a_offs, b.a_offs, hs))) return rc;
-  }
-  if ((rc = to_device_offs(ctx, io.d_mix_offs, b.mix_offs, hs))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_b_offs, b.b_offs, hs))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_frame_offs, b.frame_offs, hs))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_out_offs, b.out_offs, hs))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_ctx_frame_offs, b.ctx_frame_offs, hs))) return rc;
+  if ((rc = stage_batch(ctx, io, b.geo, mix, mix_offs, ctx_a, a_offs, ctx_b, b_offs, hs))) return rc;
   tl_mark(ctx, 1, hs);
   CK(cudaEventRecord(io.uploaded, hs));
   b.staged = true;
@@ -985,75 +1080,22 @@ int nhans_run(nhans_ctx* ctx) {
   if (!b.staged) return fail(ctx, NHANS_ERR_STATE, "nhans_upload has not staged a batch");
   CK(cudaSetDevice(ctx->device));
   int rc;
-  const int U = b.U;
-  const size_t sbytes = (size_t)b.total_frames * kBins * 4;
-  const size_t cbytes = (size_t)U * kCtxFrames * kBins * 4;
-  const int n_cols = ctx->main_net.plan.cond.n_cols;
-  CK(b.peak_mix.ensure(sizeof(int) * U));
-  CK(b.peak_a.ensure(sizeof(int) * U));
-  CK(b.peak_b.ensure(sizeof(int) * U));
-  CK(b.logmag.ensure(sbytes + 4));
-  CK(b.phase.ensure(2 * sbytes + 8));          // unit phasors (float2 per bin) between the two transforms
-  CK(b.den.ensure(sbytes + 4));
-  CK(b.ctxlm_b.ensure(cbytes));
-  CK(b.emb_b.ensure((size_t)U * 512 * 4));
-  CK(b.cond.ensure((size_t)U * n_cols * 4));
+  const Geometry& g = b.geo;
   IoSlot& io = b.io[b.cur];
-  CK(io.out_i16.ensure(b.total_out * 2 + 32));
-  CK(io.out_f32.ensure(b.total_out * 4 + 4));
-  CK(b.mixproc.ensure(b.total_out * 4 + 4));
+  CK(io.out_i16.ensure(g.total_out * 2 + 32));
+  CK(io.out_f32.ensure(g.total_out * 4 + 4));
+  CK(b.mixproc.ensure(g.total_out * 4 + 4));
   if (!b.has_a && (rc = ensure_silent(ctx))) return rc;
 
   // the inputs of this set have landed, and the outputs the set held two batches ago have reached the host
   CK(cudaStreamWaitEvent(ctx->stream, io.uploaded, 0));
   if (io.d2h_pending) CK(cudaStreamWaitEvent(ctx->stream, io.drained, 0));
   tl_mark(ctx, 2, ctx->stream);
-  // front end: a2-a4 for the mixture and the first 200 frames of each context (SN/apply.py:359-387)
-  CK(launch_peaks(ctx->stream, io.mix.as<int16_t>(), io.d_mix_offs.as<long long>(), U, b.peak_mix.as<int>()));
-  CK(launch_peaks(ctx->stream, io.b.as<int16_t>(), io.d_b_offs.as<long long>(), U, b.peak_b.as<int>()));
-  ctx->launches += 2;
+  if ((rc = run_fused<int16_t>(ctx, io))) return rc;
   {
-    ProfScope ps(ctx, 1, 0, 2.0 * b.mix_offs[U] + 3.0 * sbytes);
-    CK(launch_stft(ctx->stream, io.mix.as<int16_t>(), io.d_mix_offs.as<long long>(), io.d_frame_offs.as<long long>(), U,
-                   b.peak_mix.as<int>(), b.max_frames, b.total_frames, b.logmag.as<float>(), b.phase.as<float>(), true));
-  }
-  {
-    ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_stft(ctx->stream, io.b.as<int16_t>(), io.d_b_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U,
-                   b.peak_b.as<int>(), kCtxFrames, (long long)U * kCtxFrames, b.ctxlm_b.as<float>(), nullptr));
-  }
-  const float* emb_a = nullptr;
-  int stride_a = 0;
-  if (b.has_a) {
-    CK(b.ctxlm_a.ensure(cbytes));
-    CK(b.emb_a.ensure((size_t)U * 512 * 4));
-    CK(launch_peaks(ctx->stream, io.a.as<int16_t>(), io.d_a_offs.as<long long>(), U, b.peak_a.as<int>()));
-    ctx->launches += 1;
-    ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_stft(ctx->stream, io.a.as<int16_t>(), io.d_a_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U,
-                   b.peak_a.as<int>(), kCtxFrames, (long long)U * kCtxFrames, b.ctxlm_a.as<float>(), nullptr));
-  }
-  // embedding towers: once per distinct context clip (SURVEY.md F6), not once per window
-  if (b.has_a) {
-    if ((rc = run_tower(ctx, b.ctxlm_a.as<float>(), U, b.emb_a.as<float>()))) return rc;
-    emb_a = b.emb_a.as<float>();
-    stride_a = 512;
-  } else {
-    emb_a = ctx->silent_emb.as<float>();
-  }
-  if ((rc = run_tower(ctx, b.ctxlm_b.as<float>(), U, b.emb_b.as<float>()))) return rc;
-  {
-    ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_cond_table(ctx->stream, emb_a, stride_a, b.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb,
-                         ctx->main_net.c, n_cols, b.cond.as<float>()));
-  }
-  if ((rc = run_masknet(ctx, b.logmag.as<float>(), io.d_frame_offs.as<long long>(), b.frame_offs.data(), U, b.total_frames,
-                        b.cond.as<float>(), b.den.as<float>())))
-    return rc;
-  {
-    ProfScope ps(ctx, 2, 0, 3.0 * sbytes + 6.0 * b.total_out);
+    ProfScope ps(ctx, 2, 0, 3.0 * g.total_frames * kBins * 4 + 6.0 * g.total_out);
     CK(launch_istft(ctx->stream, b.den.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
-                    io.d_out_offs.as<long long>(), U, b.peak_mix.as<int>(), 0, b.max_frames, io.out_f32.as<float>(),
+                    io.d_out_offs.as<long long>(), g.U, b.peak_mix.as<int>(), g.max_frames, io.out_f32.as<float>(),
                     io.out_i16.as<int16_t>(), true));
   }
   tl_mark(ctx, 3, ctx->stream);
@@ -1066,20 +1108,21 @@ int nhans_download(nhans_ctx* ctx, int16_t* out_i16, float* out_f32, float* mixp
   if (!ctx) return NHANS_ERR_ARG;
   Batch& b = ctx->batch;
   if (!b.done) return fail(ctx, NHANS_ERR_STATE, "nhans_run has not produced a batch");
+  const Geometry& g = b.geo;
   CK(cudaSetDevice(ctx->device));
   IoSlot& io = b.io[b.cur];
   if (mixproc_f32) {
     // 'mixed_processed.wav' (SN/apply.py:457-458): iSTFT of the window centres, i.e. of the input spectrogram
-    ProfScope ps(ctx, 2, 0, 3.0 * b.total_frames * kBins * 4 + 4.0 * b.total_out);
+    ProfScope ps(ctx, 2, 0, 3.0 * g.total_frames * kBins * 4 + 4.0 * g.total_out);
     CK(launch_istft(ctx->stream, b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
-                    io.d_out_offs.as<long long>(), b.U, b.peak_mix.as<int>(), 0, b.max_frames, b.mixproc.as<float>(), nullptr, true));
-    CK(cudaMemcpyAsync(mixproc_f32, b.mixproc.p, b.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
+                    io.d_out_offs.as<long long>(), g.U, b.peak_mix.as<int>(), g.max_frames, b.mixproc.as<float>(), nullptr, true));
+    CK(cudaMemcpyAsync(mixproc_f32, b.mixproc.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
   }
   // the outputs leave on their own stream, so that the next batch can start computing meanwhile
   CK(cudaStreamWaitEvent(ctx->d2h_stream, io.consumed, 0));
   tl_mark(ctx, 4, ctx->d2h_stream);
-  if (out_i16) CK(cudaMemcpyAsync(out_i16, io.out_i16.p, b.total_out * 2, cudaMemcpyDeviceToHost, ctx->d2h_stream));
-  if (out_f32) CK(cudaMemcpyAsync(out_f32, io.out_f32.p, b.total_out * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+  if (out_i16) CK(cudaMemcpyAsync(out_i16, io.out_i16.p, g.total_out * 2, cudaMemcpyDeviceToHost, ctx->d2h_stream));
+  if (out_f32) CK(cudaMemcpyAsync(out_f32, io.out_f32.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->d2h_stream));
   tl_mark(ctx, 5, ctx->d2h_stream);
   CK(cudaEventRecord(io.drained, ctx->d2h_stream));
   io.d2h_pending = true;
@@ -1091,27 +1134,28 @@ int nhans_postmix(nhans_ctx* ctx, float compensate, int ac, float* mixed_f32, fl
   if (!ctx) return NHANS_ERR_ARG;
   Batch& b = ctx->batch;
   if (!b.done) return fail(ctx, NHANS_ERR_STATE, "nhans_run has not produced a batch");
+  const Geometry& g = b.geo;
   CK(cudaSetDevice(ctx->device));
   IoSlot& io = b.io[b.cur];
-  CK(b.removed.ensure(b.total_out * 4 + 4));
-  CK(b.comp.ensure(b.total_out * 4 + 4));
-  CK(b.sums.ensure(sizeof(double) * 2 * b.U));
-  CK(b.snr.ensure(sizeof(float) * b.U));
+  CK(b.removed.ensure(g.total_out * 4 + 4));
+  CK(b.comp.ensure(g.total_out * 4 + 4));
+  CK(b.sums.ensure(sizeof(double) * 2 * g.U));
+  CK(b.snr.ensure(sizeof(float) * g.U));
   {
-    ProfScope ps(ctx, 2, 0, 4.0 * b.total_frames * kBins * 4 + 12.0 * b.total_out);
+    ProfScope ps(ctx, 2, 0, 4.0 * g.total_frames * kBins * 4 + 12.0 * g.total_out);
     CK(launch_istft_post(ctx->stream, b.den.as<float>(), b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
-                         io.d_out_offs.as<long long>(), b.U, b.max_frames, nullptr, b.mixproc.as<float>(), b.removed.as<float>(),
+                         io.d_out_offs.as<long long>(), g.U, g.max_frames, nullptr, b.mixproc.as<float>(), b.removed.as<float>(),
                          b.sums.as<double>(), true));
   }
   {
     ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_compensate(ctx->stream, io.out_f32.as<float>(), b.removed.as<float>(), io.d_out_offs.as<long long>(), b.U,
+    CK(launch_compensate(ctx->stream, io.out_f32.as<float>(), b.removed.as<float>(), io.d_out_offs.as<long long>(), g.U,
                          b.sums.as<double>(), compensate, ac, compensated_f32 ? b.comp.as<float>() : nullptr, b.snr.as<float>()));
   }
-  if (mixed_f32) CK(cudaMemcpyAsync(mixed_f32, b.mixproc.p, b.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (removed_f32) CK(cudaMemcpyAsync(removed_f32, b.removed.p, b.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (compensated_f32) CK(cudaMemcpyAsync(compensated_f32, b.comp.p, b.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  if (snr_est) CK(cudaMemcpyAsync(snr_est, b.snr.p, sizeof(float) * b.U, cudaMemcpyDeviceToHost, ctx->stream));
+  if (mixed_f32) CK(cudaMemcpyAsync(mixed_f32, b.mixproc.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  if (removed_f32) CK(cudaMemcpyAsync(removed_f32, b.removed.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  if (compensated_f32) CK(cudaMemcpyAsync(compensated_f32, b.comp.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  if (snr_est) CK(cudaMemcpyAsync(snr_est, b.snr.p, sizeof(float) * g.U, cudaMemcpyDeviceToHost, ctx->stream));
   return NHANS_OK;
 }
 
@@ -1132,27 +1176,9 @@ int nhans_enhance_f32(nhans_ctx* ctx, const float* mix, const int64_t* mix_offs,
   CK(cudaSetDevice(ctx->device));
   int rc;
   if ((rc = need_weights(ctx))) return rc;
-  std::vector<long long> mo(U + 1), ao(U + 1, 0), bo(U + 1), fo(U + 1, 0), fc(U + 1, 0), oo(U + 1, 0), cfo(U + 1);
-  int max_frames = 0, max_c = 0;
-  for (int u = 0; u <= U; ++u) {
-    mo[u] = mix_offs[u] - mix_offs[0];
-    bo[u] = b_offs[u] - b_offs[0];
-    if (ctx_a) ao[u] = a_offs[u] - a_offs[0];
-    cfo[u] = (long long)u * kCtxFrames;
-  }
-  for (int u = 0; u < U; ++u) {
-    const int T = frames_of(mo[u + 1] - mo[u]);
-    if (T <= start_frame) return fail(ctx, NHANS_ERR_ARG, "utterance " + std::to_string(u) + " has " + std::to_string(T) + " <= start_frame frames");
-    if (frames_of(bo[u + 1] - bo[u]) < kCtxFrames || (ctx_a && frames_of(ao[u + 1] - ao[u]) < kCtxFrames))
-      return fail(ctx, NHANS_ERR_CONTEXT_TOO_SHORT,
-                  "context signal of utterance " + std::to_string(u) + " yields fewer than 200 STFT frames (needs >= 32240 samples)");
-    max_frames = std::max(max_frames, T);
-    max_c = std::max(max_c, T - start_frame);
-    fo[u + 1] = fo[u] + T;
-    fc[u + 1] = fc[u] + (T - start_frame);
-    oo[u + 1] = oo[u] + (long long)(T - start_frame - 1) * 160 + 400;
-  }
-  for (int u = 0; u <= U; ++u) out_offs[u] = oo[u];
+  Geometry geo;
+  if ((rc = batch_geometry(ctx, mix_offs, ctx_a ? a_offs : nullptr, b_offs, U, start_frame, geo))) return rc;
+  std::copy(geo.out_offs.begin(), geo.out_offs.end(), out_offs);
   if (!out_f32 && !mixproc_f32) return NHANS_OK;
   // the shared spectra / embedding buffers are about to be reused: nothing of an earlier batch may still be running
   CK(cudaStreamSynchronize(ctx->stream));
@@ -1160,86 +1186,28 @@ int nhans_enhance_f32(nhans_ctx* ctx, const float* mix, const int64_t* mix_offs,
   CK(cudaStreamSynchronize(ctx->d2h_stream));
   Batch& b = ctx->batch;
   b.done = false; b.staged = false;
-  DBuf* F = ctx->fbuf;
+  b.geo = std::move(geo);
+  b.has_a = ctx_a != nullptr;
+  const Geometry& g = b.geo;
   cudaStream_t st = ctx->stream;
-  const size_t sbytes = (size_t)fo[U] * kBins * 4, cbytes = (size_t)fc[U] * kBins * 4, xbytes = (size_t)U * kCtxFrames * kBins * 4;
-  const int n_cols = ctx->main_net.plan.cond.n_cols;
-  CK(F[0].ensure(mo[U] * 4 + 16));
-  CK(cudaMemcpyAsync(F[0].p, mix + mix_offs[0], mo[U] * 4, cudaMemcpyHostToDevice, st));
-  CK(F[1].ensure(bo[U] * 4 + 16));
-  CK(cudaMemcpyAsync(F[1].p, ctx_b + b_offs[0], bo[U] * 4, cudaMemcpyHostToDevice, st));
-  if ((rc = to_device_offs(ctx, F[3], mo))) return rc;
-  if ((rc = to_device_offs(ctx, F[4], bo))) return rc;
-  if ((rc = to_device_offs(ctx, F[6], fo))) return rc;
-  if ((rc = to_device_offs(ctx, F[7], fc))) return rc;
-  if ((rc = to_device_offs(ctx, F[8], oo))) return rc;
-  if ((rc = to_device_offs(ctx, F[9], cfo))) return rc;
-  CK(b.logmag.ensure(sbytes + 4));
-  CK(b.phase.ensure(2 * sbytes + 8));
-  CK(b.den.ensure(cbytes + 4));
-  CK(b.ctxlm_b.ensure(xbytes));
-  CK(b.emb_b.ensure((size_t)U * 512 * 4));
-  CK(b.cond.ensure((size_t)U * n_cols * 4));
-  CK(b.peak_mix.ensure(sizeof(int) * U));
-  CK(cudaMemsetAsync(b.peak_mix.p, 0, sizeof(int) * U, st));           // no int16 output on this path
-  {
-    ProfScope ps(ctx, 1, 0, 4.0 * mo[U] + 3.0 * sbytes);
-    CK(launch_stft_f32(st, F[0].as<float>(), F[3].as<long long>(), F[6].as<long long>(), U, max_frames, b.logmag.as<float>(),
-                       b.phase.as<float>(), true));
-  }
-  CK(launch_stft_f32(st, F[1].as<float>(), F[4].as<long long>(), F[9].as<long long>(), U, kCtxFrames, b.ctxlm_b.as<float>(), nullptr));
-  ctx->launches += 1;
-  const float* emb_a = nullptr;
-  int stride_a = 0;
-  if (ctx_a) {
-    CK(F[2].ensure(ao[U] * 4 + 16));
-    CK(cudaMemcpyAsync(F[2].p, ctx_a + a_offs[0], ao[U] * 4, cudaMemcpyHostToDevice, st));
-    if ((rc = to_device_offs(ctx, F[5], ao))) return rc;
-    CK(b.ctxlm_a.ensure(xbytes));
-    CK(b.emb_a.ensure((size_t)U * 512 * 4));
-    CK(launch_stft_f32(st, F[2].as<float>(), F[5].as<long long>(), F[9].as<long long>(), U, kCtxFrames, b.ctxlm_a.as<float>(), nullptr));
-    ctx->launches += 1;
-    if ((rc = run_tower(ctx, b.ctxlm_a.as<float>(), U, b.emb_a.as<float>()))) return rc;
-    emb_a = b.emb_a.as<float>();
-    stride_a = 512;
-  } else {
-    if ((rc = ensure_silent(ctx))) return rc;
-    emb_a = ctx->silent_emb.as<float>();
-  }
-  if ((rc = run_tower(ctx, b.ctxlm_b.as<float>(), U, b.emb_b.as<float>()))) return rc;
-  CK(launch_cond_table(st, emb_a, stride_a, b.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb, ctx->main_net.c, n_cols,
-                       b.cond.as<float>()));
-  ctx->launches += 1;
-  // frames [start_frame, T_u) of every utterance, compacted: the slice is processed like a whole utterance
-  const float* lm_c = b.logmag.as<float>();
-  const float* ph_c = b.phase.as<float>();
-  if (start_frame > 0) {
-    CK(F[10].ensure(cbytes + 4));
-    CK(F[11].ensure(2 * cbytes + 8));
-    for (int u = 0; u < U; ++u) {
-      const size_t rows = (size_t)(fc[u + 1] - fc[u]) * kBins;
-      const size_t src = (size_t)(fo[u] + start_frame) * kBins, dst = (size_t)fc[u] * kBins;
-      CK(cudaMemcpyAsync(F[10].as<float>() + dst, b.logmag.as<float>() + src, rows * 4, cudaMemcpyDeviceToDevice, st));
-      CK(cudaMemcpyAsync(F[11].as<float>() + 2 * dst, b.phase.as<float>() + 2 * src, rows * 8, cudaMemcpyDeviceToDevice, st));
-    }
-    lm_c = F[10].as<float>();
-    ph_c = F[11].as<float>();
-  }
-  if ((rc = run_masknet(ctx, lm_c, F[7].as<long long>(), fc.data(), U, fc[U], b.cond.as<float>(), b.den.as<float>()))) return rc;
   IoSlot& io = b.io[b.cur];
-  CK(io.out_f32.ensure(oo[U] * 4 + 16));
+  if ((rc = stage_batch(ctx, io, g, mix, mix_offs, ctx_a, a_offs, ctx_b, b_offs, st))) return rc;
+  if (!b.has_a && (rc = ensure_silent(ctx))) return rc;
+  if ((rc = run_fused<float>(ctx, io))) return rc;
+  const double istft_bytes = 3.0 * g.total_frames * kBins * 4 + 4.0 * g.total_out;
+  CK(io.out_f32.ensure(g.total_out * 4 + 16));
   if (out_f32) {
-    ProfScope ps(ctx, 2, 0, 3.0 * cbytes + 4.0 * oo[U]);
-    CK(launch_istft(st, b.den.as<float>(), ph_c, F[7].as<long long>(), F[8].as<long long>(), U, b.peak_mix.as<int>(), 0, max_c,
-                    io.out_f32.as<float>(), nullptr, true));
-    CK(cudaMemcpyAsync(out_f32, io.out_f32.p, oo[U] * 4, cudaMemcpyDeviceToHost, st));
+    ProfScope ps(ctx, 2, 0, istft_bytes);
+    CK(launch_istft(st, b.den.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(), io.d_out_offs.as<long long>(), U,
+                    b.peak_mix.as<int>(), g.max_frames, io.out_f32.as<float>(), nullptr, true));
+    CK(cudaMemcpyAsync(out_f32, io.out_f32.p, g.total_out * 4, cudaMemcpyDeviceToHost, st));
   }
   if (mixproc_f32) {
-    CK(b.mixproc.ensure(oo[U] * 4 + 16));
-    ProfScope ps(ctx, 2, 0, 3.0 * cbytes + 4.0 * oo[U]);
-    CK(launch_istft(st, lm_c, ph_c, F[7].as<long long>(), F[8].as<long long>(), U, b.peak_mix.as<int>(), 0, max_c, b.mixproc.as<float>(),
-                    nullptr, true));
-    CK(cudaMemcpyAsync(mixproc_f32, b.mixproc.p, oo[U] * 4, cudaMemcpyDeviceToHost, st));
+    CK(b.mixproc.ensure(g.total_out * 4 + 16));
+    ProfScope ps(ctx, 2, 0, istft_bytes);
+    CK(launch_istft(st, b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(), io.d_out_offs.as<long long>(), U,
+                    b.peak_mix.as<int>(), g.max_frames, b.mixproc.as<float>(), nullptr, true));
+    CK(cudaMemcpyAsync(mixproc_f32, b.mixproc.p, g.total_out * 4, cudaMemcpyDeviceToHost, st));
   }
   cudaError_t e = cudaStreamSynchronize(st);
   if ((rc = check_kernel_flag(ctx))) return rc;
@@ -1368,7 +1336,8 @@ int nhans_debug_read_batch(nhans_ctx* ctx, int which, float* out, int64_t n_floa
   if (!ctx || !out || which < 0 || which > 2) return NHANS_ERR_ARG;
   Batch& b = ctx->batch;
   if (!b.done) return fail(ctx, NHANS_ERR_STATE, "nhans_run has not produced a batch");
-  const long long rows = b.total_frames * kBins;
+  const Geometry& g = b.geo;
+  const long long rows = g.total_frames * kBins;
   const long long have = which == 1 ? 2 * rows : rows;            // 1: unit phasors (float2 per bin)
   if (n_floats > have) return fail(ctx, NHANS_ERR_ARG, "the batch holds fewer values than requested");
   const DBuf& src = which == 0 ? b.logmag : (which == 1 ? b.phase : b.den);

@@ -501,9 +501,7 @@ cudaError_t launch_peaks(cudaStream_t s, const int16_t* pcm, const long long* of
 }
 
 cudaError_t launch_stft(cudaStream_t s, const int16_t* pcm, const long long* offs, const long long* frame_offs, int U,
-                        const int* peak, int max_frames_per_clip, long long total_frames, float* logmag, float* phase,
-                        bool phasor) {
-  (void)total_frames;
+                        const int* peak, int max_frames_per_clip, float* logmag, float* phase, bool phasor) {
   if (U <= 0 || max_frames_per_clip <= 0) return cudaSuccess;
   dim3 grid((max_frames_per_clip + kFB - 1) / kFB, U);
   if (phasor) stft_kernel<true><<<grid, kSW * 32, 0, s>>>(pcm, nullptr, offs, frame_offs, peak, logmag, phase);
@@ -529,9 +527,8 @@ cudaError_t launch_normalise(cudaStream_t s, const int16_t* pcm, const long long
 }
 
 cudaError_t launch_istft(cudaStream_t s, const float* logmag, const float* phase, const long long* frame_offs,
-                         const long long* out_offs, int U, const int* peak, long long total_blocks_hint,
-                         int max_frames_per_clip, float* out_f32, int16_t* out_i16, bool phasor) {
-  (void)total_blocks_hint;
+                         const long long* out_offs, int U, const int* peak, int max_frames_per_clip, float* out_f32,
+                         int16_t* out_i16, bool phasor) {
   if (U <= 0 || max_frames_per_clip <= 0) return cudaSuccess;
   dim3 grid((max_frames_per_clip + 2 + kOH - 1) / kOH, U);
   if (phasor) istft_kernel<true><<<grid, kThreads, 0, s>>>(logmag, phase, frame_offs, out_offs, peak, out_f32, out_i16);

@@ -164,15 +164,15 @@ cudaError_t launch_normalise(cudaStream_t s, const int16_t* pcm, const long long
                              const int* peak, float* out);
 // frames, window, FFT-400, log(|X| + 1e-5), angle: logmag/phase rows [frame_offs[u] + t][201]
 cudaError_t launch_stft(cudaStream_t s, const int16_t* pcm, const long long* offs, const long long* frame_offs, int U,
-                        const int* peak, int max_frames_per_clip, long long total_frames, float* logmag, float* phase,
+                        const int* peak, int max_frames_per_clip, float* logmag, float* phase,
                         bool phasor = false);   // phasor: `phase` receives unit phasors (float2 per bin) instead of angles
 cudaError_t launch_eval_loss(cudaStream_t s, const float* den, const float* tgt, long long n, float* loss);
 cudaError_t launch_stft_f32(cudaStream_t s, const float* x, const long long* offs, const long long* frame_offs, int U,
                             int max_frames_per_clip, float* logmag, float* phase, bool phasor = false);
 // exp(logmag) * e^{j phase} -> irfft-400 -> synthesis window -> overlap-add -> f32 / int16 samples
 cudaError_t launch_istft(cudaStream_t s, const float* logmag, const float* phase, const long long* frame_offs,
-                         const long long* out_offs, int U, const int* peak, long long total_blocks_hint,
-                         int max_frames_per_clip, float* out_f32, int16_t* out_i16, bool phasor = false);
+                         const long long* out_offs, int U, const int* peak, int max_frames_per_clip, float* out_f32,
+                         int16_t* out_i16, bool phasor = false);
 // apply_snc post-mix outputs (SN/apply.py:456-470): both iSTFTs, removed, energy sums; then compensated / snr_est
 cudaError_t launch_istft_post(cudaStream_t s, const float* den_logmag, const float* mix_logmag, const float* phase,
                               const long long* frame_offs, const long long* out_offs, int U, int max_frames_per_clip,

@@ -26,13 +26,16 @@ def _ptr(a):
     return None if a is None else a.ctypes.data_as(ctypes.c_void_p)
 
 
-def pack(clips):
-    """List of 1-D int16 arrays -> (concatenated int16, int64 offsets [U+1])."""
+def pack(clips, dtype=np.int16, alloc=np.empty):
+    """List of 1-D arrays -> (concatenated `dtype` samples, int64 offsets [U+1]).  `alloc(n, dtype)` provides the
+    contiguous array the samples are copied into."""
     offs = np.zeros(len(clips) + 1, np.int64)
     for i, c in enumerate(clips):
         offs[i + 1] = offs[i] + len(c)
-    data = np.concatenate([np.asarray(c, np.int16) for c in clips]) if clips else np.zeros(0, np.int16)
-    return np.ascontiguousarray(data), offs
+    data = alloc(int(offs[-1]), dtype)
+    for i, c in enumerate(clips):
+        data[offs[i]:offs[i + 1]] = c
+    return data, offs
 
 
 def unpack(data, offs):
@@ -130,10 +133,7 @@ class Engine:
     def stft_f32(self, signals):
         """float32 sample arrays (already normalised / mixed) -> (logmag [F,201], phase [F,201], frame_offs [U+1])"""
         U = len(signals)
-        offs = np.zeros(U + 1, np.int64)
-        for i, c in enumerate(signals):
-            offs[i + 1] = offs[i] + len(c)
-        data = np.ascontiguousarray(np.concatenate([np.asarray(c, np.float32) for c in signals]))
+        data, offs = pack(signals, np.float32)
         fo = np.zeros(U + 1, np.int64)
         self._ck(self.lib.nhans_stft_f32(self.h, _ptr(data), _ptr(offs), U, None, None, _ptr(fo)))
         F = int(fo[-1])
@@ -147,14 +147,9 @@ class Engine:
         host; contexts = first 200 frames of ctx_a[u] / ctx_b[u] (ctx_a may be None: Silent.wav); the mask network runs
         over mixture frames [start:].  One device pass, no host round trips between the stages.
         -> (list of denoised sample arrays, list of mixture-centre sample arrays or None)"""
-        def packf(clips):
-            offs = np.zeros(len(clips) + 1, np.int64)
-            for i, c in enumerate(clips):
-                offs[i + 1] = offs[i] + len(c)
-            return np.ascontiguousarray(np.concatenate([np.asarray(c, np.float32) for c in clips])), offs
-        m, mo = packf(mixes)
-        b, bo = packf(ctx_b)
-        a, ao = packf(ctx_a) if ctx_a is not None else (None, None)
+        m, mo = pack(mixes, np.float32)
+        b, bo = pack(ctx_b, np.float32)
+        a, ao = pack(ctx_a, np.float32) if ctx_a is not None else (None, None)
         U = len(mixes)
         oo = np.zeros(U + 1, np.int64)
         self._ck(self.lib.nhans_enhance_f32(self.h, _ptr(m), _ptr(mo), U, _ptr(a), _ptr(ao), _ptr(b), _ptr(bo), int(start), None, None, _ptr(oo)))
@@ -276,13 +271,7 @@ class Engine:
         return cur.array[:n]
 
     def _pack_pinned(self, stage, key, clips):
-        offs = np.zeros(len(clips) + 1, np.int64)
-        for i, c in enumerate(clips):
-            offs[i + 1] = offs[i] + len(c)
-        buf = self._pinned(stage, key, int(offs[-1]), np.int16)
-        for i, c in enumerate(clips):
-            buf[offs[i]:offs[i + 1]] = c
-        return buf, offs
+        return pack(clips, np.int16, lambda n, dtype: self._pinned(stage, key, n, dtype))
 
     def submit(self, mix_clips, ctx_a_clips, ctx_b_clips, want_f32=True, want_i16=True, want_mixproc=False):
         """Stage a batch in pinned memory and enqueue H2D + kernels + D2H without waiting.  Up to two batches may be

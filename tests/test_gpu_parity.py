@@ -168,6 +168,11 @@ def test_fused_float_path_matches_stage_entries(engine_sn):
             ysm, _ = engine_sn.istft(sl, sp, f1)
             assert len(y[u]) == len(ys) == (T - start - 1) * 160 + 400
             assert _snr(ys, y[u]) >= 60.0 and _snr(ysm, ym[u]) >= 80.0
+    # frame t of m[160 s:] is frame t + s of m: frames [200:] of the mixture are exactly the frames of its slice
+    y, ym = engine_sn.enhance_f32(mixes, ca, cb, start=200)
+    ys, ysm = engine_sn.enhance_f32([m[160 * 200:] for m in mixes], ca, cb, start=0)
+    for u in range(2):
+        assert np.array_equal(y[u], ys[u]) and np.array_equal(ym[u], ysm[u])
     # Silent positive context (ctx_a = None) == an explicit all-zero clip
     y0, _ = engine_sn.enhance_f32(mixes[:1], None, cb[:1], start=0)
     y1, _ = engine_sn.enhance_f32(mixes[:1], [np.zeros(48000, np.float32)], cb[:1], start=0)
