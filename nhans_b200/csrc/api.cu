@@ -62,7 +62,7 @@ struct NetDev {
   NetPlan plan;
   std::vector<__half*> bufs;
   std::vector<GemmLayerDev> layers;
-  float *first_w = nullptr, *first_bias = nullptr, *first_tftab = nullptr;
+  float *first_w = nullptr, *first_bias = nullptr;
   uint16_t *first_ttab16 = nullptr, *first_ftab16 = nullptr;
   float *Pa = nullptr, *Pb = nullptr, *c = nullptr;
   int *u_frame = nullptr, *u_lo = nullptr, *u_hi = nullptr, *u_utt = nullptr;
@@ -214,8 +214,13 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
   }
   int rc;
   if (P.cond.n_cols > 0) {
-    // main net: room for the frames of one pass plus 34 virtual frames per utterance (utterances of >= 17 frames on
-    // average; a pass of shorter ones falls back to the per-window kernel)
+    // main net: its first convolution runs once per frame (kernels.h FrameConvDev), which needs this shape
+    const DirectLayer& D = P.first;
+    if (D.kh != 4 || D.kw != 4 || D.sh != 1 || D.sw != 1 || D.pt != 1 || D.pl != 1 || D.Hin != kWinFrames || D.Ho != kWinFrames ||
+        D.raw_oh != -(kWinFrames / 2) || D.N != 64)
+      return fail(ctx, NHANS_ERR_STATE, "first convolution of the mask network with an unexpected shape");
+    // per-frame table: a pass's windows plus 34 virtual frames per utterance it touches.  run_masknet sizes every pass
+    // to fit, so utterances that average fewer than 17 frames run in smaller passes.
     net.crow_cap = 3LL * P.capacity + 64;
     void* p = nullptr;
     CK(cudaMalloc(&p, (size_t)4 * net.crow_cap * kBins * 64 * sizeof(float)));
@@ -230,7 +235,6 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
   }
   if ((rc = upload(ctx, net, P.first.w, &net.first_w))) return rc;
   if ((rc = upload(ctx, net, P.first.epi.bias, &net.first_bias))) return rc;
-  if ((rc = upload(ctx, net, P.first.epi.tftab, &net.first_tftab))) return rc;
   if ((rc = upload(ctx, net, P.first.epi.ttab16, &net.first_ttab16))) return rc;
   if ((rc = upload(ctx, net, P.first.epi.ftab16, &net.first_ftab16))) return rc;
   if ((rc = upload(ctx, net, P.cond.Pa, &net.Pa))) return rc;
@@ -384,11 +388,11 @@ EpiDev make_epi(const NetDev& net, const Epilogue& E, const Grid& out, const flo
   return e;
 }
 
-struct PassInfo {                   // which frames / utterances a pass of the mask network touches
-  long long w0;                     // first window (= global frame index of its centre)
-  int u_first, u_last;
+struct PassInfo {                   // which utterances / per-frame table rows a pass of the mask network touches
   const long long* d_frame_offs;
-  int U;
+  int u_first, u_last;
+  long long crow0;                  // first table row = first window + 34 * u_first
+  int rows;                         // table rows of the pass (<= crow_cap)
 };
 
 // Runs `units` windows / context rows whose unit tables are already filled.
@@ -397,7 +401,6 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
   const NetPlan& P = net.plan;
   UnitTable ut{net.u_frame, net.u_lo, net.u_hi, net.u_utt};
   bool gen_first = false;
-  long long gen_crow0 = 0;
   {
     const DirectLayer& D = P.first;
     DirectDev d;
@@ -407,42 +410,35 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
     d.Hin = D.Hin; d.Win = D.Win; d.raw_oh = D.raw_oh; d.Ho = D.Ho; d.Wo = D.Wo; d.N = D.N;
     d.w = net.first_w;
     d.units_tab = ut;
-    d.epi = make_epi(net, D.epi, D.out, net.first_bias, net.first_tftab, nullptr, nullptr, raw, cond_table, nullptr);
+    d.epi = make_epi(net, D.epi, D.out, net.first_bias, nullptr, nullptr, nullptr, raw, cond_table, nullptr);
     d.epi.ttab16 = reinterpret_cast<const __half*>(net.first_ttab16);
     d.epi.ftab16 = reinterpret_cast<const __half*>(net.first_ftab16);
     d.epi.tab_H = D.Ho; d.epi.tab_W = D.Wo;
     ProfScope ps(ctx, 3, 2.0 * D.macs_per_unit * units, 0);
-    bool done = false;
-    if (pass && net.convC && D.kh == 4 && D.kw == 4 && D.sh == 1 && D.sw == 1 && D.pt == 1 && D.pl == 1 && D.Hin == kWinFrames &&
-        D.Ho == kWinFrames && D.raw_oh == -(kWinFrames / 2) && D.N == 64) {
+    if (pass) {
       FrameConvDev f;
       memset(&f, 0, sizeof f);
       f.raw = raw; f.frame_offs = pass->d_frame_offs;
       f.u_first = pass->u_first; f.u_last = pass->u_last;
-      f.crow0 = pass->w0 + 34LL * pass->u_first;
-      const long long last = pass->w0 + units - 1 + 34LL * pass->u_last + (kWinFrames - 1);
-      f.rows = (int)(last - f.crow0 + 1);
+      f.crow0 = pass->crow0;
+      f.rows = pass->rows;
       f.crow_cap = net.crow_cap;
       f.w = net.first_w;
       f.bias = d.epi.bias; f.bias_stride = d.epi.bias_stride; f.ftab16 = d.epi.ftab16;
       f.C = net.convC;
-      if (f.rows <= net.crow_cap) {
-        // (expanding the pass in slices so that a slice's table stays L2-resident was measured: no gain)
-        CK(launch_frame_conv(ctx->stream, f));
-        // the row-walk kernel of the next layer builds its A operand from the table (conv_walk.cu kWalkGen); otherwise
-        // the table is expanded into the (window, row) activation tensor here
-        gen_first = ctx->use_walk && ctx->use_gen && !P.gemm.empty() && P.gemm[0].walk && net.layers[0].w_walk &&
-                    P.gemm[0].a_buf[0] == D.out.buf && D.epi.relu && d.epi.ttab16;
-        if (gen_first) {
-          gen_crow0 = f.crow0;
-        } else {
-          CK(launch_window_expand(ctx->stream, d, net.convC, f.crow0, net.crow_cap, 0, units));
-          ctx->launches += 1;
-        }
-        done = true;
+      // (expanding the pass in slices so that a slice's table stays L2-resident was measured: no gain)
+      CK(launch_frame_conv(ctx->stream, f));
+      // the row-walk kernel of the next layer builds its A operand from the table (conv_walk.cu kWalkGen); otherwise
+      // the table is expanded into the (window, row) activation tensor here
+      gen_first = ctx->use_walk && ctx->use_gen && !P.gemm.empty() && P.gemm[0].walk && net.layers[0].w_walk &&
+                  P.gemm[0].a_buf[0] == D.out.buf && D.epi.relu && d.epi.ttab16;
+      if (!gen_first) {
+        CK(launch_window_expand(ctx->stream, d, net.convC, pass->crow0, net.crow_cap, 0, units));
+        ctx->launches += 1;
       }
+    } else {
+      CK(launch_direct_conv(ctx->stream, d));
     }
-    if (!done) CK(launch_direct_conv(ctx->stream, d));
   }
   for (size_t i = 0; i < P.gemm.size(); ++i) {
     const GemmLayer& L = P.gemm[i];
@@ -475,7 +471,7 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
       wd.H = L.Ho; wd.Wq = L.Wq; wd.Wo = L.Wo; wd.pt = L.c_pt; wd.pl = L.c_pl;
       wd.units = ut; wd.epi = g.epi; wd.err_flag = g.err_flag; wd.debug_stats = g.debug_stats;
       if (i == 0 && gen_first) {
-        wd.gen_C = net.convC; wd.gen_crow0 = gen_crow0; wd.gen_crow_cap = net.crow_cap;
+        wd.gen_C = net.convC; wd.gen_crow0 = pass->crow0; wd.gen_crow_cap = net.crow_cap;
         wd.gen_ttab16 = reinterpret_cast<const __half*>(net.first_ttab16);
       }
       cudaError_t le = launch_walk(ctx->stream, ctx->n_sm, D.mapA0, D.mapBwalk, wd);
@@ -518,16 +514,26 @@ int run_masknet(nhans_ctx* ctx, const float* logmag, const long long* d_frame_of
   NetDev& net = ctx->main_net;
   const int cap = net.plan.capacity;
   if (total_frames > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one batch");
-  for (long long w0 = 0; w0 < total_frames; w0 += cap) {
-    const int n = (int)std::min<long long>(cap, total_frames - w0);
-    CK(launch_units_main(ctx->stream, d_frame_offs, U, (int)w0, n, net.u_frame, net.u_lo, net.u_hi, net.u_utt));
-    ctx->launches += 1;
+  // utterance of a frame: largest u with frame_offs[u] <= frame
+  auto utt_of = [&](long long frame) { return (int)(std::upper_bound(h_frame_offs, h_frame_offs + U + 1, frame) - h_frame_offs) - 1; };
+  for (long long w0 = 0, n = 0; w0 < total_frames; w0 += n) {
     PassInfo pi;
-    pi.w0 = w0; pi.d_frame_offs = d_frame_offs; pi.U = U;
-    // utterances of the first / last window of the pass: largest u with frame_offs[u] <= frame
-    pi.u_first = (int)(std::upper_bound(h_frame_offs, h_frame_offs + U + 1, w0) - h_frame_offs) - 1;
-    pi.u_last = (int)(std::upper_bound(h_frame_offs, h_frame_offs + U + 1, w0 + n - 1) - h_frame_offs) - 1;
-    int rc = run_net(ctx, net, n, logmag, cond_table, den + (size_t)w0 * kBins, &pi);
+    pi.d_frame_offs = d_frame_offs;
+    pi.u_first = utt_of(w0);
+    pi.crow0 = w0 + 34LL * pi.u_first;
+    // the largest pass whose per-frame table rows (its windows + 34 per utterance) fit; one window always does
+    auto rows = [&](long long m) { return m + 34LL * (utt_of(w0 + m - 1) - pi.u_first + 1); };
+    long long lo = 1, hi = std::min<long long>(cap, total_frames - w0);
+    while (lo < hi) {
+      const long long mid = (lo + hi + 1) / 2;
+      if (rows(mid) <= net.crow_cap) lo = mid; else hi = mid - 1;
+    }
+    n = lo;
+    pi.u_last = utt_of(w0 + n - 1);
+    pi.rows = (int)rows(n);
+    CK(launch_units_main(ctx->stream, d_frame_offs, U, (int)w0, (int)n, net.u_frame, net.u_lo, net.u_hi, net.u_utt));
+    ctx->launches += 1;
+    int rc = run_net(ctx, net, (int)n, logmag, cond_table, den + (size_t)w0 * kBins, &pi);
     if (rc) return rc;
   }
   return 0;

@@ -113,6 +113,7 @@ constexpr int kGemmThreads = 352;     // A producer, B producer, MMA issuer, 8 e
 int gemm_smem_bytes(int BN, int num_kb, int tab_bytes, int cta2, int row, GemmCfg* cfg);
 cudaError_t launch_gemm(cudaStream_t s, int n_sm, const CUtensorMap& mapA0, const CUtensorMap& mapA1,
                         const CUtensorMap& mapB, const CUtensorMap& mapBhalf, const GemmDev& p);
+// first convolution of the towers (Cin = 1, N = 64); an epilogue with embedding tables is rejected
 cudaError_t launch_direct_conv(cudaStream_t s, const DirectDev& p);
 // mapA: the input grid as [pixels][64] (box 136 x 64), mapB: repacked weights [4 kernel-row blocks x 64][4 x 64] (box 256 x 64)
 cudaError_t launch_walk(cudaStream_t s, int n_sm, const CUtensorMap& mapA, const CUtensorMap& mapB, const WalkDev& p);
@@ -124,7 +125,8 @@ cudaError_t launch_walk(cudaStream_t s, int n_sm, const CUtensorMap& mapA, const
 // frame + 34 * utterance + row indexes the zero-extended utterance (17 virtual frames on either side), and the
 // conditioning bias of the utterance and the frequency embedding F[w] are folded in (a C row belongs to one
 // utterance).  window_expand then writes h1[n][h][w][:] = relu(C[variant(h)][crow(n) + h][w][:] + T[h]) in fp16:
-// 35x fewer multiply-adds than the per-window kernel, what remains is the 1.8 GB store stream of a pass.
+// 35x fewer multiply-adds than a per-window evaluation, what remains is the 1.8 GB store stream of a pass.
+// The host sizes every pass so that its rows fit the table (rows <= crow_cap), whatever the utterance lengths.
 struct FrameConvDev {
   const float* raw;            // [frames][201] log-magnitude
   const long long* frame_offs; // [U + 1] device

@@ -1,6 +1,6 @@
 // CUDA-core kernels around the tensor-core GEMMs: the Cin = 1 convolutions (per-frame evaluation + window
-// expansion for the mask network, per-unit kernels with the implicit window gather for the towers / fallback), the conditioning-projection table, the tower's global mean pool and the
-// per-unit lookup tables.
+// expansion for the mask network, a per-pixel kernel that reads the spectrogram rows for the towers), the
+// conditioning-projection table, the tower's global mean pool and the per-unit lookup tables.
 #include "kernels.h"
 
 namespace nhans {
@@ -12,11 +12,10 @@ __device__ __forceinline__ uint32_t pack_half2(float a, float b) {
   return *reinterpret_cast<uint32_t*>(&h);
 }
 
-// resblock1_1_conv1 (main.py:162, Cin = 1, 4x4) and embedding/noise_resblock1_1_conv1 (main.py:104, 8x4,
-// stride 3x2): one thread per output pixel, 64 output channels in registers.  Input row r of unit n is
-// frame units.frame[n] + r + raw_oh of the fp32 log-magnitude array; rows outside the clip and outside
-// [0, Hin) read 0.0, which is the zero padding of pad_1D_for_windowing (SN/apply.py:170-173) and of the
-// 'SAME' convolution at once - the [T, 35, 201] window tensor is never materialised.
+// embedding/noise_resblock1_1_conv1 (main.py:104, Cin = 1, 8x4, stride 3x2, no embedding tables): one thread per
+// output pixel, 64 output channels in registers.  Input row r of unit n is frame units.frame[n] + r + raw_oh of
+// the fp32 log-magnitude array; rows outside the unit's [lo, hi) frames and outside [0, Hin) read 0.0, the zero
+// padding of the 'SAME' convolution.
 constexpr int kDirectPitch = 68;                       // floats per staged pixel row (64 + 4: conflict-free float4 access)
 __global__ void __launch_bounds__(128)
 direct_conv64_kernel(const DirectDev p) {
@@ -61,7 +60,7 @@ direct_conv64_kernel(const DirectDev p) {
     }
   }
   // Epilogue through a warp-private shared-memory transpose: 8 lanes then cover one pixel's 64 channels, so
-  // the table loads and the fp16 stores of a warp touch whole 128-byte lines instead of 32 scattered ones.
+  // the bias loads and the fp16 stores of a warp touch whole 128-byte lines instead of 32 scattered ones.
   const int utt = p.units_tab.utt ? p.units_tab.utt[unit] : 0;
   const int yy = ho + e.o_oy, xx = wo + e.o_ox;
   const int plane = (yy % e.o_sh) * e.o_sw + (xx % e.o_sw);
@@ -69,14 +68,13 @@ direct_conv64_kernel(const DirectDev p) {
   const int lane = threadIdx.x & 31;
   float* st = s_stage + (threadIdx.x >> 5) * (32 * kDirectPitch);
   long long* s_pix = reinterpret_cast<long long*>(s_meta) + (threadIdx.x >> 5) * 32;
-  int* s_tf = s_meta + 2 * 4 * 32 + (threadIdx.x >> 5) * 64;
+  int* s_utt = s_meta + 2 * 4 * 32 + (threadIdx.x >> 5) * 32;
   __syncwarp();
 #pragma unroll
   for (int n = 0; n < 16; ++n)
     *reinterpret_cast<float4*>(st + lane * kDirectPitch + 4 * n) = make_float4(acc[4 * n], acc[4 * n + 1], acc[4 * n + 2], acc[4 * n + 3]);
   s_pix[lane] = valid ? pix : -1;
-  s_tf[2 * lane] = valid ? (ho * p.Wo + wo) : 0;
-  s_tf[2 * lane + 1] = utt;
+  s_utt[lane] = utt;
   __syncwarp();
   const int sub = lane >> 3, cg = (lane & 7) * 8;
 #pragma unroll 2
@@ -86,14 +84,8 @@ direct_conv64_kernel(const DirectDev p) {
     if (opix < 0) continue;
     const float4 a0 = *reinterpret_cast<const float4*>(st + r * kDirectPitch + cg);
     const float4 a1 = *reinterpret_cast<const float4*>(st + r * kDirectPitch + cg + 4);
-    const float4* b4 = reinterpret_cast<const float4*>(e.bias + (size_t)s_tf[2 * r + 1] * e.bias_stride + cg);
-    float4 b0 = __ldg(b4), b1 = __ldg(b4 + 1);
-    if (e.tftab) {
-      const float4* t4 = reinterpret_cast<const float4*>(e.tftab + (size_t)s_tf[2 * r] * 64 + cg);
-      const float4 t0 = __ldg(t4), t1 = __ldg(t4 + 1);
-      b0.x += t0.x; b0.y += t0.y; b0.z += t0.z; b0.w += t0.w;
-      b1.x += t1.x; b1.y += t1.y; b1.z += t1.z; b1.w += t1.w;
-    }
+    const float4* b4 = reinterpret_cast<const float4*>(e.bias + (size_t)s_utt[r] * e.bias_stride + cg);
+    const float4 b0 = __ldg(b4), b1 = __ldg(b4 + 1);
     float v[8] = {a0.x + b0.x, a0.y + b0.y, a0.z + b0.z, a0.w + b0.w, a1.x + b1.x, a1.y + b1.y, a1.z + b1.z, a1.w + b1.w};
     if (e.relu) {
 #pragma unroll
@@ -103,156 +95,6 @@ direct_conv64_kernel(const DirectDev p) {
     o.x = pack_half2(v[0], v[1]); o.y = pack_half2(v[2], v[3]);
     o.z = pack_half2(v[4], v[5]); o.w = pack_half2(v[6], v[7]);
     *reinterpret_cast<uint4*>(e.out + opix * e.out_C + cg) = o;
-  }
-}
-
-// Tensor-core version of the same convolution (legacy mma.sync path: the work is only 7 MMAC per window, but on
-// CUDA cores it cost 9 % of the step).  A warp owns 16 consecutive output pixels of one image row:
-// D[16 px][64 ch] = A[16 px][taps] . B[taps][64 ch] with mma.sync.m16n8k8 TF32, the A fragment gathered straight
-// from the fp32 spectrogram (implicit window gather and zero padding as above).  To stay at fp32 accuracy every
-// operand is split into two TF32 terms (a = a_hi + a_lo, b = b_hi + b_lo) and the three significant products are
-// accumulated (3xTF32).  Kernel width must be 4 (it is, for both layers): tap k = 4 i + j.
-__device__ __forceinline__ uint32_t to_tf32(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-__device__ __forceinline__ void mma_tf32(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-
-constexpr int kMmaWarps = 4;
-constexpr int kMmaPitch = 68;                          // floats per staged pixel row
-// A warp walks one output image row (unit, ho) in 16-pixel segments, so everything that depends on the row only -
-// the frame bounds, the per-utterance bias, the time-embedding row T[ho] folded into it, the output row address - is
-// set up once per 13 segments; per pixel only the frequency-embedding row F[wo] (fp16, 25 KB, L1 resident) is read.
-// kTab: 0 = no tables (tower), 1 = separable fp16 tables, 2 = combined fp32 table (fallback).
-__device__ __forceinline__ void add_half8(float (&b)[8], const uint4 t) {
-  const __half2* h = reinterpret_cast<const __half2*>(&t);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const float2 f = __half22float2(h[i]);
-    b[2 * i] += f.x;
-    b[2 * i + 1] += f.y;
-  }
-}
-
-template <int KSTEPS>
-__global__ void __launch_bounds__(kMmaWarps * 32)     // 80 registers; capping them for 7-8 blocks/SM spills and is 15 % slower
-direct_conv_mma_kernel(const DirectDev p, const int segs) {
-  extern __shared__ float4 s_b[];                      // [ksteps][8 n-tiles][32 lanes] {b0_hi, b1_hi, b0_lo, b1_lo}
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  float* st = reinterpret_cast<float*>(s_b + KSTEPS * 8 * 32) + warp * 16 * kMmaPitch;
-  for (int idx = threadIdx.x; idx < KSTEPS * 8 * 32; idx += blockDim.x) {
-    const int l = idx & 31, nt = (idx >> 5) & 7, ks = idx >> 8;
-    const int n = nt * 8 + (l >> 2);                   // B fragment: b0 = (k = l % 4, n), b1 = (k + 4, n)
-    const float w0 = p.w[(ks * 8 + (l & 3)) * 64 + n], w1 = p.w[(ks * 8 + (l & 3) + 4) * 64 + n];
-    const float h0 = __uint_as_float(to_tf32(w0)), h1 = __uint_as_float(to_tf32(w1));
-    s_b[idx] = make_float4(h0, h1, __uint_as_float(to_tf32(w0 - h0)), __uint_as_float(to_tf32(w1 - h1)));
-  }
-  __syncthreads();
-  const EpiDev& e = p.epi;
-  const int rows = p.units * p.Ho;
-  const int g4 = lane >> 2, t4 = lane & 3;             // fragment row / column ids
-  const int sub = lane >> 3, cg = (lane & 7) * 8;      // epilogue: 4 pixels per pass, 8 channels per lane
-  const int tab = (e.ttab16 && e.ftab16) ? 1 : (e.tftab ? 2 : 0);
-  const int xshift = e.o_sw == 1 ? 0 : (e.o_sw == 2 ? 1 : -1);
-  for (int rowid = blockIdx.x * kMmaWarps + warp; rowid < rows; rowid += gridDim.x * kMmaWarps) {
-    const int unit = rowid / p.Ho, ho = rowid - unit * p.Ho;
-    const int frame0 = p.units_tab.frame[unit] + p.raw_oh;
-    const int lo = p.units_tab.lo[unit], hi = p.units_tab.hi[unit];
-    const int utt = p.units_tab.utt ? p.units_tab.utt[unit] : 0;
-    // source rows of the 2 KSTEPS kernel rows (null when the row is padding or another utterance's frame)
-    const float* src[2 * KSTEPS];
-#pragma unroll
-    for (int i = 0; i < 2 * KSTEPS; ++i) {
-      const int r = ho * p.sh + i - p.pt;
-      const int frame = frame0 + r;
-      src[i] = (r >= 0 && r < p.Hin && frame >= lo && frame < hi) ? e.raw + (size_t)frame * 201 : nullptr;
-    }
-    float bias[8];
-    {
-      const float4* b4 = reinterpret_cast<const float4*>(e.bias + (size_t)utt * e.bias_stride + cg);
-      const float4 b0 = __ldg(b4), b1 = __ldg(b4 + 1);
-      bias[0] = b0.x; bias[1] = b0.y; bias[2] = b0.z; bias[3] = b0.w;
-      bias[4] = b1.x; bias[5] = b1.y; bias[6] = b1.z; bias[7] = b1.w;
-      if (tab == 1) add_half8(bias, __ldg(reinterpret_cast<const uint4*>(e.ttab16 + ho * 64 + cg)));
-    }
-    const int yy = ho + e.o_oy;
-    const long long row_pix = unit * e.o_ustride + (yy / e.o_sh) * e.o_rstride;
-    const int plane_y = (yy % e.o_sh) * e.o_sw;
-    for (int seg = 0; seg < segs; ++seg) {
-      const int wo0 = seg * 16;
-      float acc[8][4];
-#pragma unroll
-      for (int nt = 0; nt < 8; ++nt) { acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f; }
-      const int f0 = (wo0 + g4) * p.sw + t4 - p.pl, f1 = f0 + 8 * p.sw;
-      const bool ok0 = f0 >= 0 && f0 < p.Win, ok1 = f1 >= 0 && f1 < p.Win;
-#pragma unroll
-      for (int ks = 0; ks < KSTEPS; ++ks) {
-        // A fragment: a0 = (px g4, tap t4), a1 = (px g4 + 8, tap t4), a2 = (px g4, tap t4 + 4), a3 = (px g4 + 8, tap t4 + 4)
-        float av[4];
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {                  // h: kernel row 2 ks + h  (taps t4 and t4 + 4)
-          const float* row = src[2 * ks + h];
-          av[2 * h] = (row && ok0) ? __ldg(row + f0) : 0.f;
-          av[2 * h + 1] = (row && ok1) ? __ldg(row + f1) : 0.f;
-        }
-        uint32_t a_hi[4], a_lo[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          a_hi[k] = to_tf32(av[k]);
-          a_lo[k] = to_tf32(av[k] - __uint_as_float(a_hi[k]));
-        }
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-          const float4 b = s_b[(ks * 8 + nt) * 32 + lane];
-          mma_tf32(acc[nt], a_lo, __float_as_uint(b.x), __float_as_uint(b.y));
-          mma_tf32(acc[nt], a_hi, __float_as_uint(b.z), __float_as_uint(b.w));
-          mma_tf32(acc[nt], a_hi, __float_as_uint(b.x), __float_as_uint(b.y));
-        }
-      }
-      // C fragment -> staging: c0/c1 = (px g4, ch 8 nt + 2 t4 + {0,1}), c2/c3 = (px g4 + 8, ...)
-      __syncwarp();
-#pragma unroll
-      for (int nt = 0; nt < 8; ++nt) {
-        *reinterpret_cast<float2*>(st + g4 * kMmaPitch + nt * 8 + 2 * t4) = make_float2(acc[nt][0], acc[nt][1]);
-        *reinterpret_cast<float2*>(st + (g4 + 8) * kMmaPitch + nt * 8 + 2 * t4) = make_float2(acc[nt][2], acc[nt][3]);
-      }
-      __syncwarp();
-#pragma unroll
-      for (int g = 0; g < 4; ++g) {
-        const int px = g * 4 + sub, wo = wo0 + px;
-        if (wo >= p.Wo) continue;
-        const float4 a0 = *reinterpret_cast<const float4*>(st + px * kMmaPitch + cg);
-        const float4 a1 = *reinterpret_cast<const float4*>(st + px * kMmaPitch + cg + 4);
-        float v[8] = {bias[0], bias[1], bias[2], bias[3], bias[4], bias[5], bias[6], bias[7]};
-        if (tab == 1) {
-          add_half8(v, __ldg(reinterpret_cast<const uint4*>(e.ftab16 + wo * 64 + cg)));
-        } else if (tab == 2) {
-          const float4* t4p = reinterpret_cast<const float4*>(e.tftab + ((size_t)ho * p.Wo + wo) * 64 + cg);
-          const float4 t0 = __ldg(t4p), t1 = __ldg(t4p + 1);
-          v[0] += t0.x; v[1] += t0.y; v[2] += t0.z; v[3] += t0.w;
-          v[4] += t1.x; v[5] += t1.y; v[6] += t1.z; v[7] += t1.w;
-        }
-        v[0] += a0.x; v[1] += a0.y; v[2] += a0.z; v[3] += a0.w;
-        v[4] += a1.x; v[5] += a1.y; v[6] += a1.z; v[7] += a1.w;
-        if (e.relu) {
-#pragma unroll
-          for (int i = 0; i < 8; ++i) v[i] = fmaxf(v[i], 0.f);
-        }
-        const int xx = wo + e.o_ox;
-        long long pix;
-        if (xshift >= 0) pix = (long long)(plane_y + (xx & ((1 << xshift) - 1))) * e.o_plane + row_pix + (xx >> xshift);
-        else pix = (long long)(plane_y + (xx % e.o_sw)) * e.o_plane + row_pix + (xx / e.o_sw);
-        uint4 o;
-        o.x = pack_half2(v[0], v[1]); o.y = pack_half2(v[2], v[3]);
-        o.z = pack_half2(v[4], v[5]); o.w = pack_half2(v[6], v[7]);
-        *reinterpret_cast<uint4*>(e.out + pix * e.out_C + cg) = o;
-      }
-    }
   }
 }
 
@@ -328,6 +170,16 @@ frame_conv_kernel(const FrameConvDev p) {
 #pragma unroll
     for (int k = 0; k < 4; ++k)
       *reinterpret_cast<float4*>(out + k * vplane + (size_t)w * 64 + cg) = make_float4(v[k][0], v[k][1], v[k][2], v[k][3]);
+  }
+}
+
+__device__ __forceinline__ void add_half8(float (&b)[8], const uint4 t) {
+  const __half2* h = reinterpret_cast<const __half2*>(&t);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const float2 f = __half22float2(h[i]);
+    b[2 * i] += f.x;
+    b[2 * i + 1] += f.y;
   }
 }
 
@@ -474,21 +326,11 @@ __global__ void units_rows_kernel(int r0, int n_units, int rows, int* frame, int
 
 cudaError_t launch_direct_conv(cudaStream_t s, const DirectDev& p) {
   if (p.units <= 0) return cudaSuccess;
-  if (p.N != 64) return cudaErrorInvalidValue;
-  if (p.kw == 4 && p.kh == 4) {
-    const int segs = (p.Wo + 15) / 16;
-    const long long rows = (long long)p.units * p.Ho;
-    if (rows > 0x7fffffffLL) return cudaErrorInvalidValue;
-    const size_t smem_mma = (size_t)2 * 8 * 32 * 16 + kMmaWarps * 16 * kMmaPitch * 4;
-    long long blocks_mma = (rows + kMmaWarps - 1) / kMmaWarps;
-    if (blocks_mma > 148 * 16) blocks_mma = 148 * 16;              // grid-stride: the weight fragments are staged once per CTA
-    direct_conv_mma_kernel<2><<<(unsigned)blocks_mma, kMmaWarps * 32, smem_mma, s>>>(p, segs);
-    return cudaGetLastError();
-  }
+  if (p.N != 64 || p.epi.tftab || p.epi.ttab16 || p.epi.ftab16) return cudaErrorInvalidValue;
   const long long total = (long long)p.units * p.Ho * p.Wo;
   const int threads = 128;
   const long long blocks = (total + threads - 1) / threads;
-  const size_t smem = (size_t)p.kh * p.kw * 64 * 4 + 4 * 32 * kDirectPitch * 4 + 2 * 4 * 32 * 4 + 4 * 64 * 4;
+  const size_t smem = (size_t)p.kh * p.kw * 64 * 4 + 4 * 32 * kDirectPitch * 4 + 2 * 4 * 32 * 4 + 4 * 32 * 4;
   direct_conv64_kernel<<<(unsigned)blocks, threads, smem, s>>>(p);
   return cudaGetLastError();
 }

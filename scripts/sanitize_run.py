@@ -1,7 +1,7 @@
 """Smoke-size invocations of the hot path for compute-sanitizer (scripts/sanitize.sh): tiny capacities so that every
-kernel - STFT, towers, first convolution (per-frame table + generated operand, or the per-window fallback), row-walk
-and shifted-row GEMM layers, split-K head, iSTFT, post-mix - runs a handful of CTAs.
-   python scripts/sanitize_run.py sn|ss|fallback"""
+kernel - STFT, towers, first convolution (per-frame table + generated operand), row-walk and shifted-row GEMM layers,
+split-K head, iSTFT, post-mix - runs a handful of CTAs; `tiny` packs a batch of 2-3 frame utterances into several passes.
+   python scripts/sanitize_run.py sn|ss|tiny"""
 import os
 import sys
 
@@ -16,8 +16,8 @@ mode = sys.argv[1] if len(sys.argv) > 1 else "sn"
 variant = 1 if mode == "ss" else 0
 eng = Engine(0, variant, win_capacity=8, row_capacity=1)
 eng.load_weights(W.seeded_init(variant, 0))
-if mode == "fallback":
-    # utterances of 2-3 frames: more virtual frames than the per-frame table holds -> per-window first convolution
+if mode == "tiny":
+    # utterances of 2-3 frames: more virtual frames than one pass's per-frame table holds -> several smaller passes
     base = synth.mixture(0.5, 1)
     mixes = [base[o:o + 560 + 160 * (i % 2)] for i, o in enumerate(range(0, 4000, 400))]
     res = eng.enhance(mixes, None, [synth.noise_clip(1)] * len(mixes))
