@@ -129,6 +129,39 @@ int nhans_download(nhans_ctx* ctx, int16_t* out_i16, float* out_f32, float* mixp
 int nhans_postmix(nhans_ctx* ctx, float compensate, int ac, float* mixed_f32, float* removed_f32, float* compensated_f32,
                   float* snr_est);
 
+/* ---- streaming: live int16 mono streams, bit-identical to the batch path --------------------------------
+ *
+ * A stream is enhanced chunk by chunk as its samples arrive.  For every chunking, the concatenation of what a stream
+ * emits equals the int16 / float32 output of nhans_enhance_batch for the whole clip bit for bit, given the same peak
+ * and contexts.  Emission rule: after a stream has received N samples in all, F = 1 + (N - 400) / 160 frames (0 when
+ * N < 400), it has emitted 160 * max(0, F - 17) samples; after its final step it has emitted (F - 1) * 160 + 400 (0 when
+ * F = 0), what the batch path returns for the clip (trailing samples that fill no frame are dropped).  A window needs
+ * the 17 frames after its centre and a 400-sample frame, so the algorithmic latency is 16 * 160 + 400 = 2960 samples
+ * (185 ms at 16 kHz), plus up to 159 samples waiting for the next hop boundary.
+ * nhans_load_weights closes every open stream.  Without loaded weights the calls below return NHANS_ERR_STATE. */
+
+/* Opens n streams (one tower pass for all of them).  Stream i is conditioned on ctx_b[b_offs[i] : b_offs[i+1]] and
+ * ctx_a[a_offs[i] : a_offs[i+1]], with the rules of nhans_enhance_batch (ctx_a may be NULL for the selective-noise
+ * variant: Silent.wav; each clip must yield 200 frames, else NHANS_ERR_CONTEXT_TOO_SHORT).  peak[i] >= 0 replaces the
+ * whole-clip max|x| of SN/apply.py:150, which a live stream cannot know: pass the peak nhans_stft reports for the whole
+ * clip for output identical to the batch path, or a fixed full-scale value such as 32767.  It scales the input and the
+ * int16 output.  ids [n] receives the stream ids.  Synchronous. */
+int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t* a_offs, const int16_t* ctx_b,
+                      const int64_t* b_offs, const int32_t* peak, int* ids);
+/* Appends chunk pcm[offs[i] : offs[i+1]] (any length, 0 included) to stream ids[i] (i < n, ids distinct) and processes
+ * every window that has become computable across the n streams in the same network passes.  out_offs [n+1] is written
+ * (offsets relative to out_offs[0] = 0); out_i16 / out_f32 (either may be NULL) receive each stream's newly emitted
+ * samples there.  final may be NULL; final[i] != 0 flushes stream i, which then takes no further step.  An unknown or
+ * closed id, an id given twice or a step after the final one is NHANS_ERR_ARG.  Synchronous; leaves the results of a
+ * batch in flight (nhans_upload / nhans_run / nhans_download / nhans_postmix) untouched. */
+int nhans_stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final,
+                      int16_t* out_i16, float* out_f32, int64_t* out_offs);
+/* Releases n streams, finalised or not. */
+int nhans_stream_close(nhans_ctx* ctx, int n, const int* ids);
+/* Host only (no context, no GPU): samples one step emits for a stream that goes from `before` to `after` samples
+ * received (final != 0: its final step). */
+int nhans_stream_emit_len(int64_t before, int64_t after, int final, int64_t* emitted);
+
 /* Pinned host memory for the copies above. */
 int nhans_host_alloc(int64_t bytes, void** out);
 void nhans_host_free(void* p);

@@ -18,6 +18,7 @@ SYMBOLS = [
     "nhans_event_elapsed_ms", "nhans_profile_enable", "nhans_profile_get", "nhans_profile_reset",
     "nhans_profile_get_layer", "nhans_plan_json",
     "nhans_debug_read_buffer", "nhans_debug_read_batch", "nhans_debug_timeline", "nhans_debug_layer_stats", "nhans_device_info",
+    "nhans_stream_open", "nhans_stream_step", "nhans_stream_close", "nhans_stream_emit_len",
 ]
 
 
@@ -79,5 +80,9 @@ def load():
     lib.nhans_debug_read_batch.argtypes = [vp, i32, vp, i64]
     lib.nhans_debug_timeline.argtypes = [vp, vp, i32]
     lib.nhans_device_info.argtypes = [vp, c.POINTER(i32), c.POINTER(i32), c.POINTER(i32), c.POINTER(i64)]
+    lib.nhans_stream_open.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp]
+    lib.nhans_stream_step.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    lib.nhans_stream_close.argtypes = [vp, i32, vp]
+    lib.nhans_stream_emit_len.argtypes = [i64, i64, i32, c.POINTER(i64)]
     _lib = lib
     return lib

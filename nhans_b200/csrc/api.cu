@@ -12,6 +12,8 @@
 #include <memory>
 #include <string>
 #include <type_traits>
+#include <unordered_map>
+#include <unordered_set>
 #include <vector>
 
 #include "kernels.h"
@@ -105,14 +107,56 @@ struct Geometry {
   long long total_frames = 0, total_out = 0;
 };
 
+// Conditioning of U context pairs (run_conditioning): peaks of int16 clips, the first 200 STFT frames of each clip,
+// their embeddings and the conditioning table [U][n_cols].
+struct CondBufs {
+  DBuf peak_a, peak_b, ctxlm_a, ctxlm_b, emb_a, emb_b, cond;
+  void release() {
+    for (DBuf* d : {&peak_a, &peak_b, &ctxlm_a, &ctxlm_b, &emb_a, &emb_b, &cond}) d->release();
+  }
+};
+
 struct Batch {
   Geometry geo;
   bool has_a = false;
   bool staged = false, done = false;
   IoSlot io[2];
   int cur = 0;                      // set the staged / running batch uses
-  DBuf peak_mix, peak_a, peak_b;
-  DBuf logmag, phase, den, ctxlm_a, ctxlm_b, emb_a, emb_b, cond, mixproc, removed, comp, sums, snr;
+  DBuf peak_mix;
+  CondBufs cb;
+  DBuf logmag, phase, den, mixproc, removed, comp, sums, snr;
+};
+
+// Host side of one open stream (nhans_stream_open).  Its device state is slot `slot` of Streams::pool
+// (kernels.h StreamStepDev): the conditioning row, the last <= 34 frames (log-magnitude and phasors) its next windows
+// read, and its last two denoised frames.
+struct StreamRec {
+  int slot = -1, peak = 0;
+  bool final = false;               // the final step has run: no further chunks
+  long long n = 0;                  // samples received
+  std::vector<int16_t> tail;        // samples from 160 * frames_of(n) on, where the next frame starts
+};
+
+// Every open stream of a context, with device buffers of their own (the batch path's results stay untouched).
+struct Streams {
+  std::unordered_map<int, StreamRec> rec;
+  int next_id = 0;
+  DBuf pool;                        // slots of slot_stride floats
+  int n_slots = 0;
+  long long slot_stride = 0;
+  std::vector<int> free_slots;
+  DBuf ctx_a, ctx_b, ctx_offs;     // nhans_stream_open
+  CondBufs cb;
+  DBuf pcm, desc, new_lm, new_ph, seg_lm, seg_ph, den_win, den_seg, cond, out_i16, out_f32;   // nhans_stream_step
+  void release() {
+    for (DBuf* d : {&pool, &ctx_a, &ctx_b, &ctx_offs, &pcm, &desc, &new_lm, &new_ph, &seg_lm, &seg_ph, &den_win,
+                    &den_seg, &cond, &out_i16, &out_f32})
+      d->release();
+    cb.release();
+    rec.clear();
+    free_slots.clear();
+    n_slots = 0;
+  }
 };
 
 }  // namespace
@@ -132,6 +176,7 @@ struct nhans_ctx {
   DBuf silent_emb;
   bool silent_ready = false;
   Batch batch;
+  Streams streams;
   DBuf tmp[8];
   cudaEvent_t events[16] = {};
   bool profile = false;
@@ -391,7 +436,7 @@ EpiDev make_epi(const NetDev& net, const Epilogue& E, const Grid& out, const flo
 struct PassInfo {                   // which utterances / per-frame table rows a pass of the mask network touches
   const long long* d_frame_offs;
   int u_first, u_last;
-  long long crow0;                  // first table row = first window + 34 * u_first
+  long long crow0;                  // first table row = frame of the first window + 34 * u_first
   int rows;                         // table rows of the pass (<= crow_cap)
 };
 
@@ -508,30 +553,41 @@ int run_tower(nhans_ctx* ctx, const float* ctx_logmag, int R, float* emb) {
   return 0;
 }
 
-// Mask network over all frames (device logmag rows) -> denoised rows.
-int run_masknet(nhans_ctx* ctx, const float* logmag, const long long* d_frame_offs, const long long* h_frame_offs, int U,
-                long long total_frames, const float* cond_table, float* den) {
+// Mask network over windows -> denoised rows den[window].  Segment s stores frames [frame_offs[s], frame_offs[s + 1]) of
+// `logmag` (rows outside read as zero padding) and owns windows [win_offs[s], win_offs[s + 1]), centred on stored frames
+// frame_offs[s] + left[s] + ...  A whole utterance has one window per frame: win_offs = frame_offs and left = null.
+int run_masknet(nhans_ctx* ctx, const float* logmag, const long long* d_frame_offs, const long long* h_frame_offs,
+                const long long* d_win_offs, const long long* h_win_offs, const int* d_left, const int* h_left, int U,
+                const float* cond_table, float* den) {
   NetDev& net = ctx->main_net;
   const int cap = net.plan.capacity;
-  if (total_frames > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one batch");
-  // utterance of a frame: largest u with frame_offs[u] <= frame
-  auto utt_of = [&](long long frame) { return (int)(std::upper_bound(h_frame_offs, h_frame_offs + U + 1, frame) - h_frame_offs) - 1; };
-  for (long long w0 = 0, n = 0; w0 < total_frames; w0 += n) {
+  const long long total_windows = h_win_offs[U];
+  if (h_frame_offs[U] > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one batch");
+  // segment of a window: largest s with win_offs[s] <= window
+  auto seg_of = [&](long long w) { return (int)(std::upper_bound(h_win_offs, h_win_offs + U + 1, w) - h_win_offs) - 1; };
+  // per-frame table row of window row 0 of window w (kernels.h FrameConvDev: stored frame + 34 per earlier segment)
+  auto crow_of = [&](long long w) {
+    const int s = seg_of(w);
+    return h_frame_offs[s] + (h_left ? h_left[s] : 0) + (w - h_win_offs[s]) + 34LL * s;
+  };
+  for (long long w0 = 0, n = 0; w0 < total_windows; w0 += n) {
     PassInfo pi;
     pi.d_frame_offs = d_frame_offs;
-    pi.u_first = utt_of(w0);
-    pi.crow0 = w0 + 34LL * pi.u_first;
-    // the largest pass whose per-frame table rows (its windows + 34 per utterance) fit; one window always does
-    auto rows = [&](long long m) { return m + 34LL * (utt_of(w0 + m - 1) - pi.u_first + 1); };
-    long long lo = 1, hi = std::min<long long>(cap, total_frames - w0);
+    pi.u_first = seg_of(w0);
+    pi.crow0 = crow_of(w0);
+    // the largest pass whose per-frame table rows fit; one window always does.  For whole utterances these are its
+    // windows + 34 per utterance.
+    auto rows = [&](long long m) { return crow_of(w0 + m - 1) + 35 - pi.crow0; };
+    long long lo = 1, hi = std::min<long long>(cap, total_windows - w0);
     while (lo < hi) {
       const long long mid = (lo + hi + 1) / 2;
       if (rows(mid) <= net.crow_cap) lo = mid; else hi = mid - 1;
     }
     n = lo;
-    pi.u_last = utt_of(w0 + n - 1);
+    pi.u_last = seg_of(w0 + n - 1);
     pi.rows = (int)rows(n);
-    CK(launch_units_main(ctx->stream, d_frame_offs, U, (int)w0, (int)n, net.u_frame, net.u_lo, net.u_hi, net.u_utt));
+    CK(launch_units_main(ctx->stream, d_frame_offs, d_win_offs, d_left, U, (int)w0, (int)n, net.u_frame, net.u_lo, net.u_hi,
+                         net.u_utt));
     ctx->launches += 1;
     int rc = run_net(ctx, net, (int)n, logmag, cond_table, den + (size_t)w0 * kBins, &pi);
     if (rc) return rc;
@@ -672,6 +728,57 @@ int stage_batch(nhans_ctx* ctx, IoSlot& io, const Geometry& g, const T* mix, con
   return 0;
 }
 
+// Conditioning rows of U context pairs on the compute stream (a2-a4 of SN/apply.py:359-387 for the first 200 frames
+// of each context, the embedding towers, the conditioning table) -> c.cond [U][n_cols].  a = null: the cached
+// Silent.wav embedding (ensure_silent must have run).
+template <class T>
+int run_conditioning(nhans_ctx* ctx, CondBufs& c, const T* a, const long long* d_a_offs, const T* b, const long long* d_b_offs,
+                     const long long* d_ctx_frame_offs, int U) {
+  constexpr bool pcm = std::is_same<T, int16_t>::value;
+  const size_t cbytes = (size_t)U * kCtxFrames * kBins * 4;
+  const int n_cols = ctx->main_net.plan.cond.n_cols;
+  cudaStream_t st = ctx->stream;
+  CK(c.ctxlm_b.ensure(cbytes));
+  CK(c.emb_b.ensure((size_t)U * 512 * 4));
+  CK(c.cond.ensure((size_t)U * n_cols * 4));
+  if (a) {
+    CK(c.ctxlm_a.ensure(cbytes));
+    CK(c.emb_a.ensure((size_t)U * 512 * 4));
+  }
+  if (pcm) {
+    CK(c.peak_a.ensure(sizeof(int) * U));
+    CK(c.peak_b.ensure(sizeof(int) * U));
+    CK(launch_peaks(st, reinterpret_cast<const int16_t*>(b), d_b_offs, U, c.peak_b.as<int>()));
+    ctx->launches += 1;
+  }
+  {
+    ProfScope ps(ctx, 4, 0, 0);
+    CK(launch_stft_of(st, b, d_b_offs, d_ctx_frame_offs, U, c.peak_b.as<int>(), kCtxFrames, c.ctxlm_b.as<float>(), nullptr, false));
+  }
+  const float* emb_a = ctx->silent_emb.as<float>();
+  int stride_a = 0;
+  int rc;
+  if (a) {
+    if (pcm) {
+      CK(launch_peaks(st, reinterpret_cast<const int16_t*>(a), d_a_offs, U, c.peak_a.as<int>()));
+      ctx->launches += 1;
+    }
+    {
+      ProfScope ps(ctx, 4, 0, 0);
+      CK(launch_stft_of(st, a, d_a_offs, d_ctx_frame_offs, U, c.peak_a.as<int>(), kCtxFrames, c.ctxlm_a.as<float>(), nullptr, false));
+    }
+    // embedding towers: once per distinct context clip (SURVEY.md F6), not once per window
+    if ((rc = run_tower(ctx, c.ctxlm_a.as<float>(), U, c.emb_a.as<float>()))) return rc;
+    emb_a = c.emb_a.as<float>();
+    stride_a = 512;
+  }
+  if ((rc = run_tower(ctx, c.ctxlm_b.as<float>(), U, c.emb_b.as<float>()))) return rc;
+  ProfScope ps(ctx, 4, 0, 0);
+  CK(launch_cond_table(st, emb_a, stride_a, c.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb, ctx->main_net.c,
+                       n_cols, c.cond.as<float>()));
+  return 0;
+}
+
 // The fused path up to the inverse STFT, on the compute stream, for the batch staged in `io` (int16 or float samples):
 // a2-a4 for the mixture and the first 200 frames of each context (SN/apply.py:359-387), the embedding towers, the
 // conditioning table and the mask network.  Leaves batch.logmag / phase / den filled.
@@ -682,26 +789,14 @@ int run_fused(nhans_ctx* ctx, IoSlot& io) {
   const Geometry& g = b.geo;
   const int U = g.U;
   const size_t sbytes = (size_t)g.total_frames * kBins * 4;
-  const size_t cbytes = (size_t)U * kCtxFrames * kBins * 4;
-  const int n_cols = ctx->main_net.plan.cond.n_cols;
   cudaStream_t st = ctx->stream;
   CK(b.peak_mix.ensure(sizeof(int) * U));
   CK(b.logmag.ensure(sbytes + 4));
   CK(b.phase.ensure(2 * sbytes + 8));          // unit phasors (float2 per bin) between the two transforms
   CK(b.den.ensure(sbytes + 4));
-  CK(b.ctxlm_b.ensure(cbytes));
-  CK(b.emb_b.ensure((size_t)U * 512 * 4));
-  CK(b.cond.ensure((size_t)U * n_cols * 4));
-  if (b.has_a) {
-    CK(b.ctxlm_a.ensure(cbytes));
-    CK(b.emb_a.ensure((size_t)U * 512 * 4));
-  }
   if (pcm) {
-    CK(b.peak_a.ensure(sizeof(int) * U));
-    CK(b.peak_b.ensure(sizeof(int) * U));
     CK(launch_peaks(st, io.mix.as<int16_t>(), io.d_mix_offs.as<long long>(), U, b.peak_mix.as<int>()));
-    CK(launch_peaks(st, io.b.as<int16_t>(), io.d_b_offs.as<long long>(), U, b.peak_b.as<int>()));
-    ctx->launches += 2;
+    ctx->launches += 1;
   } else {
     CK(cudaMemsetAsync(b.peak_mix.p, 0, sizeof(int) * U, st));     // the inverse STFT reads it; no int16 output here
   }
@@ -710,37 +805,12 @@ int run_fused(nhans_ctx* ctx, IoSlot& io) {
     CK(launch_stft_of(st, io.mix.as<T>(), io.d_mix_offs.as<long long>(), io.d_frame_offs.as<long long>(), U,
                       b.peak_mix.as<int>(), g.max_frames, b.logmag.as<float>(), b.phase.as<float>(), true));
   }
-  {
-    ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_stft_of(st, io.b.as<T>(), io.d_b_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U,
-                      b.peak_b.as<int>(), kCtxFrames, b.ctxlm_b.as<float>(), nullptr, false));
-  }
-  const float* emb_a = ctx->silent_emb.as<float>();
-  int stride_a = 0;
   int rc;
-  if (b.has_a) {
-    if (pcm) {
-      CK(launch_peaks(st, io.a.as<int16_t>(), io.d_a_offs.as<long long>(), U, b.peak_a.as<int>()));
-      ctx->launches += 1;
-    }
-    {
-      ProfScope ps(ctx, 4, 0, 0);
-      CK(launch_stft_of(st, io.a.as<T>(), io.d_a_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U,
-                        b.peak_a.as<int>(), kCtxFrames, b.ctxlm_a.as<float>(), nullptr, false));
-    }
-    // embedding towers: once per distinct context clip (SURVEY.md F6), not once per window
-    if ((rc = run_tower(ctx, b.ctxlm_a.as<float>(), U, b.emb_a.as<float>()))) return rc;
-    emb_a = b.emb_a.as<float>();
-    stride_a = 512;
-  }
-  if ((rc = run_tower(ctx, b.ctxlm_b.as<float>(), U, b.emb_b.as<float>()))) return rc;
-  {
-    ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_cond_table(st, emb_a, stride_a, b.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb,
-                         ctx->main_net.c, n_cols, b.cond.as<float>()));
-  }
-  return run_masknet(ctx, b.logmag.as<float>(), io.d_frame_offs.as<long long>(), g.frame_offs.data(), U, g.total_frames,
-                     b.cond.as<float>(), b.den.as<float>());
+  if ((rc = run_conditioning(ctx, b.cb, b.has_a ? io.a.as<T>() : nullptr, io.d_a_offs.as<long long>(), io.b.as<T>(),
+                             io.d_b_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U)))
+    return rc;
+  return run_masknet(ctx, b.logmag.as<float>(), io.d_frame_offs.as<long long>(), g.frame_offs.data(), io.d_frame_offs.as<long long>(),
+                     g.frame_offs.data(), nullptr, nullptr, U, b.cb.cond.as<float>(), b.den.as<float>());
 }
 
 // nhans_stft / nhans_stft_f32
@@ -777,6 +847,53 @@ int stft_entry(nhans_ctx* ctx, const T* x, const int64_t* offs, int U, float* lo
   if (peak) CK(cudaMemcpyAsync(peak, ctx->tmp[3].p, sizeof(int) * U, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   return NHANS_OK;
+}
+
+// ---- streaming -----------------------------------------------------------------------------------
+constexpr int kHalfWin = kWinFrames / 2;      // 17: frames a window reaches on either side of its centre
+
+// Windows of a stream that has F frames: all of them after the final step, else those whose 17 right-hand frames
+// exist.  Output hop h needs denoised frames h - 2 .. h, so a stream that has windows [0, b) has emitted hops [0, b),
+// and after its final step the whole (F - 1) * 160 + 400 samples of the batch path.
+long long stream_windows(int F, bool final) { return final ? F : std::max(0, F - kHalfWin); }
+long long stream_emitted(int F, bool final) { return final ? out_len(F) : 160LL * stream_windows(F, false); }
+
+// A slot of the state pool for each of n new streams; the pool grows (keeping its contents) when none is free.
+int alloc_slots(nhans_ctx* ctx, int n, std::vector<int>& slots) {
+  Streams& S = ctx->streams;
+  if ((int)S.free_slots.size() < n) {
+    const int n_cols = ctx->main_net.plan.cond.n_cols;
+    const long long stride = (kSlotCond + n_cols + 3) / 4 * 4;
+    const int want = std::max({S.n_slots * 2, S.n_slots + n - (int)S.free_slots.size(), 16});
+    DBuf grown;
+    CK(grown.ensure((size_t)want * stride * 4));
+    if (S.n_slots) CK(cudaMemcpyAsync(grown.p, S.pool.p, (size_t)S.n_slots * stride * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    S.pool.release();
+    S.pool = grown;
+    S.slot_stride = stride;
+    for (int i = want - 1; i >= S.n_slots; --i) S.free_slots.push_back(i);
+    S.n_slots = want;
+  }
+  slots.resize(n);
+  for (int i = 0; i < n; ++i) {
+    slots[i] = S.free_slots.back();
+    S.free_slots.pop_back();
+  }
+  return 0;
+}
+
+// The streams of a step must be open, distinct and not finalised.
+int check_stream_ids(nhans_ctx* ctx, int n, const int* ids, bool for_step) {
+  std::unordered_set<int> seen;
+  for (int i = 0; i < n; ++i) {
+    auto it = ctx->streams.rec.find(ids[i]);
+    if (it == ctx->streams.rec.end()) return fail(ctx, NHANS_ERR_ARG, "stream id " + std::to_string(ids[i]) + " is not open");
+    if (!seen.insert(ids[i]).second) return fail(ctx, NHANS_ERR_ARG, "stream id " + std::to_string(ids[i]) + " appears twice");
+    if (for_step && it->second.final)
+      return fail(ctx, NHANS_ERR_ARG, "stream id " + std::to_string(ids[i]) + " has had its final step");
+  }
+  return 0;
 }
 
 }  // namespace
@@ -855,10 +972,10 @@ void nhans_destroy(nhans_ctx* ctx) {
       d->release();
     for (cudaEvent_t ev : {io.uploaded, io.consumed, io.drained}) if (ev) cudaEventDestroy(ev);
   }
-  for (DBuf* d : {&b.peak_mix, &b.peak_a, &b.peak_b, &b.logmag, &b.phase, &b.den, &b.ctxlm_a,
-                  &b.ctxlm_b, &b.emb_a, &b.emb_b, &b.cond, &b.mixproc, &b.removed, &b.comp, &b.sums,
-                  &b.snr, &ctx->silent_emb})
+  for (DBuf* d : {&b.peak_mix, &b.logmag, &b.phase, &b.den, &b.mixproc, &b.removed, &b.comp, &b.sums, &b.snr, &ctx->silent_emb})
     d->release();
+  b.cb.release();
+  ctx->streams.release();
   for (auto& t : ctx->tmp) t.release();
   for (auto& ev : ctx->events) if (ev) cudaEventDestroy(ev);
   for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -880,6 +997,7 @@ int nhans_load_weights(nhans_ctx* ctx, const char* const* names, const int64_t* 
   free_net(ctx->main_net);
   free_net(ctx->tower);
   ctx->silent_ready = false;
+  ctx->streams.release();           // their conditioning rows belong to the old weights
   try {
     ctx->main_net.plan = build_main_plan(w, ctx->variant, ctx->win_cap);
     ctx->tower.plan = build_tower_plan(w, ctx->row_cap);
@@ -1004,8 +1122,8 @@ int nhans_masknet(nhans_ctx* ctx, const float* logmag, const int64_t* frame_offs
   CK(cudaMemcpyAsync(ctx->tmp[3].p, emb_b, (size_t)U * 512 * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(launch_cond_table(ctx->stream, ctx->tmp[2].as<float>(), 512, ctx->tmp[3].as<float>(), 512, U, ctx->main_net.Pa,
                        ctx->main_net.Pb, ctx->main_net.c, n_cols, ctx->tmp[4].as<float>()));
-  if ((rc = run_masknet(ctx, ctx->tmp[0].as<float>(), ctx->tmp[5].as<long long>(), fo.data(), U, total, ctx->tmp[4].as<float>(),
-                        ctx->tmp[1].as<float>())))
+  if ((rc = run_masknet(ctx, ctx->tmp[0].as<float>(), ctx->tmp[5].as<long long>(), fo.data(), ctx->tmp[5].as<long long>(), fo.data(),
+                        nullptr, nullptr, U, ctx->tmp[4].as<float>(), ctx->tmp[1].as<float>())))
     return rc;
   CK(cudaMemcpyAsync(denoised, ctx->tmp[1].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
   cudaError_t e = cudaStreamSynchronize(ctx->stream);
@@ -1380,6 +1498,198 @@ int nhans_device_info(nhans_ctx* ctx, int* sm_count, int* cc_major, int* cc_mino
   if (cc_major) *cc_major = prop.major;
   if (cc_minor) *cc_minor = prop.minor;
   if (mem_bytes) *mem_bytes = (int64_t)prop.totalGlobalMem;
+  return NHANS_OK;
+}
+
+int nhans_stream_emit_len(int64_t before, int64_t after, int final, int64_t* emitted) {
+  if (!emitted || before < 0 || after < before) return NHANS_ERR_ARG;
+  *emitted = stream_emitted(frames_of(after), final != 0) - stream_emitted(frames_of(before), false);
+  return NHANS_OK;
+}
+
+int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t* a_offs, const int16_t* ctx_b,
+                      const int64_t* b_offs, const int32_t* peak, int* ids) {
+  if (!ctx || n <= 0 || n > 65535 || !ctx_b || !b_offs || !peak || !ids) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  if (ctx_a && !a_offs) return fail(ctx, NHANS_ERR_ARG, "ctx_a given without offsets");
+  if (!ctx_a && ctx->variant != NHANS_VARIANT_SELECTIVE_NOISE) return fail(ctx, NHANS_ERR_ARG, "the separator needs both context recordings");
+  for (int i = 0; i < n; ++i)
+    if (peak[i] < 0) return fail(ctx, NHANS_ERR_ARG, "stream " + std::to_string(i) + " has a negative peak");
+  CK(cudaSetDevice(ctx->device));
+  int rc;
+  if ((rc = need_weights(ctx))) return rc;
+  // the context clips are laid out like a batch's (a mixture of zero samples per stream)
+  std::vector<int64_t> no_mix(n + 1, 0);
+  Geometry g;
+  if ((rc = batch_geometry(ctx, no_mix.data(), ctx_a ? a_offs : nullptr, b_offs, n, kWholeClips, g))) return rc;
+  Streams& S = ctx->streams;
+  if (!ctx_a && (rc = ensure_silent(ctx))) return rc;
+  cudaStream_t st = ctx->stream;
+  auto clips = [&](DBuf& d, const int16_t* x, const int64_t* offs, long long len) {
+    CK(d.ensure(len * 2 + 32));
+    CK(cudaMemcpyAsync(d.p, x + offs[0], len * 2, cudaMemcpyHostToDevice, st));
+    return 0;
+  };
+  // device offsets: b | a | context frames, n + 1 each
+  std::vector<long long> offs(g.b_offs);
+  offs.insert(offs.end(), g.ctx_frame_offs.begin(), g.ctx_frame_offs.end());
+  if (ctx_a) offs.insert(offs.end(), g.a_offs.begin(), g.a_offs.end());
+  if ((rc = clips(S.ctx_b, ctx_b, b_offs, g.b_offs[n]))) return rc;
+  if (ctx_a && (rc = clips(S.ctx_a, ctx_a, a_offs, g.a_offs[n]))) return rc;
+  if ((rc = to_device_offs(ctx, S.ctx_offs, offs))) return rc;
+  const long long* d_offs = S.ctx_offs.as<long long>();
+  if ((rc = run_conditioning(ctx, S.cb, ctx_a ? S.ctx_a.as<int16_t>() : nullptr, d_offs + 2 * (n + 1), S.ctx_b.as<int16_t>(), d_offs,
+                             d_offs + (n + 1), n)))
+    return rc;
+  std::vector<int> slots;
+  if ((rc = alloc_slots(ctx, n, slots))) return rc;
+  const int n_cols = ctx->main_net.plan.cond.n_cols;
+  for (int i = 0; i < n; ++i)
+    CK(cudaMemcpyAsync(S.pool.as<float>() + slots[i] * S.slot_stride + kSlotCond, S.cb.cond.as<float>() + (size_t)i * n_cols,
+                       (size_t)n_cols * 4, cudaMemcpyDeviceToDevice, st));
+  cudaError_t e = cudaStreamSynchronize(st);
+  if ((rc = check_kernel_flag(ctx))) return rc;
+  CK(e);
+  for (int i = 0; i < n; ++i) {
+    StreamRec r;
+    r.slot = slots[i];
+    r.peak = peak[i];
+    ids[i] = S.next_id++;
+    S.rec.emplace(ids[i], std::move(r));
+  }
+  return NHANS_OK;
+}
+
+int nhans_stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final,
+                      int16_t* out_i16, float* out_f32, int64_t* out_offs) {
+  if (!ctx || n < 0 || n > 65535 || !out_offs || (n > 0 && (!ids || !offs))) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  out_offs[0] = 0;
+  if (n == 0) return NHANS_OK;
+  for (int i = 0; i < n; ++i)
+    if (offs[i + 1] < offs[i]) return fail(ctx, NHANS_ERR_ARG, "chunk offsets must not decrease");
+  if (offs[n] > offs[0] && !pcm) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  int rc;
+  if ((rc = need_weights(ctx))) return rc;
+  if ((rc = check_stream_ids(ctx, n, ids, true))) return rc;
+  CK(cudaSetDevice(ctx->device));
+  Streams& S = ctx->streams;
+  // Geometry of the step (kernels.h StreamStepDev).  Stream i has F0 frames before the step and F1 after it; its windows
+  // [a, b) run now.  It stores frames [cs, F1), cs = a - 17 (or 0): the carry = F0 - cs frames of its slot, then the new
+  // ones.  Its denoised frames a - dc .. b - 1 go through the inverse STFT.
+  std::vector<long long> lo64(6 * (n + 1), 0);           // pcm | new | seg | win | out offsets, staged samples
+  long long *pcm_o = &lo64[0], *new_o = pcm_o + (n + 1), *seg_o = new_o + (n + 1), *win_o = seg_o + (n + 1), *out_o = win_o + (n + 1);
+  std::vector<int> i32(7 * n);
+  int *slot = &i32[0], *carry = slot + n, *left = carry + n, *den_carry = left + n, *keep = den_carry + n, *den_keep = keep + n,
+      *peak = den_keep + n;
+  int max_new = 0, max_rows = 0, max_wins = 0, max_keep = 0;
+  long long max_out = 0;
+  std::vector<int> F1s(n);
+  for (int i = 0; i < n; ++i) {
+    const StreamRec& r = S.rec.at(ids[i]);
+    const bool fin = final && final[i];
+    const long long len = offs[i + 1] - offs[i], N1 = r.n + len;
+    const int F0 = frames_of(r.n), F1 = frames_of(N1);
+    const long long a = stream_windows(F0, false), b = std::max(a, stream_windows(F1, fin));
+    const long long cs = std::max(0LL, a - kHalfWin);
+    slot[i] = r.slot;
+    peak[i] = r.peak;
+    carry[i] = (int)(F0 - cs);
+    left[i] = (int)(a - cs);
+    den_carry[i] = (int)std::min(a, 2LL);
+    keep[i] = (int)(std::max(0LL, b - kHalfWin) - cs);
+    den_keep[i] = (int)std::min(b, 2LL);
+    F1s[i] = F1;
+    pcm_o[i + 1] = pcm_o[i] + (long long)r.tail.size() + len;
+    new_o[i + 1] = new_o[i] + (F1 - F0);
+    seg_o[i + 1] = seg_o[i] + (F1 - cs);
+    win_o[i + 1] = win_o[i] + (b - a);
+    out_o[i + 1] = out_o[i] + stream_emitted(F1, fin) - stream_emitted(F0, false);
+    max_new = std::max(max_new, F1 - F0);
+    max_rows = std::max<long long>(max_rows, F1 - cs);
+    max_wins = std::max<long long>(max_wins, b - a);
+    max_keep = std::max<long long>(max_keep, F1 - cs - keep[i]);
+    max_out = std::max(max_out, out_o[i + 1] - out_o[i]);
+  }
+  const int n_cols = ctx->main_net.plan.cond.n_cols;
+  const long long n_new = new_o[n], n_seg = seg_o[n], n_win = win_o[n], n_out = out_o[n];
+  if (n_seg > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one step");
+  // staging: each stream's unframed tail, then its chunk
+  std::vector<int16_t> staged((size_t)pcm_o[n]);
+  for (int i = 0; i < n; ++i) {
+    const StreamRec& r = S.rec.at(ids[i]);
+    std::copy(r.tail.begin(), r.tail.end(), staged.begin() + pcm_o[i]);
+    if (offs[i + 1] > offs[i]) std::copy(pcm + offs[i], pcm + offs[i + 1], staged.begin() + pcm_o[i] + r.tail.size());
+  }
+  cudaStream_t st = ctx->stream;
+  const size_t desc64 = lo64.size() * 8;
+  CK(S.pcm.ensure(staged.size() * 2 + 32));
+  CK(S.desc.ensure(desc64 + i32.size() * 4));
+  CK(S.new_lm.ensure((size_t)n_new * kBins * 4 + 4));
+  CK(S.new_ph.ensure((size_t)n_new * kBins * 8 + 8));
+  CK(S.seg_lm.ensure((size_t)n_seg * kBins * 4 + 4));
+  CK(S.seg_ph.ensure((size_t)n_seg * kBins * 8 + 8));
+  CK(S.den_seg.ensure((size_t)n_seg * kBins * 4 + 4));
+  CK(S.den_win.ensure((size_t)n_win * kBins * 4 + 4));
+  CK(S.cond.ensure((size_t)n * n_cols * 4));
+  CK(S.out_f32.ensure((size_t)n_out * 4 + 16));
+  CK(S.out_i16.ensure((size_t)n_out * 2 + 16));
+  if (!staged.empty()) CK(cudaMemcpyAsync(S.pcm.p, staged.data(), staged.size() * 2, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(S.desc.p, lo64.data(), desc64, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(S.desc.as<char>() + desc64, i32.data(), i32.size() * 4, cudaMemcpyHostToDevice, st));
+  const long long* d64 = S.desc.as<long long>();
+  const int* d32 = reinterpret_cast<const int*>(S.desc.as<char>() + desc64);
+  StreamStepDev p;
+  p.n = n;
+  p.seg_offs = d64 + 2 * (n + 1); p.new_offs = d64 + (n + 1); p.win_offs = d64 + 3 * (n + 1); p.out_offs = d64 + 4 * (n + 1);
+  p.slot = d32; p.carry = d32 + n; p.left = d32 + 2 * n; p.den_carry = d32 + 3 * n; p.keep = d32 + 4 * n; p.den_keep = d32 + 5 * n;
+  p.peak = d32 + 6 * n;
+  p.pool = S.pool.as<float>(); p.slot_stride = S.slot_stride; p.n_cols = n_cols;
+  p.new_lm = S.new_lm.as<float>(); p.new_ph = S.new_ph.as<float>(); p.den_win = S.den_win.as<float>();
+  p.seg_lm = S.seg_lm.as<float>(); p.seg_ph = S.seg_ph.as<float>(); p.den_seg = S.den_seg.as<float>(); p.cond = S.cond.as<float>();
+  {
+    ProfScope ps(ctx, 1, 0, 2.0 * pcm_o[n] + 12.0 * n_new * kBins);
+    CK(launch_stft(st, S.pcm.as<int16_t>(), d64, p.new_offs, n, p.peak, max_new, S.new_lm.as<float>(), S.new_ph.as<float>(), true));
+  }
+  CK(launch_stream_assemble(st, p, max_rows));
+  ctx->launches += 1;
+  if (n_win > 0) {
+    // (no pass when no window became computable)
+    if ((rc = run_masknet(ctx, p.seg_lm, p.seg_offs, seg_o, p.win_offs, win_o, p.left, left, n, p.cond, S.den_win.as<float>()))) return rc;
+    CK(launch_stream_den(st, p, max_wins));
+    ctx->launches += 1;
+  }
+  if (out_f32 || out_i16) {
+    ProfScope ps(ctx, 2, 0, 12.0 * n_win * kBins + 6.0 * n_out);
+    CK(launch_istft_stream(st, p, (int)max_out, out_f32 ? S.out_f32.as<float>() : nullptr, out_i16 ? S.out_i16.as<int16_t>() : nullptr));
+  }
+  CK(launch_stream_save(st, p, max_keep));
+  ctx->launches += 1;
+  if (out_f32 && n_out) CK(cudaMemcpyAsync(out_f32, S.out_f32.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+  if (out_i16 && n_out) CK(cudaMemcpyAsync(out_i16, S.out_i16.p, n_out * 2, cudaMemcpyDeviceToHost, st));
+  cudaError_t e = cudaStreamSynchronize(st);
+  if ((rc = check_kernel_flag(ctx))) return rc;
+  CK(e);
+  for (int i = 0; i < n; ++i) {
+    StreamRec& r = S.rec.at(ids[i]);
+    const long long F0 = frames_of(r.n);
+    // the next frame starts at sample 160 F1: keep the staged samples from there on
+    const long long from = 160LL * (F1s[i] - F0);
+    r.tail.assign(staged.begin() + pcm_o[i] + from, staged.begin() + pcm_o[i + 1]);
+    r.n += offs[i + 1] - offs[i];
+    r.final = final && final[i];
+    out_offs[i + 1] = out_o[i + 1];
+  }
+  return NHANS_OK;
+}
+
+int nhans_stream_close(nhans_ctx* ctx, int n, const int* ids) {
+  if (!ctx || n < 0 || (n > 0 && !ids)) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  int rc;
+  if ((rc = check_stream_ids(ctx, n, ids, false))) return rc;
+  Streams& S = ctx->streams;
+  for (int i = 0; i < n; ++i) {
+    S.free_slots.push_back(S.rec.at(ids[i]).slot);
+    S.rec.erase(ids[i]);
+  }
   return NHANS_OK;
 }
 

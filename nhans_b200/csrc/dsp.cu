@@ -376,6 +376,37 @@ istft_kernel(const float* __restrict__ logmag, const float* __restrict__ phase, 
   }
 }
 
+// The same inverse STFT over the segments of a stream step (kernels.h StreamStepDev): local frame 0 of stream s is
+// the first carried denoised frame (den_carry of them precede its windows), frames outside [0, T) are zero as at an
+// utterance edge, and local samples [lo, lo + len) with lo = 160 den_carry go to out_offs[s].  Every sample is the same
+// gather and sum as in istft_kernel, so a stream's samples are bit-identical to the whole clip's.
+// grid: (ceil((max len + 159) / 160 / kOH), n).
+__global__ void __launch_bounds__(kThreads, 4)
+istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t* __restrict__ out_i16) {
+  __shared__ __align__(16) float s_y[kNFI * kWin];
+  const int u = blockIdx.y;
+  const int dc = p.den_carry[u];
+  const int T = dc + (int)(p.win_offs[u + 1] - p.win_offs[u]);
+  const long long len = p.out_offs[u + 1] - p.out_offs[u];
+  const int h0 = dc + blockIdx.x * kOH;   // first output hop (local)
+  if (T <= 0 || (long long)blockIdx.x * kOH * kHop >= len) return;
+  istft_frames<true>(s_y, p.den_seg, p.seg_ph, p.seg_offs[u] + p.left[u] - dc, T, h0 - 2);
+  const long long lo = (long long)dc * kHop;
+  const float scale = (float)((double)p.peak[u] + 0.000001);
+  for (int i = threadIdx.x * 4; i < kOH * kHop; i += blockDim.x * 4) {
+    const long long n = (long long)h0 * kHop + i - lo;
+    if (n >= len) break;
+    const float4 acc = ola_sample4(s_y, i);
+    const long long o = p.out_offs[u] + n;
+    if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = acc;
+    if (out_i16) {
+      short4 q;
+      q.x = to_i16(acc.x * scale); q.y = to_i16(acc.y * scale); q.z = to_i16(acc.z * scale); q.w = to_i16(acc.w * scale);
+      *reinterpret_cast<short4*>(out_i16 + o) = q;
+    }
+  }
+}
+
 // Post-mix outputs of apply_snc (SN/apply.py:456-464) fused into one pass: both inverse STFTs (denoised
 // spectrum and the input spectrum = 'mixed_processed'), removed = mixed_processed - denoised, and the two
 // per-clip energy sums of snr_est = mean(denoised^2) / mean(removed^2).
@@ -533,6 +564,13 @@ cudaError_t launch_istft(cudaStream_t s, const float* logmag, const float* phase
   dim3 grid((max_frames_per_clip + 2 + kOH - 1) / kOH, U);
   if (phasor) istft_kernel<true><<<grid, kThreads, 0, s>>>(logmag, phase, frame_offs, out_offs, peak, out_f32, out_i16);
   else istft_kernel<false><<<grid, kThreads, 0, s>>>(logmag, phase, frame_offs, out_offs, peak, out_f32, out_i16);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_istft_stream(cudaStream_t s, const StreamStepDev& p, int max_samples, float* out_f32, int16_t* out_i16) {
+  if (p.n <= 0 || max_samples <= 0) return cudaSuccess;
+  dim3 grid((max_samples + kOH * kHop - 1) / (kOH * kHop), p.n);
+  istft_stream_kernel<<<grid, kThreads, 0, s>>>(p, out_f32, out_i16);
   return cudaGetLastError();
 }
 

@@ -154,8 +154,10 @@ cudaError_t launch_mean_pool(cudaStream_t s, const __half* act, int units, int p
 // out[n][c] = (sum_s scratch[s][n][c]) * scale[c] + bias[c] + raw[frame[n]][c], c < 201 (head of main.py:238-242)
 cudaError_t launch_head_reduce(cudaStream_t s, const float* scratch, int ksplit, int units, int N, const float* scale, const float* bias,
                                const float* raw, const int* frame, float* out);
-cudaError_t launch_units_main(cudaStream_t s, const long long* frame_offs, int U, int w0, int nwin, int* frame, int* lo,
-                              int* hi, int* utt);
+// windows [w0, w0 + nwin) of segments with window offsets win_offs [U + 1]; window g of segment s is centred on stored
+// frame frame_offs[s] + left[s] + (g - win_offs[s]) (left = null: 0, one window per stored frame)
+cudaError_t launch_units_main(cudaStream_t s, const long long* frame_offs, const long long* win_offs, const int* left, int U, int w0,
+                              int nwin, int* frame, int* lo, int* hi, int* utt);
 cudaError_t launch_units_rows(cudaStream_t s, int r0, int n, int rows_per_unit, int* frame, int* lo, int* hi, int* utt);
 
 // ---- DSP ----
@@ -182,5 +184,35 @@ cudaError_t launch_istft_post(cudaStream_t s, const float* den_logmag, const flo
 cudaError_t launch_compensate(cudaStream_t s, const float* den, const float* removed, const long long* out_offs, int U,
                               const double* sums, float compensate, int ac, float* out, float* snr_est);
 cudaError_t dsp_init_tables();
+
+// ---- streaming (api.cu nhans_stream_step) ----
+// One step over n streams.  Stream s stores frames [cs, F) of its recording in the step's segment, rows
+// seg_offs[s] .. seg_offs[s + 1] of seg_lm (log-magnitude, [201]) / seg_ph (unit phasors, [201] float2): the first
+// carry[s] rows come from its state slot, the others are its new frames (rows new_offs[s] .. new_offs[s + 1] of the
+// STFT output).  Its windows are centred on segment rows left[s] .. left[s] + n_win - 1 (global windows win_offs[s] ..).
+// den_seg has the layout of seg_lm: the denoised frames of the windows, preceded by den_carry[s] frames of the previous
+// step; the inverse STFT runs over those rows and emits samples [160 den_carry, 160 den_carry + out_offs[s + 1] - out_offs[s])
+// of their overlap-add.  The slot then keeps segment rows [keep[s], T) and the last den_keep[s] denoised frames.
+constexpr int kStreamCarry = 34;      // stored frames a stream carries between steps (2 x 17 window half)
+struct StreamStepDev {
+  int n;
+  const long long *seg_offs, *new_offs, *win_offs, *out_offs;   // [n + 1]
+  const int *slot, *carry, *left, *den_carry, *keep, *den_keep, *peak;   // [n]
+  // state pool: slot i at pool + i * slot_stride floats = lm [34][201] | ph [34][201][2] | den [2][201] | cond [n_cols]
+  float* pool;
+  long long slot_stride;
+  int n_cols;
+  const float *new_lm, *new_ph, *den_win;
+  float *seg_lm, *seg_ph, *den_seg, *cond;
+};
+constexpr long long kSlotPh = (long long)kStreamCarry * 201, kSlotDen = 3LL * kStreamCarry * 201, kSlotCond = kSlotDen + 2 * 201;
+// segment rows (carried + new), the carried denoised rows and the conditioning rows [n][n_cols] of the step
+cudaError_t launch_stream_assemble(cudaStream_t s, const StreamStepDev& p, int max_rows);
+// denoised rows of the windows (den_win, one per window) -> den_seg
+cudaError_t launch_stream_den(cudaStream_t s, const StreamStepDev& p, int max_wins);
+// inverse STFT of the emitted samples -> out_f32 / out_i16 (either may be null) at out_offs
+cudaError_t launch_istft_stream(cudaStream_t s, const StreamStepDev& p, int max_samples, float* out_f32, int16_t* out_i16);
+// slot state for the next step
+cudaError_t launch_stream_save(cudaStream_t s, const StreamStepDev& p, int max_rows);
 
 }  // namespace nhans

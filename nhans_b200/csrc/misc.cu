@@ -295,19 +295,20 @@ __global__ void head_reduce_kernel(const float* __restrict__ scratch, int ksplit
   }
 }
 
-// Window n of the chunk is global frame w0 + n (one window per STFT frame, SN/apply.py:378); its clip is
-// found by binary search in frame_offs.
-__global__ void units_main_kernel(const long long* __restrict__ frame_offs, int U, int w0, int nwin, int* frame, int* lo,
-                                  int* hi, int* utt) {
+// Window n of the chunk is global window g = w0 + n; its segment is found by binary search in win_offs, and its
+// centre is stored frame frame_offs[s] + left[s] + (g - win_offs[s]) (left = null: 0).  A whole utterance is a segment
+// with one window per stored frame (SN/apply.py:378); a stream segment also stores context frames without windows.
+__global__ void units_main_kernel(const long long* __restrict__ frame_offs, const long long* __restrict__ win_offs,
+                                  const int* __restrict__ left, int U, int w0, int nwin, int* frame, int* lo, int* hi, int* utt) {
   const int n = blockIdx.x * blockDim.x + threadIdx.x;
   if (n >= nwin) return;
   const long long g = (long long)w0 + n;
-  int a = 0, b = U;                                     // frame_offs[a] <= g < frame_offs[b]
+  int a = 0, b = U;                                     // win_offs[a] <= g < win_offs[b]
   while (b - a > 1) {
     const int mid = (a + b) >> 1;
-    if (frame_offs[mid] <= g) a = mid; else b = mid;
+    if (win_offs[mid] <= g) a = mid; else b = mid;
   }
-  frame[n] = (int)g;
+  frame[n] = (int)(frame_offs[a] + (left ? left[a] : 0) + (g - win_offs[a]));
   lo[n] = (int)frame_offs[a];
   hi[n] = (int)frame_offs[a + 1];
   utt[n] = a;
@@ -370,10 +371,10 @@ cudaError_t launch_head_reduce(cudaStream_t s, const float* scratch, int ksplit,
   return cudaGetLastError();
 }
 
-cudaError_t launch_units_main(cudaStream_t s, const long long* frame_offs, int U, int w0, int nwin, int* frame, int* lo,
-                              int* hi, int* utt) {
+cudaError_t launch_units_main(cudaStream_t s, const long long* frame_offs, const long long* win_offs, const int* left, int U, int w0,
+                              int nwin, int* frame, int* lo, int* hi, int* utt) {
   if (nwin <= 0) return cudaSuccess;
-  units_main_kernel<<<(nwin + 255) / 256, 256, 0, s>>>(frame_offs, U, w0, nwin, frame, lo, hi, utt);
+  units_main_kernel<<<(nwin + 255) / 256, 256, 0, s>>>(frame_offs, win_offs, left, U, w0, nwin, frame, lo, hi, utt);
   return cudaGetLastError();
 }
 

@@ -14,6 +14,7 @@ from . import _lib, weights as W
 N_BINS = 201
 CTX_FRAMES = 200
 KIND_GEMM, KIND_STFT, KIND_ISTFT, KIND_DIRECT, KIND_OTHER = range(5)
+STREAM_EMIT_SLACK = 17 * 160 + 400
 
 
 class NhansError(RuntimeError):
@@ -321,6 +322,40 @@ class Engine:
         self.sync()
         return {"mixed_processed": unpack(mixed, out_offs), "removed": unpack(removed, out_offs),
                 "compensated": unpack(comp, out_offs), "snr_est": snr}
+
+    # ---- streaming --------------------------------------------------------------------------------
+    def stream_open(self, ctx_a_clips, ctx_b_clips, peaks):
+        """Open one live int16 stream per context pair (ctx_a_clips may be None: Silent.wav).  peaks: the int16 peak each
+        stream is scaled by (the whole clip's nhans_stft peak reproduces the batch path exactly, 32767 is full scale).
+        -> list of stream ids"""
+        n = len(ctx_b_clips)
+        b, bo = pack(ctx_b_clips)
+        a, ao = pack(ctx_a_clips) if ctx_a_clips is not None else (None, None)
+        pk = np.ascontiguousarray(peaks, np.int32)
+        ids = np.zeros(n, np.int32)
+        self._ck(self.lib.nhans_stream_open(self.h, n, _ptr(a), _ptr(ao), _ptr(b), _ptr(bo), _ptr(pk), _ptr(ids)))
+        return [int(i) for i in ids]
+
+    def stream_step(self, ids, chunks, final=None, want_f32=True, want_i16=True):
+        """Append chunks[i] (int16) to stream ids[i] and run every window that became computable; final[i] flushes
+        stream i.  -> {"i16": [...], "f32": [...]}: the samples each stream emitted in this step."""
+        n = len(ids)
+        pcm, offs = pack(chunks)
+        ids_a = np.ascontiguousarray(ids, np.int32)
+        fin = np.ascontiguousarray(final, np.int32) if final is not None else None
+        # a step emits fewer than len(chunk) + 17 * 160 + 400 samples per stream (the frames it held back, plus the last
+        # frame's tail at the final step)
+        cap = int(offs[-1]) + STREAM_EMIT_SLACK * n
+        oo = np.zeros(n + 1, np.int64)
+        o16 = np.empty(cap, np.int16) if want_i16 else None
+        o32 = np.empty(cap, np.float32) if want_f32 else None
+        self._ck(self.lib.nhans_stream_step(self.h, n, _ptr(ids_a), _ptr(pcm), _ptr(offs), _ptr(fin), _ptr(o16), _ptr(o32), _ptr(oo)))
+        return {"i16": [np.array(v) for v in unpack(o16, oo)] if want_i16 else None,
+                "f32": [np.array(v) for v in unpack(o32, oo)] if want_f32 else None}
+
+    def stream_close(self, ids):
+        ids_a = np.ascontiguousarray(ids, np.int32)
+        self._ck(self.lib.nhans_stream_close(self.h, len(ids_a), _ptr(ids_a)))
 
     def upload(self, mix, mix_offs, ctx_a, a_offs, ctx_b, b_offs):
         self._ck(self.lib.nhans_upload(self.h, _ptr(mix), _ptr(mix_offs), len(mix_offs) - 1, _ptr(ctx_a), _ptr(a_offs),
