@@ -125,7 +125,9 @@ int nhans_download(nhans_ctx* ctx, int16_t* out_i16, float* out_f32, float* mixp
 /* Post-mix outputs of apply_snc for the batch nhans_run just processed (SN/apply.py:456-472), computed on the GPU
  * in one fused pass: mixed_processed = iSTFT(input spectrum), removed = mixed_processed - denoised,
  * snr_est[u] = mean(denoised^2) / mean(removed^2), compensated = denoised + removed * (ac ? snr_est / 20 : compensate).
- * Any output may be NULL; copies are enqueued on the context stream (nhans_sync). */
+ * A clip without frames (fewer than 400 samples), or whose removed signal is all zero, has snr_est = +inf; the --ac factor
+ * is then 0, and a clip without frames has empty outputs.  Any output may be NULL; copies are enqueued on the context
+ * stream (nhans_sync). */
 int nhans_postmix(nhans_ctx* ctx, float compensate, int ac, float* mixed_f32, float* removed_f32, float* compensated_f32,
                   float* snr_est);
 

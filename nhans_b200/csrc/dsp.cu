@@ -577,9 +577,10 @@ cudaError_t launch_istft_stream(cudaStream_t s, const StreamStepDev& p, int max_
 cudaError_t launch_istft_post(cudaStream_t s, const float* den_logmag, const float* mix_logmag, const float* phase,
                               const long long* frame_offs, const long long* out_offs, int U, int max_frames_per_clip,
                               float* den_f32, float* mixed_f32, float* removed_f32, double* sums, bool phasor) {
-  if (U <= 0 || max_frames_per_clip <= 0) return cudaSuccess;
+  if (U <= 0) return cudaSuccess;
+  // zeroed even when no clip has a frame: compensate_kernel reads the sums of every clip
   cudaError_t e = cudaMemsetAsync(sums, 0, sizeof(double) * 2 * U, s);
-  if (e != cudaSuccess) return e;
+  if (e != cudaSuccess || max_frames_per_clip <= 0) return e;
   dim3 grid((max_frames_per_clip + 2 + kOH - 1) / kOH, U);
   if (phasor)
     istft_post_kernel<true><<<grid, kThreads, 0, s>>>(den_logmag, mix_logmag, phase, frame_offs, out_offs, den_f32, mixed_f32, removed_f32, sums);
