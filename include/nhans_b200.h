@@ -139,7 +139,8 @@ int nhans_postmix(nhans_ctx* ctx, float compensate, int ac, float* mixed_f32, fl
  * N < 400), it has emitted 160 * max(0, F - 17) samples; after its final step it has emitted (F - 1) * 160 + 400 (0 when
  * F = 0), what the batch path returns for the clip (trailing samples that fill no frame are dropped).  A window needs
  * the 17 frames after its centre and a 400-sample frame, so the algorithmic latency is 16 * 160 + 400 = 2960 samples
- * (185 ms at 16 kHz), plus up to 159 samples waiting for the next hop boundary.
+ * (185 ms at 16 kHz), plus up to 159 samples waiting for the next hop boundary.  nhans_stream_step_post also streams
+ * the post-mix outputs of nhans_postmix (ac = 0), bit for bit, with a running snr_est.
  * nhans_load_weights closes every open stream.  Without loaded weights the calls below return NHANS_ERR_STATE. */
 
 /* Opens n streams (one tower pass for all of them).  Stream i is conditioned on ctx_b[b_offs[i] : b_offs[i+1]] and
@@ -158,6 +159,17 @@ int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t
  * batch in flight (nhans_upload / nhans_run / nhans_download / nhans_postmix) untouched. */
 int nhans_stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final,
                       int16_t* out_i16, float* out_f32, int64_t* out_offs);
+/* nhans_stream_step plus the post-mix outputs of nhans_postmix (SN/apply.py:456-470) for the same samples: the same
+ * arguments, checks, emission rule and out_offs, and mixed_f32 ('mixed_processed'), removed_f32 and compensated_f32 =
+ * denoised + removed * compensate[i], each bit-identical to nhans_postmix(compensate[i], ac = 0) of the whole clip.
+ * compensate [n] holds one factor per stream (NULL: 0; a non-finite factor counts as 0).  Every output array may be NULL.
+ * snr_est [n] (may be NULL) receives each stream's running estimate: sum(denoised^2) / sum(removed^2) in float64 over every
+ * sample the stream has emitted through nhans_stream_step_post (samples of plain nhans_stream_step calls do not count),
+ * +inf while that removed energy is 0 (no sample yet, or a clip of fewer than 400 samples).  --ac has no streaming form: its
+ * factor is the whole clip's snr_est, which only nhans_postmix knows.  Synchronous; leaves a batch in flight untouched. */
+int nhans_stream_step_post(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final,
+                           const float* compensate, int16_t* out_i16, float* out_f32, float* mixed_f32, float* removed_f32,
+                           float* compensated_f32, int64_t* out_offs, float* snr_est);
 /* Releases n streams, finalised or not. */
 int nhans_stream_close(nhans_ctx* ctx, int n, const int* ids);
 /* Host only (no context, no GPU): samples one step emits for a stream that goes from `before` to `after` samples

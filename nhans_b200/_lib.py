@@ -18,7 +18,7 @@ SYMBOLS = [
     "nhans_event_elapsed_ms", "nhans_profile_enable", "nhans_profile_get", "nhans_profile_reset",
     "nhans_profile_get_layer", "nhans_plan_json",
     "nhans_debug_read_buffer", "nhans_debug_read_batch", "nhans_debug_timeline", "nhans_debug_layer_stats", "nhans_device_info",
-    "nhans_stream_open", "nhans_stream_step", "nhans_stream_close", "nhans_stream_emit_len",
+    "nhans_stream_open", "nhans_stream_step", "nhans_stream_step_post", "nhans_stream_close", "nhans_stream_emit_len",
 ]
 
 
@@ -82,6 +82,7 @@ def load():
     lib.nhans_device_info.argtypes = [vp, c.POINTER(i32), c.POINTER(i32), c.POINTER(i32), c.POINTER(i64)]
     lib.nhans_stream_open.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp]
     lib.nhans_stream_step.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    lib.nhans_stream_step_post.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.nhans_stream_close.argtypes = [vp, i32, vp]
     lib.nhans_stream_emit_len.argtypes = [i64, i64, i32, c.POINTER(i64)]
     _lib = lib

@@ -6,6 +6,7 @@
 
 #include <algorithm>
 #include <array>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -135,6 +136,7 @@ struct StreamRec {
   bool final = false;               // the final step has run: no further chunks
   long long n = 0;                  // samples received
   std::vector<int16_t> tail;        // samples from 160 * frames_of(n) on, where the next frame starts
+  double e_den = 0, e_rem = 0;      // sum den^2, sum removed^2 of the samples emitted by nhans_stream_step_post
 };
 
 // Every open stream of a context, with device buffers of their own (the batch path's results stay untouched).
@@ -148,9 +150,10 @@ struct Streams {
   DBuf ctx_a, ctx_b, ctx_offs;     // nhans_stream_open
   CondBufs cb;
   DBuf pcm, desc, new_lm, new_ph, seg_lm, seg_ph, den_win, den_seg, cond, out_i16, out_f32;   // nhans_stream_step
+  DBuf factor, mixed, removed, comp, sums;                                                   // nhans_stream_step_post
   void release() {
     for (DBuf* d : {&pool, &ctx_a, &ctx_b, &ctx_offs, &pcm, &desc, &new_lm, &new_ph, &seg_lm, &seg_ph, &den_win,
-                    &den_seg, &cond, &out_i16, &out_f32})
+                    &den_seg, &cond, &out_i16, &out_f32, &factor, &mixed, &removed, &comp, &sums})
       d->release();
     cb.release();
     rec.clear();
@@ -896,6 +899,168 @@ int check_stream_ids(nhans_ctx* ctx, int n, const int* ids, bool for_step) {
   return 0;
 }
 
+// The post-mix outputs of nhans_stream_step_post (null: a plain step).
+struct PostOut {
+  const float* compensate;          // [n] or null (0)
+  float *mixed, *removed, *comp, *snr_est;
+};
+
+// nhans_stream_step and, with `post`, nhans_stream_step_post.
+int stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final, int16_t* out_i16,
+                float* out_f32, int64_t* out_offs, const PostOut* post) {
+  if (!ctx || n < 0 || n > 65535 || !out_offs || (n > 0 && (!ids || !offs))) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  out_offs[0] = 0;
+  if (n == 0) return NHANS_OK;
+  for (int i = 0; i < n; ++i)
+    if (offs[i + 1] < offs[i]) return fail(ctx, NHANS_ERR_ARG, "chunk offsets must not decrease");
+  if (offs[n] > offs[0] && !pcm) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
+  int rc;
+  if ((rc = need_weights(ctx))) return rc;
+  if ((rc = check_stream_ids(ctx, n, ids, true))) return rc;
+  CK(cudaSetDevice(ctx->device));
+  Streams& S = ctx->streams;
+  // Geometry of the step (kernels.h StreamStepDev).  Stream i has F0 frames before the step and F1 after it; its windows
+  // [a, b) run now.  It stores frames [cs, F1), cs = a - 17 (or 0): the carry = F0 - cs frames of its slot, then the new
+  // ones.  Its denoised frames a - dc .. b - 1 go through the inverse STFT.
+  std::vector<long long> lo64(6 * (n + 1), 0);           // pcm | new | seg | win | out offsets, staged samples
+  long long *pcm_o = &lo64[0], *new_o = pcm_o + (n + 1), *seg_o = new_o + (n + 1), *win_o = seg_o + (n + 1), *out_o = win_o + (n + 1);
+  std::vector<int> i32(7 * n);
+  int *slot = &i32[0], *carry = slot + n, *left = carry + n, *den_carry = left + n, *keep = den_carry + n, *den_keep = keep + n,
+      *peak = den_keep + n;
+  int max_new = 0, max_rows = 0, max_wins = 0, max_keep = 0;
+  long long max_out = 0;
+  std::vector<int> F1s(n);
+  for (int i = 0; i < n; ++i) {
+    const StreamRec& r = S.rec.at(ids[i]);
+    const bool fin = final && final[i];
+    const long long len = offs[i + 1] - offs[i], N1 = r.n + len;
+    const int F0 = frames_of(r.n), F1 = frames_of(N1);
+    const long long a = stream_windows(F0, false), b = std::max(a, stream_windows(F1, fin));
+    const long long cs = std::max(0LL, a - kHalfWin);
+    slot[i] = r.slot;
+    peak[i] = r.peak;
+    carry[i] = (int)(F0 - cs);
+    left[i] = (int)(a - cs);
+    den_carry[i] = (int)std::min(a, 2LL);
+    keep[i] = (int)(std::max(0LL, b - kHalfWin) - cs);
+    den_keep[i] = (int)std::min(b, 2LL);
+    F1s[i] = F1;
+    pcm_o[i + 1] = pcm_o[i] + (long long)r.tail.size() + len;
+    new_o[i + 1] = new_o[i] + (F1 - F0);
+    seg_o[i + 1] = seg_o[i] + (F1 - cs);
+    win_o[i + 1] = win_o[i] + (b - a);
+    out_o[i + 1] = out_o[i] + stream_emitted(F1, fin) - stream_emitted(F0, false);
+    max_new = std::max(max_new, F1 - F0);
+    max_rows = std::max<long long>(max_rows, F1 - cs);
+    max_wins = std::max<long long>(max_wins, b - a);
+    max_keep = std::max<long long>(max_keep, F1 - cs - keep[i]);
+    max_out = std::max(max_out, out_o[i + 1] - out_o[i]);
+  }
+  const int n_cols = ctx->main_net.plan.cond.n_cols;
+  const long long n_new = new_o[n], n_seg = seg_o[n], n_win = win_o[n], n_out = out_o[n];
+  if (n_seg > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one step");
+  // staging: each stream's unframed tail, then its chunk
+  std::vector<int16_t> staged((size_t)pcm_o[n]);
+  for (int i = 0; i < n; ++i) {
+    const StreamRec& r = S.rec.at(ids[i]);
+    std::copy(r.tail.begin(), r.tail.end(), staged.begin() + pcm_o[i]);
+    if (offs[i + 1] > offs[i]) std::copy(pcm + offs[i], pcm + offs[i + 1], staged.begin() + pcm_o[i] + r.tail.size());
+  }
+  cudaStream_t st = ctx->stream;
+  const size_t desc64 = lo64.size() * 8;
+  CK(S.pcm.ensure(staged.size() * 2 + 32));
+  CK(S.desc.ensure(desc64 + i32.size() * 4));
+  CK(S.new_lm.ensure((size_t)n_new * kBins * 4 + 4));
+  CK(S.new_ph.ensure((size_t)n_new * kBins * 8 + 8));
+  CK(S.seg_lm.ensure((size_t)n_seg * kBins * 4 + 4));
+  CK(S.seg_ph.ensure((size_t)n_seg * kBins * 8 + 8));
+  CK(S.den_seg.ensure((size_t)n_seg * kBins * 4 + 4));
+  CK(S.den_win.ensure((size_t)n_win * kBins * 4 + 4));
+  CK(S.cond.ensure((size_t)n * n_cols * 4));
+  CK(S.out_f32.ensure((size_t)n_out * 4 + 16));
+  CK(S.out_i16.ensure((size_t)n_out * 2 + 16));
+  if (!staged.empty()) CK(cudaMemcpyAsync(S.pcm.p, staged.data(), staged.size() * 2, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(S.desc.p, lo64.data(), desc64, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(S.desc.as<char>() + desc64, i32.data(), i32.size() * 4, cudaMemcpyHostToDevice, st));
+  const long long* d64 = S.desc.as<long long>();
+  const int* d32 = reinterpret_cast<const int*>(S.desc.as<char>() + desc64);
+  StreamStepDev p;
+  p.n = n;
+  p.seg_offs = d64 + 2 * (n + 1); p.new_offs = d64 + (n + 1); p.win_offs = d64 + 3 * (n + 1); p.out_offs = d64 + 4 * (n + 1);
+  p.slot = d32; p.carry = d32 + n; p.left = d32 + 2 * n; p.den_carry = d32 + 3 * n; p.keep = d32 + 4 * n; p.den_keep = d32 + 5 * n;
+  p.peak = d32 + 6 * n;
+  p.pool = S.pool.as<float>(); p.slot_stride = S.slot_stride; p.n_cols = n_cols;
+  p.new_lm = S.new_lm.as<float>(); p.new_ph = S.new_ph.as<float>(); p.den_win = S.den_win.as<float>();
+  p.seg_lm = S.seg_lm.as<float>(); p.seg_ph = S.seg_ph.as<float>(); p.den_seg = S.den_seg.as<float>(); p.cond = S.cond.as<float>();
+  {
+    ProfScope ps(ctx, 1, 0, 2.0 * pcm_o[n] + 12.0 * n_new * kBins);
+    CK(launch_stft(st, S.pcm.as<int16_t>(), d64, p.new_offs, n, p.peak, max_new, S.new_lm.as<float>(), S.new_ph.as<float>(), true));
+  }
+  CK(launch_stream_assemble(st, p, max_rows));
+  ctx->launches += 1;
+  if (n_win > 0) {
+    // (no pass when no window became computable)
+    if ((rc = run_masknet(ctx, p.seg_lm, p.seg_offs, seg_o, p.win_offs, win_o, p.left, left, n, p.cond, S.den_win.as<float>()))) return rc;
+    CK(launch_stream_den(st, p, max_wins));
+    ctx->launches += 1;
+  }
+  // the post step always runs its inverse STFT: the running snr_est covers every sample it emits, wanted or not
+  std::vector<float> factor;
+  std::vector<double> sums;
+  if (post) {
+    factor.resize(n);
+    sums.resize(2 * n);
+    for (int i = 0; i < n; ++i) {
+      const float c = post->compensate ? post->compensate[i] : 0.f;
+      factor[i] = std::isfinite(c) ? c : 0.f;             // the batch rule (compensate_kernel)
+    }
+    CK(S.factor.ensure((size_t)n * 4));
+    CK(S.sums.ensure(sizeof(double) * 2 * n));
+    CK(S.mixed.ensure((size_t)n_out * 4 + 16));
+    CK(S.removed.ensure((size_t)n_out * 4 + 16));
+    CK(S.comp.ensure((size_t)n_out * 4 + 16));
+    CK(cudaMemcpyAsync(S.factor.p, factor.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+    ProfScope ps(ctx, 2, 0, 24.0 * n_win * kBins + 18.0 * n_out);
+    CK(launch_istft_stream_post(st, p, (int)max_out, S.factor.as<float>(), out_f32 ? S.out_f32.as<float>() : nullptr,
+                                out_i16 ? S.out_i16.as<int16_t>() : nullptr, post->mixed ? S.mixed.as<float>() : nullptr,
+                                post->removed ? S.removed.as<float>() : nullptr, post->comp ? S.comp.as<float>() : nullptr,
+                                S.sums.as<double>()));
+  } else if (out_f32 || out_i16) {
+    ProfScope ps(ctx, 2, 0, 12.0 * n_win * kBins + 6.0 * n_out);
+    CK(launch_istft_stream(st, p, (int)max_out, out_f32 ? S.out_f32.as<float>() : nullptr, out_i16 ? S.out_i16.as<int16_t>() : nullptr));
+  }
+  CK(launch_stream_save(st, p, max_keep));
+  ctx->launches += 1;
+  if (out_f32 && n_out) CK(cudaMemcpyAsync(out_f32, S.out_f32.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+  if (out_i16 && n_out) CK(cudaMemcpyAsync(out_i16, S.out_i16.p, n_out * 2, cudaMemcpyDeviceToHost, st));
+  if (post) {
+    if (post->mixed && n_out) CK(cudaMemcpyAsync(post->mixed, S.mixed.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+    if (post->removed && n_out) CK(cudaMemcpyAsync(post->removed, S.removed.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+    if (post->comp && n_out) CK(cudaMemcpyAsync(post->comp, S.comp.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sums.data(), S.sums.p, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
+  }
+  cudaError_t e = cudaStreamSynchronize(st);
+  if ((rc = check_kernel_flag(ctx))) return rc;
+  CK(e);
+  for (int i = 0; i < n; ++i) {
+    StreamRec& r = S.rec.at(ids[i]);
+    const long long F0 = frames_of(r.n);
+    // the next frame starts at sample 160 F1: keep the staged samples from there on
+    const long long from = 160LL * (F1s[i] - F0);
+    r.tail.assign(staged.begin() + pcm_o[i] + from, staged.begin() + pcm_o[i + 1]);
+    r.n += offs[i + 1] - offs[i];
+    r.final = final && final[i];
+    out_offs[i + 1] = out_o[i + 1];
+    if (post) {
+      r.e_den += sums[2 * i];
+      r.e_rem += sums[2 * i + 1];
+      // both means share the sample count, so snr_est is the ratio of the sums (compensate_kernel)
+      if (post->snr_est) post->snr_est[i] = (float)(r.e_rem > 0 ? r.e_den / r.e_rem : INFINITY);
+    }
+  }
+  return NHANS_OK;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -1561,124 +1726,14 @@ int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t
 
 int nhans_stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final,
                       int16_t* out_i16, float* out_f32, int64_t* out_offs) {
-  if (!ctx || n < 0 || n > 65535 || !out_offs || (n > 0 && (!ids || !offs))) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  out_offs[0] = 0;
-  if (n == 0) return NHANS_OK;
-  for (int i = 0; i < n; ++i)
-    if (offs[i + 1] < offs[i]) return fail(ctx, NHANS_ERR_ARG, "chunk offsets must not decrease");
-  if (offs[n] > offs[0] && !pcm) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  int rc;
-  if ((rc = need_weights(ctx))) return rc;
-  if ((rc = check_stream_ids(ctx, n, ids, true))) return rc;
-  CK(cudaSetDevice(ctx->device));
-  Streams& S = ctx->streams;
-  // Geometry of the step (kernels.h StreamStepDev).  Stream i has F0 frames before the step and F1 after it; its windows
-  // [a, b) run now.  It stores frames [cs, F1), cs = a - 17 (or 0): the carry = F0 - cs frames of its slot, then the new
-  // ones.  Its denoised frames a - dc .. b - 1 go through the inverse STFT.
-  std::vector<long long> lo64(6 * (n + 1), 0);           // pcm | new | seg | win | out offsets, staged samples
-  long long *pcm_o = &lo64[0], *new_o = pcm_o + (n + 1), *seg_o = new_o + (n + 1), *win_o = seg_o + (n + 1), *out_o = win_o + (n + 1);
-  std::vector<int> i32(7 * n);
-  int *slot = &i32[0], *carry = slot + n, *left = carry + n, *den_carry = left + n, *keep = den_carry + n, *den_keep = keep + n,
-      *peak = den_keep + n;
-  int max_new = 0, max_rows = 0, max_wins = 0, max_keep = 0;
-  long long max_out = 0;
-  std::vector<int> F1s(n);
-  for (int i = 0; i < n; ++i) {
-    const StreamRec& r = S.rec.at(ids[i]);
-    const bool fin = final && final[i];
-    const long long len = offs[i + 1] - offs[i], N1 = r.n + len;
-    const int F0 = frames_of(r.n), F1 = frames_of(N1);
-    const long long a = stream_windows(F0, false), b = std::max(a, stream_windows(F1, fin));
-    const long long cs = std::max(0LL, a - kHalfWin);
-    slot[i] = r.slot;
-    peak[i] = r.peak;
-    carry[i] = (int)(F0 - cs);
-    left[i] = (int)(a - cs);
-    den_carry[i] = (int)std::min(a, 2LL);
-    keep[i] = (int)(std::max(0LL, b - kHalfWin) - cs);
-    den_keep[i] = (int)std::min(b, 2LL);
-    F1s[i] = F1;
-    pcm_o[i + 1] = pcm_o[i] + (long long)r.tail.size() + len;
-    new_o[i + 1] = new_o[i] + (F1 - F0);
-    seg_o[i + 1] = seg_o[i] + (F1 - cs);
-    win_o[i + 1] = win_o[i] + (b - a);
-    out_o[i + 1] = out_o[i] + stream_emitted(F1, fin) - stream_emitted(F0, false);
-    max_new = std::max(max_new, F1 - F0);
-    max_rows = std::max<long long>(max_rows, F1 - cs);
-    max_wins = std::max<long long>(max_wins, b - a);
-    max_keep = std::max<long long>(max_keep, F1 - cs - keep[i]);
-    max_out = std::max(max_out, out_o[i + 1] - out_o[i]);
-  }
-  const int n_cols = ctx->main_net.plan.cond.n_cols;
-  const long long n_new = new_o[n], n_seg = seg_o[n], n_win = win_o[n], n_out = out_o[n];
-  if (n_seg > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one step");
-  // staging: each stream's unframed tail, then its chunk
-  std::vector<int16_t> staged((size_t)pcm_o[n]);
-  for (int i = 0; i < n; ++i) {
-    const StreamRec& r = S.rec.at(ids[i]);
-    std::copy(r.tail.begin(), r.tail.end(), staged.begin() + pcm_o[i]);
-    if (offs[i + 1] > offs[i]) std::copy(pcm + offs[i], pcm + offs[i + 1], staged.begin() + pcm_o[i] + r.tail.size());
-  }
-  cudaStream_t st = ctx->stream;
-  const size_t desc64 = lo64.size() * 8;
-  CK(S.pcm.ensure(staged.size() * 2 + 32));
-  CK(S.desc.ensure(desc64 + i32.size() * 4));
-  CK(S.new_lm.ensure((size_t)n_new * kBins * 4 + 4));
-  CK(S.new_ph.ensure((size_t)n_new * kBins * 8 + 8));
-  CK(S.seg_lm.ensure((size_t)n_seg * kBins * 4 + 4));
-  CK(S.seg_ph.ensure((size_t)n_seg * kBins * 8 + 8));
-  CK(S.den_seg.ensure((size_t)n_seg * kBins * 4 + 4));
-  CK(S.den_win.ensure((size_t)n_win * kBins * 4 + 4));
-  CK(S.cond.ensure((size_t)n * n_cols * 4));
-  CK(S.out_f32.ensure((size_t)n_out * 4 + 16));
-  CK(S.out_i16.ensure((size_t)n_out * 2 + 16));
-  if (!staged.empty()) CK(cudaMemcpyAsync(S.pcm.p, staged.data(), staged.size() * 2, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(S.desc.p, lo64.data(), desc64, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(S.desc.as<char>() + desc64, i32.data(), i32.size() * 4, cudaMemcpyHostToDevice, st));
-  const long long* d64 = S.desc.as<long long>();
-  const int* d32 = reinterpret_cast<const int*>(S.desc.as<char>() + desc64);
-  StreamStepDev p;
-  p.n = n;
-  p.seg_offs = d64 + 2 * (n + 1); p.new_offs = d64 + (n + 1); p.win_offs = d64 + 3 * (n + 1); p.out_offs = d64 + 4 * (n + 1);
-  p.slot = d32; p.carry = d32 + n; p.left = d32 + 2 * n; p.den_carry = d32 + 3 * n; p.keep = d32 + 4 * n; p.den_keep = d32 + 5 * n;
-  p.peak = d32 + 6 * n;
-  p.pool = S.pool.as<float>(); p.slot_stride = S.slot_stride; p.n_cols = n_cols;
-  p.new_lm = S.new_lm.as<float>(); p.new_ph = S.new_ph.as<float>(); p.den_win = S.den_win.as<float>();
-  p.seg_lm = S.seg_lm.as<float>(); p.seg_ph = S.seg_ph.as<float>(); p.den_seg = S.den_seg.as<float>(); p.cond = S.cond.as<float>();
-  {
-    ProfScope ps(ctx, 1, 0, 2.0 * pcm_o[n] + 12.0 * n_new * kBins);
-    CK(launch_stft(st, S.pcm.as<int16_t>(), d64, p.new_offs, n, p.peak, max_new, S.new_lm.as<float>(), S.new_ph.as<float>(), true));
-  }
-  CK(launch_stream_assemble(st, p, max_rows));
-  ctx->launches += 1;
-  if (n_win > 0) {
-    // (no pass when no window became computable)
-    if ((rc = run_masknet(ctx, p.seg_lm, p.seg_offs, seg_o, p.win_offs, win_o, p.left, left, n, p.cond, S.den_win.as<float>()))) return rc;
-    CK(launch_stream_den(st, p, max_wins));
-    ctx->launches += 1;
-  }
-  if (out_f32 || out_i16) {
-    ProfScope ps(ctx, 2, 0, 12.0 * n_win * kBins + 6.0 * n_out);
-    CK(launch_istft_stream(st, p, (int)max_out, out_f32 ? S.out_f32.as<float>() : nullptr, out_i16 ? S.out_i16.as<int16_t>() : nullptr));
-  }
-  CK(launch_stream_save(st, p, max_keep));
-  ctx->launches += 1;
-  if (out_f32 && n_out) CK(cudaMemcpyAsync(out_f32, S.out_f32.p, n_out * 4, cudaMemcpyDeviceToHost, st));
-  if (out_i16 && n_out) CK(cudaMemcpyAsync(out_i16, S.out_i16.p, n_out * 2, cudaMemcpyDeviceToHost, st));
-  cudaError_t e = cudaStreamSynchronize(st);
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
-  for (int i = 0; i < n; ++i) {
-    StreamRec& r = S.rec.at(ids[i]);
-    const long long F0 = frames_of(r.n);
-    // the next frame starts at sample 160 F1: keep the staged samples from there on
-    const long long from = 160LL * (F1s[i] - F0);
-    r.tail.assign(staged.begin() + pcm_o[i] + from, staged.begin() + pcm_o[i + 1]);
-    r.n += offs[i + 1] - offs[i];
-    r.final = final && final[i];
-    out_offs[i + 1] = out_o[i + 1];
-  }
-  return NHANS_OK;
+  return stream_step(ctx, n, ids, pcm, offs, final, out_i16, out_f32, out_offs, nullptr);
+}
+
+int nhans_stream_step_post(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const int64_t* offs, const int* final,
+                           const float* compensate, int16_t* out_i16, float* out_f32, float* mixed_f32, float* removed_f32,
+                           float* compensated_f32, int64_t* out_offs, float* snr_est) {
+  PostOut post{compensate, mixed_f32, removed_f32, compensated_f32, snr_est};
+  return stream_step(ctx, n, ids, pcm, offs, final, out_i16, out_f32, out_offs, &post);
 }
 
 int nhans_stream_close(nhans_ctx* ctx, int n, const int* ids) {

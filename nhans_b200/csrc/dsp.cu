@@ -380,9 +380,15 @@ istft_kernel(const float* __restrict__ logmag, const float* __restrict__ phase, 
 // the first carried denoised frame (den_carry of them precede its windows), frames outside [0, T) are zero as at an
 // utterance edge, and local samples [lo, lo + len) with lo = 160 den_carry go to out_offs[s].  Every sample is the same
 // gather and sum as in istft_kernel, so a stream's samples are bit-identical to the whole clip's.
+// POST adds the post-mix outputs of istft_post_kernel / compensate_kernel: the same rows of seg_lm (the input spectrum,
+// with the same phasors) give mixed_processed, then removed = mixed - den, compensated = den + removed * factor[s], and
+// the energy sums of den and removed go to sums[s][0..1] (zeroed by the launcher).  Any output may be null.
 // grid: (ceil((max len + 159) / 160 / kOH), n).
-__global__ void __launch_bounds__(kThreads, 4)
-istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t* __restrict__ out_i16) {
+template <bool POST>
+__global__ void __launch_bounds__(kThreads, POST ? 1 : 4)
+istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t* __restrict__ out_i16, float* __restrict__ mixed_f32,
+                    float* __restrict__ removed_f32, float* __restrict__ comp_f32, const float* __restrict__ factor,
+                    double* __restrict__ sums /* [n][2] */) {
   __shared__ __align__(16) float s_y[kNFI * kWin];
   const int u = blockIdx.y;
   const int dc = p.den_carry[u];
@@ -390,19 +396,70 @@ istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t*
   const long long len = p.out_offs[u + 1] - p.out_offs[u];
   const int h0 = dc + blockIdx.x * kOH;   // first output hop (local)
   if (T <= 0 || (long long)blockIdx.x * kOH * kHop >= len) return;
-  istft_frames<true>(s_y, p.den_seg, p.seg_ph, p.seg_offs[u] + p.left[u] - dc, T, h0 - 2);
+  const long long row0 = p.seg_offs[u] + p.left[u] - dc;
+  istft_frames<true>(s_y, p.den_seg, p.seg_ph, row0, T, h0 - 2);
   const long long lo = (long long)dc * kHop;
   const float scale = (float)((double)p.peak[u] + 0.000001);
-  for (int i = threadIdx.x * 4; i < kOH * kHop; i += blockDim.x * 4) {
-    const long long n = (long long)h0 * kHop + i - lo;
-    if (n >= len) break;
-    const float4 acc = ola_sample4(s_y, i);
-    const long long o = p.out_offs[u] + n;
-    if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = acc;
-    if (out_i16) {
-      short4 q;
-      q.x = to_i16(acc.x * scale); q.y = to_i16(acc.y * scale); q.z = to_i16(acc.z * scale); q.w = to_i16(acc.w * scale);
-      *reinterpret_cast<short4*>(out_i16 + o) = q;
+  if constexpr (!POST) {
+    for (int i = threadIdx.x * 4; i < kOH * kHop; i += blockDim.x * 4) {
+      const long long n = (long long)h0 * kHop + i - lo;
+      if (n >= len) break;
+      const float4 acc = ola_sample4(s_y, i);
+      const long long o = p.out_offs[u] + n;
+      if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = acc;
+      if (out_i16) {
+        short4 q;
+        q.x = to_i16(acc.x * scale); q.y = to_i16(acc.y * scale); q.z = to_i16(acc.z * scale); q.w = to_i16(acc.w * scale);
+        *reinterpret_cast<short4*>(out_i16 + o) = q;
+      }
+    }
+  } else {
+    __shared__ float s_red[2][kThreads / 32];
+    constexpr int PER = (kOH * kHop / 4 + kThreads - 1) / kThreads;
+    float4 den[PER];
+#pragma unroll
+    for (int k = 0; k < PER; ++k) {
+      const int i = (threadIdx.x + k * kThreads) * 4;
+      den[k] = i < kOH * kHop ? ola_sample4(s_y, i) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    istft_frames<true>(s_y, p.seg_lm, p.seg_ph, row0, T, h0 - 2);
+    const float f = factor[u];
+    float e_den = 0.f, e_rem = 0.f;
+#pragma unroll
+    for (int k = 0; k < PER; ++k) {
+      const int i = (threadIdx.x + k * kThreads) * 4;
+      const long long n = (long long)h0 * kHop + i - lo;
+      if (i >= kOH * kHop || n >= len) continue;
+      const float4 mixed = ola_sample4(s_y, i);
+      const float4 d = den[k];
+      const float4 rem = make_float4(mixed.x - d.x, mixed.y - d.y, mixed.z - d.z, mixed.w - d.w);
+      const long long o = p.out_offs[u] + n;
+      if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = d;
+      if (out_i16) {
+        short4 q;
+        q.x = to_i16(d.x * scale); q.y = to_i16(d.y * scale); q.z = to_i16(d.z * scale); q.w = to_i16(d.w * scale);
+        *reinterpret_cast<short4*>(out_i16 + o) = q;
+      }
+      if (mixed_f32) *reinterpret_cast<float4*>(mixed_f32 + o) = mixed;
+      if (removed_f32) *reinterpret_cast<float4*>(removed_f32 + o) = rem;
+      // one FFMA per sample, as compensate_kernel's den + removed * factor
+      if (comp_f32)
+        *reinterpret_cast<float4*>(comp_f32 + o) = make_float4(__fmaf_rn(rem.x, f, d.x), __fmaf_rn(rem.y, f, d.y),
+                                                               __fmaf_rn(rem.z, f, d.z), __fmaf_rn(rem.w, f, d.w));
+      e_den += d.x * d.x + d.y * d.y + d.z * d.z + d.w * d.w;
+      e_rem += rem.x * rem.x + rem.y * rem.y + rem.z * rem.z + rem.w * rem.w;
+    }
+    for (int o = 16; o; o >>= 1) {
+      e_den += __shfl_xor_sync(0xffffffffu, e_den, o);
+      e_rem += __shfl_xor_sync(0xffffffffu, e_rem, o);
+    }
+    if ((threadIdx.x & 31) == 0) { s_red[0][threadIdx.x >> 5] = e_den; s_red[1][threadIdx.x >> 5] = e_rem; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double a = 0, b = 0;
+      for (int w = 0; w < kThreads / 32; ++w) { a += s_red[0][w]; b += s_red[1][w]; }
+      atomicAdd(&sums[2 * u], a);
+      atomicAdd(&sums[2 * u + 1], b);
     }
   }
 }
@@ -570,7 +627,18 @@ cudaError_t launch_istft(cudaStream_t s, const float* logmag, const float* phase
 cudaError_t launch_istft_stream(cudaStream_t s, const StreamStepDev& p, int max_samples, float* out_f32, int16_t* out_i16) {
   if (p.n <= 0 || max_samples <= 0) return cudaSuccess;
   dim3 grid((max_samples + kOH * kHop - 1) / (kOH * kHop), p.n);
-  istft_stream_kernel<<<grid, kThreads, 0, s>>>(p, out_f32, out_i16);
+  istft_stream_kernel<false><<<grid, kThreads, 0, s>>>(p, out_f32, out_i16, nullptr, nullptr, nullptr, nullptr, nullptr);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_istft_stream_post(cudaStream_t s, const StreamStepDev& p, int max_samples, const float* factor, float* out_f32,
+                                     int16_t* out_i16, float* mixed_f32, float* removed_f32, float* comp_f32, double* sums) {
+  if (p.n <= 0) return cudaSuccess;
+  // zeroed even when the step emits nothing: the caller adds the sums of every stream to its running totals
+  cudaError_t e = cudaMemsetAsync(sums, 0, sizeof(double) * 2 * p.n, s);
+  if (e != cudaSuccess || max_samples <= 0) return e;
+  dim3 grid((max_samples + kOH * kHop - 1) / (kOH * kHop), p.n);
+  istft_stream_kernel<true><<<grid, kThreads, 0, s>>>(p, out_f32, out_i16, mixed_f32, removed_f32, comp_f32, factor, sums);
   return cudaGetLastError();
 }
 

@@ -212,6 +212,11 @@ cudaError_t launch_stream_assemble(cudaStream_t s, const StreamStepDev& p, int m
 cudaError_t launch_stream_den(cudaStream_t s, const StreamStepDev& p, int max_wins);
 // inverse STFT of the emitted samples -> out_f32 / out_i16 (either may be null) at out_offs
 cudaError_t launch_istft_stream(cudaStream_t s, const StreamStepDev& p, int max_samples, float* out_f32, int16_t* out_i16);
+// the same plus the post-mix outputs of launch_istft_post / launch_compensate over the same samples: mixed_processed (inverse
+// STFT of seg_lm), removed, compensated with factor[s] per stream (device [n], already 0 where not finite), and the energy
+// sums [n][2] (sum den^2, sum removed^2) of the emitted samples, zeroed first.  Every output but sums may be null.
+cudaError_t launch_istft_stream_post(cudaStream_t s, const StreamStepDev& p, int max_samples, const float* factor, float* out_f32,
+                                     int16_t* out_i16, float* mixed_f32, float* removed_f32, float* comp_f32, double* sums);
 // slot state for the next step
 cudaError_t launch_stream_save(cudaStream_t s, const StreamStepDev& p, int max_rows);
 

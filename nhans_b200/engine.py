@@ -353,6 +353,27 @@ class Engine:
         return {"i16": [np.array(v) for v in unpack(o16, oo)] if want_i16 else None,
                 "f32": [np.array(v) for v in unpack(o32, oo)] if want_f32 else None}
 
+    def stream_step_post(self, ids, chunks, compensate, final=None):
+        """stream_step plus the post-mix outputs of postmix(compensate, ac=False) for the emitted samples.  compensate: one
+        factor for every stream or one per stream.  -> {"i16", "f32", "mixed_processed", "removed", "compensated"}: per-stream
+        lists of this step's samples, and "snr_est": each stream's running estimate over its post-step samples so far."""
+        n = len(ids)
+        pcm, offs = pack(chunks)
+        ids_a = np.ascontiguousarray(ids, np.int32)
+        fin = np.ascontiguousarray(final, np.int32) if final is not None else None
+        comp = np.ascontiguousarray(np.broadcast_to(np.asarray(compensate, np.float32), (n,)))
+        cap = int(offs[-1]) + STREAM_EMIT_SLACK * n
+        oo = np.zeros(n + 1, np.int64)
+        o16 = np.empty(cap, np.int16)
+        o32, mixed, removed, compensated = (np.empty(cap, np.float32) for _ in range(4))
+        snr = np.zeros(n, np.float32)
+        self._ck(self.lib.nhans_stream_step_post(self.h, n, _ptr(ids_a), _ptr(pcm), _ptr(offs), _ptr(fin), _ptr(comp), _ptr(o16),
+                                                 _ptr(o32), _ptr(mixed), _ptr(removed), _ptr(compensated), _ptr(oo), _ptr(snr)))
+        res = {k: [np.array(v) for v in unpack(a, oo)] for k, a in
+               (("i16", o16), ("f32", o32), ("mixed_processed", mixed), ("removed", removed), ("compensated", compensated))}
+        res["snr_est"] = snr
+        return res
+
     def stream_close(self, ids):
         ids_a = np.ascontiguousarray(ids, np.int32)
         self._ck(self.lib.nhans_stream_close(self.h, len(ids_a), _ptr(ids_a)))

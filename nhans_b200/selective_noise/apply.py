@@ -142,12 +142,13 @@ def _sibling(save_to, name):
     return root + "_" + name
 
 
+def _to_i16(f32, peak):
+    v = np.rint(f32.astype(np.float32) * np.float32(peak + 0.000001))
+    return np.clip(v, -32768, 32767).astype(np.int16)
+
+
 def _emit(save_to, f32, peak, as_float32):
-    if as_float32:
-        write_wav(save_to, f32.astype(np.float32))
-    else:
-        v = np.rint(f32.astype(np.float32) * np.float32(peak + 0.000001))
-        write_wav(save_to, np.clip(v, -32768, 32767).astype(np.int16))
+    write_wav(save_to, f32.astype(np.float32) if as_float32 else _to_i16(f32, peak))
 
 
 def _post_mix_host(den, mixed, compensate, ac):
@@ -236,6 +237,82 @@ def _pairs(inp, pos, neg, out):
     return mixed, poss, negs, outs
 
 
+# ---- live mode (--stream): raw PCM in, raw PCM out, through the engine's streaming entry points ----------------------
+def add_stream_args(ap):
+    ap.add_argument("--stream", action="store_true",
+                    help="live mode: --input is raw s16le mono 16 kHz PCM ('-' = stdin), --output raw PCM ('-' = stdout), "
+                         "s16le or f32le with --float32")
+    ap.add_argument("--peak", type=int, default=32767, help="--stream: the int16 peak that scales the input and the output")
+    ap.add_argument("--chunk-ms", type=int, default=100, help="--stream: largest read from the input, in ms of audio")
+
+
+def check_stream_args(ap, a):
+    if a.peak < 0:
+        ap.error("--peak must not be negative")
+    if a.chunk_ms < 1:
+        ap.error("--chunk-ms must be at least 1")
+
+
+def stream_context(ap, path, flag):
+    """A context wav of a live stream: it must be int16 mono, the only form the int16 stream path conditions on exactly."""
+    x = read_wav(path)
+    if not is_pcm16(x):
+        ap.error("%s %s: --stream needs an int16 mono context file (a stereo file is averaged in float64, which only the "
+                 "batch path reproduces)" % (flag, path))
+    return x
+
+
+def pcm_bytes(x):
+    """Raw little-endian bytes of int16 (s16le) or float32 (f32le) samples."""
+    return np.asarray(x, x.dtype.newbyteorder("<")).tobytes()
+
+
+def stream_pipe(step, inp, out, chunk_ms):
+    """Feed raw s16le samples from `inp` ('-' = stdin) to step(samples, final) -> bytes and write what it returns to `out`
+    ('-' = stdout), flushed after every step.  Each read takes what the pipe holds, at most one chunk, so a slow source is
+    not held back; an odd trailing byte waits for the next read.  At EOF an empty final step flushes the stream."""
+    fd = sys.stdin.fileno() if inp == "-" else os.open(inp, os.O_RDONLY)
+    dst = sys.stdout.buffer if out == "-" else open(out, "wb")
+    try:
+        want, carry = 2 * (FS // 1000) * chunk_ms, b""
+        while True:
+            data = os.read(fd, want)
+            if not data:
+                break
+            buf = carry + data
+            n = len(buf) & ~1
+            carry = buf[n:]
+            if n:
+                dst.write(step(np.frombuffer(buf[:n], "<i2").astype(np.int16), False))
+                dst.flush()
+        if carry:
+            sys.stderr.write("ignoring an odd trailing byte at the end of the input\n")
+        dst.write(step(np.zeros(0, np.int16), True))
+        dst.flush()
+    finally:
+        if inp != "-":
+            os.close(fd)
+        if out != "-":
+            dst.close()
+
+
+def stream_denoiser(ap, a):
+    """--stream: the compensated signal (denoised + removed * --compensate) of one live stream; with --compensate 0 it is
+    the denoised signal.  int16 output follows the rule of the wav outputs with --peak."""
+    neg = stream_context(ap, a.neg, "--neg")
+    pos = None if _is_silent(a.pos) else stream_context(ap, a.pos, "--pos")
+    eng = get_engine(VARIANT)
+    [sid] = eng.stream_open(None if pos is None else [pos], [neg], [a.peak])
+
+    def step(x, final):
+        comp = eng.stream_step_post([sid], [x], a.compensate, final=[int(final)])["compensated"][0]
+        return pcm_bytes(comp if a.float32 else _to_i16(comp, a.peak))
+    try:
+        stream_pipe(step, a.input, a.output, a.chunk_ms)
+    finally:
+        eng.stream_close([sid])
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="nhans_denoiser", description="N-HANS denoiser / selective noise suppression (B200 engine)")
     ap.add_argument("--input", default=FLAGS.input)
@@ -245,7 +322,15 @@ def main(argv=None):
     ap.add_argument("--compensate", type=float, default=0.0)
     ap.add_argument("--ac", action="store_true")
     ap.add_argument("--float32", action="store_true", help="write float32 wavs like the reference instead of 16-bit PCM")
+    add_stream_args(ap)
     a = ap.parse_args(argv)
+    if a.stream:
+        if a.ac:
+            ap.error("--ac cannot be used with --stream: its factor is the whole clip's snr_est, which a live stream does not "
+                     "know until it ends; use --compensate")
+        check_stream_args(ap, a)
+        stream_denoiser(ap, a)
+        return 0
     FLAGS.input, FLAGS.neg, FLAGS.pos, FLAGS.output = a.input, a.neg, a.pos, a.output
     FLAGS.compensate, FLAGS.ac, FLAGS.float32 = a.compensate, a.ac, a.float32
     if os.path.isdir(a.input):

@@ -16,7 +16,8 @@ import numpy as np
 from .. import weights as W
 from ..session import get_engine
 from ..wavio import FS, is_pcm16, read_wav, write_wav
-from ..selective_noise.apply import _emit, _fit_noise, _norm64, _seq_sum, _sibling
+from ..selective_noise.apply import (_emit, _fit_noise, _norm64, _seq_sum, _sibling, add_stream_args, check_stream_args,
+                                     pcm_bytes, stream_context, stream_pipe)
 
 Noise_Win = 200
 Mix_Win = 35
@@ -119,6 +120,22 @@ def apply_separator(mixedpath, cleanpath, noisepath, save_to):
     apply_separator_batch([mixedpath], [cleanpath], [noisepath], [save_to])
 
 
+def stream_separator(ap, a):
+    """--stream: the separated signal of one live stream (int16 scaled by --peak, or float32)."""
+    noise = stream_context(ap, a.neg, "--neg")
+    clean = stream_context(ap, a.pos, "--pos")
+    eng = get_engine(VARIANT)
+    [sid] = eng.stream_open([noise], [clean], [a.peak])                     # ctx_a = --neg, ctx_b = --pos
+
+    def step(x, final):
+        r = eng.stream_step([sid], [x], final=[int(final)], want_f32=a.float32, want_i16=not a.float32)
+        return pcm_bytes(r["f32"][0] if a.float32 else r["i16"][0])
+    try:
+        stream_pipe(step, a.input, a.output, a.chunk_ms)
+    finally:
+        eng.stream_close([sid])
+
+
 def main(argv=None):
     ap = argparse.ArgumentParser(prog="nhans_separator", description="N-HANS speech separator (B200 engine)")
     ap.add_argument("--input", default=FLAGS.input)
@@ -126,7 +143,12 @@ def main(argv=None):
     ap.add_argument("--pos", default=FLAGS.pos)
     ap.add_argument("--output", default=FLAGS.output)
     ap.add_argument("--float32", action="store_true")
+    add_stream_args(ap)
     a = ap.parse_args(argv)
+    if a.stream:
+        check_stream_args(ap, a)
+        stream_separator(ap, a)
+        return 0
     FLAGS.input, FLAGS.neg, FLAGS.pos, FLAGS.output, FLAGS.float32 = a.input, a.neg, a.pos, a.output, a.float32
     if os.path.isdir(a.input):
         names = sorted(f for f in os.listdir(a.input) if f.lower().endswith(".wav"))

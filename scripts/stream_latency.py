@@ -4,7 +4,11 @@ step: median and p99), the audio seconds pushed per second of wall clock, and th
 over p99 step latency: above 1 the GPU keeps up with S live streams).  Asserts nothing about speed.  Prints one JSON
 line with the GPU name and power limit.
 
-  python scripts/stream_latency.py [--streams 1,64,1024] [--steps 50] [--warmup 10] [--chunk-ms 100]"""
+With --post, two sets of S streams fed the same audio take plain steps (nhans_stream_step) and post-mix steps
+(nhans_stream_step_post, compensate 0.3) in turn, alternating which goes first, so that both are timed under the same
+conditions; each result row names its mode.
+
+  python scripts/stream_latency.py [--streams 1,64,1024] [--steps 50] [--warmup 10] [--chunk-ms 100] [--post]"""
 import argparse
 import json
 import os
@@ -25,6 +29,7 @@ ap.add_argument("--steps", type=int, default=50)
 ap.add_argument("--warmup", type=int, default=10)
 ap.add_argument("--chunk-ms", type=int, default=100)
 ap.add_argument("--device", type=int, default=0)
+ap.add_argument("--post", action="store_true", help="also time post-mix steps, alternating with plain steps")
 a = ap.parse_args()
 
 
@@ -42,22 +47,28 @@ negs = [synth.noise_clip(9000 + u) for u in range(n_distinct)]
 eng = Engine(a.device, W.SELECTIVE_NOISE)
 eng.load_weights(W.seeded_init(W.SELECTIVE_NOISE, 0))
 results = []
+modes = {"plain": lambda ids, chunks: eng.stream_step(ids, chunks),
+         "post": lambda ids, chunks: eng.stream_step_post(ids, chunks, 0.3)}
+if not a.post:
+    del modes["post"]
 try:
     for S in [int(s) for s in a.streams.split(",")]:
-        ids = eng.stream_open(None, [negs[u % n_distinct] for u in range(S)], [32767] * S)
-        times = []
+        ids = {m: eng.stream_open(None, [negs[u % n_distinct] for u in range(S)], [32767] * S) for m in modes}
+        times = {m: [] for m in modes}
         for k in range(a.warmup + a.steps):
             chunks = [mixes[u % n_distinct][k * chunk:(k + 1) * chunk] for u in range(S)]
-            t0 = time.perf_counter()
-            eng.stream_step(ids, chunks)
-            if k >= a.warmup:
-                times.append(time.perf_counter() - t0)
-        eng.stream_close(ids)
-        t = np.array(times)
-        results.append({"streams": S, "step_ms_median": round(1e3 * float(np.median(t)), 3),
-                        "step_ms_p99": round(1e3 * float(np.percentile(t, 99)), 3),
-                        "audio_s_per_s": round(S * chunk / 16000.0 * len(t) / float(t.sum()), 1),
-                        "rt_headroom_p99": round(chunk / 16000.0 / float(np.percentile(t, 99)), 2)})
+            for m in (list(modes) if k % 2 == 0 else list(modes)[::-1]):
+                t0 = time.perf_counter()
+                modes[m](ids[m], chunks)
+                if k >= a.warmup:
+                    times[m].append(time.perf_counter() - t0)
+        for m in modes:
+            eng.stream_close(ids[m])
+            t = np.array(times[m])
+            results.append({"mode": m, "streams": S, "step_ms_median": round(1e3 * float(np.median(t)), 3),
+                            "step_ms_p99": round(1e3 * float(np.percentile(t, 99)), 3),
+                            "audio_s_per_s": round(S * chunk / 16000.0 * len(t) / float(t.sum()), 1),
+                            "rt_headroom_p99": round(chunk / 16000.0 / float(np.percentile(t, 99)), 2)})
 finally:
     eng.close()
 print(json.dumps(dict(gpu_info(a.device), chunk_ms=a.chunk_ms, steps=a.steps, warmup=a.warmup, results=results)))
