@@ -54,6 +54,7 @@ struct DBuf {
 struct GemmLayerDev {
   __half* w = nullptr;
   KGroupDev* groups = nullptr;
+  uint32_t* row_groups = nullptr;
   float *bias = nullptr, *tftab = nullptr, *res_scale = nullptr, *r1_vec = nullptr;
   uint16_t *ttab16 = nullptr, *ftab16 = nullptr;
   CUtensorMap mapA0, mapA1, mapB, mapBhalf;
@@ -308,6 +309,9 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
       groups[j] = d;
     }
     if ((rc = upload(ctx, net, groups, &D.groups))) return rc;
+    if ((rc = upload(ctx, net, L.row_groups, &D.row_groups))) return rc;
+    if (L.epi.head && (int)L.groups.size() % kHeadSplit == 0 && !every_split_live(L, kHeadSplit))
+      return fail(ctx, NHANS_ERR_STATE, "layer " + L.name + ": a K split runs no group for some output row");
     if ((rc = upload(ctx, net, L.epi.bias, &D.bias))) return rc;
     if ((rc = upload(ctx, net, L.epi.tftab, &D.tftab))) return rc;
     if ((rc = upload(ctx, net, L.epi.ttab16, &D.ttab16))) return rc;
@@ -495,7 +499,7 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
     memset(&g, 0, sizeof g);
     long long M = (long long)units * L.Ho * L.Wq;
     if ((long long)P.capacity * L.Ho * L.Wq > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many rows in one pass");
-    g.M = (int)M; g.plane_pitch = P.capacity * L.Wq; g.plane_rows = units * L.Wq; g.N = L.N; g.BN = L.BN; g.num_kb = (int)L.kb.size(); g.num_groups = (int)L.groups.size(); g.groups = D.groups;
+    g.M = (int)M; g.plane_pitch = P.capacity * L.Wq; g.plane_rows = units * L.Wq; g.N = L.N; g.BN = L.BN; g.num_kb = (int)L.kb.size(); g.num_groups = (int)L.groups.size(); g.groups = D.groups; g.row_groups = D.row_groups;
     g.Hq = L.Hq; g.Wq = L.Wq; g.Ho = L.Ho; g.Wo = L.Wo;
     g.units = ut;
     g.epi = make_epi(net, L.epi, L.out, D.bias, D.tftab, D.res_scale, D.r1_vec, raw, cond_table, out_f32);

@@ -6,9 +6,11 @@
 // convolutions is lowered to this form by plan.cc (a group g = the kw taps of one kernel row and one
 // 64-channel chunk).  Activations live in "image-row-outer" padded grids (plan.h): a tap is a constant row
 // offset, vertical padding is TMA out-of-bounds fill, and only real output rows are enumerated; tiles are
-// ordered image-row-fastest.  Persistent CTA PAIRS (cluster of 2, cta_group::2; a single-CTA instantiation
-// serves small problems); a tile is (256 / BN) sub-tiles of 256 rows (128 per CTA) x BN columns, i.e. always
-// 256 fp32 accumulator columns in TMEM, double buffered (2 x 256 = all 512 columns).
+// ordered image-row-fastest.  A tile lies in one output row ho and runs only the groups whose kernel row reads
+// inside the image for that row (GemmDev::row_groups, at most two index ranges looked up once per tile): all three
+// roles skip the same groups, with no test per group.  Persistent CTA PAIRS (cluster of 2, cta_group::2; a
+// single-CTA instantiation serves small problems); a tile is (256 / BN) sub-tiles of 256 rows (128 per CTA) x BN
+// columns, i.e. always 256 fp32 accumulator columns in TMEM, double buffered (2 x 256 = all 512 columns).
 //
 //   warp 8   A producer     one TMA box of 136 rows x 64 channels ("slab") per (group, sub-tile): the kw taps
 //                           of a kernel row read the SAME slab through UMMA descriptors whose start address
@@ -65,6 +67,31 @@ struct __align__(8) Ctrl {
 };
 static_assert(sizeof(Ctrl) <= kCtrlBytes, "control block too large");
 
+// Output row of the tiles one CTA visits (tile0, tile0 + step, ...): ho = (tile / (ksplit n_tiles)) % Ho (kernels.h
+// GemmDev), advanced without divisions.
+struct TileRow {
+  int tpr, d_r, d_ho, Ho, r, ho;
+  __device__ __forceinline__ TileRow(int tile0, int step, int tpr_, int Ho_)
+      : tpr(tpr_), d_r(step % tpr_), d_ho((step / tpr_) % Ho_), Ho(Ho_), r(tile0 % tpr_), ho((tile0 / tpr_) % Ho_) {}
+  __device__ __forceinline__ void next() {
+    r += d_r;
+    const int carry = r >= tpr ? 1 : 0;
+    r -= carry * tpr;
+    ho += d_ho + carry;
+    if (ho >= Ho) ho -= Ho;
+  }
+};
+
+// The groups of [g_lo, g_hi) (one K split) a tile runs: [s0, e0) and then [s1, e1), from its row's entry of
+// GemmDev::row_groups (empty ranges have e = s)
+struct LiveGroups {
+  int s0, e0, s1, e1;
+  __device__ __forceinline__ LiveGroups(uint32_t w, int g_lo, int g_hi) {
+    s0 = max((int)(w & 0xffu), g_lo); e0 = max(s0, min((int)((w >> 8) & 0xffu), g_hi));
+    s1 = max((int)((w >> 16) & 0xffu), g_lo); e1 = max(s1, min((int)(w >> 24), g_hi));
+  }
+};
+
 __device__ __forceinline__ uint32_t pack_half2(float a, float b) {
   __half2 h = __floats2half2_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&h);
@@ -77,7 +104,7 @@ __device__ __forceinline__ uint32_t pack_half2(float a, float b) {
 // test in the single issuing lane's tap loop is paid in throughput (the lane is instruction bound, DESIGN.md §4).
 template <int IL, bool CTA2, bool RES>
 __device__ __forceinline__ void mma_issuer(Ctrl* ctrl, const GemmDev& p, const GemmCfg& cfg, uint8_t* smem_a, uint8_t* smem_b,
-                                           uint32_t tmem_base, int num_tiles, int b_bytes) {
+                                           uint32_t tmem_base, int num_tiles, int n_tiles, int b_bytes) {
   const int cta_shift = CTA2 ? 1 : 0;
   const int MT = cfg.mt;
   const int num_groups = p.num_groups;
@@ -101,12 +128,20 @@ __device__ __forceinline__ void mma_issuer(Ctrl* ctrl, const GemmDev& p, const G
       else ptx::mbar_wait(bar, parity, p.err_flag, tag);
     };
     const long long t_start = clock64();
-    for (int tile = blockIdx.x >> cta_shift; tile < num_tiles; tile += gridDim.x >> cta_shift, ++it) {
+    const int step = gridDim.x >> cta_shift;
+    TileRow row(blockIdx.x >> cta_shift, step, p.ksplit * n_tiles, p.Ho);
+    for (int tile = blockIdx.x >> cta_shift; tile < num_tiles; tile += step, ++it, row.next()) {
       const uint32_t acc = it & 1, acc_phase = (it >> 1) & 1;
       const int g_lo = (tile % p.ksplit) * gper, g_hi = min(num_groups, g_lo + gper);
+      const uint32_t row_w = __ldg(p.row_groups + row.ho);
       wait(&ctrl->tmem_empty[acc], acc_phase ^ 1, 2, &w_tmem);
       ptx::tc_fence_after();
-      for (int g = g_lo; g < g_hi; ++g) {
+      const LiveGroups lg(row_w, g_lo, g_hi);
+      const int g_first = lg.e0 > lg.s0 ? lg.s0 : lg.s1;             // the tile's first MMA overwrites the accumulator
+      int gb = lg.s0, ge = lg.e0;
+#pragma unroll 1
+      for (int pass = 0; pass < 2; ++pass, gb = lg.s1, ge = lg.e1)
+      for (int g = gb; g < ge; ++g) {
         const int ntaps = ctrl->groups[g].ntaps;
         // the MT slabs of a group land on the barrier of the group's first slab (MT divides the ring depth, so a
         // group never wraps): one wait per group
@@ -132,7 +167,7 @@ __device__ __forceinline__ void mma_issuer(Ctrl* ctrl, const GemmDev& p, const G
             ptx::tc_fence_after();
             const uint32_t sh = (uint32_t)ctrl->groups[g].shift[t] * 8;
             const uint32_t b_lo = b_base + bslot * b_step;
-            const uint32_t first = (uint32_t)(g != g_lo || t != 0);
+            const uint32_t first = (uint32_t)(g != g_first || t != 0);
             const uint64_t db = desc_hi | b_lo;
 #pragma unroll
             for (int k = 0; k < 4; ++k) {                         // +32 B inside the swizzle atom per K = 16
@@ -155,7 +190,8 @@ __device__ __forceinline__ void mma_issuer(Ctrl* ctrl, const GemmDev& p, const G
           if (i0 + IL >= MT) { bslot0 = bslot; bphase0 = bphase; }
         }
       }
-      b_ready = true;
+      // resident weights: a tile that ran every group has waited on the barrier of every k-block
+      if (lg.e0 - lg.s0 + lg.e1 - lg.s1 == g_hi - g_lo) b_ready = true;
       if (CTA2) ptx::umma_commit_2sm(&ctrl->tmem_full[acc]); else ptx::umma_commit(&ctrl->tmem_full[acc]);
     }
     if (p.debug_stats) {
@@ -608,10 +644,14 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     const int gper = (num_groups + p.ksplit - 1) / p.ksplit;
     for (int tile = blockIdx.x >> cta_shift; tile < num_tiles; tile += gridDim.x >> cta_shift) {
       const int mtile = (tile / p.ksplit) / n_tiles;
-      const int tchunk = mtile / p.Ho;
-      const int m0 = (mtile - tchunk * p.Ho) * p.plane_pitch + tchunk * tile_rows + (int)rank * 128;
+      const int tchunk = mtile / p.Ho, ho = mtile - tchunk * p.Ho;
+      const int m0 = ho * p.plane_pitch + tchunk * tile_rows + (int)rank * 128;
       const int g_lo = (tile % p.ksplit) * gper, g_hi = min(num_groups, g_lo + gper);
-      for (int g = g_lo; g < g_hi; ++g) {
+      const LiveGroups lg(__ldg(p.row_groups + ho), g_lo, g_hi);      // the issuer's groups, in its order
+      int gb = lg.s0, ge = lg.e0;
+#pragma unroll 1
+      for (int pass = 0; pass < 2; ++pass, gb = lg.s1, ge = lg.e1)
+      for (int g = gb; g < ge; ++g) {
         const int row_off = ctrl->groups[g].row_off, col = ctrl->groups[g].col, map = ctrl->groups[g].map;
         uint64_t* gbar = &ctrl->a_full[slot];               // the group's slabs complete on its first slab's barrier
         for (int i = 0; i < MT; ++i) {
@@ -647,10 +687,16 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     } else {
       uint32_t slot = 0, phase = 0;
       const int gper = (num_groups + p.ksplit - 1) / p.ksplit;
-      for (int tile = blockIdx.x >> cta_shift; tile < num_tiles; tile += gridDim.x >> cta_shift) {
+      const int step = gridDim.x >> cta_shift;
+      TileRow row(blockIdx.x >> cta_shift, step, p.ksplit * n_tiles, p.Ho);
+      for (int tile = blockIdx.x >> cta_shift; tile < num_tiles; tile += step, row.next()) {
         const int n0 = ((tile / p.ksplit) % n_tiles) * p.BN + (int)rank * (p.BN >> 1) * cta_shift;
         const int g_lo = (tile % p.ksplit) * gper, g_hi = min(num_groups, g_lo + gper);
-        for (int g = g_lo; g < g_hi; ++g) {
+        const LiveGroups lg(__ldg(p.row_groups + row.ho), g_lo, g_hi);   // the issuer's groups, in its order
+        int gb = lg.s0, ge = lg.e0;
+#pragma unroll 1
+        for (int pass = 0; pass < 2; ++pass, gb = lg.s1, ge = lg.e1)
+        for (int g = gb; g < ge; ++g) {
           const int ntaps = ctrl->groups[g].ntaps;
           // all B tiles of a group complete on the barrier of the group's first slot (one wait per group in the issuer)
           uint64_t* gbar = &ctrl->b_full[slot];
@@ -677,11 +723,11 @@ gemm_shift_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_consta
     if (rank != 0) {
       // the peer CTA of a pair only lends its shared memory / TMEM; the leader issues for both
     } else if (cfg.resident) {
-      if (cfg.il == 2) mma_issuer<2, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
-      else mma_issuer<1, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
+      if (cfg.il == 2) mma_issuer<2, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, n_tiles, b_bytes);
+      else mma_issuer<1, CTA2, true>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, n_tiles, b_bytes);
     } else {
-      if (cfg.il == 2) mma_issuer<2, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
-      else mma_issuer<1, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, b_bytes);
+      if (cfg.il == 2) mma_issuer<2, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, n_tiles, b_bytes);
+      else mma_issuer<1, CTA2, false>(ctrl, p, cfg, smem_a, smem_b, tmem_base, num_tiles, n_tiles, b_bytes);
     }
   } else {
     // ===================== epilogue (warps 0..7) =====================
@@ -759,7 +805,7 @@ cudaError_t launch_flavour(cudaStream_t s, int grid, int smem, const CUtensorMap
 cudaError_t launch_gemm(cudaStream_t s, int n_sm, const CUtensorMap& mapA0, const CUtensorMap& mapA1,
                         const CUtensorMap& mapB_full, const CUtensorMap& mapB_half, const GemmDev& p) {
   if (p.M <= 0) return cudaSuccess;
-  if (p.num_groups > kMaxGroups || p.BN % 16 != 0 || p.BN > 256 || p.N % p.BN != 0) return cudaErrorInvalidValue;
+  if (p.num_groups > kMaxGroups || !p.row_groups || p.BN % 16 != 0 || p.BN > 256 || p.N % p.BN != 0) return cudaErrorInvalidValue;
   const EpiDev& e = p.epi;
   GemmCfg cfg;
   // row-per-thread epilogue for the 64/128-channel layers, transposing epilogue for BN = 256 and the head

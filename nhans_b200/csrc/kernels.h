@@ -69,6 +69,7 @@ struct GemmDev {
   int num_kb;               // k-blocks (64 wide) of the packed weights
   int num_groups;
   const KGroupDev* groups;
+  const uint32_t* row_groups;   // [Ho]: groups a tile of output row ho runs, [s0, e0) + [s1, e1) (plan.h GemmLayer)
   int Hq, Wq, Ho, Wo;
   UnitTable units;
   EpiDev epi;

@@ -246,9 +246,9 @@ struct Builder {
     }
   }
 
-  // Appends the k-blocks and packed weights of a (kh x kw) convolution tap set reading grid `src`
-  // (A map `map`) with top/left pads (pt, pl); weights w[kh][kw][Cin][C] scaled per output channel.
-  void add_conv_taps(GemmLayer* L, const Grid& src, int map, const std::vector<float>& wt, int kh, int kw,
+  // Appends the k-blocks and packed weights of a (kh x kw) convolution tap set with vertical stride sh reading grid
+  // `src` (A map `map`) with top/left pads (pt, pl); weights w[kh][kw][Cin][C] scaled per output channel.
+  void add_conv_taps(GemmLayer* L, const Grid& src, int map, const std::vector<float>& wt, int kh, int kw, int sh,
                      int Cin, int C, int pt, int pl, const std::vector<double>& scale) {
     int k0 = (int)L->kb.size() * kTileK;
     L->a_rowlen[map] = Cin;
@@ -258,16 +258,24 @@ struct Builder {
     std::vector<uint16_t> nw((size_t)L->N * Knew, 0);
     for (int n = 0; n < L->N; ++n)
       for (int k = 0; k < k0; ++k) nw[(size_t)n * Knew + k] = L->w[(size_t)n * k0 + k];
-    for (int i = 0; i < kh; ++i)
+    for (int i = 0; i < kh; ++i) {
+      // output rows whose input row ho * sh + i - pt lies inside the source image (a contiguous range)
+      int lo = L->Ho, hi = 0;
+      for (int ho = 0; ho < L->Ho; ++ho) {
+        const int y = ho * sh + i - pt;
+        if (y >= 0 && y < src.H) { lo = std::min(lo, ho); hi = ho + 1; }
+      }
+      if (lo >= hi) lo = hi = 0;
       for (int j = 0; j < kw; ++j) {
         int32_t off = tap_offset(src, i - pt, j - pl);
-        for (int c0 = 0; c0 < Cin; c0 += kTileK) L->kb.push_back({off, (int16_t)map, (int16_t)c0});
+        for (int c0 = 0; c0 < Cin; c0 += kTileK) L->kb.push_back({off, (int16_t)map, (int16_t)c0, (int16_t)lo, (int16_t)hi});
         for (int c = 0; c < Cin; ++c)
           for (int n = 0; n < C; ++n) {
             double v = (double)wt[(((size_t)i * kw + j) * Cin + c) * C + n] * scale[n];
             nw[(size_t)n * Knew + k0 + (i * kw + j) * Cin + c] = f32_to_f16_bits((float)v);
           }
       }
+    }
     L->w.swap(nw);
     L->K = Knew;
   }
@@ -315,7 +323,7 @@ struct Builder {
       L.Hq = g.Hq; L.Wq = g.Wq; L.Ho = g.Ho; L.Wo = g.Wo;
       L.a_buf[0] = x.buf;
       L.N = C;
-      add_conv_taps(&L, x, 0, w1, b.kh, b.kw, Cin, C, g.pt, g.pl, bn1.s);
+      add_conv_taps(&L, x, 0, w1, b.kh, b.kw, b.sh, Cin, C, g.pt, g.pl, bn1.s);
       L.BN = pick_bn(L.N);
       L.epi = e1;
       L.out = h;
@@ -331,7 +339,7 @@ struct Builder {
     L.Hq = g.Hq; L.Wq = g.Wq; L.Ho = g.Ho; L.Wo = g.Wo;
     L.a_buf[0] = h.buf;
     L.N = C;
-    add_conv_taps(&L, h, 0, w2, b.kh, b.kw, C, C, g.pt2, g.pl2, bnA.s);
+    add_conv_taps(&L, h, 0, w2, b.kh, b.kw, 1, C, C, g.pt2, g.pl2, bnA.s);
     L.BN = pick_bn(L.N);
     L.macs_per_unit = (double)g.Ho * g.Wo * b.kh * b.kw * C * C;
     std::vector<double> constant(C);
@@ -353,7 +361,7 @@ struct Builder {
         e2.r1_sh = b.sh; e2.r1_sw = b.sw; e2.raw_oh = raw_oh;
       } else {
         L.a_buf[1] = x.buf;
-        add_conv_taps(&L, x, 1, wt, 1, 1, Cin, C, 0, 0, bnA.s);
+        add_conv_taps(&L, x, 1, wt, 1, 1, b.sh, Cin, C, 0, 0, bnA.s);      // pixel (ho sh, wo sw): every row live
       }
       L.macs_per_unit += (double)g.Ho * g.Wo * Cin * C;
     }
@@ -432,13 +440,16 @@ void build_groups(GemmLayer* L) {
   }
   L->subnormal_frac = nz ? (double)sub / (double)nz : 0.0;
   L->groups.clear();
+  if (L->Ho > 255) throw std::runtime_error(L->name + ": more than 255 output rows");
   const int n = (int)L->kb.size();
   std::vector<char> used(n, 0);
+  double live_rows = 0;                    // sum over k-blocks of the output rows they run for
   for (int a = 0; a < n; ++a) {
     if (used[a]) continue;
     KGroup g{};
     g.row_off = L->kb[a].row_off; g.map = L->kb[a].map; g.col = L->kb[a].col;
     g.ntaps = 0;
+    int lo = L->Ho, hi = 0;
     // taps of the same source / channel chunk whose rows lie within 7 rows above the first one
     for (int b = a; b < n && g.ntaps < 4; ++b) {
       if (used[b] || L->kb[b].map != g.map || L->kb[b].col != g.col) continue;
@@ -448,9 +459,42 @@ void build_groups(GemmLayer* L) {
       g.bk[g.ntaps] = b;
       g.ntaps++;
       used[b] = 1;
+      // the group is dead for a row only if every tap is (taps of one kernel row share their range)
+      if (L->kb[b].ho_lo < L->kb[b].ho_hi) { lo = std::min(lo, (int)L->kb[b].ho_lo); hi = std::max(hi, (int)L->kb[b].ho_hi); }
     }
+    if (lo >= hi) lo = hi = 0;
+    g.ho_lo = (uint8_t)lo; g.ho_hi = (uint8_t)hi;
+    live_rows += (double)g.ntaps * (hi - lo);
     L->groups.push_back(g);
   }
+  // the live groups of every output row as (at most) two index ranges
+  const int G = (int)L->groups.size();
+  if (G > 255) throw std::runtime_error(L->name + ": more than 255 k-groups");
+  L->row_groups.assign(L->Ho, 0u);
+  for (int ho = 0; ho < L->Ho; ++ho) {
+    int s[2] = {0, 0}, e[2] = {0, 0}, runs = 0;
+    for (int j = 0; j < G; ++j) {
+      if (ho < L->groups[j].ho_lo || ho >= L->groups[j].ho_hi) continue;
+      if (runs > 0 && e[runs - 1] == j) { e[runs - 1] = j + 1; continue; }
+      if (runs == 2) throw std::runtime_error(L->name + ": the live groups of a row form more than two ranges");
+      s[runs] = j; e[runs] = j + 1; ++runs;
+    }
+    if (runs == 0) throw std::runtime_error(L->name + ": output row " + std::to_string(ho) + " reads only padding");
+    L->row_groups[ho] = (uint32_t)s[0] | (uint32_t)e[0] << 8 | (uint32_t)s[1] << 16 | (uint32_t)e[1] << 24;
+  }
+  // a k-block skipped for one output row saves 64 x N x Wo MACs (the rank-1 term of macs_per_unit has no k-block)
+  L->exec_macs_per_unit = L->macs_per_unit - ((double)n * L->Ho - live_rows) * kTileK * L->N * L->Wo;
+}
+
+bool every_split_live(const GemmLayer& L, int ksplit) {
+  const int G = (int)L.groups.size(), gper = (G + ksplit - 1) / ksplit;
+  for (int sp = 0; sp < ksplit; ++sp)
+    for (int ho = 0; ho < L.Ho; ++ho) {
+      bool any = false;
+      for (int j = sp * gper; j < std::min(G, (sp + 1) * gper); ++j) any |= (ho >= L.groups[j].ho_lo && ho < L.groups[j].ho_hi);
+      if (!any) return false;
+    }
+  return true;
 }
 
 static std::string grid_json(const Grid& g) {
@@ -474,10 +518,26 @@ std::string plan_to_json(const NetPlan& p) {
     char b[512];
     snprintf(b, sizeof b,
              "%s{\"name\":\"%s\",\"Hq\":%d,\"Wq\":%d,\"Ho\":%d,\"Wo\":%d,\"N\":%d,\"BN\":%d,\"K\":%d,\"a_buf\":[%d,%d],"
-             "\"res_buf\":%d,\"cond_off\":%d,\"groups\":%d,\"macs\":%.1f,\"walk\":%d,\"out\":",
-             i ? "," : "", L.name.c_str(), L.Hq, L.Wq, L.Ho, L.Wo, L.N, L.BN, L.K, L.a_buf[0], L.a_buf[1], L.epi.res_buf,
-             L.epi.cond_off, (int)L.groups.size(), L.macs_per_unit, L.walk);
-    s += b + grid_json(L.out) + "}";
+             "\"a_rowlen\":[%d,%d],\"res_buf\":%d,\"cond_off\":%d,\"groups\":%d,\"macs\":%.1f,\"exec_macs\":%.1f,\"walk\":%d,"
+             "\"group_list\":[",
+             i ? "," : "", L.name.c_str(), L.Hq, L.Wq, L.Ho, L.Wo, L.N, L.BN, L.K, L.a_buf[0], L.a_buf[1], L.a_rowlen[0],
+             L.a_rowlen[1], L.epi.res_buf, L.epi.cond_off, (int)L.groups.size(), L.macs_per_unit, L.exec_macs_per_unit, L.walk);
+    s += b;
+    for (size_t j = 0; j < L.groups.size(); ++j) {
+      const KGroup& g = L.groups[j];
+      std::string sh;
+      for (int t = 0; t < g.ntaps; ++t) sh += (t ? "," : "") + std::to_string(g.shift[t]);
+      snprintf(b, sizeof b, "%s{\"row_off\":%d,\"map\":%d,\"col\":%d,\"shift\":[%s],\"ho\":[%d,%d]}", j ? "," : "", g.row_off,
+               g.map, g.col, sh.c_str(), g.ho_lo, g.ho_hi);
+      s += b;
+    }
+    s += "],\"row_groups\":[";
+    for (size_t j = 0; j < L.row_groups.size(); ++j) {
+      const uint32_t r = L.row_groups[j];
+      snprintf(b, sizeof b, "%s[%u,%u,%u,%u]", j ? "," : "", r & 0xffu, (r >> 8) & 0xffu, (r >> 16) & 0xffu, r >> 24);
+      s += b;
+    }
+    s += "],\"out\":" + grid_json(L.out) + "}";
   }
   s += "]}";
   return s;
@@ -511,7 +571,7 @@ NetPlan build_main_plan(const WeightMap& w, int variant, int capacity) {
     L.a_buf[0] = head_buf;
     L.a_rowlen[0] = 2560;
     L.N = 512; L.BN = 256; L.K = 2560;
-    for (int k = 0; k < 2560; k += kTileK) L.kb.push_back({0, 0, (int16_t)k});
+    for (int k = 0; k < 2560; k += kTileK) L.kb.push_back({0, 0, (int16_t)k, 0, 1});
     L.w.resize((size_t)512 * 2560);
     for (int n = 0; n < 512; ++n)
       for (int k = 0; k < 2560; ++k)     // k = h * 512 + c ; w[h][0][c][n]
@@ -535,7 +595,7 @@ NetPlan build_main_plan(const WeightMap& w, int variant, int capacity) {
     L.a_buf[0] = P.gemm.back().out.buf;
     L.a_rowlen[0] = 13312;
     L.N = 208; L.BN = 208; L.K = 13312;
-    for (int k = 0; k < 13312; k += kTileK) L.kb.push_back({0, 0, (int16_t)k});
+    for (int k = 0; k < 13312; k += kTileK) L.kb.push_back({0, 0, (int16_t)k, 0, 1});
     L.w.assign((size_t)208 * 13312, 0);
     // last_dense is zero-initialised and trained with a small learning rate (main.py:238): real checkpoints may
     // hold values below the fp16 normal range (6.1e-5).  Every output column is therefore scaled by a power of

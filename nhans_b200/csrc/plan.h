@@ -67,17 +67,21 @@ struct KBlock {                   // one 64-wide k-block of a GemmLayer
   int32_t row_off;                // pixel offset added to the tile's first row
   int16_t map;                    // 0: A0, 1: A1
   int16_t col;                    // first channel
+  int16_t ho_lo, ho_hi;           // output rows [ho_lo, ho_hi) whose kernel row of this tap lies inside the source image;
+                                  // for the other rows the tap reads only vertical padding (zeros)
 };
 
 // A group of up to 4 k-blocks whose A rows differ only by a small row shift (the kw taps of one kernel row
 // and one 64-channel chunk): the engine loads ONE slab of 128 + 8 rows and feeds every tap from it through
 // row-shifted UMMA descriptors, so A is fetched from L2 once per kernel row instead of once per tap.
+// A tile of output row ho runs the group only if ho_lo <= ho < ho_hi (the union of its taps' ranges): for the
+// other rows every A row the group reads is padding, so skipping it leaves every fp32 sum bit for bit the same.
 struct KGroup {
   int32_t row_off;                // row offset of shift 0
   int16_t map;                    // 0: A0, 1: A1
   int16_t col;                    // first channel
   int16_t ntaps;
-  int16_t pad_;
+  uint8_t ho_lo, ho_hi;           // live output rows [ho_lo, ho_hi)
   int16_t shift[4];               // extra rows of tap t (0..7)
   int32_t bk[4];                  // k-block index of tap t in the packed weights
 };
@@ -109,10 +113,15 @@ struct GemmLayer {
   int K = 0;                              // 64 * kb.size()
   std::vector<KBlock> kb;
   std::vector<KGroup> groups;             // kb regrouped for slab reuse (same k-blocks, same order of B)
+  // [Ho]: the groups a tile of output row ho runs, as two index ranges s0 | e0 << 8 | s1 << 16 | e1 << 24 =
+  // [s0, e0) + [s1, e1) (groups are ordered by kernel row, so the live conv groups are one range and the 1x1
+  // transform groups, live for every row, the other)
+  std::vector<uint32_t> row_groups;
   std::vector<uint16_t> w;                // fp16 bits, [N][K] (K contiguous)
   Epilogue epi;
   Grid out;                               // out.buf < 0 for the head
   double macs_per_unit = 0;               // algorithmic MACs per window / context row (SURVEY App. B)
+  double exec_macs_per_unit = 0;          // the part of them the engine executes: k-blocks of live groups only
   // Row-walk eligible (conv_walk.cu): a stride-1 4 x 4 convolution with 64 channels in and out and no second A
   // source.  The k-blocks / weights above stay valid (plain N = 64 GEMM, what the CPU interpreter executes); the
   // engine repacks the weights as [kernel row block][cout] x [kw][cin] and walks the image rows instead.
@@ -161,8 +170,12 @@ NetPlan build_tower_plan(const WeightMap& w, int capacity);
 // TF 'SAME' padding: out = ceil(n / s), pad = max((out - 1) s + k - n, 0), before = pad / 2
 void same_pads(int n, int k, int s, int* out, int* before, int* after);
 
-// Regroups L->kb into L->groups (call once the k-block list is complete).
+// Regroups L->kb into L->groups and fills L->row_groups (call once the k-block list is complete).
 void build_groups(GemmLayer* L);
+
+// Split-K over ksplit consecutive slices of ceil(groups / ksplit) groups (gemm_tc.cu): does every slice run at least
+// one group for every output row?  A slice that runs none would publish an accumulator no MMA has written.
+bool every_split_live(const GemmLayer& L, int ksplit);
 
 // JSON description of a plan (geometry only, no weights) for tests and DESIGN tables.
 std::string plan_to_json(const NetPlan& p);

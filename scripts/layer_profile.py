@@ -40,8 +40,12 @@ print('clocks under load: median sm %.0f MHz, median power %.0f W (%d samples)' 
 layers = eng.profile_layers(0)
 tot = sum(l["ms"] for l in layers)
 print("%d x %.0f s: %.1f ms/run -> %.1f audio-s/s" % (utts, secs, ms / 2, utts * secs / (ms / 2e3)))
-for l in layers:
-    print("%-22s K=%5d N=%3d  %8.2f ms  %5.1f%%  %7.1f TFLOP/s" % (l["name"], l["K"], l["N"], l["ms"] / 6, 100 * l["ms"] / tot, l["tflops"]))
+# TFLOP/s counts the algorithmic MACs (TF's, padding included); exec counts the MACs the kernels run, without the
+# kernel rows that fall into vertical padding (the plan of an older library has no `exec_macs`: exec = TFLOP/s there)
+for l, pg in zip(layers, eng.plan(0)["gemm"]):
+    l["exec_tflops"] = l["tflops"] * pg.get("exec_macs", pg["macs"]) / pg["macs"]
+    print("%-22s K=%5d N=%3d  %8.2f ms  %5.1f%%  %7.1f exec  %7.1f TFLOP/s" % (l["name"], l["K"], l["N"], l["ms"] / 6, 100 * l["ms"] / tot,
+                                                                            l["exec_tflops"], l["tflops"]))
 st = eng.profile_get(0)
 print("all GEMM layers: %.1f ms, %.1f TFLOP/s;  direct conv %.1f ms" % (st["ms"] / 6, st["flops"] / st["ms"] / 1e9, eng.profile_get(3)["ms"] / 6))
 if json_out:
