@@ -15,6 +15,7 @@
 #include <type_traits>
 #include <unordered_map>
 #include <unordered_set>
+#include <utility>
 #include <vector>
 
 #include "kernels.h"
@@ -30,24 +31,27 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+// One device allocation, freed by its owner's destructor.
 struct DBuf {
   void* p = nullptr;
   size_t cap = 0;
-  cudaError_t ensure(size_t bytes) {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-    size_t want = bytes + bytes / 8 + 256;
-    cudaError_t e = cudaMalloc(&p, want);
-    if (e == cudaSuccess) cap = want;
+  DBuf() = default;
+  DBuf(DBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+  DBuf& operator=(DBuf&& o) noexcept {   // the old allocation goes with `o`
+    std::swap(p, o.p);
+    std::swap(cap, o.cap);
+    return *this;
+  }
+  ~DBuf() { if (p) cudaFree(p); }
+  // replaces the allocation by one of exactly `bytes` (contents not kept)
+  cudaError_t alloc(size_t bytes) {
+    *this = DBuf();
+    cudaError_t e = cudaMalloc(&p, bytes);
+    if (e == cudaSuccess) cap = bytes; else p = nullptr;
     return e;
   }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-  }
+  // at least `bytes`, reallocated with 1/8 of headroom only when too small
+  cudaError_t ensure(size_t bytes) { return bytes <= cap ? cudaSuccess : alloc(bytes + bytes / 8 + 256); }
   template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
@@ -73,7 +77,7 @@ struct NetDev {
   float* convC = nullptr;           // main net: per-frame first-convolution table (kernels.h FrameConvDev)
   float* head_scratch = nullptr;    // main net: split-K partial sums of last_dense [kHeadSplit][capacity][208]
   long long crow_cap = 0;
-  std::vector<void*> allocs;
+  std::vector<DBuf> allocs;         // every device allocation above (net_alloc)
   bool ready = false;
 };
 
@@ -113,9 +117,6 @@ struct Geometry {
 // their embeddings and the conditioning table [U][n_cols].
 struct CondBufs {
   DBuf peak_a, peak_b, ctxlm_a, ctxlm_b, emb_a, emb_b, cond;
-  void release() {
-    for (DBuf* d : {&peak_a, &peak_b, &ctxlm_a, &ctxlm_b, &emb_a, &emb_b, &cond}) d->release();
-  }
 };
 
 struct Batch {
@@ -152,15 +153,6 @@ struct Streams {
   CondBufs cb;
   DBuf pcm, desc, new_lm, new_ph, seg_lm, seg_ph, den_win, den_seg, cond, out_i16, out_f32;   // nhans_stream_step
   DBuf factor, mixed, removed, comp, sums;                                                   // nhans_stream_step_post
-  void release() {
-    for (DBuf* d : {&pool, &ctx_a, &ctx_b, &ctx_offs, &pcm, &desc, &new_lm, &new_ph, &seg_lm, &seg_ph, &den_win,
-                    &den_seg, &cond, &out_i16, &out_f32, &factor, &mixed, &removed, &comp, &sums})
-      d->release();
-    cb.release();
-    rec.clear();
-    free_slots.clear();
-    n_slots = 0;
-  }
 };
 
 }  // namespace
@@ -196,6 +188,20 @@ struct nhans_ctx {
   bool use_gen = true;              // resblock1_1_conv2 builds its A operand from the per-frame table (NHANS_NO_GEN=1: window_expand)
   double layer_acc[128][4] = {};
   double launches = 0;              // every kernel launched by this context (counted even when not profiling)
+  // Also runs on a context nhans_create gave up on, whose later handles are still null.  The device buffers go with
+  // their DBufs.
+  ~nhans_ctx() {
+    for (IoSlot& io : batch.io)
+      for (cudaEvent_t ev : {io.uploaded, io.consumed, io.drained}) if (ev) cudaEventDestroy(ev);
+    for (cudaEvent_t ev : events) if (ev) cudaEventDestroy(ev);
+    for (auto& r : prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
+    for (cudaEvent_t ev : ev_pool) cudaEventDestroy(ev);
+    for (auto& t : tl) for (cudaEvent_t ev : t) if (ev) cudaEventDestroy(ev);
+    if (tl_origin) cudaEventDestroy(tl_origin);
+    if (err_flag_host) cudaFreeHost(err_flag_host);
+    if (debug_stats) cudaFree(debug_stats);
+    for (cudaStream_t s : {stream, h2d_stream, d2h_stream}) if (s) cudaStreamDestroy(s);
+  }
 };
 
 namespace {
@@ -213,15 +219,23 @@ int fail(nhans_ctx* c, int code, const std::string& msg) {
                                            std::to_string(__LINE__) + ")");                              \
   } while (0)
 
+// n elements of device memory owned by `net`, zeroed on the compute stream when `zero`.
+template <class T>
+int net_alloc(nhans_ctx* ctx, NetDev& net, size_t n, T** out, bool zero = false) {
+  net.allocs.emplace_back();
+  DBuf& d = net.allocs.back();
+  CK(d.alloc(n * sizeof(T)));
+  if (zero) CK(cudaMemsetAsync(d.p, 0, n * sizeof(T), ctx->stream));
+  *out = d.as<T>();
+  return 0;
+}
+
 template <class T>
 int upload(nhans_ctx* ctx, NetDev& net, const std::vector<T>& h, T** out) {
   *out = nullptr;
   if (h.empty()) return 0;
-  void* p = nullptr;
-  CK(cudaMalloc(&p, h.size() * sizeof(T)));
-  net.allocs.push_back(p);
-  CK(cudaMemcpyAsync(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-  *out = reinterpret_cast<T*>(p);
+  if (int rc = net_alloc(ctx, net, h.size(), out)) return rc;
+  CK(cudaMemcpyAsync(*out, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
   return 0;
 }
 
@@ -239,29 +253,14 @@ int make_map(nhans_ctx* ctx, CUtensorMap* map, const void* base, long long cols,
   return 0;
 }
 
-void free_net(NetDev& net) {
-  for (void* p : net.allocs) cudaFree(p);
-  net.allocs.clear();
-  net.bufs.clear();
-  net.layers.clear();
-  net.ready = false;
-}
-
 // Allocates the activation grids (zeroed once: padding positions are never written afterwards), uploads
 // packed weights and epilogue tables, encodes the TMA descriptors.
 int realise_net(nhans_ctx* ctx, NetDev& net) {
   const NetPlan& P = net.plan;
-  net.bufs.assign(P.bufs.size(), nullptr);
-  for (size_t i = 0; i < P.bufs.size(); ++i) {
-    const Grid& g = P.bufs[i];
-    size_t bytes = (size_t)g.pixels * g.C * sizeof(__half);
-    void* p = nullptr;
-    CK(cudaMalloc(&p, bytes));
-    net.allocs.push_back(p);
-    CK(cudaMemsetAsync(p, 0, bytes, ctx->stream));
-    net.bufs[i] = reinterpret_cast<__half*>(p);
-  }
   int rc;
+  net.bufs.assign(P.bufs.size(), nullptr);
+  for (size_t i = 0; i < P.bufs.size(); ++i)
+    if ((rc = net_alloc(ctx, net, (size_t)P.bufs[i].pixels * P.bufs[i].C, &net.bufs[i], true))) return rc;
   if (P.cond.n_cols > 0) {
     // main net: its first convolution runs once per frame (kernels.h FrameConvDev), which needs this shape
     const DirectLayer& D = P.first;
@@ -271,17 +270,10 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
     // per-frame table: a pass's windows plus 34 virtual frames per utterance it touches.  run_masknet sizes every pass
     // to fit, so utterances that average fewer than 17 frames run in smaller passes.
     net.crow_cap = 3LL * P.capacity + 64;
-    void* p = nullptr;
-    CK(cudaMalloc(&p, (size_t)4 * net.crow_cap * kBins * 64 * sizeof(float)));
-    net.allocs.push_back(p);
-    net.convC = reinterpret_cast<float*>(p);
+    if ((rc = net_alloc(ctx, net, (size_t)4 * net.crow_cap * kBins * 64, &net.convC))) return rc;
   }
-  if (P.cond.n_cols > 0 && !P.gemm.empty() && P.gemm.back().epi.head && !getenv("NHANS_NO_SPLITK")) {
-    void* p = nullptr;
-    CK(cudaMalloc(&p, (size_t)kHeadSplit * P.capacity * P.gemm.back().N * sizeof(float)));
-    net.allocs.push_back(p);
-    net.head_scratch = reinterpret_cast<float*>(p);
-  }
+  if (P.cond.n_cols > 0 && !P.gemm.empty() && P.gemm.back().epi.head && !getenv("NHANS_NO_SPLITK"))
+    if ((rc = net_alloc(ctx, net, (size_t)kHeadSplit * P.capacity * P.gemm.back().N, &net.head_scratch))) return rc;
   if ((rc = upload(ctx, net, P.first.w, &net.first_w))) return rc;
   if ((rc = upload(ctx, net, P.first.epi.bias, &net.first_bias))) return rc;
   if ((rc = upload(ctx, net, P.first.epi.ttab16, &net.first_ttab16))) return rc;
@@ -293,13 +285,9 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
   for (size_t i = 0; i < P.gemm.size(); ++i) {
     const GemmLayer& L = P.gemm[i];
     GemmLayerDev& D = net.layers[i];
-    {
-      void* p = nullptr;
-      CK(cudaMalloc(&p, L.w.size() * 2));
-      net.allocs.push_back(p);
-      CK(cudaMemcpyAsync(p, L.w.data(), L.w.size() * 2, cudaMemcpyHostToDevice, ctx->stream));
-      D.w = reinterpret_cast<__half*>(p);
-    }
+    uint16_t* dw = nullptr;
+    if ((rc = upload(ctx, net, L.w, &dw))) return rc;
+    D.w = reinterpret_cast<__half*>(dw);
     std::vector<KGroupDev> groups(L.groups.size());
     for (size_t j = 0; j < groups.size(); ++j) {
       const KGroup& g = L.groups[j];
@@ -336,20 +324,14 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
           for (int co = 0; co < 64; ++co)
             for (int ci = 0; ci < 64; ++ci)
               ww[(size_t)((3 - kh) * 64 + co) * 256 + kw * 64 + ci] = L.w[(size_t)co * L.K + (kh * 4 + kw) * 64 + ci];
-      uint16_t* dw = nullptr;
       if ((rc = upload(ctx, net, ww, &dw))) return rc;
       CK(cudaStreamSynchronize(ctx->stream));          // `ww` is a temporary
       D.w_walk = reinterpret_cast<__half*>(dw);
       if ((rc = make_map(ctx, &D.mapBwalk, D.w_walk, 256, 256, 256))) return rc;
     }
   }
-  const int cap = P.capacity;
-  for (int** p : {&net.u_frame, &net.u_lo, &net.u_hi, &net.u_utt}) {
-    void* q = nullptr;
-    CK(cudaMalloc(&q, sizeof(int) * (size_t)cap));
-    net.allocs.push_back(q);
-    *p = reinterpret_cast<int*>(q);
-  }
+  for (int** p : {&net.u_frame, &net.u_lo, &net.u_hi, &net.u_utt})
+    if ((rc = net_alloc(ctx, net, P.capacity, p))) return rc;
   CK(cudaStreamSynchronize(ctx->stream));
   net.ready = true;
   return 0;
@@ -643,6 +625,13 @@ int check_kernel_flag(nhans_ctx* ctx) {
   return 0;
 }
 
+// Result of a call after waiting on its work (e): a kernel that gave up waiting explains the CUDA error it leaves.
+int finish(nhans_ctx* ctx, cudaError_t e) {
+  if (int rc = check_kernel_flag(ctx)) return rc;
+  CK(e);
+  return NHANS_OK;
+}
+
 int frames_of(long long n) { return n >= 400 ? (int)(1 + (n - 400) / 160) : 0; }
 
 // samples the inverse STFT returns for T frames
@@ -700,6 +689,22 @@ int need_weights(nhans_ctx* ctx) {
   return 0;
 }
 
+// ctx_a comes with its offsets, and only the selective-noise variant may leave it out (Silent.wav conditions instead).
+int check_contexts(nhans_ctx* ctx, const void* ctx_a, const int64_t* a_offs) {
+  if (ctx_a && !a_offs) return fail(ctx, NHANS_ERR_ARG, "ctx_a given without offsets");
+  if (!ctx_a && ctx->variant != NHANS_VARIANT_SELECTIVE_NOISE)
+    return fail(ctx, NHANS_ERR_ARG, "the separator needs both context recordings");
+  return 0;
+}
+
+// Copies the n samples of x from offs[0] on into d on `stream`.
+template <class T>
+int copy_clips(nhans_ctx* ctx, DBuf& d, const T* x, const int64_t* offs, long long n, cudaStream_t stream) {
+  CK(d.ensure(n * sizeof(T) + 32));
+  CK(cudaMemcpyAsync(d.p, x + offs[0], n * sizeof(T), cudaMemcpyHostToDevice, stream));
+  return 0;
+}
+
 // STFT of int16 PCM (scaled by 1 / (peak + 1e-6) on the fly) or of float samples (as they are)
 cudaError_t launch_stft_of(cudaStream_t s, const int16_t* pcm, const long long* offs, const long long* frame_offs, int U,
                            const int* peak, int max_frames, float* logmag, float* phase, bool phasor) {
@@ -714,17 +719,12 @@ cudaError_t launch_stft_of(cudaStream_t s, const float* x, const long long* offs
 template <class T>
 int stage_batch(nhans_ctx* ctx, IoSlot& io, const Geometry& g, const T* mix, const int64_t* mix_offs, const T* ctx_a,
                 const int64_t* a_offs, const T* ctx_b, const int64_t* b_offs, cudaStream_t stream) {
-  auto clips = [&](DBuf& d, const T* x, const int64_t* offs, long long n) {
-    CK(d.ensure(n * sizeof(T) + 32));
-    CK(cudaMemcpyAsync(d.p, x + offs[0], n * sizeof(T), cudaMemcpyHostToDevice, stream));
-    return 0;
-  };
   const int U = g.U;
   int rc;
-  if ((rc = clips(io.mix, mix, mix_offs, g.mix_offs[U]))) return rc;
-  if ((rc = clips(io.b, ctx_b, b_offs, g.b_offs[U]))) return rc;
+  if ((rc = copy_clips(ctx, io.mix, mix, mix_offs, g.mix_offs[U], stream))) return rc;
+  if ((rc = copy_clips(ctx, io.b, ctx_b, b_offs, g.b_offs[U], stream))) return rc;
   if (ctx_a) {
-    if ((rc = clips(io.a, ctx_a, a_offs, g.a_offs[U]))) return rc;
+    if ((rc = copy_clips(ctx, io.a, ctx_a, a_offs, g.a_offs[U], stream))) return rc;
     if ((rc = to_device_offs(ctx, io.d_a_offs, g.a_offs, stream))) return rc;
   }
   if ((rc = to_device_offs(ctx, io.d_mix_offs, g.mix_offs, stream))) return rc;
@@ -820,6 +820,18 @@ int run_fused(nhans_ctx* ctx, IoSlot& io) {
                      g.frame_offs.data(), nullptr, nullptr, U, b.cb.cond.as<float>(), b.den.as<float>());
 }
 
+// Inverse STFT on the compute stream of the batch staged in `io`: `spec` (batch.den or batch.logmag) with the
+// phasors of batch.phase -> out_f32 / out_i16 (either may be null).
+int batch_istft(nhans_ctx* ctx, const IoSlot& io, const DBuf& spec, float* out_f32, int16_t* out_i16) {
+  const Batch& b = ctx->batch;
+  const Geometry& g = b.geo;
+  // spectrum + phasors read, samples written
+  ProfScope ps(ctx, 2, 0, 3.0 * 4 * kBins * g.total_frames + ((out_f32 ? 4.0 : 0.0) + (out_i16 ? 2.0 : 0.0)) * g.total_out);
+  CK(launch_istft(ctx->stream, spec.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(), io.d_out_offs.as<long long>(),
+                  g.U, b.peak_mix.as<int>(), g.max_frames, out_f32, out_i16, true));
+  return 0;
+}
+
 // nhans_stft / nhans_stft_f32
 template <class T>
 int stft_entry(nhans_ctx* ctx, const T* x, const int64_t* offs, int U, float* logmag, float* phase, int64_t* frame_offs,
@@ -833,8 +845,7 @@ int stft_entry(nhans_ctx* ctx, const T* x, const int64_t* offs, int U, float* lo
   std::copy(g.frame_offs.begin(), g.frame_offs.end(), frame_offs);
   if (!logmag && !phase && !peak) return NHANS_OK;
   const long long total = g.mix_offs[U];
-  CK(ctx->tmp[0].ensure(total * sizeof(T) + 32));
-  CK(cudaMemcpyAsync(ctx->tmp[0].p, x + offs[0], total * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+  if ((rc = copy_clips(ctx, ctx->tmp[0], x, offs, total, ctx->stream))) return rc;
   if ((rc = to_device_offs(ctx, ctx->tmp[1], g.mix_offs))) return rc;
   if ((rc = to_device_offs(ctx, ctx->tmp[2], g.frame_offs))) return rc;
   const size_t sbytes = (size_t)g.total_frames * kBins * 4;
@@ -876,8 +887,7 @@ int alloc_slots(nhans_ctx* ctx, int n, std::vector<int>& slots) {
     CK(grown.ensure((size_t)want * stride * 4));
     if (S.n_slots) CK(cudaMemcpyAsync(grown.p, S.pool.p, (size_t)S.n_slots * stride * 4, cudaMemcpyDeviceToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    S.pool.release();
-    S.pool = grown;
+    S.pool = std::move(grown);
     S.slot_stride = stride;
     for (int i = want - 1; i >= S.n_slots; --i) S.free_slots.push_back(i);
     S.n_slots = want;
@@ -1043,9 +1053,7 @@ int stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const
     if (post->comp && n_out) CK(cudaMemcpyAsync(post->comp, S.comp.p, n_out * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(sums.data(), S.sums.p, sizeof(double) * 2 * n, cudaMemcpyDeviceToHost, st));
   }
-  cudaError_t e = cudaStreamSynchronize(st);
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
+  if ((rc = finish(ctx, cudaStreamSynchronize(st)))) return rc;
   for (int i = 0; i < n; ++i) {
     StreamRec& r = S.rec.at(ids[i]);
     const long long F0 = frames_of(r.n);
@@ -1129,32 +1137,7 @@ int nhans_create(int device, int variant, int win_capacity, int row_capacity, nh
 void nhans_destroy(nhans_ctx* ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->device);
-  cudaStreamSynchronize(ctx->stream);
-  free_net(ctx->main_net);
-  free_net(ctx->tower);
-  Batch& b = ctx->batch;
-  if (ctx->h2d_stream) cudaStreamSynchronize(ctx->h2d_stream);
-  if (ctx->d2h_stream) cudaStreamSynchronize(ctx->d2h_stream);
-  for (IoSlot& io : b.io) {
-    for (DBuf* d : {&io.mix, &io.a, &io.b, &io.d_mix_offs, &io.d_a_offs, &io.d_b_offs, &io.d_frame_offs, &io.d_out_offs,
-                    &io.d_ctx_frame_offs, &io.out_i16, &io.out_f32})
-      d->release();
-    for (cudaEvent_t ev : {io.uploaded, io.consumed, io.drained}) if (ev) cudaEventDestroy(ev);
-  }
-  for (DBuf* d : {&b.peak_mix, &b.logmag, &b.phase, &b.den, &b.mixproc, &b.removed, &b.comp, &b.sums, &b.snr, &ctx->silent_emb})
-    d->release();
-  b.cb.release();
-  ctx->streams.release();
-  for (auto& t : ctx->tmp) t.release();
-  for (auto& ev : ctx->events) if (ev) cudaEventDestroy(ev);
-  for (auto& r : ctx->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
-  for (auto& ev : ctx->ev_pool) cudaEventDestroy(ev);
-  for (auto& ev : ctx->tl) for (auto& e : ev) if (e) cudaEventDestroy(e);
-  if (ctx->tl_origin) cudaEventDestroy(ctx->tl_origin);
-  if (ctx->err_flag_host) cudaFreeHost(ctx->err_flag_host);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  if (ctx->h2d_stream) cudaStreamDestroy(ctx->h2d_stream);
-  if (ctx->d2h_stream) cudaStreamDestroy(ctx->d2h_stream);
+  for (cudaStream_t s : {ctx->stream, ctx->h2d_stream, ctx->d2h_stream}) cudaStreamSynchronize(s);
   delete ctx;
 }
 
@@ -1163,10 +1146,14 @@ int nhans_load_weights(nhans_ctx* ctx, const char* const* names, const int64_t* 
   CK(cudaSetDevice(ctx->device));
   WeightMap w;
   for (int i = 0; i < n; ++i) w[names[i]] = std::vector<float>(data[i], data[i] + sizes[i]);
-  free_net(ctx->main_net);
-  free_net(ctx->tower);
+  ctx->main_net = NetDev{};
+  ctx->tower = NetDev{};
   ctx->silent_ready = false;
-  ctx->streams.release();           // their conditioning rows belong to the old weights
+  // open streams end, since their conditioning rows belong to the old weights; ids go on counting, so that an id from
+  // before the reload never names a new stream
+  const int next_id = ctx->streams.next_id;
+  ctx->streams = Streams{};
+  ctx->streams.next_id = next_id;
   try {
     ctx->main_net.plan = build_main_plan(w, ctx->variant, ctx->win_cap);
     ctx->tower.plan = build_tower_plan(w, ctx->row_cap);
@@ -1205,12 +1192,10 @@ int nhans_normalise(nhans_ctx* ctx, const int16_t* pcm, const int64_t* offs, int
     if (trim && n >= 400) n -= (n - 400) % 160;
     oo[u + 1] = oo[u] + n;
   }
-  const long long total = ho[U] - ho[0];
-  CK(ctx->tmp[0].ensure(total * 2 + 32));
-  CK(cudaMemcpyAsync(ctx->tmp[0].p, pcm + ho[0], total * 2, cudaMemcpyHostToDevice, ctx->stream));
+  int rc;
+  if ((rc = copy_clips(ctx, ctx->tmp[0], pcm, offs, ho[U] - ho[0], ctx->stream))) return rc;
   std::vector<long long> rel(U + 1);
   for (int u = 0; u <= U; ++u) rel[u] = ho[u] - ho[0];
-  int rc;
   if ((rc = to_device_offs(ctx, ctx->tmp[1], rel))) return rc;
   if ((rc = to_device_offs(ctx, ctx->tmp[2], oo))) return rc;
   CK(ctx->tmp[3].ensure(sizeof(int) * U));
@@ -1264,10 +1249,7 @@ int nhans_embed(nhans_ctx* ctx, const float* ctx_logmag, int R, float* emb) {
   CK(cudaMemcpyAsync(ctx->tmp[0].p, ctx_logmag, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
   if ((rc = run_tower(ctx, ctx->tmp[0].as<float>(), R, ctx->tmp[1].as<float>()))) return rc;
   CK(cudaMemcpyAsync(emb, ctx->tmp[1].p, (size_t)R * 512 * 4, cudaMemcpyDeviceToHost, ctx->stream));
-  cudaError_t e = cudaStreamSynchronize(ctx->stream);
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
-  return NHANS_OK;
+  return finish(ctx, cudaStreamSynchronize(ctx->stream));
 }
 
 int nhans_masknet(nhans_ctx* ctx, const float* logmag, const int64_t* frame_offs, int U, const float* emb_a,
@@ -1295,10 +1277,7 @@ int nhans_masknet(nhans_ctx* ctx, const float* logmag, const int64_t* frame_offs
                         nullptr, nullptr, U, ctx->tmp[4].as<float>(), ctx->tmp[1].as<float>())))
     return rc;
   CK(cudaMemcpyAsync(denoised, ctx->tmp[1].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
-  cudaError_t e = cudaStreamSynchronize(ctx->stream);
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
-  return NHANS_OK;
+  return finish(ctx, cudaStreamSynchronize(ctx->stream));
 }
 
 int nhans_istft(nhans_ctx* ctx, const float* logmag, const float* phase, const int64_t* frame_offs, int U,
@@ -1344,11 +1323,9 @@ int nhans_istft(nhans_ctx* ctx, const float* logmag, const float* phase, const i
 int nhans_upload(nhans_ctx* ctx, const int16_t* mix, const int64_t* mix_offs, int U, const int16_t* ctx_a,
                  const int64_t* a_offs, const int16_t* ctx_b, const int64_t* b_offs) {
   if (!ctx || !mix || !mix_offs || !ctx_b || !b_offs || U <= 0) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  if (ctx_a && !a_offs) return fail(ctx, NHANS_ERR_ARG, "ctx_a given without offsets");
-  if (!ctx_a && ctx->variant != NHANS_VARIANT_SELECTIVE_NOISE)
-    return fail(ctx, NHANS_ERR_ARG, "the separator needs both context recordings");
-  CK(cudaSetDevice(ctx->device));
   int rc;
+  if ((rc = check_contexts(ctx, ctx_a, a_offs))) return rc;
+  CK(cudaSetDevice(ctx->device));
   if ((rc = need_weights(ctx))) return rc;
   Batch& b = ctx->batch;
   b.staged = false; b.done = false;
@@ -1385,12 +1362,7 @@ int nhans_run(nhans_ctx* ctx) {
   if (io.d2h_pending) CK(cudaStreamWaitEvent(ctx->stream, io.drained, 0));
   tl_mark(ctx, 2, ctx->stream);
   if ((rc = run_fused<int16_t>(ctx, io))) return rc;
-  {
-    ProfScope ps(ctx, 2, 0, 3.0 * g.total_frames * kBins * 4 + 6.0 * g.total_out);
-    CK(launch_istft(ctx->stream, b.den.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
-                    io.d_out_offs.as<long long>(), g.U, b.peak_mix.as<int>(), g.max_frames, io.out_f32.as<float>(),
-                    io.out_i16.as<int16_t>(), true));
-  }
+  if ((rc = batch_istft(ctx, io, b.den, io.out_f32.as<float>(), io.out_i16.as<int16_t>()))) return rc;
   tl_mark(ctx, 3, ctx->stream);
   CK(cudaEventRecord(io.consumed, ctx->stream));
   b.done = true;
@@ -1406,9 +1378,8 @@ int nhans_download(nhans_ctx* ctx, int16_t* out_i16, float* out_f32, float* mixp
   IoSlot& io = b.io[b.cur];
   if (mixproc_f32) {
     // 'mixed_processed.wav' (SN/apply.py:457-458): iSTFT of the window centres, i.e. of the input spectrogram
-    ProfScope ps(ctx, 2, 0, 3.0 * g.total_frames * kBins * 4 + 4.0 * g.total_out);
-    CK(launch_istft(ctx->stream, b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
-                    io.d_out_offs.as<long long>(), g.U, b.peak_mix.as<int>(), g.max_frames, b.mixproc.as<float>(), nullptr, true));
+    int rc;
+    if ((rc = batch_istft(ctx, io, b.logmag, b.mixproc.as<float>(), nullptr))) return rc;
     CK(cudaMemcpyAsync(mixproc_f32, b.mixproc.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
   }
   // the outputs leave on their own stream, so that the next batch can start computing meanwhile
@@ -1438,7 +1409,7 @@ int nhans_postmix(nhans_ctx* ctx, float compensate, int ac, float* mixed_f32, fl
     ProfScope ps(ctx, 2, 0, 4.0 * g.total_frames * kBins * 4 + 12.0 * g.total_out);
     CK(launch_istft_post(ctx->stream, b.den.as<float>(), b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
                          io.d_out_offs.as<long long>(), g.U, g.max_frames, nullptr, b.mixproc.as<float>(), b.removed.as<float>(),
-                         b.sums.as<double>(), true));
+                         b.sums.as<double>()));
   }
   {
     ProfScope ps(ctx, 4, 0, 0);
@@ -1464,10 +1435,9 @@ int nhans_enhance_batch(nhans_ctx* ctx, const int16_t* mix, const int64_t* mix_o
 int nhans_enhance_f32(nhans_ctx* ctx, const float* mix, const int64_t* mix_offs, int U, const float* ctx_a, const int64_t* a_offs,
                       const float* ctx_b, const int64_t* b_offs, int start_frame, float* out_f32, float* mixproc_f32, int64_t* out_offs) {
   if (!ctx || !mix || !mix_offs || !ctx_b || !b_offs || !out_offs || U <= 0 || start_frame < 0) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  if (ctx_a && !a_offs) return fail(ctx, NHANS_ERR_ARG, "ctx_a given without offsets");
-  if (!ctx_a && ctx->variant != NHANS_VARIANT_SELECTIVE_NOISE) return fail(ctx, NHANS_ERR_ARG, "the separator needs both context recordings");
-  CK(cudaSetDevice(ctx->device));
   int rc;
+  if ((rc = check_contexts(ctx, ctx_a, a_offs))) return rc;
+  CK(cudaSetDevice(ctx->device));
   if ((rc = need_weights(ctx))) return rc;
   Geometry geo;
   if ((rc = batch_geometry(ctx, mix_offs, ctx_a ? a_offs : nullptr, b_offs, U, start_frame, geo))) return rc;
@@ -1487,25 +1457,17 @@ int nhans_enhance_f32(nhans_ctx* ctx, const float* mix, const int64_t* mix_offs,
   if ((rc = stage_batch(ctx, io, g, mix, mix_offs, ctx_a, a_offs, ctx_b, b_offs, st))) return rc;
   if (!b.has_a && (rc = ensure_silent(ctx))) return rc;
   if ((rc = run_fused<float>(ctx, io))) return rc;
-  const double istft_bytes = 3.0 * g.total_frames * kBins * 4 + 4.0 * g.total_out;
   CK(io.out_f32.ensure(g.total_out * 4 + 16));
   if (out_f32) {
-    ProfScope ps(ctx, 2, 0, istft_bytes);
-    CK(launch_istft(st, b.den.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(), io.d_out_offs.as<long long>(), U,
-                    b.peak_mix.as<int>(), g.max_frames, io.out_f32.as<float>(), nullptr, true));
+    if ((rc = batch_istft(ctx, io, b.den, io.out_f32.as<float>(), nullptr))) return rc;
     CK(cudaMemcpyAsync(out_f32, io.out_f32.p, g.total_out * 4, cudaMemcpyDeviceToHost, st));
   }
   if (mixproc_f32) {
     CK(b.mixproc.ensure(g.total_out * 4 + 16));
-    ProfScope ps(ctx, 2, 0, istft_bytes);
-    CK(launch_istft(st, b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(), io.d_out_offs.as<long long>(), U,
-                    b.peak_mix.as<int>(), g.max_frames, b.mixproc.as<float>(), nullptr, true));
+    if ((rc = batch_istft(ctx, io, b.logmag, b.mixproc.as<float>(), nullptr))) return rc;
     CK(cudaMemcpyAsync(mixproc_f32, b.mixproc.p, g.total_out * 4, cudaMemcpyDeviceToHost, st));
   }
-  cudaError_t e = cudaStreamSynchronize(st);
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
-  return NHANS_OK;
+  return finish(ctx, cudaStreamSynchronize(st));
 }
 
 int nhans_sync(nhans_ctx* ctx) {
@@ -1515,9 +1477,7 @@ int nhans_sync(nhans_ctx* ctx) {
   cudaError_t e1 = cudaStreamSynchronize(ctx->h2d_stream);
   cudaError_t e2 = cudaStreamSynchronize(ctx->d2h_stream);
   for (IoSlot& io : ctx->batch.io) io.d2h_pending = false;
-  int rc;
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
+  if (int rc = finish(ctx, e)) return rc;
   CK(e1);
   CK(e2);
   return NHANS_OK;
@@ -1530,9 +1490,7 @@ int nhans_sync_previous(nhans_ctx* ctx) {
   if (io.d2h_pending) {
     cudaError_t e = cudaEventSynchronize(io.drained);
     io.d2h_pending = false;
-    int rc;
-    if ((rc = check_kernel_flag(ctx))) return rc;
-    CK(e);
+    return finish(ctx, e);
   }
   return NHANS_OK;
 }
@@ -1679,12 +1637,11 @@ int nhans_stream_emit_len(int64_t before, int64_t after, int final, int64_t* emi
 int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t* a_offs, const int16_t* ctx_b,
                       const int64_t* b_offs, const int32_t* peak, int* ids) {
   if (!ctx || n <= 0 || n > 65535 || !ctx_b || !b_offs || !peak || !ids) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
-  if (ctx_a && !a_offs) return fail(ctx, NHANS_ERR_ARG, "ctx_a given without offsets");
-  if (!ctx_a && ctx->variant != NHANS_VARIANT_SELECTIVE_NOISE) return fail(ctx, NHANS_ERR_ARG, "the separator needs both context recordings");
+  int rc;
+  if ((rc = check_contexts(ctx, ctx_a, a_offs))) return rc;
   for (int i = 0; i < n; ++i)
     if (peak[i] < 0) return fail(ctx, NHANS_ERR_ARG, "stream " + std::to_string(i) + " has a negative peak");
   CK(cudaSetDevice(ctx->device));
-  int rc;
   if ((rc = need_weights(ctx))) return rc;
   // the context clips are laid out like a batch's (a mixture of zero samples per stream)
   std::vector<int64_t> no_mix(n + 1, 0);
@@ -1693,17 +1650,12 @@ int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t
   Streams& S = ctx->streams;
   if (!ctx_a && (rc = ensure_silent(ctx))) return rc;
   cudaStream_t st = ctx->stream;
-  auto clips = [&](DBuf& d, const int16_t* x, const int64_t* offs, long long len) {
-    CK(d.ensure(len * 2 + 32));
-    CK(cudaMemcpyAsync(d.p, x + offs[0], len * 2, cudaMemcpyHostToDevice, st));
-    return 0;
-  };
   // device offsets: b | a | context frames, n + 1 each
   std::vector<long long> offs(g.b_offs);
   offs.insert(offs.end(), g.ctx_frame_offs.begin(), g.ctx_frame_offs.end());
   if (ctx_a) offs.insert(offs.end(), g.a_offs.begin(), g.a_offs.end());
-  if ((rc = clips(S.ctx_b, ctx_b, b_offs, g.b_offs[n]))) return rc;
-  if (ctx_a && (rc = clips(S.ctx_a, ctx_a, a_offs, g.a_offs[n]))) return rc;
+  if ((rc = copy_clips(ctx, S.ctx_b, ctx_b, b_offs, g.b_offs[n], st))) return rc;
+  if (ctx_a && (rc = copy_clips(ctx, S.ctx_a, ctx_a, a_offs, g.a_offs[n], st))) return rc;
   if ((rc = to_device_offs(ctx, S.ctx_offs, offs))) return rc;
   const long long* d_offs = S.ctx_offs.as<long long>();
   if ((rc = run_conditioning(ctx, S.cb, ctx_a ? S.ctx_a.as<int16_t>() : nullptr, d_offs + 2 * (n + 1), S.ctx_b.as<int16_t>(), d_offs,
@@ -1715,9 +1667,7 @@ int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t
   for (int i = 0; i < n; ++i)
     CK(cudaMemcpyAsync(S.pool.as<float>() + slots[i] * S.slot_stride + kSlotCond, S.cb.cond.as<float>() + (size_t)i * n_cols,
                        (size_t)n_cols * 4, cudaMemcpyDeviceToDevice, st));
-  cudaError_t e = cudaStreamSynchronize(st);
-  if ((rc = check_kernel_flag(ctx))) return rc;
-  CK(e);
+  if ((rc = finish(ctx, cudaStreamSynchronize(st)))) return rc;
   for (int i = 0; i < n; ++i) {
     StreamRec r;
     r.slot = slots[i];

@@ -467,7 +467,6 @@ istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t*
 // Post-mix outputs of apply_snc (SN/apply.py:456-464) fused into one pass: both inverse STFTs (denoised
 // spectrum and the input spectrum = 'mixed_processed'), removed = mixed_processed - denoised, and the two
 // per-clip energy sums of snr_est = mean(denoised^2) / mean(removed^2).
-template <bool PHASOR>
 __global__ void __launch_bounds__(kThreads)
 istft_post_kernel(const float* __restrict__ den_logmag, const float* __restrict__ mix_logmag, const float* __restrict__ phase,
                   const long long* __restrict__ frame_offs, const long long* __restrict__ out_offs,
@@ -482,13 +481,13 @@ istft_post_kernel(const float* __restrict__ den_logmag, const float* __restrict_
   if (h0 >= T + 2) return;
   constexpr int PER = (kOH * kHop / 4 + kThreads - 1) / kThreads;
   float4 den[PER];
-  istft_frames<PHASOR>(s_y, den_logmag, phase, frame_offs[u], T, h0 - 2);
+  istft_frames<true>(s_y, den_logmag, phase, frame_offs[u], T, h0 - 2);
 #pragma unroll
   for (int k = 0; k < PER; ++k) {
     const int i = (threadIdx.x + k * kThreads) * 4;
     den[k] = i < kOH * kHop ? ola_sample4(s_y, i) : make_float4(0.f, 0.f, 0.f, 0.f);
   }
-  istft_frames<PHASOR>(s_y, mix_logmag, phase, frame_offs[u], T, h0 - 2);
+  istft_frames<true>(s_y, mix_logmag, phase, frame_offs[u], T, h0 - 2);
   const long long n_out = out_offs[u + 1] - out_offs[u];
   float e_den = 0.f, e_rem = 0.f;
 #pragma unroll
@@ -644,16 +643,13 @@ cudaError_t launch_istft_stream_post(cudaStream_t s, const StreamStepDev& p, int
 
 cudaError_t launch_istft_post(cudaStream_t s, const float* den_logmag, const float* mix_logmag, const float* phase,
                               const long long* frame_offs, const long long* out_offs, int U, int max_frames_per_clip,
-                              float* den_f32, float* mixed_f32, float* removed_f32, double* sums, bool phasor) {
+                              float* den_f32, float* mixed_f32, float* removed_f32, double* sums) {
   if (U <= 0) return cudaSuccess;
   // zeroed even when no clip has a frame: compensate_kernel reads the sums of every clip
   cudaError_t e = cudaMemsetAsync(sums, 0, sizeof(double) * 2 * U, s);
   if (e != cudaSuccess || max_frames_per_clip <= 0) return e;
   dim3 grid((max_frames_per_clip + 2 + kOH - 1) / kOH, U);
-  if (phasor)
-    istft_post_kernel<true><<<grid, kThreads, 0, s>>>(den_logmag, mix_logmag, phase, frame_offs, out_offs, den_f32, mixed_f32, removed_f32, sums);
-  else
-    istft_post_kernel<false><<<grid, kThreads, 0, s>>>(den_logmag, mix_logmag, phase, frame_offs, out_offs, den_f32, mixed_f32, removed_f32, sums);
+  istft_post_kernel<<<grid, kThreads, 0, s>>>(den_logmag, mix_logmag, phase, frame_offs, out_offs, den_f32, mixed_f32, removed_f32, sums);
   return cudaGetLastError();
 }
 

@@ -178,10 +178,10 @@ cudaError_t launch_stft_f32(cudaStream_t s, const float* x, const long long* off
 cudaError_t launch_istft(cudaStream_t s, const float* logmag, const float* phase, const long long* frame_offs,
                          const long long* out_offs, int U, const int* peak, int max_frames_per_clip, float* out_f32,
                          int16_t* out_i16, bool phasor = false);
-// apply_snc post-mix outputs (SN/apply.py:456-470): both iSTFTs, removed, energy sums; then compensated / snr_est
+// apply_snc post-mix outputs (SN/apply.py:456-470) from unit phasors: both iSTFTs, removed, energy sums; then compensated / snr_est
 cudaError_t launch_istft_post(cudaStream_t s, const float* den_logmag, const float* mix_logmag, const float* phase,
                               const long long* frame_offs, const long long* out_offs, int U, int max_frames_per_clip,
-                              float* den_f32, float* mixed_f32, float* removed_f32, double* sums, bool phasor = false);
+                              float* den_f32, float* mixed_f32, float* removed_f32, double* sums);
 cudaError_t launch_compensate(cudaStream_t s, const float* den, const float* removed, const long long* out_offs, int U,
                               const double* sums, float compensate, int ac, float* out, float* snr_est);
 cudaError_t dsp_init_tables();

@@ -215,6 +215,16 @@ def test_stream_argument_errors_leave_the_context_usable(sn, weights_sn):
         assert code(bare.stream_open, None, [neg], [1000]) == -3                              # weights not loaded
     finally:
         bare.close()
+    # a weight reload closes the open streams, and ids go on counting: an id from before it never names a new stream
+    small = _engine(W.SELECTIVE_NOISE, weights_sn, 8)
+    try:
+        [old] = small.stream_open(None, [neg], [1000])
+        small.load_weights(weights_sn)
+        assert code(small.stream_step, [old], [mix[:10]]) == -2
+        [new] = small.stream_open(None, [neg], [1000])
+        assert new > old
+    finally:
+        small.close()
     # the context still works: a fresh stream and the batch path
     _assert_equal(_stream(sn, mix, None, neg, [5000, 0, 1234, len(mix) - 6234]), want)
     assert np.array_equal(sn.enhance([mix], None, [neg])["i16"][0], want["i16"][0])
