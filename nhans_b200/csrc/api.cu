@@ -267,7 +267,7 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
     if (D.kh != 4 || D.kw != 4 || D.sh != 1 || D.sw != 1 || D.pt != 1 || D.pl != 1 || D.Hin != kWinFrames || D.Ho != kWinFrames ||
         D.raw_oh != -(kWinFrames / 2) || D.N != 64)
       return fail(ctx, NHANS_ERR_STATE, "first convolution of the mask network with an unexpected shape");
-    // per-frame table: a pass's windows plus 34 virtual frames per utterance it touches.  run_masknet sizes every pass
+    // per-frame table: a pass's windows plus kWinReach virtual frames per utterance it touches.  run_masknet sizes every pass
     // to fit, so utterances that average fewer than 17 frames run in smaller passes.
     net.crow_cap = 3LL * P.capacity + 64;
     if ((rc = net_alloc(ctx, net, (size_t)4 * net.crow_cap * kBins * 64, &net.convC))) return rc;
@@ -312,7 +312,7 @@ int realise_net(nhans_ctx* ctx, NetDev& net) {
       const Grid& g = P.bufs[buf];
       long long elems = (long long)g.pixels * g.C;
       if (elems % rowlen) return fail(ctx, NHANS_ERR_STATE, "buffer size not a multiple of the TMA row length");
-      if ((rc = make_map(ctx, a == 0 ? &D.mapA0 : &D.mapA1, net.bufs[buf], rowlen, elems / rowlen, 136))) return rc;
+      if ((rc = make_map(ctx, a == 0 ? &D.mapA0 : &D.mapA1, net.bufs[buf], rowlen, elems / rowlen, kSlabRows))) return rc;
     }
     if ((rc = make_map(ctx, &D.mapB, D.w, L.K, L.N, L.BN))) return rc;
     if ((rc = make_map(ctx, &D.mapBhalf, D.w, L.K, L.N, L.BN % 32 == 0 ? L.BN / 2 : L.BN))) return rc;   // CTA pairs load half of B each
@@ -425,7 +425,7 @@ EpiDev make_epi(const NetDev& net, const Epilogue& E, const Grid& out, const flo
 struct PassInfo {                   // which utterances / per-frame table rows a pass of the mask network touches
   const long long* d_frame_offs;
   int u_first, u_last;
-  long long crow0;                  // first table row = frame of the first window + 34 * u_first
+  long long crow0;                  // first table row = frame of the first window + kWinReach * u_first
   int rows;                         // table rows of the pass (<= crow_cap)
 };
 
@@ -554,10 +554,10 @@ int run_masknet(nhans_ctx* ctx, const float* logmag, const long long* d_frame_of
   if (h_frame_offs[U] > 0x7fffffffLL) return fail(ctx, NHANS_ERR_ARG, "too many frames in one batch");
   // segment of a window: largest s with win_offs[s] <= window
   auto seg_of = [&](long long w) { return (int)(std::upper_bound(h_win_offs, h_win_offs + U + 1, w) - h_win_offs) - 1; };
-  // per-frame table row of window row 0 of window w (kernels.h FrameConvDev: stored frame + 34 per earlier segment)
+  // per-frame table row of window row 0 of window w (kernels.h FrameConvDev: stored frame + kWinReach per earlier segment)
   auto crow_of = [&](long long w) {
     const int s = seg_of(w);
-    return h_frame_offs[s] + (h_left ? h_left[s] : 0) + (w - h_win_offs[s]) + 34LL * s;
+    return h_frame_offs[s] + (h_left ? h_left[s] : 0) + (w - h_win_offs[s]) + (long long)kWinReach * s;
   };
   for (long long w0 = 0, n = 0; w0 < total_windows; w0 += n) {
     PassInfo pi;
@@ -565,7 +565,7 @@ int run_masknet(nhans_ctx* ctx, const float* logmag, const long long* d_frame_of
     pi.u_first = seg_of(w0);
     pi.crow0 = crow_of(w0);
     // the largest pass whose per-frame table rows fit; one window always does.  For whole utterances these are its
-    // windows + 34 per utterance.
+    // windows + kWinReach per utterance.
     auto rows = [&](long long m) { return crow_of(w0 + m - 1) + 35 - pi.crow0; };
     long long lo = 1, hi = std::min<long long>(cap, total_windows - w0);
     while (lo < hi) {

@@ -36,7 +36,6 @@ namespace nhans {
 
 namespace {
 
-constexpr int kSlabRows = 136;                     // 128 + column taps, multiple of 8 (same box as gemm_tc.cu)
 constexpr int kSlabBytes = kSlabRows * 128;
 constexpr int kNA = 4;                             // A slab ring
 constexpr int kBTile = 64 * kWalkKH * 128;         // one column tap: [4 kernel rows x 64 couts] x 64 cin, fp16
@@ -62,21 +61,6 @@ struct __align__(8) WalkCtrl {
   uint32_t pad;
 };
 static_assert(sizeof(WalkCtrl) <= kCtrlBytes, "control block too large");
-
-__device__ __forceinline__ uint32_t pack_half2(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
-__device__ __forceinline__ void ldg256(const void* ptr, uint4& a, uint4& b) {
-  asm volatile("ld.global.nc.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
-               : "l"(ptr));
-}
-__device__ __forceinline__ void stg256(void* ptr, const uint4& a, const uint4& b) {
-  asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(ptr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w),
-               "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
-               : "memory");
-}
 
 template <int EPI>
 __global__ void __launch_bounds__(kWalkThreads + ((EPI & 4) ? kGenWarps * 32 : 0), 1)
@@ -159,8 +143,8 @@ conv64_walk_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
       const int unitA = (m0 < 0 ? 0 : m0) / p.Wq;
       const int xA = m0 - unitA * p.Wq;                                     // x of slab row 0 relative to unit A (may be -1)
       long long crowA = -1, crowB = -1;
-      if (unitA < n_units) crowA = (long long)p.units.frame[unitA] + 34LL * p.units.utt[unitA] - p.gen_crow0;
-      if (unitA + 1 < n_units) crowB = (long long)p.units.frame[unitA + 1] + 34LL * p.units.utt[unitA + 1] - p.gen_crow0;
+      if (unitA < n_units) crowA = (long long)p.units.frame[unitA] + (long long)kWinReach * p.units.utt[unitA] - p.gen_crow0;
+      if (unitA + 1 < n_units) crowB = (long long)p.units.frame[unitA + 1] + (long long)kWinReach * p.units.utt[unitA + 1] - p.gen_crow0;
       // per-lane source offsets of its rows (independent of the image row): -1 = zero row (margin / outside the pass)
       long long src_off[kIts];
 #pragma unroll
@@ -199,10 +183,10 @@ conv64_walk_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
           uint4 o = make_uint4(0u, 0u, 0u, 0u);
           if (src_off[it] >= 0) {
             const float4 a = va[it], b = vb[it];
-            o.x = pack_half2(fmaxf(a.x + t8[0], 0.f), fmaxf(a.y + t8[1], 0.f));
-            o.y = pack_half2(fmaxf(a.z + t8[2], 0.f), fmaxf(a.w + t8[3], 0.f));
-            o.z = pack_half2(fmaxf(b.x + t8[4], 0.f), fmaxf(b.y + t8[5], 0.f));
-            o.w = pack_half2(fmaxf(b.z + t8[6], 0.f), fmaxf(b.w + t8[7], 0.f));
+            o.x = ptx::pack_half2(fmaxf(a.x + t8[0], 0.f), fmaxf(a.y + t8[1], 0.f));
+            o.y = ptx::pack_half2(fmaxf(a.z + t8[2], 0.f), fmaxf(a.w + t8[3], 0.f));
+            o.z = ptx::pack_half2(fmaxf(b.x + t8[4], 0.f), fmaxf(b.y + t8[5], 0.f));
+            o.w = ptx::pack_half2(fmaxf(b.z + t8[6], 0.f), fmaxf(b.w + t8[7], 0.f));
           }
           *reinterpret_cast<uint4*>(slab + j * 128 + ((c8 ^ (j & 7)) << 4)) = o;
         }
@@ -329,7 +313,7 @@ conv64_walk_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
           }
           if (e.ftab16) {
             uint4 f0, f1;
-            ldg256(e.ftab16 + (size_t)wb * 64 + ch0 + 32 * ci, f0, f1);
+            ptx::ldg256(e.ftab16 + (size_t)wb * 64 + ch0 + 32 * ci, f0, f1);
             const uint4 ff[2] = {f0, f1};
             const __half2* fh = reinterpret_cast<const __half2*>(ff);
 #pragma unroll
@@ -361,8 +345,8 @@ conv64_walk_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
         if (!ok || o >= H) return;
         if (kRes) {
           const __half* rp = e.res + ((size_t)o * p.plane_pitch + m_plane) * e.res_C + ch0;
-          ldg256(rp, xn[0][0], xn[0][1]);
-          ldg256(rp + 32, xn[1][0], xn[1][1]);
+          ptx::ldg256(rp, xn[0][0], xn[0][1]);
+          ptx::ldg256(rp + 32, xn[1][0], xn[1][1]);
         }
         if (kR1) {
           const int frame = frame0 + o * e.r1_sh;
@@ -431,9 +415,9 @@ conv64_walk_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_consta
               for (int k = 0; k < 16; ++k) f[k] = fmaxf(f[k], 0.f);
             }
             uint4 o0, o1;
-            o0.x = pack_half2(f[0], f[1]); o0.y = pack_half2(f[2], f[3]); o0.z = pack_half2(f[4], f[5]); o0.w = pack_half2(f[6], f[7]);
-            o1.x = pack_half2(f[8], f[9]); o1.y = pack_half2(f[10], f[11]); o1.z = pack_half2(f[12], f[13]); o1.w = pack_half2(f[14], f[15]);
-            stg256(op + 32 * ci, o0, o1);
+            o0.x = ptx::pack_half2(f[0], f[1]); o0.y = ptx::pack_half2(f[2], f[3]); o0.z = ptx::pack_half2(f[4], f[5]); o0.w = ptx::pack_half2(f[6], f[7]);
+            o1.x = ptx::pack_half2(f[8], f[9]); o1.y = ptx::pack_half2(f[10], f[11]); o1.z = ptx::pack_half2(f[12], f[13]); o1.w = ptx::pack_half2(f[14], f[15]);
+            ptx::stg256(op + 32 * ci, o0, o1);
           }
         }
       }

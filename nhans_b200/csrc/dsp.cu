@@ -346,6 +346,16 @@ __device__ __forceinline__ float4 ola_sample4(const float* s_y, int i) {
 
 __device__ __forceinline__ int16_t to_i16(float v) { return (int16_t)__float2int_rn(fminf(fmaxf(v, -32768.f), 32767.f)); }
 
+// Samples o .. o + 3 as float32 and / or int16 PCM (v * scale, peak de-normalised); either output may be null
+__device__ __forceinline__ void store4(float* out_f32, int16_t* out_i16, long long o, float4 v, float scale) {
+  if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = v;
+  if (out_i16) {
+    short4 q;
+    q.x = to_i16(v.x * scale); q.y = to_i16(v.y * scale); q.z = to_i16(v.z * scale); q.w = to_i16(v.w * scale);
+    *reinterpret_cast<short4*>(out_i16 + o) = q;
+  }
+}
+
 // grid: (ceil((max_frames + 2) / kOH), U).  Output hop h (160 samples) sums frames h-2, h-1, h.  Clip lengths and
 // hop starts are multiples of 80 samples, so groups of four samples are aligned for 128-bit (f32) / 64-bit (int16) stores.
 template <bool PHASOR>
@@ -365,14 +375,7 @@ istft_kernel(const float* __restrict__ logmag, const float* __restrict__ phase, 
   for (int i = threadIdx.x * 4; i < kOH * kHop; i += blockDim.x * 4) {
     const long long n = (long long)h0 * kHop + i;
     if (n >= n_out) break;
-    const float4 acc = ola_sample4(s_y, i);
-    const long long o = out_offs[u] + n;
-    if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = acc;
-    if (out_i16) {
-      short4 q;
-      q.x = to_i16(acc.x * scale); q.y = to_i16(acc.y * scale); q.z = to_i16(acc.z * scale); q.w = to_i16(acc.w * scale);
-      *reinterpret_cast<short4*>(out_i16 + o) = q;
-    }
+    store4(out_f32, out_i16, out_offs[u] + n, ola_sample4(s_y, i), scale);
   }
 }
 
@@ -405,13 +408,7 @@ istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t*
       const long long n = (long long)h0 * kHop + i - lo;
       if (n >= len) break;
       const float4 acc = ola_sample4(s_y, i);
-      const long long o = p.out_offs[u] + n;
-      if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = acc;
-      if (out_i16) {
-        short4 q;
-        q.x = to_i16(acc.x * scale); q.y = to_i16(acc.y * scale); q.z = to_i16(acc.z * scale); q.w = to_i16(acc.w * scale);
-        *reinterpret_cast<short4*>(out_i16 + o) = q;
-      }
+      store4(out_f32, out_i16, p.out_offs[u] + n, acc, scale);
     }
   } else {
     __shared__ float s_red[2][kThreads / 32];
@@ -434,12 +431,7 @@ istft_stream_kernel(const StreamStepDev p, float* __restrict__ out_f32, int16_t*
       const float4 d = den[k];
       const float4 rem = make_float4(mixed.x - d.x, mixed.y - d.y, mixed.z - d.z, mixed.w - d.w);
       const long long o = p.out_offs[u] + n;
-      if (out_f32) *reinterpret_cast<float4*>(out_f32 + o) = d;
-      if (out_i16) {
-        short4 q;
-        q.x = to_i16(d.x * scale); q.y = to_i16(d.y * scale); q.z = to_i16(d.z * scale); q.w = to_i16(d.w * scale);
-        *reinterpret_cast<short4*>(out_i16 + o) = q;
-      }
+      store4(out_f32, out_i16, o, d, scale);
       if (mixed_f32) *reinterpret_cast<float4*>(mixed_f32 + o) = mixed;
       if (removed_f32) *reinterpret_cast<float4*>(removed_f32 + o) = rem;
       // one FFMA per sample, as compensate_kernel's den + removed * factor

@@ -46,7 +46,6 @@ namespace nhans {
 
 namespace {
 
-constexpr int kSlabRows = 136;                    // 128 + up to 7 rows of tap shift, multiple of 8
 constexpr int kSlabBytes = kSlabRows * 128;       // 17 KB, a multiple of the 1024-byte swizzle atom
 constexpr int kCtrlBytes = 8192;
 constexpr int kEpiWarps = 8;
@@ -91,11 +90,6 @@ struct LiveGroups {
     s1 = max((int)((w >> 16) & 0xffu), g_lo); e1 = max(s1, min((int)(w >> 24), g_hi));
   }
 };
-
-__device__ __forceinline__ uint32_t pack_half2(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
 
 // MMA issuer (one warp): walks tiles / groups / sub-tiles in the producers' order; one elected lane issues
 // tcgen05.mma.  IL sub-tiles are processed together so that consecutive MMAs target different TMEM
@@ -266,19 +260,14 @@ __device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, int 
       if (wo >= p.Wo) return make_int4(-1, 0, 0, 0);
       int pix, utt = p.units.utt[unit];
       float rawv = 0.f;
-      if (kR1) {
-        const int frame = p.units.frame[unit] + ho * e.r1_sh + e.raw_oh;
-        if (frame >= p.units.lo[unit] && frame < p.units.hi[unit]) rawv = __ldg(e.raw + (size_t)frame * 201 + wo * e.r1_sw);
-      }
+      if (kR1) rawv = epi_raw(e, p.units, unit, ho, wo);
       if (kHead) {
         pix = unit;
         utt = p.units.frame[unit];           // head: the centre frame row replaces the utterance index
       } else if (e.o_mode == 1) {
         pix = (unit * e.o_W + wo) * e.o_H + ho;
       } else {
-        const int y = ho + e.o_oy, x = wo + e.o_ox;
-        const int plane = (y % e.o_sh) * e.o_sw + (x % e.o_sw);
-        pix = (int)(plane * e.o_plane + unit * e.o_ustride + (y / e.o_sh) * e.o_rstride + (x / e.o_sw));
+        pix = (int)epi_grid_pixel(e, unit, ho, wo);
       }
       return make_int4(pix, (ho << 16) | wo, utt, __float_as_int(rawv));
     };
@@ -365,8 +354,8 @@ __device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, int 
           f.x = fmaxf(f.x, 0.f); f.y = fmaxf(f.y, 0.f); f.z = fmaxf(f.z, 0.f); f.w = fmaxf(f.w, 0.f);
         }
         uint2 o;
-        o.x = pack_half2(f.x, f.y);
-        o.y = pack_half2(f.z, f.w);
+        o.x = ptx::pack_half2(f.x, f.y);
+        o.y = ptx::pack_half2(f.z, f.w);
         *reinterpret_cast<uint2*>(e.out + o_out[g] + c0) = o;
       }
       __syncwarp();                         // staging is overwritten by the next chunk
@@ -389,17 +378,6 @@ __device__ __forceinline__ void epilogue_warp(Ctrl* ctrl, const GemmDev& p, int 
     release_acc(acc);
   }
   if (p.debug_stats && ew == 0 && lane == 0) atomicAdd(p.debug_stats + 3, (unsigned long long)w_full);
-}
-
-__device__ __forceinline__ void ldg256(const void* ptr, uint4& a, uint4& b) {
-  asm volatile("ld.global.nc.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
-               : "l"(ptr));
-}
-__device__ __forceinline__ void stg256(void* ptr, const uint4& a, const uint4& b) {
-  asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(ptr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w),
-               "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
-               : "memory");
 }
 
 // Row-per-thread epilogue.  The transposing epilogue above keeps global accesses coalesced at the price of two
@@ -457,19 +435,8 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
       size_t o_out = 0, o_bias = 0, o_res = 0;
       int o_t = 0, o_f = 0;
       if (ok) {
-        if (kR1) {
-          const int frame = p.units.frame[unit] + ho * e.r1_sh + e.raw_oh;
-          if (frame >= p.units.lo[unit] && frame < p.units.hi[unit]) rawv = __ldg(e.raw + (size_t)frame * 201 + wo * e.r1_sw);
-        }
-        long long pix;
-        if (e.o_mode == 1) {
-          pix = ((long long)unit * e.o_W + wo) * e.o_H + ho;
-        } else {
-          const int y = ho + e.o_oy, x = wo + e.o_ox;
-          const int plane = (y % e.o_sh) * e.o_sw + (x % e.o_sw);
-          pix = plane * e.o_plane + unit * e.o_ustride + (y / e.o_sh) * e.o_rstride + (x / e.o_sw);
-        }
-        o_out = (size_t)pix * e.out_C + n0;
+        if (kR1) rawv = epi_raw(e, p.units, unit, ho, wo);
+        o_out = (size_t)epi_pixel(e, unit, ho, wo) * e.out_C + n0;
         o_bias = (size_t)utt * e.bias_stride + n0;
         if (kRes) o_res = (size_t)m * e.res_C + n0;
         if (kTabS) {
@@ -481,7 +448,7 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
         if (c0 >= p.BN || !ok) return;
         const float4* bp = reinterpret_cast<const float4*>(e.bias + o_bias + c0);
         L.b[0] = __ldg(bp); L.b[1] = __ldg(bp + 1); L.b[2] = __ldg(bp + 2); L.b[3] = __ldg(bp + 3);
-        if (kRes) ldg256(e.res + o_res + c0, L.x[0], L.x[1]);
+        if (kRes) ptx::ldg256(e.res + o_res + c0, L.x[0], L.x[1]);
       };
       const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * 256 + i * p.BN;
       auto process = [&](const LoadSet& L, int c0) {
@@ -534,9 +501,9 @@ __device__ __forceinline__ void epilogue_warp_row(Ctrl* ctrl, const GemmDev& p, 
           for (int k = 0; k < 16; ++k) f[k] = fmaxf(f[k], 0.f);
         }
         uint4 o0, o1;
-        o0.x = pack_half2(f[0], f[1]); o0.y = pack_half2(f[2], f[3]); o0.z = pack_half2(f[4], f[5]); o0.w = pack_half2(f[6], f[7]);
-        o1.x = pack_half2(f[8], f[9]); o1.y = pack_half2(f[10], f[11]); o1.z = pack_half2(f[12], f[13]); o1.w = pack_half2(f[14], f[15]);
-        stg256(e.out + o_out + c0, o0, o1);
+        o0.x = ptx::pack_half2(f[0], f[1]); o0.y = ptx::pack_half2(f[2], f[3]); o0.z = ptx::pack_half2(f[4], f[5]); o0.w = ptx::pack_half2(f[6], f[7]);
+        o1.x = ptx::pack_half2(f[8], f[9]); o1.y = ptx::pack_half2(f[10], f[11]); o1.z = ptx::pack_half2(f[12], f[13]); o1.w = ptx::pack_half2(f[14], f[15]);
+        ptx::stg256(e.out + o_out + c0, o0, o1);
       };
       LoadSet A, B;
       int c0 = ((half + i) & 1) * 16;

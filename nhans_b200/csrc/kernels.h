@@ -6,7 +6,15 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "plan.h"
+
 namespace nhans {
+
+// Rows of the A operand box ("slab") of the tensor-core kernels: 128 rows + up to 7 rows of tap shift, a multiple of 8
+constexpr int kSlabRows = 136;
+// Frames a window reaches besides its centre, 17 on either side.  The per-frame table of the first convolution
+// (FrameConvDev) adds this many virtual zero rows per segment.
+constexpr int kWinReach = kWinFrames - 1;
 
 // Per-unit (window / context row) lookup: frame row of the unit in the raw fp32 spectrogram, the
 // [lo, hi) frame range of the clip it belongs to (rows outside read as 0.0, SN/apply.py:170-173) and
@@ -40,6 +48,25 @@ struct EpiDev {
   long long o_plane, o_rstride, o_ustride;   // pixel = plane * o_plane + (y / sh) * o_rstride + unit * o_ustride + x / sw
   float* out_f32;
 };
+
+// Output pixel of (unit, ho, wo) in the grid of an EpiDev: the device twin of plan.h grid_pixel.  epi_grid_pixel is
+// the phase-split grid (o_mode 0) alone, for kernels that never write the head layout (o_mode 1).
+__device__ __forceinline__ long long epi_grid_pixel(const EpiDev& e, int unit, int ho, int wo) {
+  const int y = ho + e.o_oy, x = wo + e.o_ox;
+  const int plane = (y % e.o_sh) * e.o_sw + (x % e.o_sw);
+  return plane * e.o_plane + unit * e.o_ustride + (y / e.o_sh) * e.o_rstride + (x / e.o_sw);
+}
+__device__ __forceinline__ long long epi_pixel(const EpiDev& e, int unit, int ho, int wo) {
+  if (e.o_mode == 1) return ((long long)unit * e.o_W + wo) * e.o_H + ho;
+  return epi_grid_pixel(e, unit, ho, wo);
+}
+
+// Raw spectrogram value the rank-1 transform adds at output (ho, wo) of a unit: 0.0 where its frame lies outside the
+// unit's clip frames [lo, hi)
+__device__ __forceinline__ float epi_raw(const EpiDev& e, const UnitTable& u, int unit, int ho, int wo) {
+  const int frame = u.frame[unit] + ho * e.r1_sh + e.raw_oh;
+  return (frame >= u.lo[unit] && frame < u.hi[unit]) ? __ldg(e.raw + (size_t)frame * 201 + wo * e.r1_sw) : 0.f;
+}
 
 struct KGroupDev {            // plan.h KGroup
   int32_t row_off;
@@ -94,7 +121,7 @@ struct WalkDev {
   unsigned long long* debug_stats;
   // Generated A operand (resblock1_1_conv2 only): instead of reading the first convolution's output from HBM, two
   // producer warps build every slab from the per-frame table of that convolution (FrameConvDev::C):
-  // A[unit, r, x, :] = relu(C[variant(r)][frame(unit) + 34 utt(unit) - crow0 + r][x][:] + T1[r][:]) in fp16
+  // A[unit, r, x, :] = relu(C[variant(r)][frame(unit) + kWinReach utt(unit) - crow0 + r][x][:] + T1[r][:]) in fp16
   const float* gen_C;       // null: A comes from mapA (TMA)
   long long gen_crow0, gen_crow_cap;
   const __half* gen_ttab16; // [H][64] time embedding of the first convolution
@@ -116,14 +143,14 @@ cudaError_t launch_gemm(cudaStream_t s, int n_sm, const CUtensorMap& mapA0, cons
                         const CUtensorMap& mapB, const CUtensorMap& mapBhalf, const GemmDev& p);
 // first convolution of the towers (Cin = 1, N = 64); an epilogue with embedding tables is rejected
 cudaError_t launch_direct_conv(cudaStream_t s, const DirectDev& p);
-// mapA: the input grid as [pixels][64] (box 136 x 64), mapB: repacked weights [4 kernel-row blocks x 64][4 x 64] (box 256 x 64)
+// mapA: the input grid as [pixels][64] (box kSlabRows x 64), mapB: repacked weights [4 kernel-row blocks x 64][4 x 64] (box 256 x 64)
 cudaError_t launch_walk(cudaStream_t s, int n_sm, const CUtensorMap& mapA, const CUtensorMap& mapB, const WalkDev& p);
 
 // First convolution of the mask network, computed once per FRAME instead of once per (window, row): the 35-frame
 // windows of one utterance are shifted copies of the same spectrogram, so conv(x)[window n, row h] depends only on
 // the frame n - 17 + h - except for which kernel rows fall outside the window (rows h = 0, 33, 34), which gives four
 // variants per frame.  frame_conv fills C[variant][crow][201][64] (fp32 FMA) for the frames a pass touches; crow =
-// frame + 34 * utterance + row indexes the zero-extended utterance (17 virtual frames on either side), and the
+// frame + kWinReach * utterance + row indexes the zero-extended utterance (17 virtual frames on either side), and the
 // conditioning bias of the utterance and the frequency embedding F[w] are folded in (a C row belongs to one
 // utterance).  window_expand then writes h1[n][h][w][:] = relu(C[variant(h)][crow(n) + h][w][:] + T[h]) in fp16:
 // 35x fewer multiply-adds than a per-window evaluation, what remains is the 1.8 GB store stream of a pass.
@@ -132,7 +159,7 @@ struct FrameConvDev {
   const float* raw;            // [frames][201] log-magnitude
   const long long* frame_offs; // [U + 1] device
   int u_first, u_last;         // utterances the pass touches
-  long long crow0;             // first C row of the pass = first window + 34 * u_first
+  long long crow0;             // first C row of the pass = first window + kWinReach * u_first
   int rows;                    // C rows to fill
   long long crow_cap;          // rows per variant plane of C
   const float* w;              // [16][64] taps (batch-norm scale folded)
@@ -194,7 +221,9 @@ cudaError_t dsp_init_tables();
 // den_seg has the layout of seg_lm: the denoised frames of the windows, preceded by den_carry[s] frames of the previous
 // step; the inverse STFT runs over those rows and emits samples [160 den_carry, 160 den_carry + out_offs[s + 1] - out_offs[s])
 // of their overlap-add.  The slot then keeps segment rows [keep[s], T) and the last den_keep[s] denoised frames.
-constexpr int kStreamCarry = 34;      // stored frames a stream carries between steps (2 x 17 window half)
+// stored frames a stream carries between steps: the 17 window centres still waiting for their right-hand frames and the
+// 17 left-hand frames of the first of them
+constexpr int kStreamCarry = kWinReach;
 struct StreamStepDev {
   int n;
   const long long *seg_offs, *new_offs, *win_offs, *out_offs;   // [n + 1]

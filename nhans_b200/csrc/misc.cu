@@ -2,15 +2,11 @@
 // expansion for the mask network, a per-pixel kernel that reads the spectrogram rows for the towers), the
 // conditioning-projection table, the tower's global mean pool and the per-unit lookup tables.
 #include "kernels.h"
+#include "ptx.cuh"
 
 namespace nhans {
 
 namespace {
-
-__device__ __forceinline__ uint32_t pack_half2(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
 
 // embedding/noise_resblock1_1_conv1 (main.py:104, Cin = 1, 8x4, stride 3x2, no embedding tables): one thread per
 // output pixel, 64 output channels in registers.  Input row r of unit n is frame units.frame[n] + r + raw_oh of
@@ -62,9 +58,7 @@ direct_conv64_kernel(const DirectDev p) {
   // Epilogue through a warp-private shared-memory transpose: 8 lanes then cover one pixel's 64 channels, so
   // the bias loads and the fp16 stores of a warp touch whole 128-byte lines instead of 32 scattered ones.
   const int utt = p.units_tab.utt ? p.units_tab.utt[unit] : 0;
-  const int yy = ho + e.o_oy, xx = wo + e.o_ox;
-  const int plane = (yy % e.o_sh) * e.o_sw + (xx % e.o_sw);
-  const long long pix = plane * e.o_plane + unit * e.o_ustride + (yy / e.o_sh) * e.o_rstride + (xx / e.o_sw);
+  const long long pix = epi_grid_pixel(e, unit, ho, wo);
   const int lane = threadIdx.x & 31;
   float* st = s_stage + (threadIdx.x >> 5) * (32 * kDirectPitch);
   long long* s_pix = reinterpret_cast<long long*>(s_meta) + (threadIdx.x >> 5) * 32;
@@ -92,14 +86,14 @@ direct_conv64_kernel(const DirectDev p) {
       for (int i = 0; i < 8; ++i) v[i] = fmaxf(v[i], 0.f);
     }
     uint4 o;
-    o.x = pack_half2(v[0], v[1]); o.y = pack_half2(v[2], v[3]);
-    o.z = pack_half2(v[4], v[5]); o.w = pack_half2(v[6], v[7]);
+    o.x = ptx::pack_half2(v[0], v[1]); o.y = ptx::pack_half2(v[2], v[3]);
+    o.z = ptx::pack_half2(v[4], v[5]); o.w = ptx::pack_half2(v[6], v[7]);
     *reinterpret_cast<uint4*>(e.out + opix * e.out_C + cg) = o;
   }
 }
 
 // ---- first convolution per frame + window expansion (kernels.h FrameConvDev) ----
-constexpr int kVirt = 17;                               // virtual frames on either side of an utterance (window half)
+constexpr int kVirt = kWinReach / 2;                    // virtual frames on either side of an utterance (window half)
 
 // grid: rows; block 256: items (w, 8-channel group).  Kernel rows i = 0..3 read frames vf - 1 + i of the
 // zero-extended utterance; variants: 0 = all rows, 1 = rows 1..3 (window row 0), 2 = rows 0..2 (row 33), 3 = rows 0..1 (row 34).
@@ -110,10 +104,10 @@ frame_conv_kernel(const FrameConvDev p) {
   for (int i = threadIdx.x; i < 16 * 64; i += blockDim.x) s_w[i] = p.w[i];
   const long long crow = p.crow0 + blockIdx.x;
   if (threadIdx.x == 0) {
-    int a = p.u_first, b = p.u_last + 1;               // largest u with frame_offs[u] + 34 u <= crow
+    int a = p.u_first, b = p.u_last + 1;               // largest u with frame_offs[u] + kWinReach u <= crow
     while (b - a > 1) {
       const int mid = (a + b) >> 1;
-      if (p.frame_offs[mid] + 2LL * kVirt * mid <= crow) a = mid; else b = mid;
+      if (p.frame_offs[mid] + (long long)kWinReach * mid <= crow) a = mid; else b = mid;
     }
     s_u = a;
   }
@@ -121,7 +115,7 @@ frame_conv_kernel(const FrameConvDev p) {
   const int u = s_u;
   const long long f0 = p.frame_offs[u];
   const int T = (int)(p.frame_offs[u + 1] - f0);
-  const int vf = (int)(crow - (f0 + 2LL * kVirt * u)) - kVirt;    // virtual frame of this row
+  const int vf = (int)(crow - (f0 + (long long)kWinReach * u)) - kVirt;    // virtual frame of this row
   const float* rows[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
@@ -194,7 +188,7 @@ window_expand_kernel(const DirectDev p, const float* __restrict__ C, long long c
   const EpiDev& e = p.epi;
   const int cg = (lane & 7) * 8;
   const int utt = p.units_tab.utt ? p.units_tab.utt[unit] : 0;
-  const long long crow_n = (long long)p.units_tab.frame[unit] + 2LL * kVirt * utt - crow0;   // C row of window row 0
+  const long long crow_n = (long long)p.units_tab.frame[unit] + (long long)kWinReach * utt - crow0;   // C row of window row 0
   const size_t vplane = (size_t)crow_cap * 201 * 64;
   constexpr int NIT = CW / 4;
   // per-lane pixel offsets of the column iterations (independent of the window row)
@@ -225,8 +219,8 @@ window_expand_kernel(const DirectDev p, const float* __restrict__ C, long long c
         for (int i = 0; i < 8; ++i) v[i] = fmaxf(v[i], 0.f);
       }
       uint4 o;
-      o.x = pack_half2(v[0], v[1]); o.y = pack_half2(v[2], v[3]);
-      o.z = pack_half2(v[4], v[5]); o.w = pack_half2(v[6], v[7]);
+      o.x = ptx::pack_half2(v[0], v[1]); o.y = ptx::pack_half2(v[2], v[3]);
+      o.z = ptx::pack_half2(v[4], v[5]); o.w = ptx::pack_half2(v[6], v[7]);
       // streaming store: the 1.8 GB of activations must not push the per-frame table out of L2 (-9 % kernel time)
       __stcs(reinterpret_cast<uint4*>(orow + off[it]), o);
     }

@@ -1,5 +1,5 @@
 // Thin inline-PTX wrappers for the sm_100a features the engine uses: mbarrier, TMA (cp.async.bulk.tensor),
-// tcgen05 (TMEM alloc / mma / commit / ld) and the proxy fences between them.
+// tcgen05 (TMEM alloc / mma / commit / ld), the proxy fences between them and 256-bit global loads / stores.
 #pragma once
 
 #include <cuda.h>
@@ -169,6 +169,22 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
       : "memory");
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+
+// ---- 256-bit global accesses (a full 32-byte sector per thread) and fp16 packing of the epilogues -----
+__device__ __forceinline__ void ldg256(const void* ptr, uint4& a, uint4& b) {
+  asm volatile("ld.global.nc.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w)
+               : "l"(ptr));
+}
+__device__ __forceinline__ void stg256(void* ptr, const uint4& a, const uint4& b) {
+  asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(ptr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w),
+               "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
+               : "memory");
+}
+__device__ __forceinline__ uint32_t pack_half2(float a, float b) {
+  __half2 h = __floats2half2_rn(a, b);
+  return *reinterpret_cast<uint32_t*>(&h);
+}
 
 // ---- CTA pairs (cta_group::2): two CTAs of a cluster cooperate on M = 256 MMAs ---------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
