@@ -55,6 +55,27 @@ struct DBuf {
   template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
+// Index arrays the library builds on the host (offsets, stream-step descriptors, peaks), sent to the device in one copy.
+// add() appends an array at a 16-byte-aligned offset and returns that offset; ptr() is valid only after upload(), which
+// may reallocate.  The host bytes stay here until the next use, so the copy never reads from a dead temporary.
+struct Staging {
+  std::vector<char> host;
+  DBuf dev;
+  Staging& reset() { host.clear(); return *this; }     // starts a new layout
+  template <class T> size_t add(const T* x, size_t n) {
+    const size_t off = (host.size() + 15) / 16 * 16;
+    host.resize(off + n * sizeof(T));
+    if (n) memcpy(host.data() + off, x, n * sizeof(T));
+    return off;
+  }
+  template <class T> size_t add(const std::vector<T>& v) { return add(v.data(), v.size()); }
+  cudaError_t upload(cudaStream_t s) {
+    cudaError_t e = dev.ensure(host.size());
+    return e != cudaSuccess ? e : cudaMemcpyAsync(dev.p, host.data(), host.size(), cudaMemcpyHostToDevice, s);
+  }
+  template <class T> const T* ptr(size_t off) const { return reinterpret_cast<const T*>(dev.as<char>() + off); }
+};
+
 struct GemmLayerDev {
   __half* w = nullptr;
   KGroupDev* groups = nullptr;
@@ -93,7 +114,10 @@ struct ProfRec {
 // Host <-> device staging of one batch.  There are two sets so that consecutive nhans_enhance_batch calls overlap:
 // the H2D copies of batch i + 1 and the D2H copies of batch i - 1 run on their own streams while batch i computes.
 struct IoSlot {
-  DBuf mix, a, b, d_mix_offs, d_a_offs, d_b_offs, d_frame_offs, d_out_offs, d_ctx_frame_offs;
+  DBuf mix, a, b;
+  Staging staging;                  // the batch's Geometry arrays; stage_batch records their device copies below
+  const long long *mix_offs = nullptr, *a_offs = nullptr, *b_offs = nullptr, *frame_offs = nullptr, *out_offs = nullptr,
+                  *ctx_frame_offs = nullptr;
   DBuf out_i16, out_f32;
   cudaEvent_t uploaded = nullptr;   // h2d stream: inputs of the batch staged in this set have landed
   cudaEvent_t consumed = nullptr;   // compute stream: every kernel reading / writing this set has finished
@@ -149,10 +173,10 @@ struct Streams {
   int n_slots = 0;
   long long slot_stride = 0;
   std::vector<int> free_slots;
-  DBuf ctx_a, ctx_b, ctx_offs;     // nhans_stream_open
+  DBuf ctx_a, ctx_b;                // nhans_stream_open
   CondBufs cb;
-  DBuf pcm, desc, new_lm, new_ph, seg_lm, seg_ph, den_win, den_seg, cond, out_i16, out_f32;   // nhans_stream_step
-  DBuf factor, mixed, removed, comp, sums;                                                   // nhans_stream_step_post
+  DBuf pcm, new_lm, new_ph, seg_lm, seg_ph, den_win, den_seg, cond, out_i16, out_f32;   // nhans_stream_step
+  DBuf mixed, removed, comp, sums;                                                     // nhans_stream_step_post
 };
 
 }  // namespace
@@ -174,6 +198,7 @@ struct nhans_ctx {
   Batch batch;
   Streams streams;
   DBuf tmp[8];
+  Staging staging;                  // index arrays of the calls that finish before they return (all but the batch path)
   cudaEvent_t events[16] = {};
   bool profile = false;
   std::vector<ProfRec> prof;
@@ -218,6 +243,16 @@ int fail(nhans_ctx* c, int code, const std::string& msg) {
       return fail(ctx, NHANS_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e__) + " (" + __FILE__ + ":" + \
                                            std::to_string(__LINE__) + ")");                              \
   } while (0)
+
+// Every launcher call goes through here: its result is checked and the launch counted in ctx->launches
+// (nhans_profile_get kind 5).  `what` names the launch in the error and is built only on failure.
+#define LAUNCH_AS(call, what)                                                                            \
+  do {                                                                                                   \
+    cudaError_t e__ = (call);                                                                            \
+    if (e__ != cudaSuccess) return fail(ctx, NHANS_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e__)); \
+    ctx->launches += 1;                                                                                  \
+  } while (0)
+#define LAUNCH(call) LAUNCH_AS(call, std::string(#call) + " (" + __FILE__ + ":" + std::to_string(__LINE__) + ")")
 
 // n elements of device memory owned by `net`, zeroed on the compute stream when `zero`.
 template <class T>
@@ -354,7 +389,6 @@ struct ProfScope {
   bool on;
   ProfRec r;
   ProfScope(nhans_ctx* c, int kind, double flops, double bytes, int layer = -1) : ctx(c), on(c->profile) {
-    c->launches += 1;
     if (!on) return;
     r.kind = kind; r.flops = flops; r.bytes = bytes; r.layer = layer;
     r.a = get_event(c); r.b = get_event(c);
@@ -461,17 +495,14 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
       f.bias = d.epi.bias; f.bias_stride = d.epi.bias_stride; f.ftab16 = d.epi.ftab16;
       f.C = net.convC;
       // (expanding the pass in slices so that a slice's table stays L2-resident was measured: no gain)
-      CK(launch_frame_conv(ctx->stream, f));
+      LAUNCH(launch_frame_conv(ctx->stream, f));
       // the row-walk kernel of the next layer builds its A operand from the table (conv_walk.cu kWalkGen); otherwise
       // the table is expanded into the (window, row) activation tensor here
       gen_first = ctx->use_walk && ctx->use_gen && !P.gemm.empty() && P.gemm[0].walk && net.layers[0].w_walk &&
                   P.gemm[0].a_buf[0] == D.out.buf && D.epi.relu && d.epi.ttab16;
-      if (!gen_first) {
-        CK(launch_window_expand(ctx->stream, d, net.convC, pass->crow0, net.crow_cap, 0, units));
-        ctx->launches += 1;
-      }
+      if (!gen_first) LAUNCH(launch_window_expand(ctx->stream, d, net.convC, pass->crow0, net.crow_cap, 0, units));
     } else {
-      CK(launch_direct_conv(ctx->stream, d));
+      LAUNCH(launch_direct_conv(ctx->stream, d));
     }
   }
   for (size_t i = 0; i < P.gemm.size(); ++i) {
@@ -508,20 +539,13 @@ int run_net(nhans_ctx* ctx, NetDev& net, int units, const float* raw, const floa
         wd.gen_C = net.convC; wd.gen_crow0 = pass->crow0; wd.gen_crow_cap = net.crow_cap;
         wd.gen_ttab16 = reinterpret_cast<const __half*>(net.first_ttab16);
       }
-      cudaError_t le = launch_walk(ctx->stream, ctx->n_sm, D.mapA0, D.mapBwalk, wd);
-      if (le != cudaSuccess)
-        return fail(ctx, NHANS_ERR_CUDA, "launch of row-walk layer " + L.name + ": " + cudaGetErrorString(le));
+      LAUNCH_AS(launch_walk(ctx->stream, ctx->n_sm, D.mapA0, D.mapBwalk, wd), "launch of row-walk layer " + L.name);
       continue;
     }
-    {
-      cudaError_t le = launch_gemm(ctx->stream, ctx->n_sm, D.mapA0, D.mapA1, D.mapB, D.mapBhalf, g);
-      if (le != cudaSuccess)
-        return fail(ctx, NHANS_ERR_CUDA, "launch of layer " + L.name + " (M " + std::to_string(g.M) + ", BN " + std::to_string(g.BN) + "): " + cudaGetErrorString(le));
-      if (split_head) {
-        CK(launch_head_reduce(ctx->stream, net.head_scratch, kHeadSplit, units, L.N, D.res_scale, D.bias, raw, net.u_frame, out_f32));
-        ctx->launches += 1;
-      }
-    }
+    LAUNCH_AS(launch_gemm(ctx->stream, ctx->n_sm, D.mapA0, D.mapA1, D.mapB, D.mapBhalf, g),
+              "launch of layer " + L.name + " (M " + std::to_string(g.M) + ", BN " + std::to_string(g.BN) + ")");
+    if (split_head)
+      LAUNCH(launch_head_reduce(ctx->stream, net.head_scratch, kHeadSplit, units, L.N, D.res_scale, D.bias, raw, net.u_frame, out_f32));
   }
   return 0;
 }
@@ -532,12 +556,11 @@ int run_tower(nhans_ctx* ctx, const float* ctx_logmag, int R, float* emb) {
   const int cap = net.plan.capacity;
   for (int r0 = 0; r0 < R; r0 += cap) {
     const int n = std::min(cap, R - r0);
-    CK(launch_units_rows(ctx->stream, r0, n, kCtxFrames, net.u_frame, net.u_lo, net.u_hi, net.u_utt));
-    ctx->launches += 1;
+    LAUNCH(launch_units_rows(ctx->stream, r0, n, kCtxFrames, net.u_frame, net.u_lo, net.u_hi, net.u_utt));
     int rc = run_net(ctx, net, n, ctx_logmag, nullptr, nullptr);
     if (rc) return rc;
     ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_mean_pool(ctx->stream, net.bufs[net.plan.pool_buf], n, net.plan.pool_pixels, 512, emb + (size_t)r0 * 512));
+    LAUNCH(launch_mean_pool(ctx->stream, net.bufs[net.plan.pool_buf], n, net.plan.pool_pixels, 512, emb + (size_t)r0 * 512));
   }
   return 0;
 }
@@ -575,9 +598,8 @@ int run_masknet(nhans_ctx* ctx, const float* logmag, const long long* d_frame_of
     n = lo;
     pi.u_last = seg_of(w0 + n - 1);
     pi.rows = (int)rows(n);
-    CK(launch_units_main(ctx->stream, d_frame_offs, d_win_offs, d_left, U, (int)w0, (int)n, net.u_frame, net.u_lo, net.u_hi,
-                         net.u_utt));
-    ctx->launches += 1;
+    LAUNCH(launch_units_main(ctx->stream, d_frame_offs, d_win_offs, d_left, U, (int)w0, (int)n, net.u_frame, net.u_lo,
+                             net.u_hi, net.u_utt));
     int rc = run_net(ctx, net, (int)n, logmag, cond_table, den + (size_t)w0 * kBins, &pi);
     if (rc) return rc;
   }
@@ -678,12 +700,6 @@ int batch_geometry(nhans_ctx* ctx, const int64_t* mix_offs, const int64_t* a_off
   return 0;
 }
 
-int to_device_offs(nhans_ctx* ctx, DBuf& d, const std::vector<long long>& h, cudaStream_t stream = nullptr) {
-  CK(d.ensure(h.size() * sizeof(long long)));
-  CK(cudaMemcpyAsync(d.p, h.data(), h.size() * sizeof(long long), cudaMemcpyHostToDevice, stream ? stream : ctx->stream));
-  return 0;
-}
-
 int need_weights(nhans_ctx* ctx) {
   if (!ctx->main_net.ready || !ctx->tower.ready) return fail(ctx, NHANS_ERR_STATE, "nhans_load_weights has not been called");
   return 0;
@@ -723,15 +739,13 @@ int stage_batch(nhans_ctx* ctx, IoSlot& io, const Geometry& g, const T* mix, con
   int rc;
   if ((rc = copy_clips(ctx, io.mix, mix, mix_offs, g.mix_offs[U], stream))) return rc;
   if ((rc = copy_clips(ctx, io.b, ctx_b, b_offs, g.b_offs[U], stream))) return rc;
-  if (ctx_a) {
-    if ((rc = copy_clips(ctx, io.a, ctx_a, a_offs, g.a_offs[U], stream))) return rc;
-    if ((rc = to_device_offs(ctx, io.d_a_offs, g.a_offs, stream))) return rc;
-  }
-  if ((rc = to_device_offs(ctx, io.d_mix_offs, g.mix_offs, stream))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_b_offs, g.b_offs, stream))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_frame_offs, g.frame_offs, stream))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_out_offs, g.out_offs, stream))) return rc;
-  if ((rc = to_device_offs(ctx, io.d_ctx_frame_offs, g.ctx_frame_offs, stream))) return rc;
+  if (ctx_a && (rc = copy_clips(ctx, io.a, ctx_a, a_offs, g.a_offs[U], stream))) return rc;
+  Staging& s = io.staging.reset();
+  const size_t mo = s.add(g.mix_offs), ao = s.add(g.a_offs), bo = s.add(g.b_offs), fo = s.add(g.frame_offs),
+               oo = s.add(g.out_offs), co = s.add(g.ctx_frame_offs);
+  CK(s.upload(stream));
+  io.mix_offs = s.ptr<long long>(mo); io.a_offs = ctx_a ? s.ptr<long long>(ao) : nullptr; io.b_offs = s.ptr<long long>(bo);
+  io.frame_offs = s.ptr<long long>(fo); io.out_offs = s.ptr<long long>(oo); io.ctx_frame_offs = s.ptr<long long>(co);
   return 0;
 }
 
@@ -755,24 +769,20 @@ int run_conditioning(nhans_ctx* ctx, CondBufs& c, const T* a, const long long* d
   if (pcm) {
     CK(c.peak_a.ensure(sizeof(int) * U));
     CK(c.peak_b.ensure(sizeof(int) * U));
-    CK(launch_peaks(st, reinterpret_cast<const int16_t*>(b), d_b_offs, U, c.peak_b.as<int>()));
-    ctx->launches += 1;
+    LAUNCH(launch_peaks(st, reinterpret_cast<const int16_t*>(b), d_b_offs, U, c.peak_b.as<int>()));
   }
   {
     ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_stft_of(st, b, d_b_offs, d_ctx_frame_offs, U, c.peak_b.as<int>(), kCtxFrames, c.ctxlm_b.as<float>(), nullptr, false));
+    LAUNCH(launch_stft_of(st, b, d_b_offs, d_ctx_frame_offs, U, c.peak_b.as<int>(), kCtxFrames, c.ctxlm_b.as<float>(), nullptr, false));
   }
   const float* emb_a = ctx->silent_emb.as<float>();
   int stride_a = 0;
   int rc;
   if (a) {
-    if (pcm) {
-      CK(launch_peaks(st, reinterpret_cast<const int16_t*>(a), d_a_offs, U, c.peak_a.as<int>()));
-      ctx->launches += 1;
-    }
+    if (pcm) LAUNCH(launch_peaks(st, reinterpret_cast<const int16_t*>(a), d_a_offs, U, c.peak_a.as<int>()));
     {
       ProfScope ps(ctx, 4, 0, 0);
-      CK(launch_stft_of(st, a, d_a_offs, d_ctx_frame_offs, U, c.peak_a.as<int>(), kCtxFrames, c.ctxlm_a.as<float>(), nullptr, false));
+      LAUNCH(launch_stft_of(st, a, d_a_offs, d_ctx_frame_offs, U, c.peak_a.as<int>(), kCtxFrames, c.ctxlm_a.as<float>(), nullptr, false));
     }
     // embedding towers: once per distinct context clip (SURVEY.md F6), not once per window
     if ((rc = run_tower(ctx, c.ctxlm_a.as<float>(), U, c.emb_a.as<float>()))) return rc;
@@ -781,8 +791,8 @@ int run_conditioning(nhans_ctx* ctx, CondBufs& c, const T* a, const long long* d
   }
   if ((rc = run_tower(ctx, c.ctxlm_b.as<float>(), U, c.emb_b.as<float>()))) return rc;
   ProfScope ps(ctx, 4, 0, 0);
-  CK(launch_cond_table(st, emb_a, stride_a, c.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb, ctx->main_net.c,
-                       n_cols, c.cond.as<float>()));
+  LAUNCH(launch_cond_table(st, emb_a, stride_a, c.emb_b.as<float>(), 512, U, ctx->main_net.Pa, ctx->main_net.Pb, ctx->main_net.c,
+                           n_cols, c.cond.as<float>()));
   return 0;
 }
 
@@ -801,23 +811,20 @@ int run_fused(nhans_ctx* ctx, IoSlot& io) {
   CK(b.logmag.ensure(sbytes + 4));
   CK(b.phase.ensure(2 * sbytes + 8));          // unit phasors (float2 per bin) between the two transforms
   CK(b.den.ensure(sbytes + 4));
-  if (pcm) {
-    CK(launch_peaks(st, io.mix.as<int16_t>(), io.d_mix_offs.as<long long>(), U, b.peak_mix.as<int>()));
-    ctx->launches += 1;
-  } else {
+  if (pcm)
+    LAUNCH(launch_peaks(st, io.mix.as<int16_t>(), io.mix_offs, U, b.peak_mix.as<int>()));
+  else
     CK(cudaMemsetAsync(b.peak_mix.p, 0, sizeof(int) * U, st));     // the inverse STFT reads it; no int16 output here
-  }
   {
     ProfScope ps(ctx, 1, 0, (double)sizeof(T) * g.mix_offs[U] + 3.0 * sbytes);
-    CK(launch_stft_of(st, io.mix.as<T>(), io.d_mix_offs.as<long long>(), io.d_frame_offs.as<long long>(), U,
-                      b.peak_mix.as<int>(), g.max_frames, b.logmag.as<float>(), b.phase.as<float>(), true));
+    LAUNCH(launch_stft_of(st, io.mix.as<T>(), io.mix_offs, io.frame_offs, U, b.peak_mix.as<int>(), g.max_frames,
+                          b.logmag.as<float>(), b.phase.as<float>(), true));
   }
   int rc;
-  if ((rc = run_conditioning(ctx, b.cb, b.has_a ? io.a.as<T>() : nullptr, io.d_a_offs.as<long long>(), io.b.as<T>(),
-                             io.d_b_offs.as<long long>(), io.d_ctx_frame_offs.as<long long>(), U)))
+  if ((rc = run_conditioning(ctx, b.cb, b.has_a ? io.a.as<T>() : nullptr, io.a_offs, io.b.as<T>(), io.b_offs, io.ctx_frame_offs, U)))
     return rc;
-  return run_masknet(ctx, b.logmag.as<float>(), io.d_frame_offs.as<long long>(), g.frame_offs.data(), io.d_frame_offs.as<long long>(),
-                     g.frame_offs.data(), nullptr, nullptr, U, b.cb.cond.as<float>(), b.den.as<float>());
+  return run_masknet(ctx, b.logmag.as<float>(), io.frame_offs, g.frame_offs.data(), io.frame_offs, g.frame_offs.data(), nullptr,
+                     nullptr, U, b.cb.cond.as<float>(), b.den.as<float>());
 }
 
 // Inverse STFT on the compute stream of the batch staged in `io`: `spec` (batch.den or batch.logmag) with the
@@ -827,8 +834,8 @@ int batch_istft(nhans_ctx* ctx, const IoSlot& io, const DBuf& spec, float* out_f
   const Geometry& g = b.geo;
   // spectrum + phasors read, samples written
   ProfScope ps(ctx, 2, 0, 3.0 * 4 * kBins * g.total_frames + ((out_f32 ? 4.0 : 0.0) + (out_i16 ? 2.0 : 0.0)) * g.total_out);
-  CK(launch_istft(ctx->stream, spec.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(), io.d_out_offs.as<long long>(),
-                  g.U, b.peak_mix.as<int>(), g.max_frames, out_f32, out_i16, true));
+  LAUNCH(launch_istft(ctx->stream, spec.as<float>(), b.phase.as<float>(), io.frame_offs, io.out_offs, g.U, b.peak_mix.as<int>(),
+                      g.max_frames, out_f32, out_i16, true));
   return 0;
 }
 
@@ -846,19 +853,20 @@ int stft_entry(nhans_ctx* ctx, const T* x, const int64_t* offs, int U, float* lo
   if (!logmag && !phase && !peak) return NHANS_OK;
   const long long total = g.mix_offs[U];
   if ((rc = copy_clips(ctx, ctx->tmp[0], x, offs, total, ctx->stream))) return rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[1], g.mix_offs))) return rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[2], g.frame_offs))) return rc;
+  Staging& s = ctx->staging.reset();
+  const size_t mo = s.add(g.mix_offs), fo = s.add(g.frame_offs);
+  CK(s.upload(ctx->stream));
   const size_t sbytes = (size_t)g.total_frames * kBins * 4;
   CK(ctx->tmp[4].ensure(sbytes + 4));
   CK(ctx->tmp[5].ensure(sbytes + 4));
   if (pcm) {
     CK(ctx->tmp[3].ensure(sizeof(int) * U));
-    CK(launch_peaks(ctx->stream, ctx->tmp[0].as<int16_t>(), ctx->tmp[1].as<long long>(), U, ctx->tmp[3].as<int>()));
+    LAUNCH(launch_peaks(ctx->stream, ctx->tmp[0].as<int16_t>(), s.ptr<long long>(mo), U, ctx->tmp[3].as<int>()));
   }
   {
     ProfScope ps(ctx, 1, 0, (double)sizeof(T) * total + 2.0 * sbytes);
-    CK(launch_stft_of(ctx->stream, ctx->tmp[0].as<T>(), ctx->tmp[1].as<long long>(), ctx->tmp[2].as<long long>(), U,
-                      ctx->tmp[3].as<int>(), g.max_frames, ctx->tmp[4].as<float>(), ctx->tmp[5].as<float>(), false));
+    LAUNCH(launch_stft_of(ctx->stream, ctx->tmp[0].as<T>(), s.ptr<long long>(mo), s.ptr<long long>(fo), U, ctx->tmp[3].as<int>(),
+                          g.max_frames, ctx->tmp[4].as<float>(), ctx->tmp[5].as<float>(), false));
   }
   if (logmag) CK(cudaMemcpyAsync(logmag, ctx->tmp[4].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
   if (phase) CK(cudaMemcpyAsync(phase, ctx->tmp[5].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
@@ -936,11 +944,9 @@ int stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const
   // Geometry of the step (kernels.h StreamStepDev).  Stream i has F0 frames before the step and F1 after it; its windows
   // [a, b) run now.  It stores frames [cs, F1), cs = a - 17 (or 0): the carry = F0 - cs frames of its slot, then the new
   // ones.  Its denoised frames a - dc .. b - 1 go through the inverse STFT.
-  std::vector<long long> lo64(6 * (n + 1), 0);           // pcm | new | seg | win | out offsets, staged samples
-  long long *pcm_o = &lo64[0], *new_o = pcm_o + (n + 1), *seg_o = new_o + (n + 1), *win_o = seg_o + (n + 1), *out_o = win_o + (n + 1);
-  std::vector<int> i32(7 * n);
-  int *slot = &i32[0], *carry = slot + n, *left = carry + n, *den_carry = left + n, *keep = den_carry + n, *den_keep = keep + n,
-      *peak = den_keep + n;
+  // offsets [n + 1] of the staged samples, new frames, segment rows, windows and emitted samples; the rest is per stream
+  std::vector<long long> pcm_o(n + 1, 0), new_o(n + 1, 0), seg_o(n + 1, 0), win_o(n + 1, 0), out_o(n + 1, 0);
+  std::vector<int> slot(n), carry(n), left(n), den_carry(n), keep(n), den_keep(n), peak(n);
   int max_new = 0, max_rows = 0, max_wins = 0, max_keep = 0;
   long long max_out = 0;
   std::vector<int> F1s(n);
@@ -980,10 +986,19 @@ int stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const
     std::copy(r.tail.begin(), r.tail.end(), staged.begin() + pcm_o[i]);
     if (offs[i + 1] > offs[i]) std::copy(pcm + offs[i], pcm + offs[i + 1], staged.begin() + pcm_o[i] + r.tail.size());
   }
+  std::vector<float> factor;        // post step: compensation factor of each stream
+  if (post)
+    for (int i = 0; i < n; ++i) {
+      const float c = post->compensate ? post->compensate[i] : 0.f;
+      factor.push_back(std::isfinite(c) ? c : 0.f);       // the batch rule (compensate_kernel)
+    }
   cudaStream_t st = ctx->stream;
-  const size_t desc64 = lo64.size() * 8;
+  Staging& sg = ctx->staging.reset();
+  const size_t o_pcm = sg.add(pcm_o), o_new = sg.add(new_o), o_seg = sg.add(seg_o), o_win = sg.add(win_o), o_out = sg.add(out_o);
+  const size_t o_slot = sg.add(slot), o_carry = sg.add(carry), o_left = sg.add(left), o_den_carry = sg.add(den_carry),
+               o_keep = sg.add(keep), o_den_keep = sg.add(den_keep), o_peak = sg.add(peak), o_factor = sg.add(factor);
+  CK(sg.upload(st));
   CK(S.pcm.ensure(staged.size() * 2 + 32));
-  CK(S.desc.ensure(desc64 + i32.size() * 4));
   CK(S.new_lm.ensure((size_t)n_new * kBins * 4 + 4));
   CK(S.new_ph.ensure((size_t)n_new * kBins * 8 + 8));
   CK(S.seg_lm.ensure((size_t)n_seg * kBins * 4 + 4));
@@ -994,57 +1009,46 @@ int stream_step(nhans_ctx* ctx, int n, const int* ids, const int16_t* pcm, const
   CK(S.out_f32.ensure((size_t)n_out * 4 + 16));
   CK(S.out_i16.ensure((size_t)n_out * 2 + 16));
   if (!staged.empty()) CK(cudaMemcpyAsync(S.pcm.p, staged.data(), staged.size() * 2, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(S.desc.p, lo64.data(), desc64, cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(S.desc.as<char>() + desc64, i32.data(), i32.size() * 4, cudaMemcpyHostToDevice, st));
-  const long long* d64 = S.desc.as<long long>();
-  const int* d32 = reinterpret_cast<const int*>(S.desc.as<char>() + desc64);
   StreamStepDev p;
   p.n = n;
-  p.seg_offs = d64 + 2 * (n + 1); p.new_offs = d64 + (n + 1); p.win_offs = d64 + 3 * (n + 1); p.out_offs = d64 + 4 * (n + 1);
-  p.slot = d32; p.carry = d32 + n; p.left = d32 + 2 * n; p.den_carry = d32 + 3 * n; p.keep = d32 + 4 * n; p.den_keep = d32 + 5 * n;
-  p.peak = d32 + 6 * n;
+  p.seg_offs = sg.ptr<long long>(o_seg); p.new_offs = sg.ptr<long long>(o_new); p.win_offs = sg.ptr<long long>(o_win);
+  p.out_offs = sg.ptr<long long>(o_out);
+  p.slot = sg.ptr<int>(o_slot); p.carry = sg.ptr<int>(o_carry); p.left = sg.ptr<int>(o_left); p.den_carry = sg.ptr<int>(o_den_carry);
+  p.keep = sg.ptr<int>(o_keep); p.den_keep = sg.ptr<int>(o_den_keep); p.peak = sg.ptr<int>(o_peak);
   p.pool = S.pool.as<float>(); p.slot_stride = S.slot_stride; p.n_cols = n_cols;
   p.new_lm = S.new_lm.as<float>(); p.new_ph = S.new_ph.as<float>(); p.den_win = S.den_win.as<float>();
   p.seg_lm = S.seg_lm.as<float>(); p.seg_ph = S.seg_ph.as<float>(); p.den_seg = S.den_seg.as<float>(); p.cond = S.cond.as<float>();
   {
     ProfScope ps(ctx, 1, 0, 2.0 * pcm_o[n] + 12.0 * n_new * kBins);
-    CK(launch_stft(st, S.pcm.as<int16_t>(), d64, p.new_offs, n, p.peak, max_new, S.new_lm.as<float>(), S.new_ph.as<float>(), true));
+    LAUNCH(launch_stft(st, S.pcm.as<int16_t>(), sg.ptr<long long>(o_pcm), p.new_offs, n, p.peak, max_new, S.new_lm.as<float>(),
+                       S.new_ph.as<float>(), true));
   }
-  CK(launch_stream_assemble(st, p, max_rows));
-  ctx->launches += 1;
+  LAUNCH(launch_stream_assemble(st, p, max_rows));
   if (n_win > 0) {
     // (no pass when no window became computable)
-    if ((rc = run_masknet(ctx, p.seg_lm, p.seg_offs, seg_o, p.win_offs, win_o, p.left, left, n, p.cond, S.den_win.as<float>()))) return rc;
-    CK(launch_stream_den(st, p, max_wins));
-    ctx->launches += 1;
+    if ((rc = run_masknet(ctx, p.seg_lm, p.seg_offs, seg_o.data(), p.win_offs, win_o.data(), p.left, left.data(), n, p.cond,
+                          S.den_win.as<float>())))
+      return rc;
+    LAUNCH(launch_stream_den(st, p, max_wins));
   }
   // the post step always runs its inverse STFT: the running snr_est covers every sample it emits, wanted or not
-  std::vector<float> factor;
-  std::vector<double> sums;
+  std::vector<double> sums(post ? 2 * n : 0);
   if (post) {
-    factor.resize(n);
-    sums.resize(2 * n);
-    for (int i = 0; i < n; ++i) {
-      const float c = post->compensate ? post->compensate[i] : 0.f;
-      factor[i] = std::isfinite(c) ? c : 0.f;             // the batch rule (compensate_kernel)
-    }
-    CK(S.factor.ensure((size_t)n * 4));
     CK(S.sums.ensure(sizeof(double) * 2 * n));
     CK(S.mixed.ensure((size_t)n_out * 4 + 16));
     CK(S.removed.ensure((size_t)n_out * 4 + 16));
     CK(S.comp.ensure((size_t)n_out * 4 + 16));
-    CK(cudaMemcpyAsync(S.factor.p, factor.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
     ProfScope ps(ctx, 2, 0, 24.0 * n_win * kBins + 18.0 * n_out);
-    CK(launch_istft_stream_post(st, p, (int)max_out, S.factor.as<float>(), out_f32 ? S.out_f32.as<float>() : nullptr,
-                                out_i16 ? S.out_i16.as<int16_t>() : nullptr, post->mixed ? S.mixed.as<float>() : nullptr,
-                                post->removed ? S.removed.as<float>() : nullptr, post->comp ? S.comp.as<float>() : nullptr,
-                                S.sums.as<double>()));
+    LAUNCH(launch_istft_stream_post(st, p, (int)max_out, sg.ptr<float>(o_factor), out_f32 ? S.out_f32.as<float>() : nullptr,
+                                    out_i16 ? S.out_i16.as<int16_t>() : nullptr, post->mixed ? S.mixed.as<float>() : nullptr,
+                                    post->removed ? S.removed.as<float>() : nullptr, post->comp ? S.comp.as<float>() : nullptr,
+                                    S.sums.as<double>()));
   } else if (out_f32 || out_i16) {
     ProfScope ps(ctx, 2, 0, 12.0 * n_win * kBins + 6.0 * n_out);
-    CK(launch_istft_stream(st, p, (int)max_out, out_f32 ? S.out_f32.as<float>() : nullptr, out_i16 ? S.out_i16.as<int16_t>() : nullptr));
+    LAUNCH(launch_istft_stream(st, p, (int)max_out, out_f32 ? S.out_f32.as<float>() : nullptr,
+                               out_i16 ? S.out_i16.as<int16_t>() : nullptr));
   }
-  CK(launch_stream_save(st, p, max_keep));
-  ctx->launches += 1;
+  LAUNCH(launch_stream_save(st, p, max_keep));
   if (out_f32 && n_out) CK(cudaMemcpyAsync(out_f32, S.out_f32.p, n_out * 4, cudaMemcpyDeviceToHost, st));
   if (out_i16 && n_out) CK(cudaMemcpyAsync(out_i16, S.out_i16.p, n_out * 2, cudaMemcpyDeviceToHost, st));
   if (post) {
@@ -1186,23 +1190,23 @@ int nhans_output_offsets(const int64_t* mix_offs, int U, int64_t* out_offs) {
 int nhans_normalise(nhans_ctx* ctx, const int16_t* pcm, const int64_t* offs, int U, int trim, float* out, int64_t* out_offs) {
   if (!ctx || !pcm || !offs || !out || !out_offs || U <= 0) return fail(ctx, NHANS_ERR_ARG, "bad arguments");
   CK(cudaSetDevice(ctx->device));
-  std::vector<long long> ho(offs, offs + U + 1), oo(U + 1, 0);
+  std::vector<long long> rel(U + 1), oo(U + 1, 0);      // input offsets relative to offs[0], output offsets
+  for (int u = 0; u <= U; ++u) rel[u] = offs[u] - offs[0];
   for (int u = 0; u < U; ++u) {
-    long long n = ho[u + 1] - ho[u];
+    long long n = rel[u + 1] - rel[u];
     if (trim && n >= 400) n -= (n - 400) % 160;
     oo[u + 1] = oo[u] + n;
   }
   int rc;
-  if ((rc = copy_clips(ctx, ctx->tmp[0], pcm, offs, ho[U] - ho[0], ctx->stream))) return rc;
-  std::vector<long long> rel(U + 1);
-  for (int u = 0; u <= U; ++u) rel[u] = ho[u] - ho[0];
-  if ((rc = to_device_offs(ctx, ctx->tmp[1], rel))) return rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[2], oo))) return rc;
+  if ((rc = copy_clips(ctx, ctx->tmp[0], pcm, offs, rel[U], ctx->stream))) return rc;
+  Staging& s = ctx->staging.reset();
+  const size_t ro = s.add(rel), o_oo = s.add(oo);
+  CK(s.upload(ctx->stream));
   CK(ctx->tmp[3].ensure(sizeof(int) * U));
   CK(ctx->tmp[4].ensure(oo[U] * 4 + 4));
-  CK(launch_peaks(ctx->stream, ctx->tmp[0].as<int16_t>(), ctx->tmp[1].as<long long>(), U, ctx->tmp[3].as<int>()));
-  CK(launch_normalise(ctx->stream, ctx->tmp[0].as<int16_t>(), ctx->tmp[1].as<long long>(), ctx->tmp[2].as<long long>(), U,
-                      ctx->tmp[3].as<int>(), ctx->tmp[4].as<float>()));
+  LAUNCH(launch_peaks(ctx->stream, ctx->tmp[0].as<int16_t>(), s.ptr<long long>(ro), U, ctx->tmp[3].as<int>()));
+  LAUNCH(launch_normalise(ctx->stream, ctx->tmp[0].as<int16_t>(), s.ptr<long long>(ro), s.ptr<long long>(o_oo), U,
+                          ctx->tmp[3].as<int>(), ctx->tmp[4].as<float>()));
   CK(cudaMemcpyAsync(out, ctx->tmp[4].p, oo[U] * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
   for (int u = 0; u <= U; ++u) out_offs[u] = oo[u];
@@ -1231,7 +1235,7 @@ int nhans_eval_loss(nhans_ctx* ctx, const float* denoised, const float* target, 
   CK(cudaMemcpyAsync(ctx->tmp[1].p, target, bytes, cudaMemcpyHostToDevice, ctx->stream));
   {
     ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_eval_loss(ctx->stream, ctx->tmp[0].as<float>(), ctx->tmp[1].as<float>(), n_frames, ctx->tmp[2].as<float>()));
+    LAUNCH(launch_eval_loss(ctx->stream, ctx->tmp[0].as<float>(), ctx->tmp[1].as<float>(), n_frames, ctx->tmp[2].as<float>()));
   }
   CK(cudaMemcpyAsync(example_loss, ctx->tmp[2].p, (size_t)n_frames * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK(cudaStreamSynchronize(ctx->stream));
@@ -1267,14 +1271,16 @@ int nhans_masknet(nhans_ctx* ctx, const float* logmag, const int64_t* frame_offs
   CK(ctx->tmp[2].ensure((size_t)U * 512 * 4));
   CK(ctx->tmp[3].ensure((size_t)U * 512 * 4));
   CK(ctx->tmp[4].ensure((size_t)U * n_cols * 4));
-  if ((rc = to_device_offs(ctx, ctx->tmp[5], fo))) return rc;
+  Staging& s = ctx->staging.reset();
+  const size_t o_fo = s.add(fo);
+  CK(s.upload(ctx->stream));
   CK(cudaMemcpyAsync(ctx->tmp[0].p, logmag, sbytes, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->tmp[2].p, emb_a, (size_t)U * 512 * 4, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->tmp[3].p, emb_b, (size_t)U * 512 * 4, cudaMemcpyHostToDevice, ctx->stream));
-  CK(launch_cond_table(ctx->stream, ctx->tmp[2].as<float>(), 512, ctx->tmp[3].as<float>(), 512, U, ctx->main_net.Pa,
-                       ctx->main_net.Pb, ctx->main_net.c, n_cols, ctx->tmp[4].as<float>()));
-  if ((rc = run_masknet(ctx, ctx->tmp[0].as<float>(), ctx->tmp[5].as<long long>(), fo.data(), ctx->tmp[5].as<long long>(), fo.data(),
-                        nullptr, nullptr, U, ctx->tmp[4].as<float>(), ctx->tmp[1].as<float>())))
+  LAUNCH(launch_cond_table(ctx->stream, ctx->tmp[2].as<float>(), 512, ctx->tmp[3].as<float>(), 512, U, ctx->main_net.Pa,
+                           ctx->main_net.Pb, ctx->main_net.c, n_cols, ctx->tmp[4].as<float>()));
+  if ((rc = run_masknet(ctx, ctx->tmp[0].as<float>(), s.ptr<long long>(o_fo), fo.data(), s.ptr<long long>(o_fo), fo.data(), nullptr,
+                        nullptr, U, ctx->tmp[4].as<float>(), ctx->tmp[1].as<float>())))
     return rc;
   CK(cudaMemcpyAsync(denoised, ctx->tmp[1].p, sbytes, cudaMemcpyDeviceToHost, ctx->stream));
   return finish(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1299,20 +1305,16 @@ int nhans_istft(nhans_ctx* ctx, const float* logmag, const float* phase, const i
   CK(ctx->tmp[1].ensure(sbytes + 4));
   CK(cudaMemcpyAsync(ctx->tmp[0].p, logmag, sbytes, cudaMemcpyHostToDevice, ctx->stream));
   CK(cudaMemcpyAsync(ctx->tmp[1].p, phase, sbytes, cudaMemcpyHostToDevice, ctx->stream));
-  int rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[2], fo))) return rc;
-  if ((rc = to_device_offs(ctx, ctx->tmp[3], oo))) return rc;
-  std::vector<int> pk(U, 0);
-  if (peak) for (int u = 0; u < U; ++u) pk[u] = peak[u];
-  CK(ctx->tmp[4].ensure(sizeof(int) * U));
-  CK(cudaMemcpyAsync(ctx->tmp[4].p, pk.data(), sizeof(int) * U, cudaMemcpyHostToDevice, ctx->stream));
+  Staging& s = ctx->staging.reset();
+  const size_t o_fo = s.add(fo), o_oo = s.add(oo), o_pk = peak ? s.add(peak, U) : s.add(std::vector<int>(U, 0));
+  CK(s.upload(ctx->stream));
   CK(ctx->tmp[5].ensure(oo[U] * 4 + 4));
   CK(ctx->tmp[6].ensure(oo[U] * 2 + 4));
   {
     ProfScope ps(ctx, 2, 0, 2.0 * sbytes + (wav_f32 ? 4.0 : 0.0) * oo[U] + (wav_i16 ? 2.0 : 0.0) * oo[U]);
-    CK(launch_istft(ctx->stream, ctx->tmp[0].as<float>(), ctx->tmp[1].as<float>(), ctx->tmp[2].as<long long>(),
-                    ctx->tmp[3].as<long long>(), U, ctx->tmp[4].as<int>(), max_frames, wav_f32 ? ctx->tmp[5].as<float>() : nullptr,
-                    wav_i16 ? ctx->tmp[6].as<int16_t>() : nullptr));
+    LAUNCH(launch_istft(ctx->stream, ctx->tmp[0].as<float>(), ctx->tmp[1].as<float>(), s.ptr<long long>(o_fo), s.ptr<long long>(o_oo),
+                        U, s.ptr<int>(o_pk), max_frames, wav_f32 ? ctx->tmp[5].as<float>() : nullptr,
+                        wav_i16 ? ctx->tmp[6].as<int16_t>() : nullptr));
   }
   if (wav_f32) CK(cudaMemcpyAsync(wav_f32, ctx->tmp[5].p, oo[U] * 4, cudaMemcpyDeviceToHost, ctx->stream));
   if (wav_i16) CK(cudaMemcpyAsync(wav_i16, ctx->tmp[6].p, oo[U] * 2, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1407,14 +1409,13 @@ int nhans_postmix(nhans_ctx* ctx, float compensate, int ac, float* mixed_f32, fl
   CK(b.snr.ensure(sizeof(float) * g.U));
   {
     ProfScope ps(ctx, 2, 0, 4.0 * g.total_frames * kBins * 4 + 12.0 * g.total_out);
-    CK(launch_istft_post(ctx->stream, b.den.as<float>(), b.logmag.as<float>(), b.phase.as<float>(), io.d_frame_offs.as<long long>(),
-                         io.d_out_offs.as<long long>(), g.U, g.max_frames, nullptr, b.mixproc.as<float>(), b.removed.as<float>(),
-                         b.sums.as<double>()));
+    LAUNCH(launch_istft_post(ctx->stream, b.den.as<float>(), b.logmag.as<float>(), b.phase.as<float>(), io.frame_offs, io.out_offs,
+                             g.U, g.max_frames, nullptr, b.mixproc.as<float>(), b.removed.as<float>(), b.sums.as<double>()));
   }
   {
     ProfScope ps(ctx, 4, 0, 0);
-    CK(launch_compensate(ctx->stream, io.out_f32.as<float>(), b.removed.as<float>(), io.d_out_offs.as<long long>(), g.U,
-                         b.sums.as<double>(), compensate, ac, compensated_f32 ? b.comp.as<float>() : nullptr, b.snr.as<float>()));
+    LAUNCH(launch_compensate(ctx->stream, io.out_f32.as<float>(), b.removed.as<float>(), io.out_offs, g.U, b.sums.as<double>(),
+                             compensate, ac, compensated_f32 ? b.comp.as<float>() : nullptr, b.snr.as<float>()));
   }
   if (mixed_f32) CK(cudaMemcpyAsync(mixed_f32, b.mixproc.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
   if (removed_f32) CK(cudaMemcpyAsync(removed_f32, b.removed.p, g.total_out * 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1650,16 +1651,13 @@ int nhans_stream_open(nhans_ctx* ctx, int n, const int16_t* ctx_a, const int64_t
   Streams& S = ctx->streams;
   if (!ctx_a && (rc = ensure_silent(ctx))) return rc;
   cudaStream_t st = ctx->stream;
-  // device offsets: b | a | context frames, n + 1 each
-  std::vector<long long> offs(g.b_offs);
-  offs.insert(offs.end(), g.ctx_frame_offs.begin(), g.ctx_frame_offs.end());
-  if (ctx_a) offs.insert(offs.end(), g.a_offs.begin(), g.a_offs.end());
   if ((rc = copy_clips(ctx, S.ctx_b, ctx_b, b_offs, g.b_offs[n], st))) return rc;
   if (ctx_a && (rc = copy_clips(ctx, S.ctx_a, ctx_a, a_offs, g.a_offs[n], st))) return rc;
-  if ((rc = to_device_offs(ctx, S.ctx_offs, offs))) return rc;
-  const long long* d_offs = S.ctx_offs.as<long long>();
-  if ((rc = run_conditioning(ctx, S.cb, ctx_a ? S.ctx_a.as<int16_t>() : nullptr, d_offs + 2 * (n + 1), S.ctx_b.as<int16_t>(), d_offs,
-                             d_offs + (n + 1), n)))
+  Staging& sg = ctx->staging.reset();
+  const size_t bo = sg.add(g.b_offs), co = sg.add(g.ctx_frame_offs), ao = sg.add(g.a_offs);
+  CK(sg.upload(st));
+  if ((rc = run_conditioning(ctx, S.cb, ctx_a ? S.ctx_a.as<int16_t>() : nullptr, ctx_a ? sg.ptr<long long>(ao) : nullptr,
+                             S.ctx_b.as<int16_t>(), sg.ptr<long long>(bo), sg.ptr<long long>(co), n)))
     return rc;
   std::vector<int> slots;
   if ((rc = alloc_slots(ctx, n, slots))) return rc;
