@@ -52,14 +52,9 @@ def test_masknet_layers_and_output(variant, engine_sn, engine_ss, weights_sn, we
     plan = eng.plan(0)
     assert plan["bufs"] == pe.plan(0)["bufs"]
     first_buf = plan["first"]["out"]["buf"]
-    for g in plan["bufs"]:                                   # every activation grid, every logical pixel
-        a = grid_gather(g, eng.read_buffer(0, g["buf"]).astype(np.float32), 9)
-        b = grid_gather(g, pe.read_buffer(0, g["buf"]), 9)
-        if g["buf"] == first_buf:
-            continue    # not materialised by this engine (it may hold another test's data): resblock1_1_conv2 builds its
-                        # operand from the per-frame table (conv_walk.cu kWalkGen); checked with NHANS_NO_GEN=1 below
-        assert _rel(a, b) < 1e-3, g
-    # the first convolution's output itself: the same engine path with the operand generator switched off
+    # (every tensor-core layer's grid is checked elementwise, layer-local, in test_gpu_net_flavours.py)
+    # the first convolution's output is not materialised by this engine: resblock1_1_conv2 builds its operand from the
+    # per-frame table (conv_walk.cu kWalkGen).  The same engine path with the operand generator switched off stores it
     monkeypatch.setenv("NHANS_NO_GEN", "1")
     from nhans_b200.engine import Engine
     nogen = Engine(0, variant, win_capacity=256, row_capacity=4)

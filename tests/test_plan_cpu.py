@@ -101,3 +101,56 @@ def test_tiny_last_dense_keeps_precision(weights_sn):
     assert np.abs(ref - lm).max() > 0                       # the head still contributes
     assert _rel(den - lm, ref - lm) < 2e-3                  # a plain fp16 cast of 1e-5 weights loses ~2 decimal digits
     pe.close()
+
+
+def _pass_units(fo, w0, n):
+    """Unit table of windows w0 .. w0 + n - 1 (one window per frame) of utterances with frame offsets fo."""
+    g = np.arange(w0, w0 + n)
+    utt = np.searchsorted(fo, g, side="right") - 1
+    return dict(frame=g, lo=fo[utt], hi=fo[utt + 1], utt=utt)
+
+
+def test_layer_evaluator_matches_interpreter(weights_sn):
+    """The layer-local double evaluator (planexec_layer / planexec_first), fed the interpreter's own grids, agrees with
+    the interpreter's fp32 run elementwise within the accumulation bound of tests/layercheck.py, for every layer, unit
+    and pixel of the last pass of both networks, den and the pooled embedding included; and again from grids
+    compacted to a subset of the units at another capacity (how the GPU tests feed it)."""
+    import layercheck as LC
+    rng = np.random.default_rng(7)
+    fo = np.array([0, 3, 5, 7])                                  # 3 utterances, 7 windows: passes of 4 + 3
+    lm = rng.normal(-3, 2, (7, 201)).astype(np.float32)
+    ea = rng.normal(0, 2, (3, 512)).astype(np.float32)
+    eb = rng.normal(0, 2, (3, 512)).astype(np.float32)
+    pe = PlanExec(weights_sn, 0, win_cap=4, row_cap=2)
+    small = PlanExec(weights_sn, 0, win_cap=2, row_cap=1)
+    try:
+        den = pe.masknet(lm, fo, ea, eb)
+        plan = pe.plan(0)
+        ut = _pass_units(fo, 4, 3)
+        cond = pe.cond(ea, eb)
+        read = lambda b: pe.read_buffer(0, b)
+        v, S = pe.first(0, ut, lm, cond)
+        got = grid_gather(plan["first"]["out"], read(plan["first"]["out"]["buf"]), 3)
+        assert LC.compare("first", got, v, LC.ulp16(v) + LC.C_ACC * S, str) <= 1.0
+        every = {li: range(3) for li in range(len(plan["gemm"]))}
+        r = LC.check_pass(pe, 0, plan, read, ut, every, lm, cond, den=den[4:])
+        assert len(r) == len(plan["gemm"]) and max(r.values()) <= 1.0
+        r2 = LC.check_pass(small, 0, plan, read, ut, {li: [0, 2] for li in every}, lm, cond, den=den[4:], gen_first=True)
+        assert max(r2.values()) <= 1.0
+
+        ctx = np.stack([O.context_of(O.logmag_phase(O.normalise(synth.noise_clip(u)))[0]) for u in range(3)])
+        emb = pe.embed(ctx)                                      # passes of 2 + 1 context rows
+        tplan = pe.plan(1)
+        raw = ctx.reshape(-1, 201)
+        tut = dict(frame=[400], lo=[400], hi=[600], utt=[0])
+        tread = lambda b: pe.read_buffer(1, b)
+        v, S = pe.first(1, tut, raw)
+        got = grid_gather(tplan["first"]["out"], tread(tplan["first"]["out"]["buf"]), 1)
+        assert LC.compare("tower first", got, v, LC.ulp16(v) + LC.C_ACC * S, str) <= 1.0
+        r = LC.check_pass(small, 1, tplan, tread, tut, {li: [0] for li in range(len(tplan["gemm"]))}, raw)
+        assert max(r.values()) <= 1.0
+        pool = grid_gather(tplan["bufs"][tplan["pool_buf"]], tread(tplan["pool_buf"]), 1).astype(np.float64).reshape(-1, 512)
+        assert np.all(np.abs(emb[2] - pool.mean(0)) <= LC.C_ACC * np.abs(pool).mean(0) + 2.0 ** -23 * np.abs(pool.mean(0)))
+    finally:
+        pe.close()
+        small.close()
